@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the NeuroAlpha decoder hot path (BASELINE.json: "EEG windows/sec").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic EEG: BASELINE.json configs[1],
 i.e. R=10 trials x B=4096 sessions of [625,8] windows per GPU (40,960 windows), decoder forward +
@@ -351,8 +351,8 @@ def run_gpu_arm(args):
 
     def step_device():
         with torch.inference_mode():
-            _, p = model.decode(x_flat, want_probs=True)
-            return ops.trial_mean(p.reshape(R, B, NC))
+            logits, p = model.decode(x_flat, want_probs=True)
+            return {"logits": logits, "probs": p, "avg_probs": ops.trial_mean(p.reshape(R, B, NC))}
 
     def step_e2e():
         return run_trials_batched(host, model)      # pinned host in, numpy out
@@ -360,17 +360,21 @@ def run_gpu_arm(args):
     def measure(dtype):
         model.compute_dtype = dtype
         sampler = ClockSampler(local).start() if rank == 0 else None
+        last = [None]                               # what the last step returned (--dump-outputs)
+
+        def step():
+            last[0] = step_device()
         for _ in range(args.warmup):
-            step_device()
+            step()
         l0 = ops.launch_count()
-        ms = time_steps(step_device, args.steps, 0, world, dev)
+        ms = time_steps(step, args.steps, 0, world, dev)
         launches = ops.launch_count() - l0
         clocks = sampler.stop() if sampler else None
         e_steps = max(1, min(args.steps, 10))
         ms_e2e = time_steps(step_e2e, e_steps, 2, world, dev)
         return {"value": world * n_win * args.steps / (ms * 1e-3), "ms_per_step": ms / args.steps,
                 "e2e_value": world * n_win * e_steps / (ms_e2e * 1e-3), "e2e_ms_per_step": ms_e2e / e_steps,
-                "launches": launches, "clocks": clocks}
+                "launches": launches, "clocks": clocks, "outputs": last[0]}
 
     fp = measure(torch.float32)                     # fp32-contract tier: the headline (the reference computes in fp32)
     h16 = measure(torch.bfloat16)                   # 16-bit tensor-core tier (fp16 operands, 2e-2 contract): named extra
@@ -478,6 +482,8 @@ def run_gpu_arm(args):
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**fp["outputs"], **{f"fp16_tier_{k}": v for k, v in h16["outputs"].items()}})
     # the CPU arm runs on rank 0 after every timed GPU region (it would perturb the other ranks' host threads otherwise)
     cpu = cpu_arm(3, 1) if not args.no_cpu else None
     cpu_train = cpu_train_arm() if (not args.no_cpu and not args.no_train) else None
@@ -594,6 +600,16 @@ def run_gpu_arm(args):
     if config1:
         line["config1"] = config1
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, arrays):
+    """Rank 0's results of the last timed step, one float32 ``<name>.npy`` each: per tier the [40960, 3] logits and
+    probabilities and the [4096, 3] 10-trial means (2.6 MB in all).  The inputs are seeded, so two builds run with the
+    same arguments can be compared output for output."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.float().cpu().numpy())
 
 
 X3_MUFU_PER_CELL, V2_MUFU_PER_CELL = 7, 5
@@ -772,7 +788,13 @@ def main():
     ap.add_argument("--no-stress", action="store_true")
     ap.add_argument("--train-batch", type=int, default=65536, help="GLOBAL batch of the train leg (configs[2])")
     ap.add_argument("--train-micro", type=int, default=148 * 128, help="windows per micro-batch (default: one 128-window tile per SM)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (both tiers) to DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
         return

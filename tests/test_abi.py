@@ -57,5 +57,7 @@ def test_python_wrapper_raises_runtime_error(lib):
 
 def test_sass_is_sm100(built_lib):
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", str(built_lib)], capture_output=True, text=True).stdout
+    from neural_speech_decoding_b200.build import find_nvcc
+    cuobjdump = Path(find_nvcc()).resolve().parent / "cuobjdump"      # the toolkit that built the library, on PATH or not
+    out = subprocess.run([str(cuobjdump), "-lelf", str(built_lib)], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
