@@ -143,6 +143,28 @@ int na_head_fwd_f32(const float* h, const float* attn_w, const float* attn_b,
                     float* logits, float* probs, float* stats, float* zpool,
                     int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream);
 
+/* ---- intermediates of the eval forward (lstm_eeg_model.py:35-38: what forward hooks on attn / ln would see) -----------
+ * Every *_ex entry point takes the arguments of its sibling plus three optional outputs after `probs`; each may be NULL,
+ * and with all three NULL the call is exactly the sibling.  They are written by the same launch as the logits:
+ *   scores_tm  [T][B] fp32, TIME-MAJOR (row t = the B windows' scores s_t = attn.weight . h_t + attn.bias of step t;
+ *              the kernels hold 32 consecutive windows per warp, so each step is one contiguous run of stores)
+ *   pooled     [B][H] fp32, sum_t alpha_t h_t (the attention-pooled vector before LayerNorm)
+ *   embedding  [B][H] fp32, LayerNorm(pooled) (the input of fc)
+ * Only rows b < B are written; 16-byte alignment as for the other outputs.
+ * na_attention_softmax_f32: scores_tm [T][B] -> attn [B][T] = softmax over time per window (exp(s - max) / sum in fp32,
+ * torch.softmax's formula; a NaN score gives the window a NaN row).  In the 16-bit tier (na_decoder_infer_bf16_ex and
+ * _x32_ex, na_decoder_infer_wide_bf16_ex) the intermediates carry that tier's 2e-2 contract; the v1 kernel
+ * (na_set_tuning("tc_infer_hs", 1 | 2)) does not write them: a non-NULL extra returns NA_EUNSUPPORTED.
+ */
+int na_head_fwd_f32_ex(const float* h, const float* attn_w, const float* attn_b,
+                       const float* ln_w, const float* ln_b,
+                       const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                       const float* rrelu_slope, const float* drop_mask, float drop_scale,
+                       float* logits, float* probs, float* scores_tm, float* pooled, float* embedding,
+                       float* stats, float* zpool,
+                       int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream);
+int na_attention_softmax_f32(const float* scores_tm, float* attn, int64_t T, int64_t B, na_stream_t stream);
+
 /* Backward of na_head_fwd_f32.  dlogits [B,NC] -> dh TMP [T][Bp][H] (padding rows zeroed)
  * and the 8 head parameter gradients, packed in `dparams` as
  * [attn_w H | attn_b 1 | ln_w H | ln_b H | fc0_w 32H | fc0_b 32 | fc3_w 32NC | fc3_b NC].
@@ -216,6 +238,17 @@ int na_decoder_infer_bf16_x32(const float* x, const void* packed,
                               const float* attn_w, const float* attn_b, const float* ln_w, const float* ln_b,
                               const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
                               float* logits, float* probs, int64_t T, int64_t B, int64_t NC, na_stream_t stream);
+/* The same two with the intermediates outputs (see na_head_fwd_f32_ex). */
+int na_decoder_infer_bf16_ex(const void* x_bf16_tmp, const void* packed,
+                             const float* attn_w, const float* attn_b, const float* ln_w, const float* ln_b,
+                             const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                             float* logits, float* probs, float* scores_tm, float* pooled, float* embedding,
+                             int64_t T, int64_t B, int64_t Bp, int64_t NC, na_stream_t stream);
+int na_decoder_infer_bf16_x32_ex(const float* x, const void* packed,
+                                 const float* attn_w, const float* attn_b, const float* ln_w, const float* ln_b,
+                                 const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                                 float* logits, float* probs, float* scores_tm, float* pooled, float* embedding,
+                                 int64_t T, int64_t B, int64_t NC, na_stream_t stream);
 
 /* ---- exact tier on the tensor cores (fp32 accuracy, 1e-5 contract) ------------------------------------
  * The same forward as na_decoder_infer_bf16_x32 at fp32 accuracy: every operand is split into fp16 hi + lo halves and
@@ -232,6 +265,12 @@ int na_decoder_infer_x3(const float* x, const void* packed,
                         const float* attn_w, const float* attn_b, const float* ln_w, const float* ln_b,
                         const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
                         float* logits, float* probs, int64_t T, int64_t B, int64_t NC, na_stream_t stream);
+/* ... with the intermediates outputs (see na_head_fwd_f32_ex). */
+int na_decoder_infer_x3_ex(const float* x, const void* packed,
+                           const float* attn_w, const float* attn_b, const float* ln_w, const float* ln_b,
+                           const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                           float* logits, float* probs, float* scores_tm, float* pooled, float* embedding,
+                           int64_t T, int64_t B, int64_t NC, na_stream_t stream);
 
 /* ---- tensor-core tier, wide hidden sizes (H = 96, 144, 192; BASELINE configs[4]: H = 192, T = 2500) --------
  * Same contract as na_decoder_infer_bf16 (lstm_eeg_model.py:32-39 + :97, eval mode; input_size 8, 2 layers),
@@ -253,6 +292,12 @@ int na_decoder_infer_wide_bf16(const void* x_bf16_tmp, const void* packed, const
                                const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
                                void* state, float* logits, float* probs,
                                int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream);
+/* ... with the intermediates outputs (see na_head_fwd_f32_ex; pooled / embedding are [B][H]). */
+int na_decoder_infer_wide_bf16_ex(const void* x_bf16_tmp, const void* packed, const float* ln_w, const float* ln_b,
+                                  const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                                  void* state, float* logits, float* probs, float* scores_tm, float* pooled,
+                                  float* embedding, int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC,
+                                  na_stream_t stream);
 
 /* ---- tensor-core tier, training (bf16 operands; fp32 accumulate, cell state, gradients) ------------
  * Layouts: TMP fp32 [T][Bp][48]; TCL bf16 [T][Bp/128][F/8][128][8] (tile-chunk layout: a tile's

@@ -29,6 +29,8 @@ SIGNATURES = {
     "na_wgrad_partial_floats": (c_int64, [I64, I64]),
     "na_lstm_layer_wgrad_f32": (c_int, [P, P, P, P, P, P, P, I64, I64, I64, I64, P]),
     "na_head_fwd_f32": (c_int, [P] * 9 + [P, P, F32, P, P, P, P, I64, I64, I64, I64, I64, P]),
+    "na_head_fwd_f32_ex": (c_int, [P] * 9 + [P, P, F32, P, P, P, P, P, P, P, I64, I64, I64, I64, I64, P]),
+    "na_attention_softmax_f32": (c_int, [P, P, I64, I64, P]),
     "na_head_param_floats": (c_int64, [I64, I64]),
     "na_head_partial_floats": (c_int64, [I64, I64, I64]),
     "na_head_bwd_f32": (c_int, [P] * 12 + [P, P, F32, P, P, P, I64, I64, I64, I64, I64, P]),
@@ -36,13 +38,17 @@ SIGNATURES = {
     "na_decoder_pack_bf16": (c_int, [P] * 9 + [P]),
     "na_decoder_infer_bf16": (c_int, [P] * 12 + [I64, I64, I64, I64, P]),
     "na_decoder_infer_bf16_x32": (c_int, [P] * 12 + [I64, I64, I64, P]),
+    "na_decoder_infer_bf16_ex": (c_int, [P] * 15 + [I64, I64, I64, I64, P]),
+    "na_decoder_infer_bf16_x32_ex": (c_int, [P] * 15 + [I64, I64, I64, P]),
     "na_decoder_packed_x3_bytes": (c_int64, []),
     "na_decoder_pack_x3": (c_int, [P] * 9 + [P]),
     "na_decoder_infer_x3": (c_int, [P] * 12 + [I64, I64, I64, P]),
+    "na_decoder_infer_x3_ex": (c_int, [P] * 15 + [I64, I64, I64, P]),
     "na_decoder_wide_packed_bytes": (c_int64, [I64]),
     "na_decoder_wide_state_bytes": (c_int64, [I64]),
     "na_decoder_pack_wide_bf16": (c_int, [P] * 11 + [I64, P]),
     "na_decoder_infer_wide_bf16": (c_int, [P] * 11 + [I64, I64, I64, I64, I64, P]),
+    "na_decoder_infer_wide_bf16_ex": (c_int, [P] * 14 + [I64, I64, I64, I64, I64, P]),
     "na_train_bf16_partial_floats": (c_int64, []),
     "na_dropout_mask_u8": (c_int, [ctypes.c_uint64, I64, I64, I64, P, P]),
     "na_lstm2_fwd_train_bf16": (c_int, [P, P, P, ctypes.c_uint64, I64, F32, P, P, P, P, P, P, P, P, P, P, I64, I64, I64, I64, P]),

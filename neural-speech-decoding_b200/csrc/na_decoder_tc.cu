@@ -402,7 +402,7 @@ int launch_pack_v2(const float*, const float*, const float*, const float*, const
                    void*, cudaStream_t);
 int launch_infer_v2(const void*, const unsigned char*, const float*, const float*, const float*, const float*, const float*,
                     const float*, const float*, const float*, float*, float*, int, int64_t, int64_t, int, int, cudaStream_t,
-                    const float*);
+                    const float*, float*, float*, float*);
 constexpr int64_t kPackedV1Bytes = (int64_t)(kK0Chunks + kK1Chunks) * kBChunk;
 
 }  // namespace tc
@@ -427,10 +427,11 @@ extern "C" int na_decoder_pack_bf16(const float* w_ih0, const float* w_hh0, cons
                               reinterpret_cast<unsigned char*>(packed) + tc::kPackedV1Bytes, as_stream(stream));
 }
 
-extern "C" int na_decoder_infer_bf16(const void* x_bf16_tmp, const void* packed, const float* attn_w,
-                                     const float* attn_b, const float* ln_w, const float* ln_b, const float* fc0_w,
-                                     const float* fc0_b, const float* fc3_w, const float* fc3_b, float* logits,
-                                     float* probs, int64_t T, int64_t B, int64_t Bp, int64_t NC, na_stream_t stream) {
+extern "C" int na_decoder_infer_bf16_ex(const void* x_bf16_tmp, const void* packed, const float* attn_w,
+                                        const float* attn_b, const float* ln_w, const float* ln_b, const float* fc0_w,
+                                        const float* fc0_b, const float* fc3_w, const float* fc3_b, float* logits,
+                                        float* probs, float* scores_tm, float* pooled, float* embedding, int64_t T, int64_t B,
+                                        int64_t Bp, int64_t NC, na_stream_t stream) {
     using namespace na;
     NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1 && Bp >= B && Bp % tc::kRows == 0, NA_EINVAL,
                "na_decoder_infer_bf16: bad shape T=%lld B=%lld Bp=%lld (Bp must be a multiple of %d)", (long long)T,
@@ -438,8 +439,11 @@ extern "C" int na_decoder_infer_bf16(const void* x_bf16_tmp, const void* packed,
     NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_infer_bf16: num_classes=%lld", (long long)NC);
     NA_REQUIRE_PTR(x_bf16_tmp); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(logits);
     NA_OPTIONAL_PTR(probs);
+    NA_OPTIONAL_PTR(scores_tm); NA_OPTIONAL_PTR(pooled); NA_OPTIONAL_PTR(embedding);
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
                "na_decoder_infer_bf16: null parameter pointer");
+    NA_REQUIRE(tc::g_infer_hs == 3 || !(scores_tm || pooled || embedding), NA_EUNSUPPORTED,
+               "na_decoder_infer_bf16_ex: the v1 kernel (tc_infer_hs = %d) does not write intermediates", tc::g_infer_hs);
     static int sms = 0;
     if (sms == 0) {
         int dev = 0;
@@ -451,7 +455,7 @@ extern "C" int na_decoder_infer_bf16(const void* x_bf16_tmp, const void* packed,
     if (hs == 3)
         return tc::launch_infer_v2(x_bf16_tmp, reinterpret_cast<const unsigned char*>(packed) + tc::kPackedV1Bytes, attn_w, attn_b,
                                    ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, (int)T, B, Bp, (int)NC, sms,
-                                   as_stream(stream), nullptr);
+                                   as_stream(stream), nullptr, scores_tm, pooled, embedding);
     const size_t smem = sizeof(tc::Smem) + 1024;
     cudaError_t e = hs == 2 ? cudaFuncSetAttribute(tc::decoder_infer_bf16_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
                             : cudaFuncSetAttribute(tc::decoder_infer_bf16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -471,17 +475,27 @@ extern "C" int na_decoder_infer_bf16(const void* x_bf16_tmp, const void* packed,
     return check_launch("na_decoder_infer_bf16");
 }
 
+extern "C" int na_decoder_infer_bf16(const void* x_bf16_tmp, const void* packed, const float* attn_w,
+                                     const float* attn_b, const float* ln_w, const float* ln_b, const float* fc0_w,
+                                     const float* fc0_b, const float* fc3_w, const float* fc3_b, float* logits,
+                                     float* probs, int64_t T, int64_t B, int64_t Bp, int64_t NC, na_stream_t stream) {
+    return na_decoder_infer_bf16_ex(x_bf16_tmp, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs,
+                                    nullptr, nullptr, nullptr, T, B, Bp, NC, stream);
+}
+
 // The same forward straight from the caller's batch-first fp32 windows x [B][T][8] (lstm_eeg_model.py:32: `forward(x)`):
 // the fp32 -> fp16 time-major pack of na_window_zscore is fused into the kernel's producer warp.
-extern "C" int na_decoder_infer_bf16_x32(const float* x, const void* packed, const float* attn_w, const float* attn_b,
-                                         const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
-                                         const float* fc3_w, const float* fc3_b, float* logits, float* probs, int64_t T,
-                                         int64_t B, int64_t NC, na_stream_t stream) {
+extern "C" int na_decoder_infer_bf16_x32_ex(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                            const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                            const float* fc3_w, const float* fc3_b, float* logits, float* probs,
+                                            float* scores_tm, float* pooled, float* embedding, int64_t T, int64_t B, int64_t NC,
+                                            na_stream_t stream) {
     using namespace na;
     NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_infer_bf16_x32: bad shape T=%lld B=%lld", (long long)T, (long long)B);
     NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_infer_bf16_x32: num_classes=%lld", (long long)NC);
     NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(logits);
     NA_OPTIONAL_PTR(probs);
+    NA_OPTIONAL_PTR(scores_tm); NA_OPTIONAL_PTR(pooled); NA_OPTIONAL_PTR(embedding);
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
                "na_decoder_infer_bf16_x32: null parameter pointer");
     static int sms = 0;
@@ -492,5 +506,14 @@ extern "C" int na_decoder_infer_bf16_x32(const float* x, const void* packed, con
         if (sms <= 0) sms = 148;
     }
     return tc::launch_infer_v2(nullptr, reinterpret_cast<const unsigned char*>(packed) + tc::kPackedV1Bytes, attn_w, attn_b, ln_w, ln_b,
-                               fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, (int)T, B, 0, (int)NC, sms, as_stream(stream), x);
+                               fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, (int)T, B, 0, (int)NC, sms, as_stream(stream), x,
+                               scores_tm, pooled, embedding);
+}
+
+extern "C" int na_decoder_infer_bf16_x32(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                         const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                         const float* fc3_w, const float* fc3_b, float* logits, float* probs, int64_t T,
+                                         int64_t B, int64_t NC, na_stream_t stream) {
+    return na_decoder_infer_bf16_x32_ex(x, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, nullptr,
+                                        nullptr, nullptr, T, B, NC, stream);
 }

@@ -178,15 +178,20 @@ __device__ __forceinline__ void cell_granule(const uint32_t* v, float* c, uint32
 // Epilogue of one tile for one warp: both layers of (lane quarter q, unit group g).  R = row replication:
 // the tile holds 128 / R distinct windows; copy rp = q / (4 / R) of source quarter qs = q % (4 / R) takes
 // granules [4 g + rp * (4 / R), + 4 / R) of the 12 four-unit granules.
-template <int R, int NT>
+// kEx: also store the attention scores (time-major [T][B]) and the pooled vector / LayerNorm output ([B][48]) of every
+// window b < B, in the reference's scale (h, not H = 2h): the scores and the LayerNorm output by the first row copy of
+// the g == 0 warps (the one that runs the head), the pooled vector by every thread for the units it pooled.
+template <int R, int NT, bool kEx>
 __device__ __forceinline__ void epilogue_tile(Smem2& S, const int q, const int g, const int lane, const int nq, const int T,
                                               const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                               const int64_t b0, const int64_t B, const int NC, float* __restrict__ logits,
-                                              float* __restrict__ probs) {
+                                              float* __restrict__ probs, float* __restrict__ scores_tm,
+                                              float* __restrict__ pooled, float* __restrict__ embedding) {
     constexpr int kQ = 4 / R;                      // distinct source quarters = granules per warp
     constexpr int kSlots = 4 / R, kU = 4 * kSlots; // granules / units owned by this thread
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
+    const bool ex_writer = kEx && g == 0 && rp == 0 && b0 + wrow < B;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     const int gr0 = 4 * g + rp * kSlots;           // first granule
     if (qs >= nq) {                                // idle quarter: keep the barrier protocol only
@@ -274,6 +279,10 @@ __device__ __forceinline__ void epilogue_tile(Smem2& S, const int q, const int g
             fence_proxy_async_smem();
             mbar_arrive(&S.h1_ready);
             if (t >= 2) pool(__uint_as_float(sc2[0]) + __uint_as_float(sc2[1]));
+            // the score columns hold w_a / 2 . H1 + b_a = w_a . h1 + b_a: no rescaling
+            if constexpr (kEx)
+                if (t >= 2 && ex_writer && scores_tm)
+                    scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]) + __uint_as_float(sc2[1]);
 #pragma unroll
             for (int u = 0; u < 2 * kSlots; ++u) hprev[u] = hb[u];
         }
@@ -285,10 +294,22 @@ __device__ __forceinline__ void epilogue_tile(Smem2& S, const int q, const int g
         tmem_ld2(tmem_d1 + lane_base + kN, sc2);
         tc_fence_before();
         pool(__uint_as_float(sc2[0]) + __uint_as_float(sc2[1]));
+        if constexpr (kEx)
+            if (ex_writer && scores_tm) scores_tm[(int64_t)(T - 1) * B + b0 + wrow] = __uint_as_float(sc2[0]) + __uint_as_float(sc2[1]);
     }
     // ---- head for this window: LN -> fc0 -> RReLU(eval) -> fc3 -> softmax ----------------------
 #pragma unroll
     for (int j = 0; j < kU; ++j) S.zx[wrow][gr0 * 4 + j] = z[j];
+    if constexpr (kEx)
+        // every copy stores the units it pooled, from its own registers: a further use of the head's products would
+        // change which of them the assembler contracts into FMAs, and the logits would no longer be the default's
+        if (pooled && b0 + wrow < B) {
+            float zp[kU];
+            const float inv = 0.5f / l;            // z accumulated H = 2h
+#pragma unroll
+            for (int j = 0; j < kU; ++j) zp[j] = z[j] * inv;
+            store_row<kU>(pooled + (b0 + wrow) * kH + gr0 * 4, zp);
+        }
     named_bar_sync(1 + qs, 96 * R);                // the 3 R warps that share source quarter qs
     if (g == 0 && rp == 0) {
         const int64_t b = b0 + wrow;
@@ -304,6 +325,8 @@ __device__ __forceinline__ void epilogue_tile(Smem2& S, const int q, const int g
         const float rstd = rsqrtf(var * (1.0f / kH) + kLnEps);
 #pragma unroll
         for (int j = 0; j < kH; ++j) zf[j] = fmaf((zf[j] - mean) * rstd, S.head.lnw[j], S.head.lnb[j]);
+        if constexpr (kEx)
+            if (ex_writer && embedding) store_row<kH>(embedding + b * kH, zf);
         float lg[NA_MAX_CLASSES];
 #pragma unroll
         for (int k = 0; k < NA_MAX_CLASSES; ++k) lg[k] = (k < NC) ? S.head.b3[k] : -INFINITY;
@@ -333,7 +356,7 @@ __device__ __forceinline__ void epilogue_tile(Smem2& S, const int q, const int g
     }
 }
 
-template <int NT>
+template <int NT, bool kEx = false>
 __global__ void __launch_bounds__(kV2Threads, 1)
 decoder_infer_v2_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T][Bp][8] fp16 bits
                         const unsigned char* __restrict__ packed,   // v2 section: B0 | B1 (pack_decoder_v2_kernel)
@@ -343,7 +366,9 @@ decoder_infer_v2_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T][B
                         const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
                         float* __restrict__ logits, float* __restrict__ probs,
                         int T, int64_t B, int64_t Bp, int NC, int nquarters, int allow_rep,
-                        const float* __restrict__ x32) {       // != NULL: the caller's [B][T][8] fp32 windows, read directly (x unused)
+                        const float* __restrict__ x32,         // != NULL: the caller's [B][T][8] fp32 windows, read directly (x unused)
+                        float* __restrict__ scores_tm,         // kEx: [T][B] scores, [B][48] pooled / LayerNorm output
+                        float* __restrict__ pooled, float* __restrict__ embedding) {
     constexpr int kMmaWarp = 12, kTmaWarp = 13;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     Smem2& S = *reinterpret_cast<Smem2*>(smem_raw);
@@ -547,9 +572,9 @@ decoder_infer_v2_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T][B
         } else {
             // ================= epilogue: both layers of (quarter q, unit group g) ========================
             const int q = warp & 3, g = warp >> 2;
-            if (R == 1) epilogue_tile<1, NT>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs);
-            else if (R == 2) epilogue_tile<2, NT>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs);
-            else epilogue_tile<4, NT>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs);
+            if (R == 1) epilogue_tile<1, NT, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs, scores_tm, pooled, embedding);
+            else if (R == 2) epilogue_tile<2, NT, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs, scores_tm, pooled, embedding);
+            else epilogue_tile<4, NT, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, logits, probs, scores_tm, pooled, embedding);
         }
         __syncthreads();       // tile done: every MMA has completed (the epilogue saw the flush d1_full)
         q0 += nq;
@@ -581,9 +606,11 @@ int launch_pack_v2(const float* w_ih0, const float* w_hh0, const float* b_ih0, c
 int launch_infer_v2(const void* x, const unsigned char* packed_v2, const float* attn_w, const float* attn_b, const float* ln_w,
                     const float* ln_b, const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
                     float* logits, float* probs, int T, int64_t B, int64_t Bp, int NC, int sms, cudaStream_t stream,
-                    const float* x32) {
+                    const float* x32, float* scores_tm, float* pooled, float* embedding) {
     const size_t smem = infer_v2_smem_bytes();
-    auto kern = g_infer_tanh_fma ? decoder_infer_v2_kernel<1> : decoder_infer_v2_kernel<0>;
+    const bool ex = scores_tm || pooled || embedding;
+    auto kern = g_infer_tanh_fma ? (ex ? decoder_infer_v2_kernel<1, true> : decoder_infer_v2_kernel<1>)
+                                 : (ex ? decoder_infer_v2_kernel<0, true> : decoder_infer_v2_kernel<0>);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_bf16: shared memory opt-in failed (%s)", cudaGetErrorString(e));
     const int nquarters = (int)((B + 31) / 32);            // padding quarters beyond B are never scheduled
@@ -591,7 +618,7 @@ int launch_infer_v2(const void* x, const unsigned char* packed_v2, const float* 
     const int grid = nquarters < sms ? nquarters : sms;
     kern<<<grid, kV2Threads, smem, stream>>>(reinterpret_cast<const __nv_bfloat16*>(x), packed_v2, attn_w, attn_b,
                                              ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, T, B, Bp, NC,
-                                             nquarters, g_infer_rep, x32);
+                                             nquarters, g_infer_rep, x32, scores_tm, pooled, embedding);
     count_launch();
     return check_launch("na_decoder_infer_bf16 (v2)");
 }

@@ -196,7 +196,9 @@ __device__ __forceinline__ uint4 ld_shared_v4(const void* p) {
     return r;
 }
 
-template <int NCH>
+// kEx: also store the attention scores (time-major [T][B]) and the pooled vector / LayerNorm output ([B][H]) of every
+// window b < B, in the reference's scale (h, not H = 2h); the g == 0 warp of the window's lane quarter writes them.
+template <int NCH, bool kEx = false>
 __global__ void __launch_bounds__(kWThreads, 1)
 decoder_infer_wide_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T][Bp][8] fp16 bits
                           const unsigned char* __restrict__ packed,   // pack_wide_kernel image
@@ -205,7 +207,9 @@ decoder_infer_wide_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T]
                           const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
                           float* __restrict__ state,                  // [grid][3][kStateFloats]: c0, c1, z
                           float* __restrict__ logits, float* __restrict__ probs,
-                          int T, int64_t B, int64_t Bp, int NC, int nquarters, int cs, int dbg) {
+                          int T, int64_t B, int64_t Bp, int NC, int nquarters, int cs, int dbg,
+                          float* __restrict__ scores_tm,              // kEx: [T][B] scores, [B][H] pooled / LayerNorm output
+                          float* __restrict__ pooled, float* __restrict__ embedding) {
     // dbg (timing experiments only, results invalid): 1 = skip the cell update, 2 = skip the gate MMAs, 4 = skip the weight loads
     // cs = thread-block-cluster size (1, 2 or 4): the CTAs of a cluster stream the SAME weight image in lockstep, so
     // each ring stage is fetched from L2 once per cluster -- rank r loads 1/cs of it and multicasts it to all.
@@ -457,6 +461,8 @@ decoder_infer_wide_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T]
                             e = __expf(score - mnew);
                             l = fmaf(l, scl, e);
                             mx = mnew;
+                            if constexpr (kEx)      // the score columns hold w_a / 2 . H1 + b_a = w_a . h1 + b_a
+                                if (g == 0 && scores_tm && b0 + row < B) scores_tm[(int64_t)(t - 1) * B + b0 + row] = score;
                         }
                     }
                     if (flush) {
@@ -535,10 +541,14 @@ decoder_infer_wide_kernel(const __nv_bfloat16* __restrict__ x,        // TMP [T]
                     mean += (a0 + a1) + (a2 + a3);
                 }
                 mean *= (1.0f / H);
+                if constexpr (kEx)
+                    if (pooled && b0 + row < B) for (int k = 0; k < H; ++k) pooled[(b0 + row) * H + k] = zf[k];
                 float var = 0.f;
                 for (int k = 0; k < H; ++k) { const float d = zf[k] - mean; var = fmaf(d, d, var); }
                 const float rstd = rsqrtf(var * (1.0f / H) + kLnEps);
                 for (int k = 0; k < H; ++k) zf[k] = fmaf((zf[k] - mean) * rstd, S.lnw[k], S.lnb[k]);
+                if constexpr (kEx)
+                    if (embedding && b0 + row < B) for (int k = 0; k < H; ++k) embedding[(b0 + row) * H + k] = zf[k];
                 float lg[NA_MAX_CLASSES];
 #pragma unroll
                 for (int k = 0; k < NA_MAX_CLASSES; ++k) lg[k] = (k < NC) ? S.b3[k] : -INFINITY;
@@ -588,12 +598,13 @@ void set_wide_dbg(int v) { g_wide_dbg = v; }
 int g_wide_cluster = 1;      // na_set_tuning("tc_wide_cluster", 1 | 2 | 4)
 void set_wide_cluster(int v) { g_wide_cluster = (v == 1 || v == 2 || v == 4) ? v : 1; }
 
-template <int NCH>
+template <int NCH, bool kEx>
 static int launch_wide(const void* x, const void* packed, const float* ln_w, const float* ln_b, const float* fc0_w,
                        const float* fc0_b, const float* fc3_w, const float* fc3_b, float* state, float* logits, float* probs,
-                       int T, int64_t B, int64_t Bp, int NC, int sms, cudaStream_t stream) {
+                       int T, int64_t B, int64_t Bp, int NC, int sms, cudaStream_t stream, float* scores_tm, float* pooled,
+                       float* embedding) {
     const size_t smem = sizeof(WideSmem<NCH>) + 1024;
-    cudaError_t e = cudaFuncSetAttribute(decoder_infer_wide_kernel<NCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(decoder_infer_wide_kernel<NCH, kEx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_wide_bf16: shared memory opt-in failed (%s)", cudaGetErrorString(e));
     const int nquarters = (int)((B + 31) / 32);
     const int ntiles = (nquarters + 3) / 4;
@@ -612,9 +623,9 @@ static int launch_wide(const void* x, const void* packed, const float* ln_w, con
     attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, decoder_infer_wide_kernel<NCH>, reinterpret_cast<const __nv_bfloat16*>(x),
+    e = cudaLaunchKernelEx(&cfg, decoder_infer_wide_kernel<NCH, kEx>, reinterpret_cast<const __nv_bfloat16*>(x),
                            reinterpret_cast<const unsigned char*>(packed), ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, state, logits, probs,
-                           T, B, Bp, NC, nquarters, cs, g_wide_dbg);
+                           T, B, Bp, NC, nquarters, cs, g_wide_dbg, scores_tm, pooled, embedding);
     if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_wide_bf16: launch failed (%s)", cudaGetErrorString(e));
     count_launch();
     return check_launch("na_decoder_infer_wide_bf16");
@@ -670,10 +681,11 @@ extern "C" int na_decoder_pack_wide_bf16(const float* w_ih0, const float* w_hh0,
     return check_launch("na_decoder_pack_wide_bf16");
 }
 
-extern "C" int na_decoder_infer_wide_bf16(const void* x_bf16_tmp, const void* packed, const float* ln_w, const float* ln_b,
-                                          const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
-                                          void* state, float* logits, float* probs, int64_t T, int64_t B, int64_t Bp,
-                                          int64_t H, int64_t NC, na_stream_t stream) {
+extern "C" int na_decoder_infer_wide_bf16_ex(const void* x_bf16_tmp, const void* packed, const float* ln_w, const float* ln_b,
+                                             const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                                             void* state, float* logits, float* probs, float* scores_tm, float* pooled,
+                                             float* embedding, int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC,
+                                             na_stream_t stream) {
     using namespace na;
     NA_REQUIRE(H == 96 || H == 144 || H == 192, NA_EUNSUPPORTED, "na_decoder_infer_wide_bf16: hidden_size=%lld (96, 144, 192)", (long long)H);
     NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1 && Bp >= B && Bp % tc::kRows == 0, NA_EINVAL,
@@ -682,10 +694,25 @@ extern "C" int na_decoder_infer_wide_bf16(const void* x_bf16_tmp, const void* pa
     NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_infer_wide_bf16: num_classes=%lld", (long long)NC);
     NA_REQUIRE_PTR(x_bf16_tmp); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(state); NA_REQUIRE_PTR(logits);
     NA_OPTIONAL_PTR(probs);
+    NA_OPTIONAL_PTR(scores_tm); NA_OPTIONAL_PTR(pooled); NA_OPTIONAL_PTR(embedding);
     NA_REQUIRE(ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL, "na_decoder_infer_wide_bf16: null parameter pointer");
     int rc = NA_EUNSUPPORTED;
-    NA_WIDE_DISPATCH(H, rc = tc::launch_wide<NCH>(x_bf16_tmp, packed, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b,
-                                                  reinterpret_cast<float*>(state), logits, probs, (int)T, B, Bp, (int)NC,
-                                                  tc::wide_sms(), as_stream(stream)));
+    if (!(scores_tm || pooled || embedding)) {
+        NA_WIDE_DISPATCH(H, (rc = tc::launch_wide<NCH, false>(x_bf16_tmp, packed, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b,
+                                                              reinterpret_cast<float*>(state), logits, probs, (int)T, B, Bp, (int)NC,
+                                                              tc::wide_sms(), as_stream(stream), nullptr, nullptr, nullptr)));
+    } else {
+        NA_WIDE_DISPATCH(H, (rc = tc::launch_wide<NCH, true>(x_bf16_tmp, packed, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b,
+                                                             reinterpret_cast<float*>(state), logits, probs, (int)T, B, Bp, (int)NC,
+                                                             tc::wide_sms(), as_stream(stream), scores_tm, pooled, embedding)));
+    }
     return rc;
+}
+
+extern "C" int na_decoder_infer_wide_bf16(const void* x_bf16_tmp, const void* packed, const float* ln_w, const float* ln_b,
+                                          const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
+                                          void* state, float* logits, float* probs, int64_t T, int64_t B, int64_t Bp,
+                                          int64_t H, int64_t NC, na_stream_t stream) {
+    return na_decoder_infer_wide_bf16_ex(x_bf16_tmp, packed, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, state, logits, probs,
+                                         nullptr, nullptr, nullptr, T, B, Bp, H, NC, stream);
 }

@@ -77,17 +77,23 @@ __global__ void pack_decoder_x3_kernel(const float* __restrict__ w_ih0, const fl
 // Epilogue of one tile for one warp: both layers of (lane quarter q, unit group g).  R = row replication as in
 // decoder_infer_v2_kernel: the tile holds 128 / R distinct windows, copy rp = q / (4 / R) of source quarter qs = q % (4 / R)
 // takes granules [4 g + rp * (4 / R), + 4 / R) of the 12 four-unit granules and stores its h (hi and lo) to every copy.
-template <int R, int NR>
+// kEx: also store the attention scores (time-major [T][B]) and the pooled vector / LayerNorm output ([B][48]) of every
+// window b < B: the scores and the LayerNorm output by the first row copy of the g == 0 warps (the one that runs the
+// head), the pooled vector by every thread for the units it pooled.
+template <int R, int NR, bool kEx>
 __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const int g, const int lane, const int nq, const int T,
                                                  const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                                  const int64_t b0, const int64_t B, const int NC,
                                                  const float* __restrict__ ln_w, const float* __restrict__ ln_b,
                                                  const float* __restrict__ fc0_w, const float* __restrict__ fc0_b,
                                                  const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
-                                                 float* __restrict__ logits, float* __restrict__ probs) {
+                                                 float* __restrict__ logits, float* __restrict__ probs,
+                                                 float* __restrict__ scores_tm, float* __restrict__ pooled,
+                                                 float* __restrict__ embedding) {
     constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
+    const bool ex_writer = kEx && g == 0 && rp == 0 && b0 + wrow < B;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     const int gr0 = 4 * g + rp * kSlots;           // first granule
     if (qs >= nq) {                                // idle quarter: keep the barrier protocol only
@@ -176,6 +182,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             uint32_t sc2[2];
             x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
             if (t >= 2) pool(__uint_as_float(sc2[0]));     // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
+            if constexpr (kEx)
+                if (t >= 2 && ex_writer && scores_tm) scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]);
             layer_phase(tmem_d1, c1, S.h1, hprev);
             tc_fence_before();
             fence_proxy_async_smem();
@@ -189,11 +197,23 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
         tc_fence_before();
         pool(__uint_as_float(sc2[0]));
+        if constexpr (kEx)
+            if (ex_writer && scores_tm) scores_tm[(int64_t)(T - 1) * B + b0 + wrow] = __uint_as_float(sc2[0]);
     }
     // ---- head: LN -> fc0 -> RReLU(eval) -> fc3 -> softmax (fp32; parameters from global memory) ------
     float* zx = reinterpret_cast<float*>(S.h0[0]);             // [128][49] floats <= the two h0 buffers
 #pragma unroll
     for (int j = 0; j < kU; ++j) zx[wrow * (kH + 1) + gr0 * 4 + j] = z[j];
+    if constexpr (kEx)
+        // every copy stores the units it pooled, from its own registers: a further use of the head's products would
+        // change which of them the assembler contracts into FMAs, and the logits would no longer be the default's
+        if (pooled && b0 + wrow < B) {
+            float zp[kU];
+            const float inv = 1.0f / l;
+#pragma unroll
+            for (int j = 0; j < kU; ++j) zp[j] = z[j] * inv;
+            store_row<kU>(pooled + (b0 + wrow) * kH + gr0 * 4, zp);
+        }
     named_bar_sync(1 + qs, 96 * R);                // the 3 R warps that share source quarter qs
     if (g == 0 && rp == 0) {
         const int64_t b = b0 + wrow;
@@ -209,6 +229,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         const float rstd = 1.0f / sqrtf(var * (1.0f / kH) + kLnEps);
 #pragma unroll
         for (int j = 0; j < kH; ++j) zf[j] = fmaf((zf[j] - mean) * rstd, __ldg(ln_w + j), __ldg(ln_b + j));
+        if constexpr (kEx)
+            if (ex_writer && embedding) store_row<kH>(embedding + b * kH, zf);
         float lg[NA_MAX_CLASSES];
 #pragma unroll
         for (int k = 0; k < NA_MAX_CLASSES; ++k) lg[k] = (k < NC) ? __ldg(fc3_b + k) : -INFINITY;
@@ -238,7 +260,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
     }
 }
 
-template <int NR>
+template <int NR, bool kEx = false>
 __global__ void __launch_bounds__(kX3Threads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
@@ -247,7 +269,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         const float* __restrict__ fc0_w, const float* __restrict__ fc0_b,
                         const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
                         float* __restrict__ logits, float* __restrict__ probs,
-                        int T, int64_t B, int NC, int nquarters) {
+                        int T, int64_t B, int NC, int nquarters,
+                        float* __restrict__ scores_tm,              // kEx: [T][B] scores, [B][48] pooled / LayerNorm output
+                        float* __restrict__ pooled, float* __restrict__ embedding) {
     constexpr int kMmaWarp = 12, kTmaWarp = 13;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     SmemX3& S = *reinterpret_cast<SmemX3*>(smem_raw);
@@ -450,9 +474,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
         } else {
             // ================= epilogue: both layers of (quarter q, unit group g) ================================
             const int q = warp & 3, g = warp >> 2;
-            if (R == 1) x3_epilogue_tile<1, NR>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs);
-            else if (R == 2) x3_epilogue_tile<2, NR>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs);
-            else x3_epilogue_tile<4, NR>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs);
+            if (R == 1) x3_epilogue_tile<1, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
+            else if (R == 2) x3_epilogue_tile<2, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
+            else x3_epilogue_tile<4, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
         }
         __syncthreads();       // tile done: every MMA has completed; the z exchange in h0 has been consumed
         q0 += nq;
@@ -491,17 +515,19 @@ extern "C" int na_decoder_pack_x3(const float* w_ih0, const float* w_hh0, const 
     return check_launch("na_decoder_pack_x3");
 }
 
-extern "C" int na_decoder_infer_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
-                                   const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
-                                   const float* fc3_w, const float* fc3_b, float* logits, float* probs, int64_t T,
-                                   int64_t B, int64_t NC, na_stream_t stream) {
+extern "C" int na_decoder_infer_x3_ex(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                      const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                      const float* fc3_w, const float* fc3_b, float* logits, float* probs, float* scores_tm,
+                                      float* pooled, float* embedding, int64_t T, int64_t B, int64_t NC, na_stream_t stream) {
     using namespace na;
     NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_infer_x3: bad shape T=%lld B=%lld", (long long)T, (long long)B);
     NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_infer_x3: num_classes=%lld", (long long)NC);
     NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(logits);
     NA_OPTIONAL_PTR(probs);
+    NA_OPTIONAL_PTR(scores_tm); NA_OPTIONAL_PTR(pooled); NA_OPTIONAL_PTR(embedding);
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
                "na_decoder_infer_x3: null parameter pointer");
+    const bool ex = scores_tm || pooled || embedding;
     static int sms = 0;
     if (sms == 0) {
         int dev = 0;
@@ -512,21 +538,34 @@ extern "C" int na_decoder_infer_x3(const float* x, const void* packed, const flo
     const size_t smem = sizeof(tc::SmemX3) + 1024;
     const int nquarters = (int)((B + 31) / 32);
     const int grid = nquarters < sms ? nquarters : sms;    // < 4 quarters per CTA run as row-replicated tiles
-#define NA_X3_LAUNCH(NRV)                                                                                                            \
+#define NA_X3_LAUNCH(NRV, EXV)                                                                                                       \
     {                                                                                                                                \
-        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, EXV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e));    \
-        tc::decoder_infer_x3_kernel<NRV><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                                         \
+        tc::decoder_infer_x3_kernel<NRV, EXV><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                                    \
             x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, \
-            (int)T, B, (int)NC, nquarters);                                                                                          \
+            (int)T, B, (int)NC, nquarters, scores_tm, pooled, embedding);                                                            \
     }
-    switch (tc::g_x3_rcp_fma) {
-        case 0: NA_X3_LAUNCH(0) break;
-        case 2: NA_X3_LAUNCH(2) break;
-        case 3: NA_X3_LAUNCH(3) break;
-        default: NA_X3_LAUNCH(1) break;
+    switch (tc::g_x3_rcp_fma * 2 + (ex ? 1 : 0)) {
+        case 0: NA_X3_LAUNCH(0, false) break;
+        case 1: NA_X3_LAUNCH(0, true) break;
+        case 4: NA_X3_LAUNCH(2, false) break;
+        case 5: NA_X3_LAUNCH(2, true) break;
+        case 6: NA_X3_LAUNCH(3, false) break;
+        case 7: NA_X3_LAUNCH(3, true) break;
+        default:
+            if (ex) NA_X3_LAUNCH(1, true) else NA_X3_LAUNCH(1, false)
+            break;
     }
 #undef NA_X3_LAUNCH
     count_launch();
     return check_launch("na_decoder_infer_x3");
+}
+
+extern "C" int na_decoder_infer_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                   const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                   const float* fc3_w, const float* fc3_b, float* logits, float* probs, int64_t T,
+                                   int64_t B, int64_t NC, na_stream_t stream) {
+    return na_decoder_infer_x3_ex(x, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, nullptr,
+                                  nullptr, nullptr, T, B, NC, stream);
 }

@@ -63,12 +63,14 @@ __device__ __forceinline__ void head_tail(const float (&zp)[JPL], const HeadPara
     a_post = (a >= 0.f ? a : a * slope) * keep;
 }
 
-template <int JPL, int CH>
+// kEx: also store the attention scores (time-major [T][B], lane 0), the pooled vector and the LayerNorm output ([B][H]).
+template <int JPL, int CH, bool kEx = false>
 __global__ void __launch_bounds__(kHeadWarps * 32)
 head_fwd_kernel(const float* __restrict__ h, HeadParams p, float* __restrict__ logits,
                 float* __restrict__ probs, float* __restrict__ stats, float* __restrict__ zpool,
                 const float* __restrict__ zpool_in,      // != NULL: tail only (pooling was done upstream)
-                int T, int64_t B, int64_t Bp, int H, int NC) {
+                int T, int64_t B, int64_t Bp, int H, int NC,
+                float* __restrict__ scores_tm, float* __restrict__ pooled, float* __restrict__ embedding) {
     extern __shared__ float smem[];
     float* w0t = smem;                               // [H][33]  fc0_w transposed
     float* zs = smem + H * (kFc + 1);                // [warps][H]
@@ -120,6 +122,8 @@ head_fwd_kernel(const float* __restrict__ h, HeadParams p, float* __restrict__ l
             for (int i = 0; i < JPL; ++i) d = fmaf(hv[u][i], wa[i], d);
             s[u] = (t0 + u < T) ? warp_sum(d) + ba : -INFINITY;
             cm = fmaxf(cm, s[u]);
+            if constexpr (kEx)
+                if (scores_tm && lane == 0 && t0 + u < T) scores_tm[(int64_t)(t0 + u) * B + b] = s[u];
         }
         const float mn = fmaxf(m, cm);
         const float sc = expf(m - mn);     // first chunk: exp(-inf) = 0
@@ -141,11 +145,16 @@ head_fwd_kernel(const float* __restrict__ h, HeadParams p, float* __restrict__ l
         zp[i] = z[i] / l;
         const int j = lane + 32 * i;
         if (zpool && j < H) zpool[b * H + j] = zp[i];
+        if constexpr (kEx)
+            if (pooled && j < H) pooled[b * H + j] = zp[i];
     }
     if (stats && lane == 0) { stats[2 * b] = m; stats[2 * b + 1] = l; }
 
     float rstd, a_pre, a_post, act_grad;
     head_tail<JPL>(zp, p, w0t, zs + warp * H, b, H, lane, xhat, rstd, a_pre, a_post, act_grad);
+    if constexpr (kEx)
+        if (embedding)
+            for (int j = lane; j < H; j += 32) embedding[b * H + j] = zs[warp * H + j];
     float lg = -INFINITY;
     for (int k = 0; k < NC; ++k) {
         const float v = warp_sum(a_post * p.fc3_w[k * kFc + lane]) + p.fc3_b[k];
@@ -316,16 +325,17 @@ head_bwd_kernel(const float* __restrict__ dlogits, const float* __restrict__ h, 
     }
 }
 
-template <int JPL, int CH>
+template <int JPL, int CH, bool kEx = false>
 int launch_head_fwd(const float* h, const HeadParams& p, float* logits, float* probs, float* stats, float* zpool,
                     int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, cudaStream_t st,
-                    const float* zpool_in = nullptr) {
+                    const float* zpool_in = nullptr, float* scores_tm = nullptr, float* pooled = nullptr,
+                    float* embedding = nullptr) {
     const size_t smem = sizeof(float) * (H * (kFc + 1) + kHeadWarps * H);
     if (smem > 48 * 1024)
-        cudaFuncSetAttribute(head_fwd_kernel<JPL, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(head_fwd_kernel<JPL, CH, kEx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const unsigned grid = (unsigned)((B + kHeadWarps - 1) / kHeadWarps);
-    head_fwd_kernel<JPL, CH><<<grid, kHeadWarps * 32, smem, st>>>(h, p, logits, probs, stats, zpool, zpool_in, (int)T, B, Bp,
-                                                                (int)H, (int)NC);
+    head_fwd_kernel<JPL, CH, kEx><<<grid, kHeadWarps * 32, smem, st>>>(h, p, logits, probs, stats, zpool, zpool_in, (int)T, B, Bp,
+                                                                     (int)H, (int)NC, scores_tm, pooled, embedding);
     count_launch();
     return check_launch("na_head_fwd_f32");
 }
@@ -355,23 +365,103 @@ static int check_head_shape(const char* fn, int64_t T, int64_t B, int64_t Bp, in
 
 }  // namespace na
 
-extern "C" int na_head_fwd_f32(const float* h, const float* attn_w, const float* attn_b, const float* ln_w,
-                               const float* ln_b, const float* fc0_w, const float* fc0_b, const float* fc3_w,
-                               const float* fc3_b, const float* rrelu_slope, const float* drop_mask,
-                               float drop_scale, float* logits, float* probs, float* stats, float* zpool,
-                               int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream) {
+extern "C" int na_head_fwd_f32_ex(const float* h, const float* attn_w, const float* attn_b, const float* ln_w,
+                                  const float* ln_b, const float* fc0_w, const float* fc0_b, const float* fc3_w,
+                                  const float* fc3_b, const float* rrelu_slope, const float* drop_mask,
+                                  float drop_scale, float* logits, float* probs, float* scores_tm, float* pooled,
+                                  float* embedding, float* stats, float* zpool, int64_t T, int64_t B, int64_t Bp, int64_t H,
+                                  int64_t NC, na_stream_t stream) {
     using namespace na;
     if (int rc = check_head_shape("na_head_fwd_f32", T, B, Bp, H, NC)) return rc;
     NA_REQUIRE_PTR(h); NA_REQUIRE_PTR(logits);
+    NA_OPTIONAL_PTR(scores_tm); NA_OPTIONAL_PTR(pooled); NA_OPTIONAL_PTR(embedding);
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
                "na_head_fwd_f32: null parameter pointer");
     HeadParams p{attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, rrelu_slope, drop_mask, drop_scale};
     cudaStream_t st = as_stream(stream);
+    if (scores_tm || pooled || embedding) {
+#define NA_HEAD_EX(JPL, CH) \
+        launch_head_fwd<JPL, CH, true>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st, nullptr, scores_tm, pooled, embedding)
+        if (H <= 64) return NA_HEAD_EX(2, 8);
+        if (H <= 128) return NA_HEAD_EX(4, 4);
+        if (H <= 256) return NA_HEAD_EX(8, 2);
+        if (H <= 512) return NA_HEAD_EX(16, 1);
+        return NA_HEAD_EX(32, 1);
+#undef NA_HEAD_EX
+    }
     if (H <= 64) return launch_head_fwd<2, 8>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st);
     if (H <= 128) return launch_head_fwd<4, 4>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st);
     if (H <= 256) return launch_head_fwd<8, 2>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st);
     if (H <= 512) return launch_head_fwd<16, 1>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st);
     return launch_head_fwd<32, 1>(h, p, logits, probs, stats, zpool, T, B, Bp, H, NC, st);
+}
+
+extern "C" int na_head_fwd_f32(const float* h, const float* attn_w, const float* attn_b, const float* ln_w,
+                               const float* ln_b, const float* fc0_w, const float* fc0_b, const float* fc3_w,
+                               const float* fc3_b, const float* rrelu_slope, const float* drop_mask,
+                               float drop_scale, float* logits, float* probs, float* stats, float* zpool,
+                               int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream) {
+    return na_head_fwd_f32_ex(h, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, rrelu_slope, drop_mask, drop_scale,
+                              logits, probs, nullptr, nullptr, nullptr, stats, zpool, T, B, Bp, H, NC, stream);
+}
+
+namespace na {
+// Attention weights from the time-major scores the inference kernels wrote: scores [T][B] -> attn [B][T], per window
+// alpha_t = exp(s_t - max_t s) / sum_t exp(s_t - max_t s) in fp32 (torch.softmax's two passes; a NaN score makes the
+// window's whole row NaN, as in torch).  A CTA owns 32 windows: lane = window for the reads (one 128-byte run per step),
+// the 8 warps stride over time, partial maxima / sums are combined in a fixed order; the write pass transposes 32 x 32
+// blocks through shared memory so that lane = step for the stores.
+constexpr int kSmWarps = 8;
+__global__ void __launch_bounds__(kSmWarps * 32) attention_softmax_kernel(const float* __restrict__ s, float* __restrict__ a,
+                                                                          int64_t T, int64_t B) {
+    __shared__ float red[kSmWarps][32];
+    __shared__ float tile[kSmWarps][32][33];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t b0 = (int64_t)blockIdx.x * 32, b = b0 + lane;
+    const bool live = b < B;
+    auto nan_max = [](float m, float v) { return (v > m || v != v) ? v : m; };     // NaN wins, as torch.max
+    float m = -INFINITY;
+    if (live)
+        for (int64_t t = warp; t < T; t += kSmWarps) m = nan_max(m, __ldg(s + t * B + b));
+    red[warp][lane] = m;
+    __syncthreads();
+    m = red[0][lane];
+#pragma unroll
+    for (int w = 1; w < kSmWarps; ++w) m = nan_max(m, red[w][lane]);
+    __syncthreads();
+    float l = 0.f;
+    if (live)
+        for (int64_t t = warp; t < T; t += kSmWarps) l += expf(__ldg(s + t * B + b) - m);
+    red[warp][lane] = l;
+    __syncthreads();
+    l = 0.f;
+#pragma unroll
+    for (int w = 0; w < kSmWarps; ++w) l += red[w][lane];
+    // write pass: warp w handles steps [32 k, 32 k + 32) for k = w, w + 8, ...
+    __shared__ float mrow[32], lrow[32];
+    if (warp == 0) { mrow[lane] = m; lrow[lane] = l; }
+    __syncthreads();
+    const int nb = B - b0 < 32 ? (int)(B - b0) : 32;
+    for (int64_t t0 = (int64_t)warp * 32; t0 < T; t0 += kSmWarps * 32) {
+        const int nt = T - t0 < 32 ? (int)(T - t0) : 32;
+        for (int i = 0; i < nt; ++i)                       // row i = step t0 + i, lane = window
+            if (live) tile[warp][i][lane] = __ldg(s + (t0 + i) * B + b);
+        __syncwarp();
+        for (int r = 0; r < nb; ++r)                       // row r = window b0 + r, lane = step
+            if (lane < nt) a[(b0 + r) * T + t0 + lane] = expf(tile[warp][lane][r] - mrow[r]) / lrow[r];
+        __syncwarp();
+    }
+}
+}  // namespace na
+
+extern "C" int na_attention_softmax_f32(const float* scores_tm, float* attn, int64_t T, int64_t B, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T <= INT32_MAX && B >= 1, NA_EINVAL, "na_attention_softmax_f32: bad shape T=%lld B=%lld", (long long)T,
+               (long long)B);
+    NA_REQUIRE_PTR(scores_tm); NA_REQUIRE_PTR(attn);
+    attention_softmax_kernel<<<(unsigned)((B + 31) / 32), kSmWarps * 32, 0, as_stream(stream)>>>(scores_tm, attn, T, B);
+    count_launch();
+    return check_launch("na_attention_softmax_f32");
 }
 
 extern "C" int64_t na_head_param_floats(int64_t H, int64_t NC) {

@@ -122,6 +122,15 @@ __device__ __forceinline__ void st_shared_v4(void* p, uint32_t a, uint32_t b, ui
                  : "memory");
 }
 
+// One window's row of N fp32 values (N % 4 == 0) to global memory, 16 B per store (the row starts 16-byte aligned:
+// the intermediates outputs of the inference kernels, [B][H] with H a multiple of 4).
+template <int N>
+__device__ __forceinline__ void store_row(float* dst, const float* v) {
+    static_assert(N % 4 == 0, "row length");
+#pragma unroll
+    for (int j = 0; j < N; j += 4) *reinterpret_cast<float4*>(dst + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
+}
+
 // One LSTM cell update for the 8 units of a block; v = [i x8 | f x8 | g x8 | o x8] pre-activations.
 // Returns h packed as 4 x bf16x2.
 __device__ __forceinline__ void cell_block(const uint32_t (&v)[32], float* c, uint32_t (&hp)[4]) {

@@ -9,7 +9,7 @@ hand-written sm_100a kernels (libneuroalpha_b200.so).  There is no CPU compute p
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Optional
+from typing import Dict, List, NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -18,6 +18,17 @@ import torch.nn as nn
 from . import ops
 
 CLASS_NAMES = ["Food", "Water", "BG-Noise"]      # reference lstm_eeg_model.py:11, verbatim
+
+
+class DecoderOutputs(NamedTuple):
+    """``EEG_LSTM.decode_intermediates``: everything the eval forward computes per window, fp32 on the device of ``x``.
+    ``attention`` = softmax over time of ``attn(out)`` (reference lstm_eeg_model.py:36), ``pooled`` = the attention-weighted
+    sum of the last LSTM layer's h (:37), ``embedding`` = ``ln(pooled)``, the input of ``fc`` (:38)."""
+    logits: torch.Tensor        # [B, K]
+    probs: torch.Tensor         # [B, K]
+    attention: torch.Tensor     # [B, T]
+    pooled: torch.Tensor        # [B, H]
+    embedding: torch.Tensor     # [B, H]
 
 
 class LSTMParameters(nn.Module):
@@ -69,7 +80,8 @@ class EEG_LSTM(nn.Module):
         self.lstm = LSTMParameters(input_size, hidden_size, num_layers, dropout if num_layers > 1 else 0.0)
         self.ln = nn.LayerNorm(hidden_size)
         self.attn = nn.Linear(hidden_size, 1)
-        # containers only (names fc.0.* / fc.3.* as in the reference); never called
+        # containers only (names fc.0.* / fc.3.* as in the reference); never called, so forward hooks registered on
+        # attn / ln / fc never fire -- decode_intermediates() returns what they would see
         self.fc = nn.Sequential(
             nn.Linear(hidden_size, 32),
             nn.RReLU(),
@@ -169,6 +181,40 @@ class EEG_LSTM(nn.Module):
             return ops.decoder_infer(x, [self.lstm.layer(l) for l in range(L)],
                                      [ops._f32c(t) for t in self._head_params()], want_probs, self.zscore_input,
                                      [self._packed(l) for l in range(L)])
+
+    def decode_intermediates(self, x: torch.Tensor) -> DecoderOutputs:
+        """Eval-mode forward without autograd that also returns the attention weights over time, the pooled vector and
+        its LayerNorm output (``DecoderOutputs``, all fp32 on the device of ``x``).
+
+        In the reference these are read with forward hooks on ``model.attn`` / ``model.ln``.  Here ``attn``, ``ln`` and
+        ``fc`` are parameter containers that the fused kernels never call, so such hooks do not fire: this method
+        replaces them.  The intermediates come from the same kernel launch as the logits, on the tier ``decode`` picks
+        (same ``compute_dtype`` / input dtype / ``zscore_input`` handling), and carry that tier's accuracy contract;
+        logits and probs are those of ``decode(x)``."""
+        ops._require_cuda(x)
+        B, T = x.shape[0], x.shape[1]
+        if B == 0:
+            H, K = self.lstm.hidden_size, self.fc[3].out_features
+            e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=x.device)
+            return DecoderOutputs(e(0, K), e(0, K), e(0, T), e(0, H), e(0, H))
+        bf16 = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
+                or self.attn.weight.dtype == torch.bfloat16)
+        with torch.no_grad():
+            if bf16 and self.tc_supported():
+                return DecoderOutputs(*ops.decoder_infer_tc_intermediates(x, self._packed_tc(), self._head_params(),
+                                                                          self.zscore_input))
+            if bf16 and self.tc_wide_supported():
+                return DecoderOutputs(*ops.decoder_infer_wide_intermediates(x, self._packed_tc_wide(), self._head_params(),
+                                                                            self.lstm.hidden_size, self.zscore_input))
+            if ops.EXACT_TC and not bf16 and self.tc_supported() and x.dtype == torch.float32:
+                if self.zscore_input:
+                    x = ops.window_zscore(x, x.shape[1], x.shape[1], True, False, ops.NA_F32)
+                return DecoderOutputs(*ops.decoder_infer_x3_intermediates(x.contiguous(), self._packed_x3(),
+                                                                          self._head_params()))
+            L = self.lstm.num_layers
+            return DecoderOutputs(*ops.decoder_infer_intermediates(
+                x, [self.lstm.layer(l) for l in range(L)], [ops._f32c(t) for t in self._head_params()],
+                self.zscore_input, [self._packed(l) for l in range(L)]))
 
     def inject_noise(self, drop1: Optional[torch.Tensor] = None, rrelu_slope: Optional[torch.Tensor] = None,
                      drop2: Optional[torch.Tensor] = None) -> None:
@@ -323,6 +369,20 @@ class SimplePredictor:
             probs = probs[0].detach().cpu().numpy().astype(np.float32)
         y_idx = int(np.argmax(probs))
         return probs, self.class_names[y_idx]
+
+    def explain(self, chunk_TxC: np.ndarray):
+        """``predict`` plus the attention weights over time: chunk [T,C] -> (probs float32[K], label, attention
+        float32[T]), with the same preprocessing.  The attention curve shows which part of the window drove the
+        decision (forward hooks on ``model.attn`` do not fire in this implementation; see
+        ``EEG_LSTM.decode_intermediates``)."""
+        x = self.pre.transform(chunk_TxC)
+        x_t = torch.from_numpy(np.ascontiguousarray(x[None, ...])).float().to(self.compute_device)
+        with self._no_grad():
+            out = self.model.decode_intermediates(x_t)
+            probs = out.probs[0].detach().cpu().numpy().astype(np.float32)
+            attention = out.attention[0].detach().cpu().numpy().astype(np.float32)
+        y_idx = int(np.argmax(probs))
+        return probs, self.class_names[y_idx], attention
 
     def predict_batch(self, chunks_BxTxC: np.ndarray, preprocess: bool = True) -> np.ndarray:
         """Batched sibling of ``predict``: [B,T,C] -> probs [B,K] (one H2D, one launch sequence, one D2H)."""

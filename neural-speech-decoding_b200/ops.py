@@ -93,7 +93,8 @@ def all_custom_ops():
             head_bwd, trial_mean, decoder_pack_bf16, decoder_infer_bf16, lstm2_fwd_train_bf16, lstm_bwd_bf16,
             dropout_mask_u8, head_tail_fwd, head_tail_bwd, decoder_infer_bf16_x32, decoder_pack_x3, decoder_infer_x3,
             decoder_pack_wide_bf16, decoder_infer_wide_bf16, x3_split_input, lstm_fwd_train_x3, lstm_bwd_x3, lstm_wgrad_x3,
-            lstm_wide_fwd_train, lstm_wide_bwd]
+            lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
+            decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex]
 
 
 def launch_count() -> int:
@@ -265,6 +266,57 @@ def _(h, B, params, rrelu_slope, drop_mask, drop_scale, want_probs, save):
             h.new_empty((B, 2) if save else (0,)), h.new_empty((B, H) if save else (0,)))
 
 
+def _ex_outputs(B: int, T: int, H: int, dev) -> Tuple[Tensor, Tensor, Tensor]:
+    """Intermediates outputs of the *_ex entry points: scores (time-major [T,B]), pooled [B,H], embedding [B,H]."""
+    return (torch.empty((T, B), dtype=torch.float32, device=dev), torch.empty((B, H), dtype=torch.float32, device=dev),
+            torch.empty((B, H), dtype=torch.float32, device=dev))
+
+
+def _ex_fake(like: Tensor, B: int, T: int, H: int, NC: int):
+    f = torch.float32
+    return (like.new_empty((B, NC), dtype=f), like.new_empty((B, NC), dtype=f), like.new_empty((T, B), dtype=f),
+            like.new_empty((B, H), dtype=f), like.new_empty((B, H), dtype=f))
+
+
+@torch.library.custom_op("neuroalpha::head_fwd_ex", mutates_args=(), device_types="cuda")
+@_device_guard
+def head_fwd_ex(h: Tensor, B: int, params: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """K4 in eval mode with its intermediates.  h TMP [T,Bp,H] -> (logits [B,NC], probs [B,NC], scores [T,B] time-major,
+    pooled [B,H] (before LayerNorm), embedding [B,H] (LayerNorm output))."""
+    _require_cuda(h, *params)
+    T, Bp, H = h.shape
+    NC = params[6].shape[0]
+    dev = h.device
+    logits = torch.empty((B, NC), dtype=torch.float32, device=dev)
+    probs = torch.empty((B, NC), dtype=torch.float32, device=dev)
+    scores, pooled, emb = _ex_outputs(B, T, H, dev)
+    _lib.call("na_head_fwd_f32_ex", h.data_ptr(), *[p.data_ptr() for p in params], None, None, 1.0, logits.data_ptr(),
+              probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), None, None, T, B, Bp, H, NC, _stream())
+    return logits, probs, scores, pooled, emb
+
+
+@head_fwd_ex.register_fake
+def _(h, B, params):
+    return _ex_fake(h, B, h.shape[0], h.shape[2], params[6].shape[0])
+
+
+@torch.library.custom_op("neuroalpha::attention_softmax", mutates_args=(), device_types="cuda")
+@_device_guard
+def attention_softmax(scores_tm: Tensor) -> Tensor:
+    """Time-major attention scores [T,B] -> attention weights [B,T] (softmax over time per window, fp32)."""
+    _require_cuda(scores_tm)
+    T, B = scores_tm.shape
+    attn = torch.empty((B, T), dtype=torch.float32, device=scores_tm.device)
+    if attn.numel():
+        _lib.call("na_attention_softmax_f32", _f32c(scores_tm).data_ptr(), attn.data_ptr(), T, B, _stream())
+    return attn
+
+
+@attention_softmax.register_fake
+def _(scores_tm):
+    return scores_tm.new_empty((scores_tm.shape[1], scores_tm.shape[0]), dtype=torch.float32)
+
+
 @torch.library.custom_op("neuroalpha::head_bwd", mutates_args=(), device_types="cuda")
 @_device_guard
 def head_bwd(dlogits: Tensor, h: Tensor, stats: Tensor, zpool: Tensor, params: Sequence[Tensor],
@@ -383,6 +435,67 @@ def _(x, packed, head, want_probs):
     return x.new_empty((x.shape[0], NC), dtype=torch.float32), x.new_empty((x.shape[0], NC) if want_probs else (0,), dtype=torch.float32)
 
 
+@torch.library.custom_op("neuroalpha::decoder_infer_bf16_ex", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_infer_bf16_ex(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor],
+                          B: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_bf16 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,48], embedding [B,48])."""
+    _require_cuda(x_tmp, packed, *head)
+    T, Bp, C = x_tmp.shape
+    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
+        raise RuntimeError("decoder_infer_bf16_ex: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
+    head = [_f32c(t) for t in head]
+    NC = head[6].shape[0]
+    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
+    probs = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
+    scores, pooled, emb = _ex_outputs(B, T, 48, x_tmp.device)
+    _lib.call("na_decoder_infer_bf16_ex", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, Bp, NC, _stream())
+    return logits, probs, scores, pooled, emb
+
+
+@decoder_infer_bf16_ex.register_fake
+def _(x_tmp, packed, head, B):
+    return _ex_fake(x_tmp, B, x_tmp.shape[0], 48, head[6].shape[0])
+
+
+@torch.library.custom_op("neuroalpha::decoder_infer_bf16_x32_ex", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_infer_bf16_x32_ex(x: Tensor, packed: Tensor, head: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_bf16_x32 with its intermediates: (logits, probs, scores [T,B] time-major, pooled, embedding)."""
+    _require_cuda(x, packed, *head)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
+        raise RuntimeError("decoder_infer_bf16_x32_ex: x must be contiguous fp32 [B, T, 8]")
+    head = [_f32c(t) for t in head]
+    NC = head[6].shape[0]
+    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
+    probs = torch.empty((B, NC), dtype=torch.float32, device=x.device)
+    scores, pooled, emb = _ex_outputs(B, T, 48, x.device)
+    _lib.call("na_decoder_infer_bf16_x32_ex", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, NC, _stream())
+    return logits, probs, scores, pooled, emb
+
+
+@decoder_infer_bf16_x32_ex.register_fake
+def _(x, packed, head):
+    return _ex_fake(x, x.shape[0], x.shape[1], 48, head[6].shape[0])
+
+
+def decoder_infer_tc_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor],
+                                   zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_tc with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48]).
+    Same input handling as decoder_infer_tc; the attention weights come from the kernel's scores by attention_softmax."""
+    _require_cuda(x)
+    B, T, C = x.shape
+    if FUSED_INPUT and not zscore and x.dtype == torch.float32 and C == 8 and B > 0:
+        lg, pr, sc, zp, emb = decoder_infer_bf16_x32_ex(x.contiguous(), packed, list(head_params))
+    else:
+        xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
+        lg, pr, sc, zp, emb = decoder_infer_bf16_ex(xt, packed, list(head_params), B)
+    return lg, pr, attention_softmax(sc), zp, emb
+
+
 FUSED_INPUT = True          # decoder_infer_tc: read fp32 [B,T,8] directly (False: K1 pack + time-major kernel; A/B timing)
 
 
@@ -442,6 +555,36 @@ def decoder_infer_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], want_pro
 def _(x, packed, head, want_probs):
     NC = head[6].shape[0]
     return x.new_empty((x.shape[0], NC), dtype=torch.float32), x.new_empty((x.shape[0], NC) if want_probs else (0,), dtype=torch.float32)
+
+
+@torch.library.custom_op("neuroalpha::decoder_infer_x3_ex", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_infer_x3_ex(x: Tensor, packed: Tensor, head: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_x3 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,48], embedding [B,48])."""
+    _require_cuda(x, packed, *head)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
+        raise RuntimeError("decoder_infer_x3_ex: x must be contiguous fp32 [B, T, 8]")
+    head = [_f32c(t) for t in head]
+    NC = head[6].shape[0]
+    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
+    probs = torch.empty((B, NC), dtype=torch.float32, device=x.device)
+    scores, pooled, emb = _ex_outputs(B, T, 48, x.device)
+    _lib.call("na_decoder_infer_x3_ex", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, NC, _stream())
+    return logits, probs, scores, pooled, emb
+
+
+@decoder_infer_x3_ex.register_fake
+def _(x, packed, head):
+    return _ex_fake(x, x.shape[0], x.shape[1], 48, head[6].shape[0])
+
+
+def decoder_infer_x3_intermediates(x: Tensor, packed: Tensor,
+                                   head_params: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_x3 with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48])."""
+    lg, pr, sc, zp, emb = decoder_infer_x3_ex(x, packed, list(head_params))
+    return lg, pr, attention_softmax(sc), zp, emb
 
 
 WIDE_HIDDEN = (96, 144, 192)          # hidden sizes of the streamed-weight tensor-core kernel (na_decoder_wide.cu)
@@ -510,6 +653,42 @@ def _(x_tmp, packed, head, B, H, want_probs):
     return x_tmp.new_empty((B, NC), dtype=torch.float32), x_tmp.new_empty((B, NC) if want_probs else (0,), dtype=torch.float32)
 
 
+@torch.library.custom_op("neuroalpha::decoder_infer_wide_bf16_ex", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_infer_wide_bf16_ex(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor], B: int,
+                               H: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_wide_bf16 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,H], embedding [B,H])."""
+    _require_cuda(x_tmp, packed, *head)
+    T, Bp, C = x_tmp.shape
+    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
+        raise RuntimeError("decoder_infer_wide_bf16_ex: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
+    head = [_f32c(t) for t in head]
+    NC = head[4].shape[0]
+    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
+    probs = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
+    scores, pooled, emb = _ex_outputs(B, T, H, x_tmp.device)
+    state = _wide_state(H, x_tmp.device)
+    _lib.call("na_decoder_infer_wide_bf16_ex", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              state.data_ptr(), logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(),
+              T, B, Bp, H, NC, _stream())
+    return logits, probs, scores, pooled, emb
+
+
+@decoder_infer_wide_bf16_ex.register_fake
+def _(x_tmp, packed, head, B, H):
+    return _ex_fake(x_tmp, B, x_tmp.shape[0], H, head[4].shape[0])
+
+
+def decoder_infer_wide_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int,
+                                     zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_wide with the intermediates: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H])."""
+    _require_cuda(x)
+    B, T, C = x.shape
+    xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
+    lg, pr, sc, zp, emb = decoder_infer_wide_bf16_ex(xt, packed, list(head_params[2:]), B, H)
+    return lg, pr, attention_softmax(sc), zp, emb
+
+
 def decoder_infer_wide(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int, want_probs: bool = False,
                        zscore: bool = False) -> Tuple[Tensor, Tensor]:
     """Eval forward of a wide decoder on the tensor-core tier.  head_params in EEG_LSTM._head_params() order."""
@@ -544,6 +723,21 @@ def decoder_infer(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_param
         cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
     logits, probs, _, _ = head_fwd(cur, B, list(head_params), None, None, 1.0, want_probs, False)
     return logits, probs
+
+
+def decoder_infer_intermediates(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
+                                zscore: bool = False, packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None
+                                ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer with the intermediates of the head: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H]).
+    The LSTM layers are the same launches; the head kernel writes the scores, the pooled vector and the LayerNorm output."""
+    _require_cuda(x)
+    B, T, C = x.shape
+    cur = window_zscore(x, T, T, zscore, True, False)
+    for l, (w_ih, w_hh, b_ih, b_hh) in enumerate(lstm_params):
+        wt, bias = packed[l] if packed is not None else pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
+        cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
+    lg, pr, sc, zp, emb = head_fwd_ex(cur, B, list(head_params))
+    return lg, pr, attention_softmax(sc), zp, emb
 
 
 class DecoderFunction(torch.autograd.Function):
