@@ -127,6 +127,33 @@ int na_lstm_layer_wgrad_f32(const float* dgates, const float* in, const float* h
                             float* dw_ih, float* dw_hh, float* db, float* partials,
                             int64_t T, int64_t Bp, int64_t K, int64_t H, na_stream_t stream);
 
+/* ---- K3 with an initial state (nn.LSTM's hx) -----------------------------------------------
+ * The three calls above with the layer's initial state and its gradients; every extra pointer is
+ * TMP-row [Bp][H] fp32 (rows >= B zero), optional, and with all of them NULL each call is exactly
+ * its sibling.
+ *   fwd:   h_init / c_init = h_{-1} / c_{-1} (both or neither).  With them the generic kernel runs
+ *          for every shape (the H = 48 kernels start from zeros).
+ *   bwd:   c_init = c_{-1} (it enters d(forget gate) at t = 0); dh_last / dc_last = dLoss/dh_{T-1}
+ *          / dLoss/dc_{T-1} from outside the sequence output (nn.LSTM's h_n / c_n), added at
+ *          t = T-1; dh_init / dc_init receive dLoss/dh_{-1} / dLoss/dc_{-1}.
+ *   wgrad: h_init adds the step-0 term dgates_0^T h_init to dW_hh.
+ */
+int na_lstm_layer_fwd_f32_hx(const float* in, const float* wt, const float* bias,
+                             float* hout, float* cout, float* gates,
+                             const float* drop_mask, float drop_scale, float* hout_drop,
+                             int64_t T, int64_t Bp, int64_t K, int64_t H,
+                             const float* h_init, const float* c_init, na_stream_t stream);
+int na_lstm_layer_bwd_f32_hx(const float* dh_out, const float* gates, const float* cstate,
+                             const float* w_ih, const float* w_hh,
+                             float* dgates, float* din, const float* in_drop_mask, float drop_scale,
+                             int64_t T, int64_t Bp, int64_t K, int64_t H,
+                             const float* c_init, const float* dh_last, const float* dc_last,
+                             float* dh_init, float* dc_init, na_stream_t stream);
+int na_lstm_layer_wgrad_f32_hx(const float* dgates, const float* in, const float* h,
+                               float* dw_ih, float* dw_hh, float* db, float* partials,
+                               int64_t T, int64_t Bp, int64_t K, int64_t H,
+                               const float* h_init, na_stream_t stream);
+
 /* ---- K4: attention pool + LayerNorm + MLP head (+ softmax) -------------------------------
  * Replaces lstm_eeg_model.py:35-39 and, when probs != NULL, F.softmax at :97.
  *   h TMP [T][Bp][H];  attn_w [H], attn_b [1], ln_w [H], ln_b [H],
@@ -271,6 +298,14 @@ int na_decoder_infer_x3_ex(const float* x, const void* packed,
                            const float* fc0_w, const float* fc0_b, const float* fc3_w, const float* fc3_b,
                            float* logits, float* probs, float* scores_tm, float* pooled, float* embedding,
                            int64_t T, int64_t B, int64_t NC, na_stream_t stream);
+/* The two LSTM layers alone, as nn.LSTM(8, 48, num_layers=2, batch_first=True) in eval mode, with the same arithmetic:
+ * no pooling and no head.  Accuracy against float64 (max|d| / max|ref| per tensor): h_n / c_n within 1e-5; the per-step
+ * out carries the operand split's error (about 22 bits per operand) through the recurrence: 6.2e-5 over 625 steps of
+ * the shipped EEG windows, where fp32 FFMA arithmetic gives 6.5e-6 (na_lstm_layer_fwd_f32).  h_init / c_init [2][B][48] = the initial state (both or neither; NULL = zeros);
+ * out [B][T][48] = the last layer's h at every step; h_n / c_n [2][B][48] = both layers' h and c after the last step.
+ * Only rows b < B are written; every pointer 16-byte aligned. */
+int na_decoder_lstm_x3(const float* x, const void* packed, const float* h_init, const float* c_init, float* out,
+                       float* h_n, float* c_n, int64_t T, int64_t B, na_stream_t stream);
 
 /* ---- tensor-core tier, wide hidden sizes (H = 96, 144, 192; BASELINE configs[4]: H = 192, T = 2500) --------
  * Same contract as na_decoder_infer_bf16 (lstm_eeg_model.py:32-39 + :97, eval mode; input_size 8, 2 layers),

@@ -28,6 +28,9 @@ SIGNATURES = {
     "na_lstm_layer_bwd_f32": (c_int, [P, P, P, P, P, P, P, P, F32, I64, I64, I64, I64, P]),
     "na_wgrad_partial_floats": (c_int64, [I64, I64]),
     "na_lstm_layer_wgrad_f32": (c_int, [P, P, P, P, P, P, P, I64, I64, I64, I64, P]),
+    "na_lstm_layer_fwd_f32_hx": (c_int, [P, P, P, P, P, P, P, F32, P, I64, I64, I64, I64, P, P, P]),
+    "na_lstm_layer_bwd_f32_hx": (c_int, [P, P, P, P, P, P, P, P, F32, I64, I64, I64, I64, P, P, P, P, P, P]),
+    "na_lstm_layer_wgrad_f32_hx": (c_int, [P, P, P, P, P, P, P, I64, I64, I64, I64, P, P]),
     "na_head_fwd_f32": (c_int, [P] * 9 + [P, P, F32, P, P, P, P, I64, I64, I64, I64, I64, P]),
     "na_head_fwd_f32_ex": (c_int, [P] * 9 + [P, P, F32, P, P, P, P, P, P, P, I64, I64, I64, I64, I64, P]),
     "na_attention_softmax_f32": (c_int, [P, P, I64, I64, P]),
@@ -44,6 +47,7 @@ SIGNATURES = {
     "na_decoder_pack_x3": (c_int, [P] * 9 + [P]),
     "na_decoder_infer_x3": (c_int, [P] * 12 + [I64, I64, I64, P]),
     "na_decoder_infer_x3_ex": (c_int, [P] * 15 + [I64, I64, I64, P]),
+    "na_decoder_lstm_x3": (c_int, [P] * 7 + [I64, I64, P]),
     "na_decoder_wide_packed_bytes": (c_int64, [I64]),
     "na_decoder_wide_state_bytes": (c_int64, [I64]),
     "na_decoder_pack_wide_bf16": (c_int, [P] * 11 + [I64, P]),

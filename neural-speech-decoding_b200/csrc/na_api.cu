@@ -31,10 +31,12 @@ int check_launch(const char* what) {
 
 int lstm_layer_fwd_generic(const float* in, const float* wt, const float* bias, float* hout, float* cout,
                            float* gates, const float* drop_mask, float drop_scale, float* hout_drop,
-                           int64_t T, int64_t Bp, int64_t K, int64_t H, cudaStream_t st);
+                           int64_t T, int64_t Bp, int64_t K, int64_t H, const float* h_init, const float* c_init,
+                           cudaStream_t st);
 int lstm_layer_bwd_generic(const float* dh_out, const float* gates, const float* cstate, const float* w_ih,
                            const float* w_hh, float* dgates, float* din, const float* in_drop_mask,
-                           float drop_scale, int64_t T, int64_t Bp, int64_t K, int64_t H, cudaStream_t st);
+                           float drop_scale, int64_t T, int64_t Bp, int64_t K, int64_t H, const float* c_init,
+                           const float* dh_last, const float* dc_last, float* dh_init, float* dc_init, cudaStream_t st);
 
 bool lstm_h48_supported(int64_t K, int64_t H, bool save_c, bool save_g);
 int lstm_layer_fwd_h48(const float* in, const float* wt, const float* bias, float* hout, float* cout,
@@ -84,23 +86,34 @@ static int check_lstm_shape(const char* fn, int64_t T, int64_t Bp, int64_t K, in
     return NA_OK;
 }
 
-extern "C" int na_lstm_layer_fwd_f32(const float* in, const float* wt, const float* bias, float* hout,
-                                     float* cout, float* gates, const float* drop_mask, float drop_scale,
-                                     float* hout_drop, int64_t T, int64_t Bp, int64_t K, int64_t H,
-                                     na_stream_t stream) {
+extern "C" int na_lstm_layer_fwd_f32_hx(const float* in, const float* wt, const float* bias, float* hout,
+                                        float* cout, float* gates, const float* drop_mask, float drop_scale,
+                                        float* hout_drop, int64_t T, int64_t Bp, int64_t K, int64_t H,
+                                        const float* h_init, const float* c_init, na_stream_t stream) {
     using namespace na;
     if (int rc = check_lstm_shape("na_lstm_layer_fwd_f32", T, Bp, K, H)) return rc;
     NA_REQUIRE_PTR(in); NA_REQUIRE_PTR(wt); NA_REQUIRE_PTR(bias); NA_REQUIRE_PTR(hout);
     NA_OPTIONAL_PTR(cout); NA_OPTIONAL_PTR(gates); NA_OPTIONAL_PTR(drop_mask); NA_OPTIONAL_PTR(hout_drop);
+    NA_OPTIONAL_PTR(h_init); NA_OPTIONAL_PTR(c_init);
     NA_REQUIRE((drop_mask == nullptr) == (hout_drop == nullptr), NA_EINVAL,
                "na_lstm_layer_fwd_f32: drop_mask and hout_drop must be given together");
-    if (g_lstm_tier == 0 && lstm_h48_supported(K, H, cout != nullptr, gates != nullptr)) {
+    NA_REQUIRE((h_init == nullptr) == (c_init == nullptr), NA_EINVAL,
+               "na_lstm_layer_fwd_f32_hx: h_init and c_init must be given together");
+    if (g_lstm_tier == 0 && h_init == nullptr && lstm_h48_supported(K, H, cout != nullptr, gates != nullptr)) {
         if (int rc = lstm_layer_fwd_h48(in, wt, bias, hout, cout, gates, T, Bp, K, as_stream(stream))) return rc;
         if (drop_mask) return mask_scale(hout, drop_mask, drop_scale, hout_drop, T * Bp * H, as_stream(stream));
         return NA_OK;
     }
     return lstm_layer_fwd_generic(in, wt, bias, hout, cout, gates, drop_mask, drop_scale, hout_drop, T, Bp, K, H,
-                                  as_stream(stream));
+                                  h_init, c_init, as_stream(stream));
+}
+
+extern "C" int na_lstm_layer_fwd_f32(const float* in, const float* wt, const float* bias, float* hout,
+                                     float* cout, float* gates, const float* drop_mask, float drop_scale,
+                                     float* hout_drop, int64_t T, int64_t Bp, int64_t K, int64_t H,
+                                     na_stream_t stream) {
+    return na_lstm_layer_fwd_f32_hx(in, wt, bias, hout, cout, gates, drop_mask, drop_scale, hout_drop, T, Bp, K, H,
+                                    nullptr, nullptr, stream);
 }
 
 extern "C" int na_set_tuning(const char* key, int64_t value) {
@@ -148,15 +161,26 @@ extern "C" int na_ffma_probe(float* out, int64_t blocks, int64_t iters, na_strea
     return check_launch("na_ffma_probe");
 }
 
-extern "C" int na_lstm_layer_bwd_f32(const float* dh_out, const float* gates, const float* cstate,
-                                     const float* w_ih, const float* w_hh, float* dgates, float* din,
-                                     const float* in_drop_mask, float drop_scale, int64_t T, int64_t Bp,
-                                     int64_t K, int64_t H, na_stream_t stream) {
+extern "C" int na_lstm_layer_bwd_f32_hx(const float* dh_out, const float* gates, const float* cstate,
+                                        const float* w_ih, const float* w_hh, float* dgates, float* din,
+                                        const float* in_drop_mask, float drop_scale, int64_t T, int64_t Bp,
+                                        int64_t K, int64_t H, const float* c_init, const float* dh_last,
+                                        const float* dc_last, float* dh_init, float* dc_init, na_stream_t stream) {
     using namespace na;
     if (int rc = check_lstm_shape("na_lstm_layer_bwd_f32", T, Bp, K, H)) return rc;
     NA_REQUIRE_PTR(dh_out); NA_REQUIRE_PTR(gates); NA_REQUIRE_PTR(cstate); NA_REQUIRE_PTR(w_ih);
     NA_REQUIRE_PTR(w_hh); NA_REQUIRE_PTR(dgates);
     NA_OPTIONAL_PTR(din); NA_OPTIONAL_PTR(in_drop_mask);
+    NA_OPTIONAL_PTR(c_init); NA_OPTIONAL_PTR(dh_last); NA_OPTIONAL_PTR(dc_last); NA_OPTIONAL_PTR(dh_init);
+    NA_OPTIONAL_PTR(dc_init);
     return lstm_layer_bwd_generic(dh_out, gates, cstate, w_ih, w_hh, dgates, din, in_drop_mask, drop_scale, T, Bp,
-                                  K, H, as_stream(stream));
+                                  K, H, c_init, dh_last, dc_last, dh_init, dc_init, as_stream(stream));
+}
+
+extern "C" int na_lstm_layer_bwd_f32(const float* dh_out, const float* gates, const float* cstate,
+                                     const float* w_ih, const float* w_hh, float* dgates, float* din,
+                                     const float* in_drop_mask, float drop_scale, int64_t T, int64_t Bp,
+                                     int64_t K, int64_t H, na_stream_t stream) {
+    return na_lstm_layer_bwd_f32_hx(dh_out, gates, cstate, w_ih, w_hh, dgates, din, in_drop_mask, drop_scale, T, Bp,
+                                    K, H, nullptr, nullptr, nullptr, nullptr, nullptr, stream);
 }

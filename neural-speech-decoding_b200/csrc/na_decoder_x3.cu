@@ -74,13 +74,68 @@ __global__ void pack_decoder_x3_kernel(const float* __restrict__ w_ih0, const fl
     }
 }
 
+// The h values of this thread's granules as fp16 hi / lo into every row copy of the A operand `buf` (row replication R as
+// in x3_epilogue_tile): four units (R = 4) or the 8-unit K chunk `pr` (R = 1, 2).
+template <int R>
+__device__ __forceinline__ void x3_store_h(unsigned char* buf, const int gr0, const int wrow, const int pr, const float* hv) {
+    if constexpr (R == 4) {
+        const uint32_t hi0 = pack_val(hv[0], hv[1]), hi1 = pack_val(hv[2], hv[3]);
+        const uint32_t lo0 = pack_val(hv[0] - val_lo(hi0), hv[1] - val_hi(hi0));
+        const uint32_t lo1 = pack_val(hv[2] - val_lo(hi1), hv[3] - val_hi(hi1));
+        unsigned char* dst = buf + (gr0 >> 1) * kAChunk + wrow * 16 + (gr0 & 1) * 8;
+#pragma unroll
+        for (int rep = 0; rep < 4; ++rep) {
+            asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(smem_u32(dst + rep * 32 * 16)), "r"(hi0), "r"(hi1) : "memory");
+            asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(smem_u32(dst + 6 * kAChunk + rep * 32 * 16)), "r"(lo0), "r"(lo1) : "memory");
+        }
+    } else {
+        uint32_t hi[4], lo[4];
+        split_pack8(hv, hi, lo);
+        unsigned char* dst = buf + ((gr0 >> 1) + pr) * kAChunk + wrow * 16;
+#pragma unroll
+        for (int rep = 0; rep < R; ++rep) {
+            st_shared_v4(dst + rep * (kRows / R) * 16, hi[0], hi[1], hi[2], hi[3]);
+            st_shared_v4(dst + 6 * kAChunk + rep * (kRows / R) * 16, lo[0], lo[1], lo[2], lo[3]);
+        }
+    }
+}
+
+// Sequence mode with an initial state: h_init [2][B][48] of this thread's units into the A operands the first recurrent
+// MMAs of the tile read (layer 0: h0[(n0 - 1) & 1], layer 1: h1), zeros for rows b >= B.  Runs before the tile's role
+// split; the caller orders the stores before the MMAs with fence.proxy.async and a barrier.
+template <int R>
+__device__ __forceinline__ void x3_seq_init(SmemX3& S, const int q, const int g, const int lane, const int nq, const int n0,
+                                            const int64_t b0, const int64_t B, const float* __restrict__ h_init) {
+    constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
+    const int qs = q % kQ, rp = q / kQ;
+    if (qs >= nq) return;
+    const int wrow = qs * 32 + lane, gr0 = 4 * g + rp * kSlots;
+    const int64_t b = b0 + wrow;
+#pragma unroll
+    for (int l = 0; l < 2; ++l) {
+        float hv[kU];
+#pragma unroll
+        for (int j = 0; j < kU; j += 4) {
+            const float4 v = b < B ? *reinterpret_cast<const float4*>(h_init + (l * B + b) * kH + gr0 * 4 + j)
+                                   : make_float4(0.f, 0.f, 0.f, 0.f);
+            hv[j] = v.x; hv[j + 1] = v.y; hv[j + 2] = v.z; hv[j + 3] = v.w;
+        }
+        unsigned char* buf = l == 0 ? S.h0[(n0 - 1) & 1] : S.h1;
+#pragma unroll
+        for (int pr = 0; pr < (R == 4 ? 1 : kSlots / 2); ++pr) x3_store_h<R>(buf, gr0, wrow, pr, hv + pr * 8);
+    }
+}
+
 // Epilogue of one tile for one warp: both layers of (lane quarter q, unit group g).  R = row replication as in
 // decoder_infer_v2_kernel: the tile holds 128 / R distinct windows, copy rp = q / (4 / R) of source quarter qs = q % (4 / R)
 // takes granules [4 g + rp * (4 / R), + 4 / R) of the 12 four-unit granules and stores its h (hi and lo) to every copy.
 // kEx: also store the attention scores (time-major [T][B]) and the pooled vector / LayerNorm output ([B][48]) of every
 // window b < B: the scores and the LayerNorm output by the first row copy of the g == 0 warps (the one that runs the
 // head), the pooled vector by every thread for the units it pooled.
-template <int R, int NR, bool kEx>
+// kSeq (never together with kEx): no pooling and no head.  The cell states start from c_init [2][B][48] when it is given,
+// and every thread stores, for its own units and rows b < B, the last layer's h of every step into seq_out [B][T][48]
+// and both layers' h and c of the last step into h_n / c_n [2][B][48].
+template <int R, int NR, bool kEx, bool kSeq>
 __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const int g, const int lane, const int nq, const int T,
                                                  const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                                  const int64_t b0, const int64_t B, const int NC,
@@ -89,7 +144,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                                                  const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
                                                  float* __restrict__ logits, float* __restrict__ probs,
                                                  float* __restrict__ scores_tm, float* __restrict__ pooled,
-                                                 float* __restrict__ embedding) {
+                                                 float* __restrict__ embedding, const float* __restrict__ c_init,
+                                                 float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
     constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
@@ -106,12 +162,23 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             }
             if (t >= 1) { mbar_wait(&S.d1_full, k1 & 1); ++k1; mbar_arrive(&S.h1_ready); }
         }
-        mbar_wait(&S.d1_full, k1 & 1); ++k1;
+        if constexpr (!kSeq) { mbar_wait(&S.d1_full, k1 & 1); ++k1; }
         return;
     }
     float c0[kU], c1[kU], z[kU], hprev[kU];
 #pragma unroll
     for (int j = 0; j < kU; ++j) { c0[j] = 0.f; c1[j] = 0.f; z[j] = 0.f; hprev[j] = 0.f; }
+    const int64_t brow = b0 + wrow;
+    if constexpr (kSeq)
+        if (c_init && brow < B) {
+#pragma unroll
+            for (int j = 0; j < kU; j += 4) {
+                const float4 u = *reinterpret_cast<const float4*>(c_init + brow * kH + gr0 * 4 + j);
+                const float4 v = *reinterpret_cast<const float4*>(c_init + (B + brow) * kH + gr0 * 4 + j);
+                c0[j] = u.x; c0[j + 1] = u.y; c0[j + 2] = u.z; c0[j + 3] = u.w;
+                c1[j] = v.x; c1[j + 1] = v.y; c1[j + 2] = v.z; c1[j + 3] = v.w;
+            }
+        }
     float mx = -INFINITY, l = 0.f;
     auto pool = [&](float score) {                 // online softmax over time (lstm_eeg_model.py:35-37), fp32
         if (score > mx) {
@@ -138,29 +205,15 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                 : "memory");
             asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
             cell_granule_exact<NR>(v, c, hout);
-            const uint32_t hi0 = pack_val(hout[0], hout[1]), hi1 = pack_val(hout[2], hout[3]);
-            const uint32_t lo0 = pack_val(hout[0] - val_lo(hi0), hout[1] - val_hi(hi0));
-            const uint32_t lo1 = pack_val(hout[2] - val_lo(hi1), hout[3] - val_hi(hi1));
-            unsigned char* dst = buf + (gr0 >> 1) * kAChunk + wrow * 16 + (gr0 & 1) * 8;
-#pragma unroll
-            for (int rep = 0; rep < 4; ++rep) {
-                asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(smem_u32(dst + rep * 32 * 16)), "r"(hi0), "r"(hi1) : "memory");
-                asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(smem_u32(dst + 6 * kAChunk + rep * 32 * 16)), "r"(lo0), "r"(lo1) : "memory");
-            }
+            x3_store_h<R>(buf, gr0, wrow, 0, hout);
         } else {
 #pragma unroll
             for (int pr = 0; pr < kSlots / 2; ++pr) {       // pairs of granules = one 8-unit K chunk
-                uint32_t v[32], hi[4], lo[4];
+                uint32_t v[32];
                 tmem_ld32(tmem_d + lane_base + (gr0 + 2 * pr) * 16, v);
                 cell_granule_exact<NR>(v, c + pr * 8, hout + pr * 8);
                 cell_granule_exact<NR>(v + 16, c + pr * 8 + 4, hout + pr * 8 + 4);
-                split_pack8(hout + pr * 8, hi, lo);
-                unsigned char* dst = buf + ((gr0 >> 1) + pr) * kAChunk + wrow * 16;
-#pragma unroll
-                for (int rep = 0; rep < R; ++rep) {
-                    st_shared_v4(dst + rep * (kRows / R) * 16, hi[0], hi[1], hi[2], hi[3]);
-                    st_shared_v4(dst + 6 * kAChunk + rep * (kRows / R) * 16, lo[0], lo[1], lo[2], lo[3]);
-                }
+                x3_store_h<R>(buf, gr0, wrow, pr, hout + pr * 8);
             }
         }
     };
@@ -170,26 +223,42 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             mbar_wait(&S.d0_full, n & 1);
             if (q == 0 && g == 0 && lane == 0) mbar_arrive(&S.x_empty[n % kX3XStages]);
             tc_fence_after();
-            float hdummy[kU];
-            layer_phase(tmem_d0, c0, S.h0[n & 1], hdummy);
+            float hl0[kU];                         // layer-0 h: the next step reads it from shared memory
+            layer_phase(tmem_d0, c0, S.h0[n & 1], hl0);
             tc_fence_before();
             fence_proxy_async_smem();
             mbar_arrive(&S.h0_ready[n & 1]);
+            if constexpr (kSeq)
+                if (t == T - 1 && brow < B) {
+                    store_row<kU>(h_n + brow * kH + gr0 * 4, hl0);
+                    store_row<kU>(c_n + brow * kH + gr0 * 4, c0);
+                }
         }
         if (t >= 1) {                              // ---- layer 1, step t-1 (+ pooling of step t-2)
             mbar_wait(&S.d1_full, k1 & 1); ++k1;
             tc_fence_after();
-            uint32_t sc2[2];
-            x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
-            if (t >= 2) pool(__uint_as_float(sc2[0]));     // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
-            if constexpr (kEx)
-                if (t >= 2 && ex_writer && scores_tm) scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]);
+            if constexpr (!kSeq) {
+                uint32_t sc2[2];
+                x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
+                if (t >= 2) pool(__uint_as_float(sc2[0]));     // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
+                if constexpr (kEx)
+                    if (t >= 2 && ex_writer && scores_tm) scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]);
+            }
             layer_phase(tmem_d1, c1, S.h1, hprev);
             tc_fence_before();
             fence_proxy_async_smem();
             mbar_arrive(&S.h1_ready);
+            if constexpr (kSeq)
+                if (brow < B) {
+                    store_row<kU>(seq_out + (brow * T + (t - 1)) * kH + gr0 * 4, hprev);
+                    if (t == T) {
+                        store_row<kU>(h_n + (B + brow) * kH + gr0 * 4, hprev);
+                        store_row<kU>(c_n + (B + brow) * kH + gr0 * 4, c1);
+                    }
+                }
         }
     }
+    if constexpr (kSeq) return;
     {                                              // flush: score of the last step
         mbar_wait(&S.d1_full, k1 & 1); ++k1;
         tc_fence_after();
@@ -260,7 +329,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
     }
 }
 
-template <int NR, bool kEx = false>
+template <int NR, bool kEx = false, bool kSeq = false>
 __global__ void __launch_bounds__(kX3Threads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
@@ -271,8 +340,13 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         float* __restrict__ logits, float* __restrict__ probs,
                         int T, int64_t B, int NC, int nquarters,
                         float* __restrict__ scores_tm,              // kEx: [T][B] scores, [B][48] pooled / LayerNorm output
-                        float* __restrict__ pooled, float* __restrict__ embedding) {
+                        float* __restrict__ pooled, float* __restrict__ embedding,
+                        const float* __restrict__ h_init,           // kSeq: initial state [2][B][48] (both or neither),
+                        const float* __restrict__ c_init,           // the last layer's h [B][T][48], final state [2][B][48]
+                        float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
+    static_assert(!(kEx && kSeq), "the intermediates and the sequence output are separate instantiations");
     constexpr int kMmaWarp = 12, kTmaWarp = 13;
+    const bool seq_init = kSeq && h_init != nullptr;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     SmemX3& S = *reinterpret_cast<SmemX3*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
@@ -296,7 +370,7 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
 #pragma unroll
             for (int e = 0; e < 8; ++e) {
                 uint16_t val = 0;
-                if (r == 0) {
+                if (!kSeq && r == 0) {
                     uint16_t hi, lo;
                     if (ch >= 6 && ch <= 11) { split16(attn_w[(ch - 6) * 8 + e], hi, lo); val = hi; }
                     else if (ch >= 19) { split16(attn_w[(ch - 19) * 8 + e], hi, lo); val = lo; }
@@ -341,6 +415,15 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
         const int nq = min(4, q_end - q0);                 // active source quarters of this tile
         const int R = nq == 1 ? 4 : (nq == 2 ? 2 : 1);     // short tiles are row-replicated (see x3_epilogue_tile)
         const int64_t b0 = (int64_t)q0 * 32;
+        if (seq_init) {
+            if (warp < kMmaWarp) {
+                if (R == 1) x3_seq_init<1>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
+                else if (R == 2) x3_seq_init<2>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
+                else x3_seq_init<4>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
+            }
+            fence_proxy_async_smem();
+            __syncthreads();       // the previous tile is complete (barrier at its end): h0 / h1 are free
+        }
 
         if (warp == kTmaWarp) {
             // ================= producer: fp32 rows -> x_hi / x_lo chunks (rows of step t+1 are in flight) ========
@@ -413,7 +496,7 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         umma_bf16(tmem_d0, umma_desc(xs, a_zero - xs, 128), desc_adv(d_b0, 8 * kBChunk), 1u);
                         umma_bf16(tmem_d0, umma_desc(xs + 2 * kAChunk, a_zero - (xs + 2 * kAChunk), 128), d_b0, 1u);
                     }
-                    if (t >= 1) {
+                    if (t >= 1 || seq_init) {                   // h_{-1} = 0 unless an initial state was stored
                         const uint64_t hp = d_h0[(n - 1) & 1];
 #pragma unroll
                         for (int i = 0; i < 3; ++i) {
@@ -442,7 +525,7 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                             umma_bf16_i(tmem_d1, desc_adv(hin, (6 + 2 * i) * kAChunk), desc_adv(d_b1, 2 * i * kX3B1Chunk), kX3IdescL1, 1u);
                         }
                     }
-                    if (t >= 2) {
+                    if (t >= 2 || seq_init) {
 #pragma unroll
                         for (int i = 0; i < 3; ++i) {
                             if (leader) {
@@ -455,7 +538,7 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                     if (leader) umma_commit(&S.d1_full);
                 }
             }
-            {   // flush: score of the last step into the 16 score columns (rows 192..207 of the h1-part chunks + bias)
+            if constexpr (!kSeq) {   // flush: score of the last step into the 16 score columns (rows 192..207 of the h1-part chunks + bias)
                 const int m = n0 + T - 1;
                 mbar_wait(&S.h1_ready, m & 1);
                 tc_fence_after();
@@ -474,9 +557,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
         } else {
             // ================= epilogue: both layers of (quarter q, unit group g) ================================
             const int q = warp & 3, g = warp >> 2;
-            if (R == 1) x3_epilogue_tile<1, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
-            else if (R == 2) x3_epilogue_tile<2, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
-            else x3_epilogue_tile<4, NR, kEx>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding);
+            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
+            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
+            else x3_epilogue_tile<4, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
         }
         __syncthreads();       // tile done: every MMA has completed; the z exchange in h0 has been consumed
         q0 += nq;
@@ -496,6 +579,17 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
 namespace na { namespace tc {
 int g_x3_rcp_fma = kX3DefaultNR;
 void set_x3_rcp_fma(int v) { g_x3_rcp_fma = v; }
+
+static int x3_sms() {
+    static int sms = 0;
+    if (sms == 0) {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        if (sms <= 0) sms = 148;
+    }
+    return sms;
+}
 } }
 
 extern "C" int64_t na_decoder_packed_x3_bytes(void) {
@@ -528,13 +622,7 @@ extern "C" int na_decoder_infer_x3_ex(const float* x, const void* packed, const 
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
                "na_decoder_infer_x3: null parameter pointer");
     const bool ex = scores_tm || pooled || embedding;
-    static int sms = 0;
-    if (sms == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (sms <= 0) sms = 148;
-    }
+    const int sms = tc::x3_sms();
     const size_t smem = sizeof(tc::SmemX3) + 1024;
     const int nquarters = (int)((B + 31) / 32);
     const int grid = nquarters < sms ? nquarters : sms;    // < 4 quarters per CTA run as row-replicated tiles
@@ -544,7 +632,7 @@ extern "C" int na_decoder_infer_x3_ex(const float* x, const void* packed, const 
         if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e));    \
         tc::decoder_infer_x3_kernel<NRV, EXV><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                                    \
             x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, \
-            (int)T, B, (int)NC, nquarters, scores_tm, pooled, embedding);                                                            \
+            (int)T, B, (int)NC, nquarters, scores_tm, pooled, embedding, nullptr, nullptr, nullptr, nullptr, nullptr);               \
     }
     switch (tc::g_x3_rcp_fma * 2 + (ex ? 1 : 0)) {
         case 0: NA_X3_LAUNCH(0, false) break;
@@ -568,4 +656,34 @@ extern "C" int na_decoder_infer_x3(const float* x, const void* packed, const flo
                                    int64_t B, int64_t NC, na_stream_t stream) {
     return na_decoder_infer_x3_ex(x, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, nullptr,
                                   nullptr, nullptr, T, B, NC, stream);
+}
+
+extern "C" int na_decoder_lstm_x3(const float* x, const void* packed, const float* h_init, const float* c_init, float* out,
+                                  float* h_n, float* c_n, int64_t T, int64_t B, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_lstm_x3: bad shape T=%lld B=%lld", (long long)T, (long long)B);
+    NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(out); NA_REQUIRE_PTR(h_n); NA_REQUIRE_PTR(c_n);
+    NA_OPTIONAL_PTR(h_init); NA_OPTIONAL_PTR(c_init);
+    NA_REQUIRE((h_init == nullptr) == (c_init == nullptr), NA_EINVAL, "na_decoder_lstm_x3: h_init and c_init must be given together");
+    const size_t smem = sizeof(tc::SmemX3) + 1024;
+    const int nquarters = (int)((B + 31) / 32);
+    const int sms = tc::x3_sms();
+    const int grid = nquarters < sms ? nquarters : sms;
+#define NA_X3_SEQ_LAUNCH(NRV)                                                                                                        \
+    {                                                                                                                                \
+        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (e != cudaSuccess) return fail((int)e, "na_decoder_lstm_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e));     \
+        tc::decoder_infer_x3_kernel<NRV, false, true><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                            \
+            x, reinterpret_cast<const unsigned char*>(packed), nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,  \
+            nullptr, nullptr, (int)T, B, 1, nquarters, nullptr, nullptr, nullptr, h_init, c_init, out, h_n, c_n);                     \
+    }
+    switch (tc::g_x3_rcp_fma) {
+        case 0: NA_X3_SEQ_LAUNCH(0) break;
+        case 2: NA_X3_SEQ_LAUNCH(2) break;
+        case 3: NA_X3_SEQ_LAUNCH(3) break;
+        default: NA_X3_SEQ_LAUNCH(1) break;
+    }
+#undef NA_X3_SEQ_LAUNCH
+    count_launch();
+    return check_launch("na_decoder_lstm_x3");
 }

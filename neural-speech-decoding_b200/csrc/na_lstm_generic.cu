@@ -25,13 +25,14 @@ __global__ void pack_lstm_layer_kernel(const float* __restrict__ w_ih, const flo
 
 // Thread j owns hidden unit j for all kGenTile windows of the tile: the four weight columns of
 // a k-step are loaded once (coalesced over j) and reused for every window; [x_t | h_{t-1}] is
-// broadcast from shared memory.
+// broadcast from shared memory.  h_init / c_init [Bp][H] (optional) are h_{-1} / c_{-1}; zeros without them.
 __global__ void lstm_fwd_generic_kernel(const float* __restrict__ in, const float* __restrict__ wt,
                                         const float* __restrict__ bias, float* __restrict__ hout,
                                         float* __restrict__ cout, float* __restrict__ gates,
                                         const float* __restrict__ drop_mask, float drop_scale,
                                         float* __restrict__ hout_drop,
-                                        int T, int64_t Bp, int K, int H) {
+                                        int T, int64_t Bp, int K, int H,
+                                        const float* __restrict__ h_init, const float* __restrict__ c_init) {
     extern __shared__ float smem[];
     const int KH = K + H, G = 4 * H;
     float* a_s = smem;                       // [kGenTile][KH]
@@ -41,8 +42,11 @@ __global__ void lstm_fwd_generic_kernel(const float* __restrict__ in, const floa
 
     float c[kGenTile];
 #pragma unroll
-    for (int b = 0; b < kGenTile; ++b) c[b] = 0.f;
-    for (int idx = threadIdx.x; idx < kGenTile * KH; idx += blockDim.x) a_s[idx] = 0.f;
+    for (int b = 0; b < kGenTile; ++b) c[b] = (c_init && unit) ? c_init[(b0 + b) * H + j] : 0.f;
+    for (int idx = threadIdx.x; idx < kGenTile * KH; idx += blockDim.x) {
+        const int b = idx / KH, k = idx % KH;
+        a_s[idx] = (h_init && k >= K) ? h_init[(b0 + b) * H + (k - K)] : 0.f;
+    }
     float bi = 0.f, bf = 0.f, bg = 0.f, bo = 0.f;
     if (unit) { bi = bias[j]; bf = bias[H + j]; bg = bias[2 * H + j]; bo = bias[3 * H + j]; }
     __syncthreads();
@@ -96,11 +100,16 @@ __global__ void lstm_fwd_generic_kernel(const float* __restrict__ in, const floa
 
 // Reverse-time pass.  Threads j < H do the elementwise gate backward of unit j; then thread
 // jj < K+H produces column jj of dgates . [W_ih | W_hh]  (din for jj < K, recurrent dh otherwise).
+// Optional, [Bp][H] each: c_init = c_{-1} (zeros without it); dh_last / dc_last = the gradients w.r.t. this layer's
+// final h / c, which enter at t = T-1; dh_init / dc_init receive the gradients w.r.t. h_{-1} / c_{-1}.
 __global__ void lstm_bwd_generic_kernel(const float* __restrict__ dh_out, const float* __restrict__ gates,
                                         const float* __restrict__ cstate, const float* __restrict__ w_ih,
                                         const float* __restrict__ w_hh, float* __restrict__ dgates,
                                         float* __restrict__ din, const float* __restrict__ in_drop_mask,
-                                        float drop_scale, int T, int64_t Bp, int K, int H) {
+                                        float drop_scale, int T, int64_t Bp, int K, int H,
+                                        const float* __restrict__ c_init, const float* __restrict__ dh_last,
+                                        const float* __restrict__ dc_last, float* __restrict__ dh_init,
+                                        float* __restrict__ dc_init) {
     extern __shared__ float smem[];
     const int G = 4 * H;
     float* dg_s = smem;                         // [kGenTile][G]
@@ -113,8 +122,9 @@ __global__ void lstm_bwd_generic_kernel(const float* __restrict__ dh_out, const 
 
     float dc[kGenTile];
 #pragma unroll
-    for (int b = 0; b < kGenTile; ++b) dc[b] = 0.f;
-    for (int idx = threadIdx.x; idx < kGenTile * H; idx += blockDim.x) dhrec_s[idx] = 0.f;
+    for (int b = 0; b < kGenTile; ++b) dc[b] = (dc_last && unit) ? dc_last[(b0 + b) * H + j] : 0.f;
+    for (int idx = threadIdx.x; idx < kGenTile * H; idx += blockDim.x)
+        dhrec_s[idx] = dh_last ? dh_last[(b0 + idx / H) * H + idx % H] : 0.f;
     __syncthreads();
 
     for (int t = T - 1; t >= 0; --t) {
@@ -127,7 +137,7 @@ __global__ void lstm_bwd_generic_kernel(const float* __restrict__ dh_out, const 
                 const float* gr = gates + row * G + j;
                 const float i = gr[0], f = gr[H], g = gr[2 * H], o = gr[3 * H];
                 const float ct = cstate[row * H + j];
-                const float cp = (t > 0) ? cstate[(row - Bp) * H + j] : 0.f;
+                const float cp = (t > 0) ? cstate[(row - Bp) * H + j] : (c_init ? c_init[(b0 + b) * H + j] : 0.f);
                 const float tc = tanh_acc(ct);
                 const float dh = dh_out[row * H + j] + dhrec_s[b * H + j];
                 const float d_o = dh * tc;
@@ -178,6 +188,12 @@ __global__ void lstm_bwd_generic_kernel(const float* __restrict__ dh_out, const 
         }
         __syncthreads();
     }
+    if (dh_init)
+        for (int idx = threadIdx.x; idx < kGenTile * H; idx += blockDim.x) dh_init[(b0 + idx / H) * H + idx % H] = dhrec_s[idx];
+    if (dc_init && unit) {
+#pragma unroll
+        for (int b = 0; b < kGenTile; ++b) dc_init[(b0 + b) * H + j] = dc[b];
+    }
 }
 
 }  // namespace na
@@ -198,21 +214,23 @@ extern "C" int na_pack_lstm_layer(const float* w_ih, const float* w_hh, const fl
 namespace na {
 int lstm_layer_fwd_generic(const float* in, const float* wt, const float* bias, float* hout, float* cout,
                            float* gates, const float* drop_mask, float drop_scale, float* hout_drop,
-                           int64_t T, int64_t Bp, int64_t K, int64_t H, cudaStream_t st) {
+                           int64_t T, int64_t Bp, int64_t K, int64_t H, const float* h_init, const float* c_init,
+                           cudaStream_t st) {
     const int threads = (int)((H + 31) / 32 * 32);
     const size_t smem = sizeof(float) * kGenTile * (K + H);
     NA_REQUIRE(smem <= 200 * 1024, NA_EUNSUPPORTED, "na_lstm_layer_fwd_f32: K+H too large for the generic tier");
     if (smem > 48 * 1024)
         cudaFuncSetAttribute(lstm_fwd_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     lstm_fwd_generic_kernel<<<(unsigned)(Bp / kGenTile), threads, smem, st>>>(
-        in, wt, bias, hout, cout, gates, drop_mask, drop_scale, hout_drop, (int)T, Bp, (int)K, (int)H);
+        in, wt, bias, hout, cout, gates, drop_mask, drop_scale, hout_drop, (int)T, Bp, (int)K, (int)H, h_init, c_init);
     count_launch();
     return check_launch("na_lstm_layer_fwd_f32(generic)");
 }
 
 int lstm_layer_bwd_generic(const float* dh_out, const float* gates, const float* cstate, const float* w_ih,
                            const float* w_hh, float* dgates, float* din, const float* in_drop_mask,
-                           float drop_scale, int64_t T, int64_t Bp, int64_t K, int64_t H, cudaStream_t st) {
+                           float drop_scale, int64_t T, int64_t Bp, int64_t K, int64_t H, const float* c_init,
+                           const float* dh_last, const float* dc_last, float* dh_init, float* dc_init, cudaStream_t st) {
     const int threads = (int)((K + H + 31) / 32 * 32);
     NA_REQUIRE(threads <= 1024, NA_EUNSUPPORTED, "na_lstm_layer_bwd_f32: K+H=%lld > 1024 in the generic tier",
                (long long)(K + H));
@@ -221,7 +239,8 @@ int lstm_layer_bwd_generic(const float* dh_out, const float* gates, const float*
     if (smem > 48 * 1024)
         cudaFuncSetAttribute(lstm_bwd_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     lstm_bwd_generic_kernel<<<(unsigned)(Bp / kGenTile), threads, smem, st>>>(
-        dh_out, gates, cstate, w_ih, w_hh, dgates, din, in_drop_mask, drop_scale, (int)T, Bp, (int)K, (int)H);
+        dh_out, gates, cstate, w_ih, w_hh, dgates, din, in_drop_mask, drop_scale, (int)T, Bp, (int)K, (int)H, c_init, dh_last,
+        dc_last, dh_init, dc_init);
     count_launch();
     return check_launch("na_lstm_layer_bwd_f32(generic)");
 }

@@ -100,14 +100,15 @@ __global__ void colsum_partial_kernel(const float* __restrict__ G, int64_t ldg, 
     partial[(size_t)blockIdx.x * M + m] = (s0 + s1) + (s2 + s3);
 }
 
-// out[i] = sum_c partial[c][i], c ascending (fixed order).
+// out[i] = sum_c partial[c][i], c ascending (fixed order); kAdd: out[i] += that sum.
+template <bool kAdd = false>
 __global__ void reduce_partials_kernel(const float* __restrict__ partial, float* __restrict__ out,
                                        int nchunks, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     float s = 0.f;
     for (int c = 0; c < nchunks; ++c) s += partial[(size_t)c * n + i];
-    out[i] = s;
+    out[i] = kAdd ? out[i] + s : s;
 }
 
 int wgrad_nchunks(int64_t M, int64_t N, int64_t R) {
@@ -120,18 +121,24 @@ int wgrad_nchunks(int64_t M, int64_t N, int64_t R) {
     return (int)n;
 }
 
-// out[M][N] = G^T A over R rows.  `partial` must hold wgrad_nchunks(M,N,R)*M*N floats.
-int gemm_tn(const float* G, int64_t ldg, const float* A, int64_t lda, int64_t R, int64_t M, int64_t N,
-            float* out, float* partial, cudaStream_t st) {
+// out[M][N] = G^T A over R rows (add: out += G^T A).  `partial` must hold wgrad_nchunks(M,N,R)*M*N floats.
+static int gemm_tn_impl(const float* G, int64_t ldg, const float* A, int64_t lda, int64_t R, int64_t M, int64_t N,
+                        float* out, float* partial, bool add, cudaStream_t st) {
     const int nch = wgrad_nchunks(M, N, R);
     int64_t rpc = (R + nch - 1) / nch;
     rpc = (rpc + kTnRows - 1) / kTnRows * kTnRows;
     const dim3 grid(nch, (unsigned)((M + kTnTile - 1) / kTnTile), (unsigned)((N + kTnTile - 1) / kTnTile));
     gemm_tn_partial_kernel<false><<<grid, kTnThreads, 0, st>>>(G, ldg, A, lda, R, (int)M, (int)N, partial, rpc, (int)N, nullptr, 0, 0);
     const int64_t n = M * N;
-    reduce_partials_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partial, out, nch, n);
+    if (add) reduce_partials_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partial, out, nch, n);
+    else reduce_partials_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partial, out, nch, n);
     count_launch(2);
     return check_launch("gemm_tn");
+}
+
+int gemm_tn(const float* G, int64_t ldg, const float* A, int64_t lda, int64_t R, int64_t M, int64_t N,
+            float* out, float* partial, cudaStream_t st) {
+    return gemm_tn_impl(G, ldg, A, lda, R, M, N, out, partial, false, st);
 }
 
 // out1[M][N1] = G^T A1 over rows [0, R),  out2[M][N2] = G[shift:]^T A2[:R-shift]  in ONE pass over G.
@@ -188,13 +195,14 @@ extern "C" int64_t na_wgrad_partial_floats(int64_t K, int64_t H) {
     return (a > b ? (a > c ? a : c) : (b > c ? b : c)) + 64;
 }
 
-extern "C" int na_lstm_layer_wgrad_f32(const float* dgates, const float* in, const float* h, float* dw_ih,
-                                       float* dw_hh, float* db, float* partials, int64_t T, int64_t Bp,
-                                       int64_t K, int64_t H, na_stream_t stream) {
+extern "C" int na_lstm_layer_wgrad_f32_hx(const float* dgates, const float* in, const float* h, float* dw_ih,
+                                          float* dw_hh, float* db, float* partials, int64_t T, int64_t Bp,
+                                          int64_t K, int64_t H, const float* h_init, na_stream_t stream) {
     using namespace na;
     NA_REQUIRE(T >= 1 && Bp >= 1 && K >= 1 && H >= 1, NA_EINVAL, "na_lstm_layer_wgrad_f32: bad shape");
     NA_REQUIRE_PTR(dgates); NA_REQUIRE_PTR(in); NA_REQUIRE_PTR(h);
     NA_REQUIRE_PTR(dw_ih); NA_REQUIRE_PTR(dw_hh); NA_REQUIRE_PTR(db); NA_REQUIRE_PTR(partials);
+    NA_OPTIONAL_PTR(h_init);
     cudaStream_t st = as_stream(stream);
     const int64_t R = T * Bp, G = 4 * H;
     int rc;
@@ -209,5 +217,13 @@ extern "C" int na_lstm_layer_wgrad_f32(const float* dgates, const float* in, con
         else rc = (int)cudaMemsetAsync(dw_hh, 0, sizeof(float) * G * H, st);
     }
     if (rc) return rc;
+    // step 0 pairs with h_{-1} = h_init (zero without it): dW_hh += dgates_0^T h_init
+    if (h_init && (rc = gemm_tn_impl(dgates, G, h_init, H, Bp, G, H, dw_hh, partials, true, st))) return rc;
     return colsum(dgates, G, R, G, db, partials, st);
+}
+
+extern "C" int na_lstm_layer_wgrad_f32(const float* dgates, const float* in, const float* h, float* dw_ih,
+                                       float* dw_hh, float* db, float* partials, int64_t T, int64_t Bp,
+                                       int64_t K, int64_t H, na_stream_t stream) {
+    return na_lstm_layer_wgrad_f32_hx(dgates, in, h, dw_ih, dw_hh, db, partials, T, Bp, K, H, nullptr, stream);
 }

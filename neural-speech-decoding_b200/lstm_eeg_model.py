@@ -9,7 +9,7 @@ hand-written sm_100a kernels (libneuroalpha_b200.so).  There is no CPU compute p
 from __future__ import annotations
 
 import math
-from typing import Dict, List, NamedTuple, Optional
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import numpy as np
 import torch
@@ -36,7 +36,10 @@ class LSTMParameters(nn.Module):
     (U(-1/sqrt(H), 1/sqrt(H)) for every tensor, drawn in registration order), so that
     ``torch.manual_seed(s); EEG_LSTM()`` reproduces the reference's weights and the 16-key
     ``state_dict`` loads with ``strict=True`` (reference lstm_eeg_model.py:16-22, 81).
-    It holds no compute: the recurrence is ``torch.ops.neuroalpha.lstm_layer_fwd``.
+
+    Calling it is ``nn.LSTM(batch_first=True)``'s forward (see ``forward``).  ``EEG_LSTM.forward``,
+    ``decode`` and ``decode_intermediates`` run their own fused kernels and never call it, so a forward
+    hook on ``model.lstm`` fires only when the user calls ``model.lstm(...)``.
     """
 
     def __init__(self, input_size: int, hidden_size: int, num_layers: int, dropout: float):
@@ -45,6 +48,7 @@ class LSTMParameters(nn.Module):
         self.dropout = float(dropout)
         self.batch_first = True
         self.bidirectional = False
+        self._pack_cache: Dict[object, tuple] = {}         # shared with the owning EEG_LSTM (same dict object)
         for l in range(num_layers):
             k = input_size if l == 0 else hidden_size
             self.register_parameter(f"weight_ih_l{l}", nn.Parameter(torch.empty(4 * hidden_size, k)))
@@ -63,6 +67,87 @@ class LSTMParameters(nn.Module):
 
     def extra_repr(self) -> str:
         return f"{self.input_size}, {self.hidden_size}, num_layers={self.num_layers}, batch_first=True, dropout={self.dropout}"
+
+    def _cached_pack(self, slot, ps, make):
+        key = tuple((p.data_ptr(), p._version, p.dtype) for p in ps)
+        hit = self._pack_cache.get(slot)
+        if hit is None or hit[0] != key:
+            with torch.no_grad():
+                hit = (key, make())
+            self._pack_cache[slot] = hit
+        return hit[1]
+
+    def _packed_x3(self):
+        ps = self.layer(0) + self.layer(1)
+        return self._cached_pack("x3", ps, lambda: ops.decoder_pack_x3(ps))
+
+    def forward(self, input: torch.Tensor, hx: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+        """``nn.LSTM(batch_first=True)``: ``input`` [B,T,C] (or unbatched [T,C]) on a CUDA device, ``hx = (h_0, c_0)``
+        [L,B,H] each ([L,H] unbatched; None = zeros) -> ``(output [B,T,H], (h_n, c_n))``, ``output`` = the last layer's
+        h at every step, ``h_n`` / ``c_n`` [L,B,H] after the last step (``h_n`` before dropout).  Same argument checks
+        and exceptions as nn.LSTM.  The result has the dtype of ``input``; the arithmetic is fp32.  Accuracy against
+        float64 nn.LSTM (max|d| / max|ref| per tensor): 1e-5 on the FFMA path and for ``h_n`` / ``c_n``; on the fused
+        path the per-step ``output`` of long windows is looser -- 6.2e-5 over the 625 steps of the shipped windows,
+        tested at 1e-4 -- because the fp16 hi + lo operand split carries about 22 bits; ``ops.EXACT_TC = False`` selects
+        the FFMA path for every call.
+
+        In ``.train()`` mode with ``dropout > 0`` the output of every layer but the last is multiplied by a keep-mask
+        ``torch.rand((B, T, H), device=input.device) >= dropout`` (drawn in layer order) and scaled by 1/(1-dropout).
+        The owning model's ``compute_dtype`` and ``zscore_input`` do not apply: this sees the raw ``input``, as
+        ``self.lstm(x)`` does in the reference.  The flagship shape (8 -> 48, 2 layers) in fp32 without autograd runs
+        on the exact tensor-core kernel (``ops.EXACT_TC``); everything else, and every call that needs gradients, on the
+        FFMA / generic kernels under ``ops.LSTMSequenceFunction`` (gradients w.r.t. input, weights and ``hx``)."""
+        if input.dim() not in (2, 3):
+            raise ValueError(f"LSTM: Expected input to be 2D or 3D, got {input.dim()}D instead")
+        batched = input.dim() == 3
+        x = input if batched else input.unsqueeze(0)
+        h0 = c0 = None
+        if hx is not None:
+            h0, c0 = hx
+            if batched and (h0.dim() != 3 or c0.dim() != 3):
+                raise RuntimeError("For batched 3-D input, hx and cx should "
+                                   f"also be 3-D but got ({h0.dim()}-D, {c0.dim()}-D) tensors")
+            if not batched:
+                if h0.dim() != 2 or c0.dim() != 2:
+                    raise RuntimeError("For unbatched 2-D input, hx and cx should "
+                                       f"also be 2-D but got ({h0.dim()}-D, {c0.dim()}-D) tensors")
+                h0, c0 = h0.unsqueeze(1), c0.unsqueeze(1)
+        w = self.weight_ih_l0
+        if x.dtype != w.dtype:
+            raise ValueError(f"RNN input dtype ({x.dtype}) does not match weight dtype ({w.dtype}). "
+                             f"Convert input: input.to({w.dtype}), or convert model: model.to({x.dtype})")
+        if x.size(-1) != self.input_size:
+            raise RuntimeError(f"input.size(-1) must be equal to input_size. Expected {self.input_size}, "
+                               f"got {x.size(-1)}")
+        L, H = self.num_layers, self.hidden_size
+        expected = (L, x.size(0), H)
+        if h0 is not None:
+            if h0.size() != expected:
+                raise RuntimeError(f"Expected hidden[0] size {expected}, got {list(h0.size())}")
+            if c0.size() != expected:
+                raise RuntimeError(f"Expected hidden[1] size {expected}, got {list(c0.size())}")
+        ops._require_cuda(x, h0, c0)          # raises on CPU tensors: there is no CPU fallback
+        B, T = x.shape[0], x.shape[1]
+        if B == 0:
+            out, h_n, c_n = x.new_empty((0, T, H)), x.new_empty((L, 0, H)), x.new_empty((L, 0, H))
+        else:
+            needs_grad = torch.is_grad_enabled() and (
+                x.requires_grad or any(p.requires_grad for p in self.parameters())
+                or (h0 is not None and (h0.requires_grad or c0.requires_grad)))
+            if (ops.EXACT_TC and (self.input_size, H, L) == (8, 48, 2) and x.dtype == torch.float32 and not needs_grad
+                    and (not self.training or self.dropout == 0.0)):
+                with torch.no_grad():
+                    out, h_n, c_n = ops.decoder_lstm_x3(x.contiguous(), self._packed_x3(), h0, c0)
+            else:
+                masks = None
+                if self.training and self.dropout > 0.0 and L > 1:
+                    masks = [(torch.rand((B, T, H), device=x.device) >= self.dropout).float() for _ in range(L - 1)]
+                flat = [t for l in range(L) for t in self.layer(l)]
+                out, h_n, c_n = ops.LSTMSequenceFunction.apply(x, h0, c0, self.dropout, masks, *flat)
+        out, h_n, c_n = (t if t.dtype == x.dtype else t.to(x.dtype) for t in (out, h_n, c_n))
+        if not batched:
+            return out.squeeze(0), (h_n.squeeze(1), c_n.squeeze(1))
+        return out, (h_n, c_n)
 
 
 class EEG_LSTM(nn.Module):
@@ -96,7 +181,7 @@ class EEG_LSTM(nn.Module):
         # "bf16 path"); also selected by bf16 inputs or a .bfloat16() module.  Both tiers train.
         self.compute_dtype = torch.float32
         self._injected_noise: Optional[Dict[str, torch.Tensor]] = None
-        self._pack_cache: Dict[object, tuple] = {}
+        self._pack_cache = self.lstm._pack_cache           # one cache: model.lstm(x) reuses the exact tier's weight image
 
     # -- helpers ---------------------------------------------------------------------------
     def _head_params(self) -> List[torch.Tensor]:
@@ -125,13 +210,7 @@ class EEG_LSTM(nn.Module):
         return out
 
     def _cached_pack(self, slot, ps, make):
-        key = tuple((p.data_ptr(), p._version, p.dtype) for p in ps)
-        hit = self._pack_cache.get(slot)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                hit = (key, make())
-            self._pack_cache[slot] = hit
-        return hit[1]
+        return self.lstm._cached_pack(slot, ps, make)
 
     def _packed(self, l: int):
         ps = self.lstm.layer(l)
@@ -152,8 +231,7 @@ class EEG_LSTM(nn.Module):
         return self._cached_pack("tc_wide", ps, lambda: ops.decoder_pack_wide_bf16(ps[:8], ps[8], ps[9]))
 
     def _packed_x3(self):
-        ps = self.lstm.layer(0) + self.lstm.layer(1)
-        return self._cached_pack("x3", ps, lambda: ops.decoder_pack_x3(ps))
+        return self.lstm._packed_x3()
 
     def _packed_tc(self):
         ps = self.lstm.layer(0) + self.lstm.layer(1)

@@ -54,6 +54,12 @@ def _f32c(t: Tensor) -> Tensor:
     return t.contiguous()
 
 
+def _aligned16(t: Tensor) -> Tensor:
+    """t, or a copy of it when its data is not 16-byte aligned (a view at an odd offset): the kernels load 16 bytes at a
+    time and the C ABI rejects such pointers."""
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 def _ptr(t: Optional[Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
@@ -94,7 +100,8 @@ def all_custom_ops():
             dropout_mask_u8, head_tail_fwd, head_tail_bwd, decoder_infer_bf16_x32, decoder_pack_x3, decoder_infer_x3,
             decoder_pack_wide_bf16, decoder_infer_wide_bf16, x3_split_input, lstm_fwd_train_x3, lstm_bwd_x3, lstm_wgrad_x3,
             lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
-            decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex]
+            decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex, lstm_layer_fwd_hx, lstm_layer_bwd_hx,
+            lstm_layer_wgrad_hx, decoder_lstm_x3]
 
 
 def launch_count() -> int:
@@ -235,6 +242,88 @@ def lstm_layer_wgrad(dgates: Tensor, inp: Tensor, h: Tensor) -> Tuple[Tensor, Te
 
 @lstm_layer_wgrad.register_fake
 def _(dgates, inp, h):
+    G = dgates.shape[2]
+    return dgates.new_empty((G, inp.shape[2])), dgates.new_empty((G, h.shape[2])), dgates.new_empty((G,))
+
+
+@torch.library.custom_op("neuroalpha::lstm_layer_fwd_hx", mutates_args=(), device_types="cuda")
+@_device_guard
+def lstm_layer_fwd_hx(inp: Tensor, wt: Tensor, bias: Tensor, drop_mask: Optional[Tensor], drop_scale: float,
+                      h0: Optional[Tensor], c0: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """lstm_layer_fwd with save=True, starting from the initial state h0 / c0 [Bp,H] (both or neither; None = zeros):
+    (h, c, gates, h_drop or empty)."""
+    _require_cuda(inp, wt, bias, drop_mask, h0, c0)
+    T, Bp, K = inp.shape
+    H = bias.numel() // 4
+    dev = inp.device
+    h = torch.empty((T, Bp, H), dtype=torch.float32, device=dev)
+    c = torch.empty((T, Bp, H), dtype=torch.float32, device=dev)
+    gates = torch.empty((T, Bp, 4 * H), dtype=torch.float32, device=dev)
+    h_drop = torch.empty((T, Bp, H) if drop_mask is not None else (0,), dtype=torch.float32, device=dev)
+    _lib.call("na_lstm_layer_fwd_f32_hx", inp.data_ptr(), wt.data_ptr(), bias.data_ptr(), h.data_ptr(), c.data_ptr(),
+              gates.data_ptr(), _ptr(drop_mask), float(drop_scale), _ptr(h_drop) if drop_mask is not None else None,
+              T, Bp, K, H, _ptr(h0), _ptr(c0), _stream())
+    return h, c, gates, h_drop
+
+
+@lstm_layer_fwd_hx.register_fake
+def _(inp, wt, bias, drop_mask, drop_scale, h0, c0):
+    T, Bp, K = inp.shape
+    H = bias.numel() // 4
+    return (inp.new_empty((T, Bp, H)), inp.new_empty((T, Bp, H)), inp.new_empty((T, Bp, 4 * H)),
+            inp.new_empty((T, Bp, H)) if drop_mask is not None else inp.new_empty((0,)))
+
+
+@torch.library.custom_op("neuroalpha::lstm_layer_bwd_hx", mutates_args=(), device_types="cuda")
+@_device_guard
+def lstm_layer_bwd_hx(dh: Tensor, gates: Tensor, c: Tensor, w_ih: Tensor, w_hh: Tensor, in_drop_mask: Optional[Tensor],
+                      drop_scale: float, need_din: bool, c0: Optional[Tensor], dh_last: Tensor, dc_last: Tensor,
+                      need_dhx: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """lstm_layer_bwd of a layer that started from c0 [Bp,H] (None = zeros), with the gradients w.r.t. its final h / c
+    (dh_last / dc_last [Bp,H]) added at the last step: (dgates, din or empty, dh0 [Bp,H], dc0 [Bp,H]; both empty unless
+    ``need_dhx``)."""
+    _require_cuda(dh, gates, c, w_ih, w_hh, in_drop_mask, c0, dh_last, dc_last)
+    T, Bp, H = dh.shape
+    K = w_ih.shape[1]
+    dev = dh.device
+    dgates = torch.empty((T, Bp, 4 * H), dtype=torch.float32, device=dev)
+    din = torch.empty((T, Bp, K) if need_din else (0,), dtype=torch.float32, device=dev)
+    dh0 = torch.empty((Bp, H) if need_dhx else (0,), dtype=torch.float32, device=dev)
+    dc0 = torch.empty((Bp, H) if need_dhx else (0,), dtype=torch.float32, device=dev)
+    _lib.call("na_lstm_layer_bwd_f32_hx", dh.data_ptr(), gates.data_ptr(), c.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(),
+              dgates.data_ptr(), _ptr(din) if need_din else None, _ptr(in_drop_mask), float(drop_scale), T, Bp, K, H,
+              _ptr(c0), dh_last.data_ptr(), dc_last.data_ptr(), _ptr(dh0) if need_dhx else None,
+              _ptr(dc0) if need_dhx else None, _stream())
+    return dgates, din, dh0, dc0
+
+
+@lstm_layer_bwd_hx.register_fake
+def _(dh, gates, c, w_ih, w_hh, in_drop_mask, drop_scale, need_din, c0, dh_last, dc_last, need_dhx):
+    T, Bp, H = dh.shape
+    st = (Bp, H) if need_dhx else (0,)
+    return (dh.new_empty((T, Bp, 4 * H)), dh.new_empty((T, Bp, w_ih.shape[1]) if need_din else (0,)), dh.new_empty(st),
+            dh.new_empty(st))
+
+
+@torch.library.custom_op("neuroalpha::lstm_layer_wgrad_hx", mutates_args=(), device_types="cuda")
+@_device_guard
+def lstm_layer_wgrad_hx(dgates: Tensor, inp: Tensor, h: Tensor, h0: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor]:
+    """lstm_layer_wgrad of a layer that started from h0 [Bp,H] (None = zeros): dW_hh includes dgates_0^T h0."""
+    _require_cuda(dgates, inp, h, h0)
+    T, Bp, G = dgates.shape
+    K, H = inp.shape[2], h.shape[2]
+    dev = dgates.device
+    dw_ih = torch.empty((G, K), dtype=torch.float32, device=dev)
+    dw_hh = torch.empty((G, H), dtype=torch.float32, device=dev)
+    db = torch.empty((G,), dtype=torch.float32, device=dev)
+    partials = torch.empty((_lib.query("na_wgrad_partial_floats", K, H),), dtype=torch.float32, device=dev)
+    _lib.call("na_lstm_layer_wgrad_f32_hx", dgates.data_ptr(), inp.data_ptr(), h.data_ptr(), dw_ih.data_ptr(),
+              dw_hh.data_ptr(), db.data_ptr(), partials.data_ptr(), T, Bp, K, H, _ptr(h0), _stream())
+    return dw_ih, dw_hh, db
+
+
+@lstm_layer_wgrad_hx.register_fake
+def _(dgates, inp, h, h0):
     G = dgates.shape[2]
     return dgates.new_empty((G, inp.shape[2])), dgates.new_empty((G, h.shape[2])), dgates.new_empty((G,))
 
@@ -580,6 +669,40 @@ def _(x, packed, head):
     return _ex_fake(x, x.shape[0], x.shape[1], 48, head[6].shape[0])
 
 
+@torch.library.custom_op("neuroalpha::decoder_lstm_x3", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_lstm_x3(x: Tensor, packed: Tensor, h0: Optional[Tensor], c0: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor]:
+    """The two LSTM layers of decoder_infer_x3 alone (same kernel and arithmetic; no pooling, no head): x [B,T,8] fp32,
+    optional initial state h0 / c0 [2,B,48] (both or neither) -> (out [B,T,48] = the last layer's h at every step,
+    h_n [2,B,48], c_n [2,B,48]).  Accuracy: see na_decoder_lstm_x3 in include/neuroalpha.h.  Inputs whose data is not
+    16-byte aligned (a contiguous view at an odd offset) are copied: the kernel reads them with 16-byte loads."""
+    _require_cuda(x, packed, h0, c0)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8:
+        raise RuntimeError("decoder_lstm_x3: x must be fp32 [B, T, 8]")
+    if (h0 is None) != (c0 is None):
+        raise RuntimeError("decoder_lstm_x3: h0 and c0 must be given together")
+    x = _aligned16(x.contiguous())
+    if h0 is not None:
+        if tuple(h0.shape) != (2, B, 48) or tuple(c0.shape) != (2, B, 48):
+            raise RuntimeError(f"decoder_lstm_x3: h0 / c0 must be [2, {B}, 48]")
+        h0, c0 = _aligned16(_f32c(h0)), _aligned16(_f32c(c0))
+    dev = x.device
+    out = torch.empty((B, T, 48), dtype=torch.float32, device=dev)
+    h_n = torch.empty((2, B, 48), dtype=torch.float32, device=dev)
+    c_n = torch.empty((2, B, 48), dtype=torch.float32, device=dev)
+    _lib.call("na_decoder_lstm_x3", x.data_ptr(), packed.data_ptr(), _ptr(h0), _ptr(c0), out.data_ptr(), h_n.data_ptr(),
+              c_n.data_ptr(), T, B, _stream())
+    return out, h_n, c_n
+
+
+@decoder_lstm_x3.register_fake
+def _(x, packed, h0, c0):
+    B, T = x.shape[0], x.shape[1]
+    f = torch.float32
+    return x.new_empty((B, T, 48), dtype=f), x.new_empty((2, B, 48), dtype=f), x.new_empty((2, B, 48), dtype=f)
+
+
 def decoder_infer_x3_intermediates(x: Tensor, packed: Tensor,
                                    head_params: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_x3 with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48])."""
@@ -811,6 +934,89 @@ class DecoderFunction(torch.autograd.Function):
             dx = dh[:, :B].permute(1, 0, 2).contiguous().reshape(xshape)
         grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip([*lstm_grads, *head_grads], ctx.param_dtypes)]
         return (dx, None, None, None, None, None, None, *grads)
+
+
+class LSTMSequenceFunction(torch.autograd.Function):
+    """x [B,T,K], initial state h0 / c0 [L,B,H] (both or neither; None = zeros), 4*L LSTM tensors ->
+    (out [B,T,H], h_n [L,B,H], c_n [L,B,H]): nn.LSTM(batch_first=True) on the FFMA / generic kernels, with the backward
+    written out by hand (fused BPTT + time-parallel weight-gradient reductions) in the style of DecoderFunction.
+    ``drop_masks``: None, or L-1 keep-masks [B,T,H] of 0/1; layer l+1 then reads h_l * mask_l / (1 - p).  All outputs
+    fp32."""
+
+    @staticmethod
+    def forward(ctx, x, h0, c0, p, drop_masks, *params):
+        _require_cuda(x, h0, c0, *params)
+        ctx.param_dtypes = [t.dtype for t in params]
+        ctx.hx_dtypes = None if h0 is None else (h0.dtype, c0.dtype)
+        L = len(params) // 4
+        B, T, _ = x.shape
+        H = params[1].shape[1]
+        Bp = padded_batch(B)
+        scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0
+
+        def rows(t, lead):                  # [..., B, H] -> zero-padded [..., Bp, H] fp32 (TMP rows)
+            z = torch.zeros((*lead, Bp, H), dtype=torch.float32, device=x.device)
+            z[..., :B, :] = t.detach()
+            return z
+
+        h0p = rows(h0, (L,)) if h0 is not None else None
+        c0p = rows(c0, (L,)) if c0 is not None else None
+        masks = [rows(m.permute(1, 0, 2), (T,)) for m in drop_masks] if drop_masks is not None else None
+        saved, h_n, c_n = [], [], []
+        layer_in = window_zscore(_aligned16(_f32c(x.detach())), T, T, False, True, False)     # TMP copy of x, fp32
+        for l in range(L):
+            w_ih, w_hh, b_ih, b_hh = (_f32c(t.detach()) for t in params[4 * l:4 * l + 4])
+            wt, bias = pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
+            mask = masks[l] if (masks is not None and l < L - 1) else None
+            h, c, gates, h_drop = lstm_layer_fwd_hx(layer_in, wt, bias, mask, scale,
+                                                    None if h0p is None else h0p[l], None if c0p is None else c0p[l])
+            saved += [layer_in, h, c, gates, w_ih, w_hh]
+            h_n.append(h[T - 1, :B])
+            c_n.append(c[T - 1, :B])
+            layer_in = h_drop if mask is not None else h
+        ctx.save_for_backward(*saved, *([h0p, c0p] if h0p is not None else []), *(masks or []))
+        ctx.meta = (L, scale, B, tuple(x.shape), h0p is not None, masks is not None)
+        return h[:, :B].permute(1, 0, 2).contiguous(), torch.stack(h_n), torch.stack(c_n)
+
+    @staticmethod
+    def backward(ctx, dout, dh_n, dc_n):
+        L, scale, B, xshape, has_hx, has_masks = ctx.meta
+        sv = list(ctx.saved_tensors)
+        layers = [sv[6 * l:6 * l + 6] for l in range(L)]
+        pos = 6 * L
+        h0p, c0p = (sv[pos], sv[pos + 1]) if has_hx else (None, None)
+        pos += 2 if has_hx else 0
+        masks = sv[pos:pos + L - 1] if has_masks else None
+        T, Bp, H = layers[-1][1].shape
+
+        def rows(t):
+            z = torch.zeros((Bp, H), dtype=torch.float32, device=t.device)
+            z[:B] = t
+            return z
+
+        dh = torch.zeros((T, Bp, H), dtype=torch.float32, device=dout.device)
+        dh[:, :B] = dout.permute(1, 0, 2)                    # the top layer's h is the output
+        need_dx = ctx.needs_input_grad[0]
+        need_dhx = has_hx and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
+        lstm_grads: List[Tensor] = [None] * (4 * L)
+        dh0, dc0 = [None] * L, [None] * L
+        for l in range(L - 1, -1, -1):
+            layer_in, h, c, gates, w_ih, w_hh = layers[l]
+            in_mask = masks[l - 1] if (has_masks and l > 0) else None
+            need_din = l > 0 or need_dx
+            dgates, din, dh0[l], dc0[l] = lstm_layer_bwd_hx(
+                dh, gates, c, w_ih, w_hh, in_mask, scale, need_din, None if c0p is None else c0p[l],
+                rows(dh_n[l].float()), rows(dc_n[l].float()), need_dhx)
+            dw_ih, dw_hh, db = lstm_layer_wgrad_hx(dgates, layer_in, h, None if h0p is None else h0p[l])
+            lstm_grads[4 * l:4 * l + 4] = [dw_ih, dw_hh, db, db.clone()]
+            dh = din
+        dx = dh[:, :B].permute(1, 0, 2).contiguous().reshape(xshape) if need_dx else None
+        dh0_out = dc0_out = None
+        if need_dhx:
+            dh0_out = torch.stack([g[:B] for g in dh0]).to(ctx.hx_dtypes[0])
+            dc0_out = torch.stack([g[:B] for g in dc0]).to(ctx.hx_dtypes[1])
+        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip(lstm_grads, ctx.param_dtypes)]
+        return (dx, dh0_out, dc0_out, None, None, *grads)
 
 
 def decoder_train_forward(x: Tensor, lstm_params, head_params, p: float, zscore: bool = False,

@@ -44,7 +44,7 @@ da, db = demangle(list(a)), demangle(list(b))
 def key(d):
     # "void na::tc::decoder_infer_x3_kernel<0, false>(...)" -> "decoder_infer_x3_kernel<0>"
     d = d.split("(")[0].replace("void ", "")
-    d = re.sub(r", false>", ">", d)
+    d = re.sub(r"(, false)+>", ">", d)
     return d
 ka = {key(da[n]): n for n in a}
 kb = {key(db[n]): n for n in b}
