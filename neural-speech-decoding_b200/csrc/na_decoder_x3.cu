@@ -11,9 +11,17 @@
 // tanh.approx of the 16-bit tier is 5e-4 and cannot be used), 10 per cell update -> 7,680 MUFU cycles per step.
 //
 // Structure = decoder_infer_v2_kernel (na_decoder_tc2.cu): 12 epilogue warps own both layers of (lane quarter, 16-unit
-// group) and alternate layer-0 step t / layer-1 step t-1; one elected MMA lane; the producer warp reads the caller's
-// fp32 [B][T][8] windows directly and writes x_hi / x_lo; the attention score is an extra accumulator column of the
+// group) and alternate layer-0 step t / layer-1 step t-1; one elected MMA lane; two producer warps read the caller's
+// fp32 [B][T][8] windows directly and write x_hi / x_lo; the attention score is an extra accumulator column of the
 // next layer-1 MMA (3-term split as well); cell state, pooling, LayerNorm, MLP and softmax in fp32.
+// 512 threads: after the setup the control warpgroup (MMA, producers, TMEM allocator) gives registers to the epilogue
+// warpgroups with setmaxnreg (56 / 152 per thread instead of 128 for all), so an epilogue phase issues all of its TMEM
+// loads before one wait without spilling.  The epilogue reports "accumulator read" (d*_drained) separately from
+// "h written" (h*_ready): the input half of the next step's MMAs (x or h0 and the bias: 3 of layer 0's 12, 10 of
+// layer 1's 19) runs while the epilogue still computes, and only the recurrent half waits for h.  Measured on one B200
+// (1000 W power limit, 1965 MHz SM clock), alternating with the 14-warp / 128-register kernel: 40,960 windows
+// 6.36-6.39 -> 5.86-5.89 ms (the register split alone: 6.04), one 32-window quarter per SM 1.44-1.47 -> 1.35-1.39 ms
+// (all of it from the early input MMAs); DESIGN 6a.
 //   A chunks ([128 rows][8] fp16 = 2 KB):  x stage = [x_hi | ones | x_lo];  h0[2], h1 = 6 hi chunks + 6 lo chunks
 //   B0 (15 chunks x 192 rows): Wih_hi | bias(hi,lo) | Whh_hi x6 | Wih_lo | Whh_lo x6
 //   B1 (25 chunks x 208 rows): Wih_hi x6 | Whh_hi x6 | bias(hi,lo) | Wih_lo x6 | Whh_lo x6;  rows 192.. = attention
@@ -33,8 +41,16 @@ struct SmemX3 {
     alignas(128) unsigned char onez[2 * kAChunk];                  // [ones | zeros]
     alignas(8) uint64_t x_full[kX3XStages], x_empty[kX3XStages];
     uint64_t d0_full, d1_full, h0_ready[2], h1_ready;
+    uint64_t d0_drained, d1_drained;                               // the epilogue has read the accumulator out of TMEM
     uint32_t tmem_base;
 };
+
+// 4 warpgroups: 0-2 = the 12 epilogue warps, 3 = MMA warp, two producer warps and the TMEM allocator.  Warp w sits on SM
+// sub-partition w % 4, so each sub-partition holds 3 epilogue warps and 1 control warp and its 512 registers per thread
+// slot split as 3 x kX3EpiRegs + kX3CtlRegs (setmaxnreg after the setup; the launch gives every warp 128).
+constexpr int kX3InferThreads = 16 * 32;
+constexpr int kX3EpiRegs = 152, kX3CtlRegs = 56;
+static_assert(3 * kX3EpiRegs + kX3CtlRegs <= 512, "register file of one SM sub-partition");
 
 // ---- weight image: [B0 15 chunks][192][8] | [B1 25 chunks][192][8] fp16, row n = (j/4)*16 + gate*4 + j%4 ------------------
 __global__ void pack_decoder_x3_kernel(const float* __restrict__ w_ih0, const float* __restrict__ w_hh0,
@@ -126,6 +142,38 @@ __device__ __forceinline__ void x3_seq_init(SmemX3& S, const int q, const int g,
     }
 }
 
+// TMEM loads without the wait: a phase issues all of its loads and waits once (x3_drained).
+__device__ __forceinline__ void x3_tmem_ld16_nowait(uint32_t taddr, uint32_t* v) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+        : "r"(taddr)
+        : "memory");
+}
+__device__ __forceinline__ void x3_tmem_ld32_nowait(uint32_t taddr, uint32_t* v) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+          "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+          "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+        : "r"(taddr)
+        : "memory");
+}
+__device__ __forceinline__ void x3_tmem_ld2_nowait(uint32_t taddr, uint32_t* v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(v[0]), "=r"(v[1]) : "r"(taddr) : "memory");
+}
+// The warp's loads of this phase have landed: one arrival of the warp on `bar` (the MMA warp may overwrite the accumulator).
+__device__ __forceinline__ void x3_drained(uint64_t* bar, const int lane) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(bar);
+}
+
 // Epilogue of one tile for one warp: both layers of (lane quarter q, unit group g).  R = row replication as in
 // decoder_infer_v2_kernel: the tile holds 128 / R distinct windows, copy rp = q / (4 / R) of source quarter qs = q % (4 / R)
 // takes granules [4 g + rp * (4 / R), + 4 / R) of the 12 four-unit granules and stores its h (hi and lo) to every copy.
@@ -158,9 +206,14 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             if (t < T) {
                 mbar_wait(&S.d0_full, n & 1);
                 if (q == 0 && g == 0 && lane == 0) mbar_arrive(&S.x_empty[n % kX3XStages]);
+                x3_drained(&S.d0_drained, lane);
                 mbar_arrive(&S.h0_ready[n & 1]);
             }
-            if (t >= 1) { mbar_wait(&S.d1_full, k1 & 1); ++k1; mbar_arrive(&S.h1_ready); }
+            if (t >= 1) {
+                mbar_wait(&S.d1_full, k1 & 1); ++k1;
+                x3_drained(&S.d1_drained, lane);
+                mbar_arrive(&S.h1_ready);
+            }
         }
         if constexpr (!kSeq) { mbar_wait(&S.d1_full, k1 & 1); ++k1; }
         return;
@@ -193,26 +246,26 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
 #pragma unroll
         for (int j = 0; j < kU; ++j) z[j] = fmaf(e, hprev[j], z[j]);
     };
-    // gates of this thread's granules -> cell update -> h (fp32, kept in hout) -> hi / lo fp16 into every row copy of `buf`
-    auto layer_phase = [&](const uint32_t tmem_d, float* c, unsigned char* buf, float* hout) {
+    // Every TMEM load of a phase is issued before its single wait (x3_drained), which also releases the accumulator to
+    // the MMA warp; the gates of this thread's granules then go through the cell update -> h (fp32, kept in hout) ->
+    // hi / lo fp16 into every row copy of `buf`.
+    auto gates_ld = [&](const uint32_t tmem_d, uint32_t* v) {
         if constexpr (R == 4) {
-            uint32_t v[16];
-            asm volatile(
-                "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                  "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                : "r"(tmem_d + lane_base + gr0 * 16)
-                : "memory");
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            x3_tmem_ld16_nowait(tmem_d + lane_base + gr0 * 16, v);
+        } else {
+#pragma unroll
+            for (int pr = 0; pr < kSlots / 2; ++pr) x3_tmem_ld32_nowait(tmem_d + lane_base + (gr0 + 2 * pr) * 16, v + 32 * pr);
+        }
+    };
+    auto cells = [&](const uint32_t* v, float* c, unsigned char* buf, float* hout) {
+        if constexpr (R == 4) {
             cell_granule_exact<NR>(v, c, hout);
             x3_store_h<R>(buf, gr0, wrow, 0, hout);
         } else {
 #pragma unroll
             for (int pr = 0; pr < kSlots / 2; ++pr) {       // pairs of granules = one 8-unit K chunk
-                uint32_t v[32];
-                tmem_ld32(tmem_d + lane_base + (gr0 + 2 * pr) * 16, v);
-                cell_granule_exact<NR>(v, c + pr * 8, hout + pr * 8);
-                cell_granule_exact<NR>(v + 16, c + pr * 8 + 4, hout + pr * 8 + 4);
+                cell_granule_exact<NR>(v + 32 * pr, c + pr * 8, hout + pr * 8);
+                cell_granule_exact<NR>(v + 32 * pr + 16, c + pr * 8 + 4, hout + pr * 8 + 4);
                 x3_store_h<R>(buf, gr0, wrow, pr, hout + pr * 8);
             }
         }
@@ -223,9 +276,11 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             mbar_wait(&S.d0_full, n & 1);
             if (q == 0 && g == 0 && lane == 0) mbar_arrive(&S.x_empty[n % kX3XStages]);
             tc_fence_after();
+            uint32_t v[16 * kSlots];
+            gates_ld(tmem_d0, v);
+            x3_drained(&S.d0_drained, lane);
             float hl0[kU];                         // layer-0 h: the next step reads it from shared memory
-            layer_phase(tmem_d0, c0, S.h0[n & 1], hl0);
-            tc_fence_before();
+            cells(v, c0, S.h0[n & 1], hl0);
             fence_proxy_async_smem();
             mbar_arrive(&S.h0_ready[n & 1]);
             if constexpr (kSeq)
@@ -237,15 +292,16 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         if (t >= 1) {                              // ---- layer 1, step t-1 (+ pooling of step t-2)
             mbar_wait(&S.d1_full, k1 & 1); ++k1;
             tc_fence_after();
+            uint32_t v[16 * kSlots], sc2[2];
+            gates_ld(tmem_d1, v);
+            if constexpr (!kSeq) x3_tmem_ld2_nowait(tmem_d1 + lane_base + kN, sc2);
+            x3_drained(&S.d1_drained, lane);
             if constexpr (!kSeq) {
-                uint32_t sc2[2];
-                x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
                 if (t >= 2) pool(__uint_as_float(sc2[0]));     // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
                 if constexpr (kEx)
                     if (t >= 2 && ex_writer && scores_tm) scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]);
             }
-            layer_phase(tmem_d1, c1, S.h1, hprev);
-            tc_fence_before();
+            cells(v, c1, S.h1, hprev);
             fence_proxy_async_smem();
             mbar_arrive(&S.h1_ready);
             if constexpr (kSeq)
@@ -329,8 +385,11 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
     }
 }
 
+// Barrier 0 over the whole CTA from code that differs between warps (the tile loops of the two register budgets).
+__device__ __forceinline__ void x3_cta_sync() { asm volatile("barrier.sync 0;" ::: "memory"); }
+
 template <int NR, bool kEx = false, bool kSeq = false>
-__global__ void __launch_bounds__(kX3Threads, 1)
+__global__ void __launch_bounds__(kX3InferThreads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
                         const float* __restrict__ attn_w, const float* __restrict__ attn_b,
@@ -345,7 +404,7 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         const float* __restrict__ c_init,           // the last layer's h [B][T][48], final state [2][B][48]
                         float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
     static_assert(!(kEx && kSeq), "the intermediates and the sequence output are separate instantiations");
-    constexpr int kMmaWarp = 12, kTmaWarp = 13;
+    constexpr int kMmaWarp = 12, kProdWarp = 13, kTmemWarp = 15;     // producers: warps 13 and 14
     const bool seq_init = kSeq && h_init != nullptr;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     SmemX3& S = *reinterpret_cast<SmemX3*>(smem_raw);
@@ -357,14 +416,14 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
         const uint4* src = reinterpret_cast<const uint4*>(packed);
         uint4* d0 = reinterpret_cast<uint4*>(S.b0);
         constexpr int n0_16 = kX3B0Chunks * kBChunk / 16;
-        for (int i = tid; i < n0_16; i += kX3Threads) d0[i] = src[i];
-        for (int i = tid; i < kX3B1Chunks * kN; i += kX3Threads) {
+        for (int i = tid; i < n0_16; i += kX3InferThreads) d0[i] = src[i];
+        for (int i = tid; i < kX3B1Chunks * kN; i += kX3InferThreads) {
             const int ch = i / kN, r = i % kN;
             reinterpret_cast<uint4*>(S.b1 + ch * kX3B1Chunk)[r] = src[n0_16 + i];
         }
         // rows 192..207 of every layer-1 chunk: row 192 = the attention vector split like the weights (hi in the hi
         // chunks of the h1 part, lo in its lo chunks, the bias pair on the ones chunk); everything else zero
-        for (int i = tid; i < kX3B1Chunks * 16; i += kX3Threads) {
+        for (int i = tid; i < kX3B1Chunks * 16; i += kX3InferThreads) {
             const int ch = i / 16, r = i % 16;
             uint16_t w[8];
 #pragma unroll
@@ -385,20 +444,21 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
         }
         const uint4 ones = make_uint4(kValOnes2, 0u, 0u, 0u);     // fp16 {1,1,0,0,0,0,0,0}
         const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-        for (int i = tid; i < kRows; i += kX3Threads) {
+        for (int i = tid; i < kRows; i += kX3InferThreads) {
 #pragma unroll
             for (int s = 0; s < kX3XStages; ++s) reinterpret_cast<uint4*>(S.x[s] + kAChunk)[i] = ones;
             reinterpret_cast<uint4*>(S.onez)[i] = ones;
             reinterpret_cast<uint4*>(S.onez + kAChunk)[i] = zero;
         }
         if (tid == 0) {
-            for (int s = 0; s < kX3XStages; ++s) { mbar_init(&S.x_full[s], 1); mbar_init(&S.x_empty[s], 1); }
+            for (int s = 0; s < kX3XStages; ++s) { mbar_init(&S.x_full[s], 2); mbar_init(&S.x_empty[s], 1); }
             mbar_init(&S.d0_full, 1); mbar_init(&S.d1_full, 1);
             mbar_init(&S.h0_ready[0], 384); mbar_init(&S.h0_ready[1], 384);
             mbar_init(&S.h1_ready, 384);
+            mbar_init(&S.d0_drained, 12); mbar_init(&S.d1_drained, 12);
             fence_mbar_init();
         }
-        if (warp == kTmaWarp) tmem_alloc_all(&S.tmem_base);
+        if (warp == kTmemWarp) tmem_alloc_all(&S.tmem_base);
         tc_fence_before();
         fence_proxy_async_smem();
         __syncthreads();
@@ -407,167 +467,195 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
     const uint32_t tmem = __shfl_sync(0xffffffffu, S.tmem_base, 0);
     const uint32_t tmem_d0 = tmem, tmem_d1 = tmem + kN;
 
-    const int q_begin = (int)(((int64_t)blockIdx.x * nquarters) / gridDim.x);
-    const int q_end = (int)(((int64_t)(blockIdx.x + 1) * nquarters) / gridDim.x);
-    int n0 = 0;
-    uint32_t k1 = 0;
-    for (int q0 = q_begin; q0 < q_end; n0 += T) {
-        const int nq = min(4, q_end - q0);                 // active source quarters of this tile
-        const int R = nq == 1 ? 4 : (nq == 2 ? 2 : 1);     // short tiles are row-replicated (see x3_epilogue_tile)
-        const int64_t b0 = (int64_t)q0 * 32;
-        if (seq_init) {
-            if (warp < kMmaWarp) {
-                if (R == 1) x3_seq_init<1>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
-                else if (R == 2) x3_seq_init<2>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
-                else x3_seq_init<4>(S, warp & 3, warp >> 2, lane, nq, n0, b0, B, h_init);
-            }
-            fence_proxy_async_smem();
-            __syncthreads();       // the previous tile is complete (barrier at its end): h0 / h1 are free
+    // body(nq, R, b0, n0) once per tile of this CTA, then the tile barrier.  Every role runs its own copy of the loop: code
+    // that both register budgets reach is held to the smaller one, and values one role keeps across tiles (the MMA
+    // descriptors) would occupy registers in the other.
+    auto for_each_tile = [&](auto&& body) {
+        const int q_begin = (int)(((int64_t)blockIdx.x * nquarters) / gridDim.x);
+        const int q_end = (int)(((int64_t)(blockIdx.x + 1) * nquarters) / gridDim.x);
+        int n0 = 0;
+        for (int q0 = q_begin; q0 < q_end; n0 += T) {
+            const int nq = min(4, q_end - q0);                 // active source quarters of this tile
+            const int R = nq == 1 ? 4 : (nq == 2 ? 2 : 1);     // short tiles are row-replicated (see x3_epilogue_tile)
+            body(nq, R, (int64_t)q0 * 32, n0);
+            x3_cta_sync();     // tile done: every MMA has completed; the z exchange in h0 has been consumed
+            q0 += nq;
         }
-
-        if (warp == kTmaWarp) {
-            // ================= producer: fp32 rows -> x_hi / x_lo chunks (rows of step t+1 are in flight) ========
-            const int nrows = nq * 32;
-            float4 cur[4][2], nxt[4][2];
-            auto fetch = [&](int t, float4 (&v)[4][2]) {
-#pragma unroll
-                for (int rr = 0; rr < 4; ++rr) {
-                    const int row = rr * 32 + lane;
-                    const int64_t b = b0 + row;
-                    if (row < nrows && b < B) {
-                        const float4* src = reinterpret_cast<const float4*>(x32 + (b * T + t) * 8);
-                        v[rr][0] = __ldg(src);
-                        v[rr][1] = __ldg(src + 1);
-                    } else {
-                        v[rr][0] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        v[rr][1] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    }
-                }
-            };
-            fetch(0, cur);
-            for (int t = 0; t < T; ++t) {
-                const int n = n0 + t, s = n % kX3XStages, u = n / kX3XStages;
-                if (t + 1 < T) fetch(t + 1, nxt);
-                mbar_wait(&S.x_empty[s], (u & 1) ^ 1);
-#pragma unroll
-                for (int rr = 0; rr < 4; ++rr) {
-                    const int row = rr * 32 + lane;
-                    if (row < nrows) {
-                        const float f[8] = {kX3XScale * cur[rr][0].x, kX3XScale * cur[rr][0].y, kX3XScale * cur[rr][0].z, kX3XScale * cur[rr][0].w,
-                                            kX3XScale * cur[rr][1].x, kX3XScale * cur[rr][1].y, kX3XScale * cur[rr][1].z, kX3XScale * cur[rr][1].w};
-                        uint32_t hi[4], lo[4];
-                        split_pack8(f, hi, lo);
-                        for (int rep = 0; rep < R; ++rep) {
-                            const int rr2 = rep * (kRows / R) + row;
-                            st_shared_v4(S.x[s] + rr2 * 16, hi[0], hi[1], hi[2], hi[3]);
-                            st_shared_v4(S.x[s] + 2 * kAChunk + rr2 * 16, lo[0], lo[1], lo[2], lo[3]);
-                        }
-                    }
-                }
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&S.x_full[s]);
-#pragma unroll
-                for (int rr = 0; rr < 4; ++rr) { cur[rr][0] = nxt[rr][0]; cur[rr][1] = nxt[rr][1]; }
-            }
-        } else if (warp == kMmaWarp) {
+    };
+    if (warp >= kMmaWarp) {
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kX3CtlRegs));
+        if (warp == kMmaWarp) {
             // ================= MMA issuer (whole warp, one elected lane) ========================================
             const bool leader = elect_one();
             // descriptors pair two K chunks through the leading byte offset (LBO): adjacent chunks, or chunk + zeros
             const uint32_t a_x0 = smem_u32(S.x[0]), a_zero = smem_u32(S.onez + kAChunk), a_ones = smem_u32(S.onez);
             const uint64_t d_b0 = umma_desc(smem_u32(S.b0), kBChunk, 128), d_b1 = umma_desc(smem_u32(S.b1), kX3B1Chunk, 128);
-            const uint64_t d_h0[2] = {umma_desc(smem_u32(S.h0[0]), kAChunk, 128), umma_desc(smem_u32(S.h0[1]), kAChunk, 128)};
+            const uint64_t d_h0 = umma_desc(smem_u32(S.h0[0]), kAChunk, 128);        // buffer i: desc_adv(d_h0, i * 12 * kAChunk)
             const uint64_t d_h1 = umma_desc(smem_u32(S.h1), kAChunk, 128);
             const uint64_t d_bias = umma_desc(a_ones, kAChunk, 128);                                // (ones | zeros)
-            for (int t = 0; t <= T; ++t) {
-                const int n = n0 + t;
-                if (t >= 1) {                                  // h0_{t-1} (hi and lo) written, D0 drained
-                    mbar_wait(&S.h0_ready[(n - 1) & 1], ((n - 1) >> 1) & 1);
-                    tc_fence_after();
-                }
-                if (t < T) {                                   // layer 0, step t
-                    const int s = n % kX3XStages, u = n / kX3XStages;
-                    mbar_wait(&S.x_full[s], u & 1);
-                    tc_fence_after();
-                    const uint32_t xs = a_x0 + s * 3 * kAChunk;
-                    if (leader) {
-                        // (x_hi | ones) . (Wih_hi | bias);  (x_hi | zeros) . (Wih_lo | *);  (x_lo | zeros) . (Wih_hi | *)
-                        umma_bf16(tmem_d0, umma_desc(xs, kAChunk, 128), d_b0, 0u);
-                        umma_bf16(tmem_d0, umma_desc(xs, a_zero - xs, 128), desc_adv(d_b0, 8 * kBChunk), 1u);
-                        umma_bf16(tmem_d0, umma_desc(xs + 2 * kAChunk, a_zero - (xs + 2 * kAChunk), 128), d_b0, 1u);
+            for_each_tile([&](const int, const int, const int64_t, const int n0) {
+                if (seq_init) x3_cta_sync();                      // the epilogue warps have stored the initial state
+                // Each accumulator gets its input part (x or h0_m, and the bias) as soon as the epilogue has read the previous
+                // step out of it (d*_drained), and its recurrent part once the h it needs is written (h*_ready); the order of
+                // the products into an accumulator stays input part first, recurrent part last.
+                for (int t = 0; t <= T; ++t) {
+                    const int n = n0 + t;
+                    if (t < T) {                                   // layer 0, step t: input part
+                        const int s = n % kX3XStages, u = n / kX3XStages;
+                        if (t >= 1) mbar_wait(&S.d0_drained, (n - 1) & 1);
+                        mbar_wait(&S.x_full[s], u & 1);
+                        tc_fence_after();
+                        const uint32_t xs = a_x0 + s * 3 * kAChunk;
+                        if (leader) {
+                            // (x_hi | ones) . (Wih_hi | bias);  (x_hi | zeros) . (Wih_lo | *);  (x_lo | zeros) . (Wih_hi | *)
+                            umma_bf16(tmem_d0, umma_desc(xs, kAChunk, 128), d_b0, 0u);
+                            umma_bf16(tmem_d0, umma_desc(xs, a_zero - xs, 128), desc_adv(d_b0, 8 * kBChunk), 1u);
+                            umma_bf16(tmem_d0, umma_desc(xs + 2 * kAChunk, a_zero - (xs + 2 * kAChunk), 128), d_b0, 1u);
+                        }
                     }
-                    if (t >= 1 || seq_init) {                   // h_{-1} = 0 unless an initial state was stored
-                        const uint64_t hp = d_h0[(n - 1) & 1];
+                    if (t >= 1) {                                  // h0_{t-1} (hi and lo) written
+                        mbar_wait(&S.h0_ready[(n - 1) & 1], ((n - 1) >> 1) & 1);
+                        tc_fence_after();
+                    }
+                    if (t < T) {                                   // layer 0, step t: recurrent part
+                        if (t >= 1 || seq_init) {                   // h_{-1} = 0 unless an initial state was stored
+                            const uint64_t hp = desc_adv(d_h0, ((n - 1) & 1) * 12 * kAChunk);
+#pragma unroll
+                            for (int i = 0; i < 3; ++i) {
+                                if (leader) {
+                                    umma_bf16(tmem_d0, desc_adv(hp, 2 * i * kAChunk), desc_adv(d_b0, (2 + 2 * i) * kBChunk), 1u);        // hi . hi
+                                    umma_bf16(tmem_d0, desc_adv(hp, 2 * i * kAChunk), desc_adv(d_b0, (9 + 2 * i) * kBChunk), 1u);        // hi . lo
+                                    umma_bf16(tmem_d0, desc_adv(hp, (6 + 2 * i) * kAChunk), desc_adv(d_b0, (2 + 2 * i) * kBChunk), 1u);  // lo . hi
+                                }
+                            }
+                        }
+                        if (leader) umma_commit(&S.d0_full);
+                    }
+                    if (t >= 1) {                                  // layer 1, step m = t - 1
+                        const int m = n - 1;
+                        if (t >= 2) {
+                            mbar_wait(&S.d1_drained, (m - 1) & 1);
+                            tc_fence_after();
+                        }
+                        const uint64_t hin = desc_adv(d_h0, (m & 1) * 12 * kAChunk);
+                        if (leader) umma_bf16_i(tmem_d1, d_bias, desc_adv(d_b1, 12 * kX3B1Chunk), kX3IdescL1, 0u);
 #pragma unroll
                         for (int i = 0; i < 3; ++i) {
                             if (leader) {
-                                umma_bf16(tmem_d0, desc_adv(hp, 2 * i * kAChunk), desc_adv(d_b0, (2 + 2 * i) * kBChunk), 1u);        // hi . hi
-                                umma_bf16(tmem_d0, desc_adv(hp, 2 * i * kAChunk), desc_adv(d_b0, (9 + 2 * i) * kBChunk), 1u);        // hi . lo
-                                umma_bf16(tmem_d0, desc_adv(hp, (6 + 2 * i) * kAChunk), desc_adv(d_b0, (2 + 2 * i) * kBChunk), 1u);  // lo . hi
+                                umma_bf16_i(tmem_d1, desc_adv(hin, 2 * i * kAChunk), desc_adv(d_b1, 2 * i * kX3B1Chunk), kX3IdescL1, 1u);
+                                umma_bf16_i(tmem_d1, desc_adv(hin, 2 * i * kAChunk), desc_adv(d_b1, (13 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
+                                umma_bf16_i(tmem_d1, desc_adv(hin, (6 + 2 * i) * kAChunk), desc_adv(d_b1, 2 * i * kX3B1Chunk), kX3IdescL1, 1u);
                             }
                         }
+                        if (t >= 2) {
+                            mbar_wait(&S.h1_ready, (m - 1) & 1);
+                            tc_fence_after();
+                        }
+                        if (t >= 2 || seq_init) {
+#pragma unroll
+                            for (int i = 0; i < 3; ++i) {
+                                if (leader) {
+                                    umma_bf16_i(tmem_d1, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1, (6 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
+                                    umma_bf16_i(tmem_d1, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1, (19 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
+                                    umma_bf16_i(tmem_d1, desc_adv(d_h1, (6 + 2 * i) * kAChunk), desc_adv(d_b1, (6 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
+                                }
+                            }
+                        }
+                        if (leader) umma_commit(&S.d1_full);
                     }
-                    if (leader) umma_commit(&S.d0_full);
                 }
-                if (t >= 1) {                                  // layer 1, step m = t - 1
-                    const int m = n - 1;
-                    if (t >= 2) {
-                        mbar_wait(&S.h1_ready, (m - 1) & 1);
-                        tc_fence_after();
-                    }
-                    const uint64_t hin = d_h0[m & 1];
-                    if (leader) umma_bf16_i(tmem_d1, d_bias, desc_adv(d_b1, 12 * kX3B1Chunk), kX3IdescL1, 0u);
+                if constexpr (!kSeq) {   // flush: score of the last step into the 16 score columns (rows 192..207 of the h1-part chunks + bias)
+                    const int m = n0 + T - 1;
+                    mbar_wait(&S.h1_ready, m & 1);
+                    tc_fence_after();
+                    const uint64_t d_b1s = desc_adv(d_b1, kN * 16);
+                    if (leader) umma_bf16_i(tmem_d1 + kN, d_bias, desc_adv(d_b1s, 12 * kX3B1Chunk), kX3IdescFlush, 0u);
 #pragma unroll
                     for (int i = 0; i < 3; ++i) {
                         if (leader) {
-                            umma_bf16_i(tmem_d1, desc_adv(hin, 2 * i * kAChunk), desc_adv(d_b1, 2 * i * kX3B1Chunk), kX3IdescL1, 1u);
-                            umma_bf16_i(tmem_d1, desc_adv(hin, 2 * i * kAChunk), desc_adv(d_b1, (13 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
-                            umma_bf16_i(tmem_d1, desc_adv(hin, (6 + 2 * i) * kAChunk), desc_adv(d_b1, 2 * i * kX3B1Chunk), kX3IdescL1, 1u);
-                        }
-                    }
-                    if (t >= 2 || seq_init) {
-#pragma unroll
-                        for (int i = 0; i < 3; ++i) {
-                            if (leader) {
-                                umma_bf16_i(tmem_d1, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1, (6 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
-                                umma_bf16_i(tmem_d1, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1, (19 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
-                                umma_bf16_i(tmem_d1, desc_adv(d_h1, (6 + 2 * i) * kAChunk), desc_adv(d_b1, (6 + 2 * i) * kX3B1Chunk), kX3IdescL1, 1u);
-                            }
+                            umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1s, (6 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
+                            umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1s, (19 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
+                            umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, (6 + 2 * i) * kAChunk), desc_adv(d_b1s, (6 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
                         }
                     }
                     if (leader) umma_commit(&S.d1_full);
                 }
-            }
-            if constexpr (!kSeq) {   // flush: score of the last step into the 16 score columns (rows 192..207 of the h1-part chunks + bias)
-                const int m = n0 + T - 1;
-                mbar_wait(&S.h1_ready, m & 1);
-                tc_fence_after();
-                const uint64_t d_b1s = desc_adv(d_b1, kN * 16);
-                if (leader) umma_bf16_i(tmem_d1 + kN, d_bias, desc_adv(d_b1s, 12 * kX3B1Chunk), kX3IdescFlush, 0u);
-#pragma unroll
-                for (int i = 0; i < 3; ++i) {
-                    if (leader) {
-                        umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1s, (6 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
-                        umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, 2 * i * kAChunk), desc_adv(d_b1s, (19 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
-                        umma_bf16_i(tmem_d1 + kN, desc_adv(d_h1, (6 + 2 * i) * kAChunk), desc_adv(d_b1s, (6 + 2 * i) * kX3B1Chunk), kX3IdescFlush, 1u);
-                    }
-                }
-                if (leader) umma_commit(&S.d1_full);
-            }
+            });
         } else {
-            // ================= epilogue: both layers of (quarter q, unit group g) ================================
-            const int q = warp & 3, g = warp >> 2;
+            for_each_tile([&](const int nq, const int R, const int64_t b0, const int n0) {
+                if (seq_init) x3_cta_sync();
+                if (warp == kTmemWarp) return;
+                // ================= producers: fp32 rows -> x_hi / x_lo chunks (rows of step t+1 are in flight) =======
+                // each of the two warps owns two row quarters; x_full counts both
+                const int nrows = nq * 32, rq0 = 2 * (warp - kProdWarp);
+                float4 cur[2][2], nxt[2][2];
+                auto fetch = [&](int t, float4 (&v)[2][2]) {
+#pragma unroll
+                    for (int rr = 0; rr < 2; ++rr) {
+                        const int row = (rq0 + rr) * 32 + lane;
+                        const int64_t b = b0 + row;
+                        if (row < nrows && b < B) {
+                            const float4* src = reinterpret_cast<const float4*>(x32 + (b * T + t) * 8);
+                            v[rr][0] = __ldg(src);
+                            v[rr][1] = __ldg(src + 1);
+                        } else {
+                            v[rr][0] = make_float4(0.f, 0.f, 0.f, 0.f);
+                            v[rr][1] = make_float4(0.f, 0.f, 0.f, 0.f);
+                        }
+                    }
+                };
+                fetch(0, cur);
+                for (int t = 0; t < T; ++t) {
+                    const int n = n0 + t, s = n % kX3XStages, u = n / kX3XStages;
+                    if (t + 1 < T) fetch(t + 1, nxt);
+                    mbar_wait(&S.x_empty[s], (u & 1) ^ 1);
+#pragma unroll
+                    for (int rr = 0; rr < 2; ++rr) {
+                        const int row = (rq0 + rr) * 32 + lane;
+                        if (row < nrows) {
+                            const float f[8] = {kX3XScale * cur[rr][0].x, kX3XScale * cur[rr][0].y, kX3XScale * cur[rr][0].z, kX3XScale * cur[rr][0].w,
+                                                kX3XScale * cur[rr][1].x, kX3XScale * cur[rr][1].y, kX3XScale * cur[rr][1].z, kX3XScale * cur[rr][1].w};
+                            uint32_t hi[4], lo[4];
+                            split_pack8(f, hi, lo);
+                            for (int rep = 0; rep < R; ++rep) {
+                                const int rr2 = rep * (kRows / R) + row;
+                                st_shared_v4(S.x[s] + rr2 * 16, hi[0], hi[1], hi[2], hi[3]);
+                                st_shared_v4(S.x[s] + 2 * kAChunk + rr2 * 16, lo[0], lo[1], lo[2], lo[3]);
+                            }
+                        }
+                    }
+                    fence_proxy_async_smem();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&S.x_full[s]);
+#pragma unroll
+                    for (int rr = 0; rr < 2; ++rr) { cur[rr][0] = nxt[rr][0]; cur[rr][1] = nxt[rr][1]; }
+                }
+            });
+        }
+    } else {
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kX3EpiRegs));
+        // ================= epilogue: both layers of (quarter q, unit group g) ====================================
+        const int q = warp & 3, g = warp >> 2;
+        int lane;                    // read again: a value kept from the setup would be spilled across setmaxnreg
+        asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane));
+        uint32_t k1 = 0;
+        for_each_tile([&](const int nq, const int R, const int64_t b0, const int n0) {
+            if (seq_init) {
+                if (R == 1) x3_seq_init<1>(S, q, g, lane, nq, n0, b0, B, h_init);
+                else if (R == 2) x3_seq_init<2>(S, q, g, lane, nq, n0, b0, B, h_init);
+                else x3_seq_init<4>(S, q, g, lane, nq, n0, b0, B, h_init);
+                fence_proxy_async_smem();
+                x3_cta_sync();     // the previous tile is complete (barrier at its end): h0 / h1 are free
+            }
             if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
             else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
             else x3_epilogue_tile<4, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
-        }
-        __syncthreads();       // tile done: every MMA has completed; the z exchange in h0 has been consumed
-        q0 += nq;
+        });
     }
 
     tc_fence_before();
     __syncthreads();
-    if (warp == kTmaWarp) {
+    if (warp == kTmemWarp) {
         tc_fence_after();
         tmem_free_all(tmem);
     }
@@ -630,7 +718,7 @@ extern "C" int na_decoder_infer_x3_ex(const float* x, const void* packed, const 
     {                                                                                                                                \
         cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, EXV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return fail((int)e, "na_decoder_infer_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e));    \
-        tc::decoder_infer_x3_kernel<NRV, EXV><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                                    \
+        tc::decoder_infer_x3_kernel<NRV, EXV><<<grid, tc::kX3InferThreads, smem, as_stream(stream)>>>(                                    \
             x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, \
             (int)T, B, (int)NC, nquarters, scores_tm, pooled, embedding, nullptr, nullptr, nullptr, nullptr, nullptr);               \
     }
@@ -673,7 +761,7 @@ extern "C" int na_decoder_lstm_x3(const float* x, const void* packed, const floa
     {                                                                                                                                \
         cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return fail((int)e, "na_decoder_lstm_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e));     \
-        tc::decoder_infer_x3_kernel<NRV, false, true><<<grid, tc::kX3Threads, smem, as_stream(stream)>>>(                            \
+        tc::decoder_infer_x3_kernel<NRV, false, true><<<grid, tc::kX3InferThreads, smem, as_stream(stream)>>>(                            \
             x, reinterpret_cast<const unsigned char*>(packed), nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,  \
             nullptr, nullptr, (int)T, B, 1, nquarters, nullptr, nullptr, nullptr, h_init, c_init, out, h_n, c_n);                     \
     }
