@@ -237,28 +237,58 @@ class EEG_LSTM(nn.Module):
         ps = self.lstm.layer(0) + self.lstm.layer(1)
         return self._cached_pack("tc", ps, lambda: ops.decoder_pack_bf16(ps))
 
+    def _tier(self, x: torch.Tensor, train: bool) -> str:
+        """The kernel tier that runs ``x``: "tc" (16-bit tensor cores, flagship shape), "wide" (16-bit tensor cores,
+        streamed weights), "x3" (fp32-accurate tensor cores, flagship shape) or "ffma" (FFMA / generic kernels, any
+        shape).  The 16-bit tier is chosen by ``compute_dtype``, a bf16 ``x`` or a .bfloat16() module.  ``train``:
+        ``forward``'s autograd path, where the tensor-core tiers give no d/dx and x3 has its own switch
+        (``ops.EXACT_TC_TRAIN``) and also takes fp16 / bf16 ``x``; otherwise the eval path of ``decode``."""
+        half = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
+                or self.attn.weight.dtype == torch.bfloat16)
+        if half and not (train and x.requires_grad):
+            if self.tc_supported():
+                return "tc"
+            if self.tc_wide_supported():
+                return "wide"
+        if train:
+            if (ops.EXACT_TC_TRAIN and not half and self.tc_supported() and not x.requires_grad
+                    and x.dtype in (torch.float32, torch.float16, torch.bfloat16)):
+                return "x3"
+        elif ops.EXACT_TC and not half and self.tc_supported() and x.dtype == torch.float32 and x.shape[0] > 0:
+            return "x3"
+        return "ffma"
+
+    def _decode(self, x: torch.Tensor, ex: bool, want_probs: bool = True):
+        """``decode`` (``ex`` False: (logits, probs)) and ``decode_intermediates`` (``ex`` True: the five fields of
+        ``DecoderOutputs``, the op families' ``*_intermediates``) on the tier ``_tier`` picks.  The two families take
+        the same arguments except ``want_probs``, which only the plain ones have."""
+        probs = () if ex else (want_probs,)
+        z = self.zscore_input
+        tier = self._tier(x, train=False)
+        with torch.no_grad():
+            if tier == "tc":
+                op = ops.decoder_infer_tc_intermediates if ex else ops.decoder_infer_tc
+                return op(x, self._packed_tc(), self._head_params(), *probs, z)
+            if tier == "wide":
+                op = ops.decoder_infer_wide_intermediates if ex else ops.decoder_infer_wide
+                return op(x, self._packed_tc_wide(), self._head_params(), self.lstm.hidden_size, *probs, z)
+            if tier == "x3":
+                # exact tier, flagship shape: fp32-accurate tensor-core kernel (fp16 hi/lo operand split); the optional
+                # z-score stage is one K1 pass that leaves the windows batch-first in fp32
+                if z:
+                    x = ops.window_zscore(x, x.shape[1], x.shape[1], True, False, ops.NA_F32)
+                op = ops.decoder_infer_x3_intermediates if ex else ops.decoder_infer_x3
+                return op(x.contiguous(), self._packed_x3(), self._head_params(), *probs)
+            L = self.lstm.num_layers
+            op = ops.decoder_infer_intermediates if ex else ops.decoder_infer
+            return op(x, [self.lstm.layer(l) for l in range(L)], [ops._f32c(t) for t in self._head_params()], *probs,
+                      z, [self._packed(l) for l in range(L)])
+
     def decode(self, x: torch.Tensor, want_probs: bool = True):
         """Eval-mode forward without autograd: x [B,T,C] on CUDA -> (logits fp32 [B,K], probs fp32 [B,K] or
         empty).  Picks the tier from ``compute_dtype`` / the dtype of ``x`` / the parameters."""
         ops._require_cuda(x)
-        bf16 = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
-                or self.attn.weight.dtype == torch.bfloat16)
-        with torch.no_grad():
-            if bf16 and self.tc_supported():
-                return ops.decoder_infer_tc(x, self._packed_tc(), self._head_params(), want_probs, self.zscore_input)
-            if bf16 and self.tc_wide_supported():
-                return ops.decoder_infer_wide(x, self._packed_tc_wide(), self._head_params(), self.lstm.hidden_size,
-                                              want_probs, self.zscore_input)
-            if (ops.EXACT_TC and not bf16 and self.tc_supported() and x.dtype == torch.float32 and x.shape[0] > 0):
-                # exact tier, flagship shape: fp32-accurate tensor-core kernel (fp16 hi/lo operand split); the optional
-                # z-score stage is one K1 pass that leaves the windows batch-first in fp32
-                if self.zscore_input:
-                    x = ops.window_zscore(x, x.shape[1], x.shape[1], True, False, ops.NA_F32)
-                return ops.decoder_infer_x3(x.contiguous(), self._packed_x3(), self._head_params(), want_probs)
-            L = self.lstm.num_layers
-            return ops.decoder_infer(x, [self.lstm.layer(l) for l in range(L)],
-                                     [ops._f32c(t) for t in self._head_params()], want_probs, self.zscore_input,
-                                     [self._packed(l) for l in range(L)])
+        return self._decode(x, False, want_probs)
 
     def decode_intermediates(self, x: torch.Tensor) -> DecoderOutputs:
         """Eval-mode forward without autograd that also returns the attention weights over time, the pooled vector and
@@ -275,24 +305,7 @@ class EEG_LSTM(nn.Module):
             H, K = self.lstm.hidden_size, self.fc[3].out_features
             e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=x.device)
             return DecoderOutputs(e(0, K), e(0, K), e(0, T), e(0, H), e(0, H))
-        bf16 = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
-                or self.attn.weight.dtype == torch.bfloat16)
-        with torch.no_grad():
-            if bf16 and self.tc_supported():
-                return DecoderOutputs(*ops.decoder_infer_tc_intermediates(x, self._packed_tc(), self._head_params(),
-                                                                          self.zscore_input))
-            if bf16 and self.tc_wide_supported():
-                return DecoderOutputs(*ops.decoder_infer_wide_intermediates(x, self._packed_tc_wide(), self._head_params(),
-                                                                            self.lstm.hidden_size, self.zscore_input))
-            if ops.EXACT_TC and not bf16 and self.tc_supported() and x.dtype == torch.float32:
-                if self.zscore_input:
-                    x = ops.window_zscore(x, x.shape[1], x.shape[1], True, False, ops.NA_F32)
-                return DecoderOutputs(*ops.decoder_infer_x3_intermediates(x.contiguous(), self._packed_x3(),
-                                                                          self._head_params()))
-            L = self.lstm.num_layers
-            return DecoderOutputs(*ops.decoder_infer_intermediates(
-                x, [self.lstm.layer(l) for l in range(L)], [ops._f32c(t) for t in self._head_params()],
-                self.zscore_input, [self._packed(l) for l in range(L)]))
+        return DecoderOutputs(*self._decode(x, True))
 
     def inject_noise(self, drop1: Optional[torch.Tensor] = None, rrelu_slope: Optional[torch.Tensor] = None,
                      drop2: Optional[torch.Tensor] = None) -> None:
@@ -353,10 +366,10 @@ class EEG_LSTM(nn.Module):
             logits, _ = self.decode(x, want_probs=False)
         else:
             d1 = rr = d2 = None
-            bf16 = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
-                    or self.attn.weight.dtype == torch.bfloat16)
-            if bf16 and self.tc_supported() and not x.requires_grad:
-                # tensor-core tier: tcgen05 forward + fused BPTT (bf16 operands, 2e-2 contract)
+            tier = self._tier(x, train=True)
+            if tier in ("tc", "x3"):
+                # flagship shape on the tensor cores: tcgen05 forward + fused BPTT; tc with bf16 operands (2e-2 contract),
+                # x3 fp32-accurate (operands split into fp16 hi + lo)
                 drop1 = None
                 if self.training:
                     injected = (self._injected_noise or {}).get("drop1") is not None
@@ -367,9 +380,9 @@ class EEG_LSTM(nn.Module):
                         # no mask tensor: the kernels generate (and the backward re-generates) the keep-bits from
                         # a counter-based hash; the seed comes from torch's CPU generator (torch.manual_seed)
                         drop1 = (int(torch.randint(0, 2 ** 62, (1,)).item()), int(round((1.0 - self.dropout_p) * 65536)))
-                logits = ops.decoder_train_forward_tc(x, lstm_params, head, self.dropout_p, self.zscore_input,
-                                                      drop1, rr, d2)
-            elif bf16 and self.tc_wide_supported() and not x.requires_grad:
+                train_forward = ops.decoder_train_forward_tc if tier == "tc" else ops.decoder_train_forward_x3
+                logits = train_forward(x, lstm_params, head, self.dropout_p, self.zscore_input, drop1, rr, d2)
+            elif tier == "wide":
                 # wide shapes (BASELINE configs[4]) on the 16-bit tier: streamed-weight recurrence kernels + cuBLAS for the
                 # time-parallel GEMMs; dropout / RReLU noise as tensors (time-major padded to 128)
                 drop1 = None
@@ -377,19 +390,6 @@ class EEG_LSTM(nn.Module):
                     d1, rr, d2 = self._draw_noise(B, T, x.device, ops.TC_TILE)
                     drop1 = d1[0] if d1 is not None else None
                 logits = ops.decoder_train_forward_wide_tc(x, lstm_params, head, self.dropout_p, self.zscore_input, drop1, rr, d2)
-            elif (ops.EXACT_TC_TRAIN and not bf16 and self.tc_supported() and not x.requires_grad
-                  and x.dtype in (torch.float32, torch.float16, torch.bfloat16)):
-                # exact tier, flagship shape: fp32-accurate tensor-core training (operands split into fp16 hi + lo)
-                drop1 = None
-                if self.training:
-                    injected = (self._injected_noise or {}).get("drop1") is not None
-                    d1, rr, d2 = self._draw_noise(B, T, x.device, ops.TC_TILE, torch.uint8, skip_drop1=not injected)
-                    if injected:
-                        drop1 = d1[0]
-                    elif self.lstm.dropout > 0.0:
-                        drop1 = (int(torch.randint(0, 2 ** 62, (1,)).item()), int(round((1.0 - self.dropout_p) * 65536)))
-                logits = ops.decoder_train_forward_x3(x, lstm_params, head, self.dropout_p, self.zscore_input,
-                                                      drop1, rr, d2)
             else:
                 if self.training:
                     d1, rr, d2 = self._draw_noise(B, T, x.device)

@@ -355,16 +355,63 @@ def _(h, B, params, rrelu_slope, drop_mask, drop_scale, want_probs, save):
             h.new_empty((B, 2) if save else (0,)), h.new_empty((B, H) if save else (0,)))
 
 
-def _ex_outputs(B: int, T: int, H: int, dev) -> Tuple[Tensor, Tensor, Tensor]:
-    """Intermediates outputs of the *_ex entry points: scores (time-major [T,B]), pooled [B,H], embedding [B,H]."""
-    return (torch.empty((T, B), dtype=torch.float32, device=dev), torch.empty((B, H), dtype=torch.float32, device=dev),
-            torch.empty((B, H), dtype=torch.float32, device=dev))
-
-
 def _ex_fake(like: Tensor, B: int, T: int, H: int, NC: int):
     f = torch.float32
     return (like.new_empty((B, NC), dtype=f), like.new_empty((B, NC), dtype=f), like.new_empty((T, B), dtype=f),
             like.new_empty((B, H), dtype=f), like.new_empty((B, H), dtype=f))
+
+
+def _infer_fake(like: Tensor, B: int, NC: int, want_probs: bool):
+    f = torch.float32
+    return like.new_empty((B, NC), dtype=f), like.new_empty((B, NC) if want_probs else (0,), dtype=f)
+
+
+def _infer_outputs(B: int, NC: int, dev, want_probs: bool = True, ex: Optional[Tuple[int, int]] = None) -> List[Tensor]:
+    """Outputs of an eval kernel: logits [B,NC] and probs [B,NC] (empty unless ``want_probs``), then with ``ex`` = (T, H)
+    the intermediates of its *_ex entry point: scores (time-major [T,B]), pooled [B,H], embedding [B,H]."""
+    shapes = [(B, NC), (B, NC) if want_probs else (0,)] + ([(ex[0], B), (B, ex[1]), (B, ex[1])] if ex is not None else [])
+    return [torch.empty(s, dtype=torch.float32, device=dev) for s in shapes]
+
+
+def _out_ptrs(out: Sequence[Tensor], want_probs: bool) -> List[Optional[int]]:
+    return [out[0].data_ptr(), _ptr(out[1]) if want_probs else None] + [t.data_ptr() for t in out[2:]]
+
+
+def _infer_x32(op: str, x: Tensor, packed: Tensor, head: Sequence[Tensor], want_probs: bool, ex: bool):
+    """Body of the eval ops that read the batch-first fp32 windows x [B,T,8] (entry point ``na_<op>``)."""
+    _require_cuda(x, packed, *head)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
+        raise RuntimeError(f"{op}: x must be contiguous fp32 [B, T, 8]")
+    head = [_f32c(t) for t in head]
+    NC = head[6].shape[0]
+    out = _infer_outputs(B, NC, x.device, want_probs, (T, 48) if ex else None)
+    _lib.call("na_" + op, x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head], *_out_ptrs(out, want_probs),
+              T, B, NC, _stream())
+    return tuple(out)
+
+
+def _infer_tmp(op: str, x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor], B: int, H: Optional[int], want_probs: bool,
+               ex: bool):
+    """Body of the eval ops that read the time-major fp16 windows x_tmp [T,Bp,8] (entry point ``na_<op>``).  ``H``: the
+    wide kernel's hidden size (it also takes its workspace), None for the flagship kernel."""
+    _require_cuda(x_tmp, packed, *head)
+    T, Bp, C = x_tmp.shape
+    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
+        raise RuntimeError(f"{op}: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
+    head = [_f32c(t) for t in head]
+    NC = head[-2].shape[0]                                       # fc.3.weight (the wide kernel takes no attention vector)
+    out = _infer_outputs(B, NC, x_tmp.device, want_probs, (T, H or 48) if ex else None)
+    state = [] if H is None else [_wide_state(H, x_tmp.device).data_ptr()]
+    _lib.call("na_" + op, x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head], *state,
+              *_out_ptrs(out, want_probs), T, B, Bp, *([] if H is None else [H]), NC, _stream())
+    return tuple(out)
+
+
+def _with_attention(out) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """(logits, probs, scores [T,B], pooled, embedding) of a *_ex op -> the same with the attention weights [B,T]."""
+    lg, pr, sc, zp, emb = out
+    return lg, pr, attention_softmax(sc), zp, emb
 
 
 @torch.library.custom_op("neuroalpha::head_fwd_ex", mutates_args=(), device_types="cuda")
@@ -375,10 +422,7 @@ def head_fwd_ex(h: Tensor, B: int, params: Sequence[Tensor]) -> Tuple[Tensor, Te
     _require_cuda(h, *params)
     T, Bp, H = h.shape
     NC = params[6].shape[0]
-    dev = h.device
-    logits = torch.empty((B, NC), dtype=torch.float32, device=dev)
-    probs = torch.empty((B, NC), dtype=torch.float32, device=dev)
-    scores, pooled, emb = _ex_outputs(B, T, H, dev)
+    logits, probs, scores, pooled, emb = _infer_outputs(B, NC, h.device, ex=(T, H))
     _lib.call("na_head_fwd_f32_ex", h.data_ptr(), *[p.data_ptr() for p in params], None, None, 1.0, logits.data_ptr(),
               probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), None, None, T, B, Bp, H, NC, _stream())
     return logits, probs, scores, pooled, emb
@@ -481,23 +525,12 @@ def decoder_infer_bf16(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor], B:
                        want_probs: bool) -> Tuple[Tensor, Tensor]:
     """Whole decoder forward on tcgen05 (bf16 operands, fp32 accumulate).  x_tmp: TMP bf16 [T,Bp,8]
     with Bp a multiple of 128 (window_zscore(..., time_major=True, bf16=True, pad_to=128))."""
-    _require_cuda(x_tmp, packed, *head)
-    T, Bp, C = x_tmp.shape
-    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
-        raise RuntimeError("decoder_infer_bf16: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    probs = torch.empty((B, NC) if want_probs else (0,), dtype=torch.float32, device=x_tmp.device)
-    _lib.call("na_decoder_infer_bf16", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), _ptr(probs) if want_probs else None, T, B, Bp, NC, _stream())
-    return logits, probs
+    return _infer_tmp("decoder_infer_bf16", x_tmp, packed, head, B, None, want_probs, False)
 
 
 @decoder_infer_bf16.register_fake
 def _(x_tmp, packed, head, B, want_probs):
-    NC = head[6].shape[0]
-    return x_tmp.new_empty((B, NC), dtype=torch.float32), x_tmp.new_empty((B, NC) if want_probs else (0,), dtype=torch.float32)
+    return _infer_fake(x_tmp, B, head[6].shape[0], want_probs)
 
 
 @torch.library.custom_op("neuroalpha::decoder_infer_bf16_x32", mutates_args=(), device_types="cuda")
@@ -505,23 +538,12 @@ def _(x_tmp, packed, head, B, want_probs):
 def decoder_infer_bf16_x32(x: Tensor, packed: Tensor, head: Sequence[Tensor], want_probs: bool) -> Tuple[Tensor, Tensor]:
     """Whole decoder forward on tcgen05 straight from the batch-first fp32 windows x [B,T,8] (the fp32 -> fp16
     time-major pack is fused into the kernel's producer warp)."""
-    _require_cuda(x, packed, *head)
-    B, T, C = x.shape
-    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
-        raise RuntimeError("decoder_infer_bf16_x32: x must be contiguous fp32 [B, T, 8]")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    probs = torch.empty((B, NC) if want_probs else (0,), dtype=torch.float32, device=x.device)
-    _lib.call("na_decoder_infer_bf16_x32", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), _ptr(probs) if want_probs else None, T, B, NC, _stream())
-    return logits, probs
+    return _infer_x32("decoder_infer_bf16_x32", x, packed, head, want_probs, False)
 
 
 @decoder_infer_bf16_x32.register_fake
 def _(x, packed, head, want_probs):
-    NC = head[6].shape[0]
-    return x.new_empty((x.shape[0], NC), dtype=torch.float32), x.new_empty((x.shape[0], NC) if want_probs else (0,), dtype=torch.float32)
+    return _infer_fake(x, x.shape[0], head[6].shape[0], want_probs)
 
 
 @torch.library.custom_op("neuroalpha::decoder_infer_bf16_ex", mutates_args=(), device_types="cuda")
@@ -529,18 +551,7 @@ def _(x, packed, head, want_probs):
 def decoder_infer_bf16_ex(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor],
                           B: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_bf16 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,48], embedding [B,48])."""
-    _require_cuda(x_tmp, packed, *head)
-    T, Bp, C = x_tmp.shape
-    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
-        raise RuntimeError("decoder_infer_bf16_ex: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    probs = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    scores, pooled, emb = _ex_outputs(B, T, 48, x_tmp.device)
-    _lib.call("na_decoder_infer_bf16_ex", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, Bp, NC, _stream())
-    return logits, probs, scores, pooled, emb
+    return _infer_tmp("decoder_infer_bf16_ex", x_tmp, packed, head, B, None, True, True)
 
 
 @decoder_infer_bf16_ex.register_fake
@@ -552,18 +563,7 @@ def _(x_tmp, packed, head, B):
 @_device_guard
 def decoder_infer_bf16_x32_ex(x: Tensor, packed: Tensor, head: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_bf16_x32 with its intermediates: (logits, probs, scores [T,B] time-major, pooled, embedding)."""
-    _require_cuda(x, packed, *head)
-    B, T, C = x.shape
-    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
-        raise RuntimeError("decoder_infer_bf16_x32_ex: x must be contiguous fp32 [B, T, 8]")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    probs = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    scores, pooled, emb = _ex_outputs(B, T, 48, x.device)
-    _lib.call("na_decoder_infer_bf16_x32_ex", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, NC, _stream())
-    return logits, probs, scores, pooled, emb
+    return _infer_x32("decoder_infer_bf16_x32_ex", x, packed, head, True, True)
 
 
 @decoder_infer_bf16_x32_ex.register_fake
@@ -571,21 +571,23 @@ def _(x, packed, head):
     return _ex_fake(x, x.shape[0], x.shape[1], 48, head[6].shape[0])
 
 
-def decoder_infer_tc_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor],
-                                   zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
-    """decoder_infer_tc with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48]).
-    Same input handling as decoder_infer_tc; the attention weights come from the kernel's scores by attention_softmax."""
+FUSED_INPUT = True          # decoder_infer_tc: read fp32 [B,T,8] directly (False: K1 pack + time-major kernel; A/B timing)
+
+
+def _infer_tc(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], want_probs: bool, zscore: bool, ex: bool):
+    """decoder_infer_tc (``ex`` False) and decoder_infer_tc_intermediates (``ex`` True, the *_ex kernels)."""
     _require_cuda(x)
     B, T, C = x.shape
+    head = list(head_params)
     if FUSED_INPUT and not zscore and x.dtype == torch.float32 and C == 8 and B > 0:
-        lg, pr, sc, zp, emb = decoder_infer_bf16_x32_ex(x.contiguous(), packed, list(head_params))
-    else:
-        xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
-        lg, pr, sc, zp, emb = decoder_infer_bf16_ex(xt, packed, list(head_params), B)
-    return lg, pr, attention_softmax(sc), zp, emb
-
-
-FUSED_INPUT = True          # decoder_infer_tc: read fp32 [B,T,8] directly (False: K1 pack + time-major kernel; A/B timing)
+        x = x.contiguous()
+        if ex:
+            return _with_attention(decoder_infer_bf16_x32_ex(x, packed, head))
+        return decoder_infer_bf16_x32(x, packed, head, want_probs)
+    xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
+    if ex:
+        return _with_attention(decoder_infer_bf16_ex(xt, packed, head, B))
+    return decoder_infer_bf16(xt, packed, head, B, want_probs)
 
 
 def decoder_infer_tc(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], want_probs: bool = False,
@@ -593,12 +595,14 @@ def decoder_infer_tc(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], w
     """Eval forward on the tensor-core tier.  x [B,T,8] fp32 (or bf16) -> (logits fp32, probs or empty).
     fp32 contiguous input without the z-score stage goes straight into the kernel; otherwise K1 packs the windows
     time-major in fp16 first (one read of x, one half-size write)."""
-    _require_cuda(x)
-    B, T, C = x.shape
-    if FUSED_INPUT and not zscore and x.dtype == torch.float32 and C == 8 and B > 0:
-        return decoder_infer_bf16_x32(x.contiguous(), packed, list(head_params), want_probs)
-    xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
-    return decoder_infer_bf16(xt, packed, list(head_params), B, want_probs)
+    return _infer_tc(x, packed, head_params, want_probs, zscore, False)
+
+
+def decoder_infer_tc_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor],
+                                   zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_tc with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48]).
+    Same input handling as decoder_infer_tc; the attention weights come from the kernel's scores by attention_softmax."""
+    return _infer_tc(x, packed, head_params, True, zscore, True)
 
 
 EXACT_TC = True             # exact tier, flagship shape, eval: fp16-split tcgen05 kernel (False: the FFMA kernels; A/B timing)
@@ -627,41 +631,19 @@ def _(lstm_flat):
 def decoder_infer_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], want_probs: bool) -> Tuple[Tensor, Tensor]:
     """Whole decoder forward at fp32 accuracy on tcgen05 (operands split into fp16 hi + lo, three MMAs per product),
     straight from the batch-first fp32 windows x [B,T,8]."""
-    _require_cuda(x, packed, *head)
-    B, T, C = x.shape
-    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
-        raise RuntimeError("decoder_infer_x3: x must be contiguous fp32 [B, T, 8]")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    probs = torch.empty((B, NC) if want_probs else (0,), dtype=torch.float32, device=x.device)
-    _lib.call("na_decoder_infer_x3", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), _ptr(probs) if want_probs else None, T, B, NC, _stream())
-    return logits, probs
+    return _infer_x32("decoder_infer_x3", x, packed, head, want_probs, False)
 
 
 @decoder_infer_x3.register_fake
 def _(x, packed, head, want_probs):
-    NC = head[6].shape[0]
-    return x.new_empty((x.shape[0], NC), dtype=torch.float32), x.new_empty((x.shape[0], NC) if want_probs else (0,), dtype=torch.float32)
+    return _infer_fake(x, x.shape[0], head[6].shape[0], want_probs)
 
 
 @torch.library.custom_op("neuroalpha::decoder_infer_x3_ex", mutates_args=(), device_types="cuda")
 @_device_guard
 def decoder_infer_x3_ex(x: Tensor, packed: Tensor, head: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_x3 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,48], embedding [B,48])."""
-    _require_cuda(x, packed, *head)
-    B, T, C = x.shape
-    if x.dtype != torch.float32 or C != 8 or not x.is_contiguous():
-        raise RuntimeError("decoder_infer_x3_ex: x must be contiguous fp32 [B, T, 8]")
-    head = [_f32c(t) for t in head]
-    NC = head[6].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    probs = torch.empty((B, NC), dtype=torch.float32, device=x.device)
-    scores, pooled, emb = _ex_outputs(B, T, 48, x.device)
-    _lib.call("na_decoder_infer_x3_ex", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(), T, B, NC, _stream())
-    return logits, probs, scores, pooled, emb
+    return _infer_x32("decoder_infer_x3_ex", x, packed, head, True, True)
 
 
 @decoder_infer_x3_ex.register_fake
@@ -706,8 +688,7 @@ def _(x, packed, h0, c0):
 def decoder_infer_x3_intermediates(x: Tensor, packed: Tensor,
                                    head_params: Sequence[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_x3 with the intermediates: (logits, probs, attention [B,T], pooled [B,48], embedding [B,48])."""
-    lg, pr, sc, zp, emb = decoder_infer_x3_ex(x, packed, list(head_params))
-    return lg, pr, attention_softmax(sc), zp, emb
+    return _with_attention(decoder_infer_x3_ex(x, packed, list(head_params)))
 
 
 WIDE_HIDDEN = (96, 144, 192)          # hidden sizes of the streamed-weight tensor-core kernel (na_decoder_wide.cu)
@@ -756,24 +737,12 @@ def decoder_infer_wide_bf16(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor
                             want_probs: bool) -> Tuple[Tensor, Tensor]:
     """Whole wide-decoder forward on tcgen05 with streamed weights.  x_tmp as for decoder_infer_bf16;
     head = [ln.w, ln.b, fc0.w, fc0.b, fc3.w, fc3.b] (the attention vector is part of `packed`)."""
-    _require_cuda(x_tmp, packed, *head)
-    T, Bp, C = x_tmp.shape
-    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
-        raise RuntimeError("decoder_infer_wide_bf16: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
-    head = [_f32c(t) for t in head]
-    NC = head[4].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    probs = torch.empty((B, NC) if want_probs else (0,), dtype=torch.float32, device=x_tmp.device)
-    state = _wide_state(H, x_tmp.device)
-    _lib.call("na_decoder_infer_wide_bf16", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              state.data_ptr(), logits.data_ptr(), _ptr(probs) if want_probs else None, T, B, Bp, H, NC, _stream())
-    return logits, probs
+    return _infer_tmp("decoder_infer_wide_bf16", x_tmp, packed, head, B, H, want_probs, False)
 
 
 @decoder_infer_wide_bf16.register_fake
 def _(x_tmp, packed, head, B, H, want_probs):
-    NC = head[4].shape[0]
-    return x_tmp.new_empty((B, NC), dtype=torch.float32), x_tmp.new_empty((B, NC) if want_probs else (0,), dtype=torch.float32)
+    return _infer_fake(x_tmp, B, head[4].shape[0], want_probs)
 
 
 @torch.library.custom_op("neuroalpha::decoder_infer_wide_bf16_ex", mutates_args=(), device_types="cuda")
@@ -781,20 +750,7 @@ def _(x_tmp, packed, head, B, H, want_probs):
 def decoder_infer_wide_bf16_ex(x_tmp: Tensor, packed: Tensor, head: Sequence[Tensor], B: int,
                                H: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer_wide_bf16 with its intermediates: (logits, probs, scores [T,B] time-major, pooled [B,H], embedding [B,H])."""
-    _require_cuda(x_tmp, packed, *head)
-    T, Bp, C = x_tmp.shape
-    if x_tmp.dtype != TC_VALUE_DTYPE or C != 8 or Bp % TC_TILE:
-        raise RuntimeError("decoder_infer_wide_bf16_ex: x_tmp must be fp16 [T, Bp % 128 == 0, 8] (the tier's value format)")
-    head = [_f32c(t) for t in head]
-    NC = head[4].shape[0]
-    logits = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    probs = torch.empty((B, NC), dtype=torch.float32, device=x_tmp.device)
-    scores, pooled, emb = _ex_outputs(B, T, H, x_tmp.device)
-    state = _wide_state(H, x_tmp.device)
-    _lib.call("na_decoder_infer_wide_bf16_ex", x_tmp.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              state.data_ptr(), logits.data_ptr(), probs.data_ptr(), scores.data_ptr(), pooled.data_ptr(), emb.data_ptr(),
-              T, B, Bp, H, NC, _stream())
-    return logits, probs, scores, pooled, emb
+    return _infer_tmp("decoder_infer_wide_bf16_ex", x_tmp, packed, head, B, H, True, True)
 
 
 @decoder_infer_wide_bf16_ex.register_fake
@@ -802,26 +758,30 @@ def _(x_tmp, packed, head, B, H):
     return _ex_fake(x_tmp, B, x_tmp.shape[0], H, head[4].shape[0])
 
 
-def decoder_infer_wide_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int,
-                                     zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
-    """decoder_infer_wide with the intermediates: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H])."""
-    _require_cuda(x)
-    B, T, C = x.shape
-    xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
-    lg, pr, sc, zp, emb = decoder_infer_wide_bf16_ex(xt, packed, list(head_params[2:]), B, H)
-    return lg, pr, attention_softmax(sc), zp, emb
-
-
-def decoder_infer_wide(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int, want_probs: bool = False,
-                       zscore: bool = False) -> Tuple[Tensor, Tensor]:
-    """Eval forward of a wide decoder on the tensor-core tier.  head_params in EEG_LSTM._head_params() order."""
+def _infer_wide(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int, want_probs: bool, zscore: bool,
+                ex: bool):
+    """decoder_infer_wide (``ex`` False) and decoder_infer_wide_intermediates (``ex`` True, the *_ex kernel)."""
     _require_cuda(x)
     B, T, C = x.shape
     # (Fusing the input pack into the wide kernel, as in decoder_infer_tc, was built and measured: bit-identical but slower --
     # 59.1 vs 56.0 ms at H = 192, T = 2500 -- because the producer warp's weight stream is that kernel's critical path; and the
     # extra code cost the default path 7 % through the instruction cache, so it was removed again.)
     xt = window_zscore(x, T, T, zscore, True, NA_F16, TC_TILE)
+    if ex:
+        return _with_attention(decoder_infer_wide_bf16_ex(xt, packed, list(head_params[2:]), B, H))
     return decoder_infer_wide_bf16(xt, packed, list(head_params[2:]), B, H, want_probs)
+
+
+def decoder_infer_wide(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int, want_probs: bool = False,
+                       zscore: bool = False) -> Tuple[Tensor, Tensor]:
+    """Eval forward of a wide decoder on the tensor-core tier.  head_params in EEG_LSTM._head_params() order."""
+    return _infer_wide(x, packed, head_params, H, want_probs, zscore, False)
+
+
+def decoder_infer_wide_intermediates(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], H: int,
+                                     zscore: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_infer_wide with the intermediates: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H])."""
+    return _infer_wide(x, packed, head_params, H, True, zscore, True)
 
 
 # ------------------------------------------------------------------------------------------
@@ -834,18 +794,26 @@ def split_head_grads(dparams: Tensor, H: int, NC: int) -> List[Tensor]:
     return [p.reshape(s) for p, s in zip(dparams.split(sizes), shapes)]
 
 
-def decoder_infer(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
-                  want_probs: bool = False, zscore: bool = False,
-                  packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None) -> Tuple[Tensor, Tensor]:
-    """Eval-mode forward, nothing saved.  x [B,T,C] -> (logits [B,NC], probs or empty)."""
+def _infer_ffma(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor], want_probs: bool,
+                zscore: bool, packed: Optional[Sequence[Tuple[Tensor, Tensor]]], ex: bool):
+    """decoder_infer (``ex`` False) and decoder_infer_intermediates (``ex`` True: the same LSTM launches, head_fwd_ex)."""
     _require_cuda(x)
     B, T, C = x.shape
     cur = window_zscore(x, T, T, zscore, True, False)
     for l, (w_ih, w_hh, b_ih, b_hh) in enumerate(lstm_params):
         wt, bias = packed[l] if packed is not None else pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
         cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
+    if ex:
+        return _with_attention(head_fwd_ex(cur, B, list(head_params)))
     logits, probs, _, _ = head_fwd(cur, B, list(head_params), None, None, 1.0, want_probs, False)
     return logits, probs
+
+
+def decoder_infer(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
+                  want_probs: bool = False, zscore: bool = False,
+                  packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None) -> Tuple[Tensor, Tensor]:
+    """Eval-mode forward, nothing saved.  x [B,T,C] -> (logits [B,NC], probs or empty)."""
+    return _infer_ffma(x, lstm_params, head_params, want_probs, zscore, packed, False)
 
 
 def decoder_infer_intermediates(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
@@ -853,14 +821,26 @@ def decoder_infer_intermediates(x: Tensor, lstm_params: Sequence[Sequence[Tensor
                                 ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """decoder_infer with the intermediates of the head: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H]).
     The LSTM layers are the same launches; the head kernel writes the scores, the pooled vector and the LayerNorm output."""
-    _require_cuda(x)
-    B, T, C = x.shape
-    cur = window_zscore(x, T, T, zscore, True, False)
-    for l, (w_ih, w_hh, b_ih, b_hh) in enumerate(lstm_params):
-        wt, bias = packed[l] if packed is not None else pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
-        cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
-    lg, pr, sc, zp, emb = head_fwd_ex(cur, B, list(head_params))
-    return lg, pr, attention_softmax(sc), zp, emb
+    return _infer_ffma(x, lstm_params, head_params, True, zscore, packed, True)
+
+
+def _save(ctx, tensors: Sequence[Tensor], optional: Sequence[Optional[Tensor]]) -> None:
+    """ctx.save_for_backward of ``tensors`` and of the ``optional`` ones that are not None; ``_saved`` restores both."""
+    ctx.optional_given = [t is not None for t in optional]
+    ctx.save_for_backward(*tensors, *[t for t in optional if t is not None])
+
+
+def _saved(ctx) -> Tuple[List[Tensor], List[Optional[Tensor]]]:
+    """(tensors, optional) as given to ``_save``, with None in place of each optional tensor that was not given."""
+    sv = list(ctx.saved_tensors)
+    n = len(sv) - sum(ctx.optional_given)
+    given = iter(sv[n:])
+    return sv[:n], [next(given) if g else None for g in ctx.optional_given]
+
+
+def _cast_grads(grads: Sequence[Tensor], dtypes: Sequence[torch.dtype]) -> List[Tensor]:
+    """Each gradient in the dtype of its parameter (the kernels produce fp32; .bfloat16() modules want bf16)."""
+    return [g.to(dt) if g.dtype != dt else g for g, dt in zip(grads, dtypes)]
 
 
 class DecoderFunction(torch.autograd.Function):
@@ -885,33 +865,19 @@ class DecoderFunction(torch.autograd.Function):
             saved += [layer_in, h, c, gates, w_ih, w_hh]
             layer_in = h_drop if mask is not None else h
         logits, _, stats, zpool = head_fwd(layer_in, B, head, rrelu_slope, drop2_mask, scale, False, True)
-        ctx.save_for_backward(*saved, stats, zpool, *head,
-                              *([m for m in drop1_masks] if drop1_masks is not None else []),
-                              *([rrelu_slope] if rrelu_slope is not None else []),
-                              *([drop2_mask] if drop2_mask is not None else []))
-        ctx.meta = (num_layers, scale, B, x.shape, zscore, drop1_masks is not None,
-                    rrelu_slope is not None, drop2_mask is not None)
+        _save(ctx, [*saved, stats, zpool, *head], [*(drop1_masks or ()), rrelu_slope, drop2_mask])
+        ctx.meta = (num_layers, scale, B, x.shape, zscore)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        num_layers, scale, B, xshape, zscore, has_d1, has_rr, has_d2 = ctx.meta
-        sv = list(ctx.saved_tensors)
+        num_layers, scale, B, xshape, zscore = ctx.meta
+        sv, (*d1, rr, d2) = _saved(ctx)
         layers = [sv[6 * l:6 * l + 6] for l in range(num_layers)]
-        pos = 6 * num_layers
-        stats, zpool = sv[pos], sv[pos + 1]
-        head = sv[pos + 2:pos + 10]
-        pos += 10
-        d1 = sv[pos:pos + num_layers - 1] if has_d1 else None
-        pos += (num_layers - 1) if has_d1 else 0
-        rr = sv[pos] if has_rr else None
-        pos += 1 if has_rr else 0
-        d2 = sv[pos] if has_d2 else None
+        stats, zpool = sv[6 * num_layers:6 * num_layers + 2]
+        head = sv[6 * num_layers + 2:]
 
-        top_in = layers[-1][1]
-        if has_d1 and num_layers > 1:
-            # the head consumed the raw h of the last layer (dropout is never applied after it)
-            pass
+        top_in = layers[-1][1]          # the head consumed the raw h of the last layer (dropout is never applied after it)
         H = top_in.shape[2]
         NC = dlogits.shape[1]
         dh, dparams = head_bwd(dlogits.contiguous(), top_in, stats, zpool, head, rr, d2, scale)
@@ -922,7 +888,7 @@ class DecoderFunction(torch.autograd.Function):
         dx = None
         for l in range(num_layers - 1, -1, -1):
             layer_in, h, c, gates, w_ih, w_hh = layers[l]
-            in_mask = d1[l - 1] if (has_d1 and l > 0) else None
+            in_mask = d1[l - 1] if (d1 and l > 0) else None
             need_din = l > 0 or need_dx
             dgates, din = lstm_layer_bwd(dh, gates, c, w_ih, w_hh, in_mask, scale, need_din)
             dw_ih, dw_hh, db = lstm_layer_wgrad(dgates, layer_in, h)
@@ -932,8 +898,7 @@ class DecoderFunction(torch.autograd.Function):
             if zscore:
                 raise RuntimeError("gradient w.r.t. x through the z-score front stage is not implemented")
             dx = dh[:, :B].permute(1, 0, 2).contiguous().reshape(xshape)
-        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip([*lstm_grads, *head_grads], ctx.param_dtypes)]
-        return (dx, None, None, None, None, None, None, *grads)
+        return (dx, None, None, None, None, None, None, *_cast_grads([*lstm_grads, *head_grads], ctx.param_dtypes))
 
 
 class LSTMSequenceFunction(torch.autograd.Function):
@@ -974,19 +939,15 @@ class LSTMSequenceFunction(torch.autograd.Function):
             h_n.append(h[T - 1, :B])
             c_n.append(c[T - 1, :B])
             layer_in = h_drop if mask is not None else h
-        ctx.save_for_backward(*saved, *([h0p, c0p] if h0p is not None else []), *(masks or []))
-        ctx.meta = (L, scale, B, tuple(x.shape), h0p is not None, masks is not None)
+        _save(ctx, saved, [h0p, c0p, *(masks or ())])
+        ctx.meta = (L, scale, B, tuple(x.shape))
         return h[:, :B].permute(1, 0, 2).contiguous(), torch.stack(h_n), torch.stack(c_n)
 
     @staticmethod
     def backward(ctx, dout, dh_n, dc_n):
-        L, scale, B, xshape, has_hx, has_masks = ctx.meta
-        sv = list(ctx.saved_tensors)
+        L, scale, B, xshape = ctx.meta
+        sv, (h0p, c0p, *masks) = _saved(ctx)
         layers = [sv[6 * l:6 * l + 6] for l in range(L)]
-        pos = 6 * L
-        h0p, c0p = (sv[pos], sv[pos + 1]) if has_hx else (None, None)
-        pos += 2 if has_hx else 0
-        masks = sv[pos:pos + L - 1] if has_masks else None
         T, Bp, H = layers[-1][1].shape
 
         def rows(t):
@@ -997,12 +958,12 @@ class LSTMSequenceFunction(torch.autograd.Function):
         dh = torch.zeros((T, Bp, H), dtype=torch.float32, device=dout.device)
         dh[:, :B] = dout.permute(1, 0, 2)                    # the top layer's h is the output
         need_dx = ctx.needs_input_grad[0]
-        need_dhx = has_hx and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
+        need_dhx = h0p is not None and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
         lstm_grads: List[Tensor] = [None] * (4 * L)
         dh0, dc0 = [None] * L, [None] * L
         for l in range(L - 1, -1, -1):
             layer_in, h, c, gates, w_ih, w_hh = layers[l]
-            in_mask = masks[l - 1] if (has_masks and l > 0) else None
+            in_mask = masks[l - 1] if (masks and l > 0) else None
             need_din = l > 0 or need_dx
             dgates, din, dh0[l], dc0[l] = lstm_layer_bwd_hx(
                 dh, gates, c, w_ih, w_hh, in_mask, scale, need_din, None if c0p is None else c0p[l],
@@ -1015,8 +976,7 @@ class LSTMSequenceFunction(torch.autograd.Function):
         if need_dhx:
             dh0_out = torch.stack([g[:B] for g in dh0]).to(ctx.hx_dtypes[0])
             dc0_out = torch.stack([g[:B] for g in dc0]).to(ctx.hx_dtypes[1])
-        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip(lstm_grads, ctx.param_dtypes)]
-        return (dx, dh0_out, dc0_out, None, None, *grads)
+        return (dx, dh0_out, dc0_out, None, None, *_cast_grads(lstm_grads, ctx.param_dtypes))
 
 
 def decoder_train_forward(x: Tensor, lstm_params, head_params, p: float, zscore: bool = False,
@@ -1201,6 +1161,50 @@ def _sm_count(device) -> int:
     return _SM_COUNT[idx]
 
 
+def _drop1_args(drop1, scale: float) -> Tuple[Optional[Tensor], int, int, float]:
+    """``drop1`` of DecoderFunctionTC / X3 -> (mask, seed, thresh16, scale1) of the layer-0 training kernels: None (no
+    inter-layer dropout), a u8 keep-mask (scaled like the head dropout), or ``(seed, thresh16)`` of the in-kernel
+    counter-based generator."""
+    if isinstance(drop1, tuple):
+        seed, thresh16 = int(drop1[0]), int(drop1[1])
+        return None, seed, thresh16, 65536.0 / thresh16 if thresh16 > 0 else 0.0   # exactly unbiased for the quantised keep-rate
+    if drop1 is not None:
+        return drop1, 0, 65536, scale
+    return None, 0, 65536, 1.0
+
+
+def _half_stride(B: int, device, half_tiles: bool) -> int:
+    """``half_stride`` of the flagship training kernels: 0 for full tiles, else the padded batch for half tiles (64 windows
+    per 128-row tile, the two row copies split the hidden units).  Half tiles are used (when ``half_tiles``, the tier's
+    TC_HALF_TILES / X3_HALF_TILES) if the batch would leave more than half of the SMs without a tile: a tile then costs
+    about half a step (strong scaling at small batches)."""
+    half = half_tiles and 2 * ((B + TC_TILE - 1) // TC_TILE) <= _sm_count(device)
+    return padded_batch(B, TC_TILE) if half else 0
+
+
+def _half_tile_rows(mask: Tensor, B: int, Bp: int) -> Tensor:
+    """A time-major keep-mask [T, >= B, 48] in the half-tile row layout [T, Bp, 48]: window b -> row (b // 64) * 128 + b % 64."""
+    b_idx = torch.arange(B, device=mask.device)
+    remapped = mask.new_zeros((mask.shape[0], Bp, mask.shape[2]))
+    remapped[:, (b_idx // 64) * TC_TILE + b_idx % 64] = mask[:, :B]
+    return remapped
+
+
+def _tc_backward(ctx, dlogits: Tensor, zpool: Tensor, head: Sequence[Tensor], rr: Optional[Tensor], d2: Optional[Tensor],
+                 scale: float, layers_bwd):
+    """Backward of DecoderFunctionTC / X3 around the tier's two layer backwards.  The head tail backward (fp32, unscaled)
+    gives dz, which _scale_dz scales; ``layers_bwd(dz)`` runs layer 1 (with the time loop of the head backward -- dh_t,
+    d attn -- fused) and layer 0 and returns the scaled (dW_ih0, dW_hh0, db0, dW_ih1, dW_hh1, db1, d_attn)."""
+    H, NC = 48, dlogits.shape[1]
+    dz, dparams = head_tail_bwd(dlogits.contiguous(), zpool, head, rr, d2, scale)
+    dz, _, inv_s = _scale_dz(dz)
+    dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn = layers_bwd(dz)
+    torch._foreach_mul_([dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn], inv_s)      # ONE launch unscales every scaled gradient
+    head_grads = split_head_grads(torch.cat([d_attn, dparams[H + 1:]]), H, NC)
+    grads = [dw_ih0, dw_hh0, db0, db0.clone(), dw_ih1, dw_hh1, db1, db1.clone(), *head_grads]
+    return (None, None, None, None, None, None, *_cast_grads(grads, ctx.param_dtypes))
+
+
 class DecoderFunctionTC(torch.autograd.Function):
     """Training step of the flagship decoder on the tensor-core tier: tcgen05 forward that saves h / c,
     fp32 head kernels, tcgen05 BPTT with the weight gradients accumulated in TMEM.  bf16 contract
@@ -1217,27 +1221,15 @@ class DecoderFunctionTC(torch.autograd.Function):
         B, T, C = x.shape
         lstm_flat, head = [t.detach() for t in params[:8]], [_f32c(t.detach()) for t in params[8:]]
         scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0          # head dropout (and mask-tensor mode)
-        mask, seed, thresh16, scale1 = None, 0, 65536, 1.0
-        if isinstance(drop1, tuple):
-            seed, thresh16 = int(drop1[0]), int(drop1[1])
-            scale1 = 65536.0 / thresh16 if thresh16 > 0 else 0.0   # exactly unbiased for the quantised keep-rate
-        elif drop1 is not None:
-            mask, scale1 = drop1, scale
-        # half tiles (64 windows per 128-row tile, the two row copies split the hidden units) when the batch would leave
-        # more than half of the SMs without a tile: a tile then costs about half a step (strong scaling at small batches)
-        half = TC_HALF_TILES and 2 * ((B + TC_TILE - 1) // TC_TILE) <= _sm_count(x.device)
-        half_stride = padded_batch(B, TC_TILE) if half else 0
+        mask, seed, thresh16, scale1 = _drop1_args(drop1, scale)
+        half_stride = _half_stride(B, x.device, TC_HALF_TILES)
         xin = x.detach()
-        if half:
+        if half_stride:
             nt = (B + 63) // 64
             if nt * 64 != B:
                 xin = torch.cat([xin, xin.new_zeros((nt * 64 - B, T, C))])
-            if mask is not None:                                                                 # window b -> row (b // 64) * 128 + b % 64
-                b_idx = torch.arange(B, device=x.device)
-                remapped = mask.new_zeros((T, nt * TC_TILE, mask.shape[2]))
-                remapped[:, (b_idx // 64) * TC_TILE + b_idx % 64] = mask[:, :B]
-                mask = remapped
-        if half:
+            if mask is not None:
+                mask = _half_tile_rows(mask, B, nt * TC_TILE)
             # pack first (fp16, time-major, 64 windows per tile), then mirror: rows 64..127 of every tile repeat rows 0..63 -- on
             # the 16-byte packed rows this copies a quarter of the bytes that mirroring the fp32 windows did
             xt = window_zscore(xin, T, T, zscore, True, NA_F16, 64)
@@ -1249,36 +1241,26 @@ class DecoderFunctionTC(torch.autograd.Function):
         h0, h0d, c0, h1, c1, zpool, stats = lstm2_fwd_train_bf16(xt, packed, mask, seed, thresh16, scale1, head[0], head[1], B, half_stride)
         logits, _ = head_tail_fwd(zpool, head, rrelu_slope, drop2_mask, scale, False)
         w = [_f32c(t) for t in lstm_flat]
-        opt = [t for t in (mask, rrelu_slope, drop2_mask) if t is not None]
-        ctx.save_for_backward(xt, h0, h0d, c0, h1, c1, packed, stats, zpool, w[0], w[1], w[4], w[5], *head, *opt)
-        ctx.meta = (scale, B, mask is not None, rrelu_slope is not None, drop2_mask is not None, seed, thresh16, scale1, half_stride)
+        _save(ctx, [xt, h0, h0d, c0, h1, c1, packed, stats, zpool, w[0], w[1], w[4], w[5], *head],
+              [mask, rrelu_slope, drop2_mask])
+        ctx.meta = (scale, B, seed, thresh16, scale1, half_stride)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        scale, B, has_d1, has_rr, has_d2, seed, thresh16, scale1, half_stride = ctx.meta
-        has_drop = has_d1 or thresh16 < 65536
-        sv = list(ctx.saved_tensors)
+        scale, B, seed, thresh16, scale1, half_stride = ctx.meta
+        sv, (d1, rr, d2) = _saved(ctx)
         xt, h0, h0d, c0, h1, c1, packed, stats, zpool, w_ih0, w_hh0, w_ih1, w_hh1 = sv[:13]
-        head = sv[13:21]
-        rest = sv[21:]
-        d1 = rest.pop(0) if has_d1 else None
-        rr = rest.pop(0) if has_rr else None
-        d2 = rest.pop(0) if has_d2 else None
-        H, NC = 48, dlogits.shape[1]
-        # head tail backward (fp32, unscaled) -> dz; the time loop of the head backward (dh_t, d attn) runs inside the
-        # layer-1 BPTT kernel
-        dz, dparams = head_tail_bwd(dlogits.contiguous(), zpool, head, rr, d2, scale)
-        dz, s, inv_s = _scale_dz(dz)
-        din1, dw_ih1, dw_hh1, db1, d_attn = lstm_bwd_bf16(1, h0d if has_drop else h0, h1, c1, None, packed, w_ih1, w_hh1,
-                                                          d1, seed, thresh16, scale1, [dz, stats, zpool, head[0], head[1]], B, half_stride)
-        _, dw_ih0, dw_hh0, db0, _ = lstm_bwd_bf16(0, xt, h0, c0, din1, packed, w_ih0, w_hh0, None, 0, 65536, 1.0, [], B, half_stride)
-        torch._foreach_mul_([dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn], inv_s)      # ONE launch unscales every scaled gradient
-        dparams = torch.cat([d_attn, dparams[H + 1:]])
-        head_grads = split_head_grads(dparams, H, NC)
-        grads = [dw_ih0, dw_hh0, db0, db0.clone(), dw_ih1, dw_hh1, db1, db1.clone(), *head_grads]
-        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip(grads, ctx.param_dtypes)]   # .bfloat16() modules
-        return (None, None, None, None, None, None, *grads)
+        head = sv[13:]
+        in1 = h0d if d1 is not None or thresh16 < 65536 else h0
+
+        def layers_bwd(dz):
+            din1, dw_ih1, dw_hh1, db1, d_attn = lstm_bwd_bf16(1, in1, h1, c1, None, packed, w_ih1, w_hh1, d1, seed, thresh16,
+                                                              scale1, [dz, stats, zpool, head[0], head[1]], B, half_stride)
+            _, dw_ih0, dw_hh0, db0, _ = lstm_bwd_bf16(0, xt, h0, c0, din1, packed, w_ih0, w_hh0, None, 0, 65536, 1.0, [], B,
+                                                      half_stride)
+            return dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn
+        return _tc_backward(ctx, dlogits, zpool, head, rr, d2, scale, layers_bwd)
 
 
 def decoder_train_forward_tc(x: Tensor, lstm_params, head_params, p: float, zscore: bool = False,
@@ -1419,65 +1401,43 @@ class DecoderFunctionX3(torch.autograd.Function):
         B, T, C = x.shape
         lstm_flat, head = [t.detach() for t in params[:8]], [_f32c(t.detach()) for t in params[8:]]
         scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0          # head dropout (and mask-tensor mode)
-        mask, seed, thresh16, scale1 = None, 0, 65536, 1.0
-        if isinstance(drop1, tuple):
-            seed, thresh16 = int(drop1[0]), int(drop1[1])
-            scale1 = 65536.0 / thresh16 if thresh16 > 0 else 0.0
-        elif drop1 is not None:
-            mask, scale1 = drop1, scale
+        mask, seed, thresh16, scale1 = _drop1_args(drop1, scale)
         xin = x.detach()
         if xin.dtype != torch.float32:
             xin = xin.float()
         if zscore:
             xin = window_zscore(xin, T, T, True, False, NA_F32)
-        # half tiles (see DecoderFunctionTC) when the batch would leave more than half of the SMs without a tile
-        half = X3_HALF_TILES and 2 * ((B + TC_TILE - 1) // TC_TILE) <= _sm_count(x.device)
-        half_stride = padded_batch(B, TC_TILE) if half else 0
-        Bp = ((B + 63) // 64) * TC_TILE if half else padded_batch(B, TC_TILE)
-        if half and mask is not None:                                    # window b -> row (b // 64) * 128 + b % 64
-            b_idx = torch.arange(B, device=x.device)
-            remapped = mask.new_zeros((T, Bp, mask.shape[2]))
-            remapped[:, (b_idx // 64) * TC_TILE + b_idx % 64] = mask[:, :B]
-            mask = remapped
+        half_stride = _half_stride(B, x.device, X3_HALF_TILES)
+        Bp = ((B + 63) // 64) * TC_TILE if half_stride else padded_batch(B, TC_TILE)
+        if half_stride and mask is not None:
+            mask = _half_tile_rows(mask, B, Bp)
         xs = x3_split_input(xin.contiguous(), Bp, half_stride)
         packed = decoder_pack_x3(lstm_flat)
         h0, h0d, c0, _, _ = lstm_fwd_train_x3(0, xs, packed, head[0], head[1], mask, seed, thresh16, scale1, B, half_stride)
         has_drop = mask is not None or thresh16 < 65536
         h1, _, c1, zpool, stats = lstm_fwd_train_x3(1, h0d if has_drop else h0, packed, head[0], head[1], None, 0, 65536, 1.0, B, half_stride)
         logits, _ = head_tail_fwd(zpool, head, rrelu_slope, drop2_mask, scale, False)
-        opt = [t for t in (mask, rrelu_slope, drop2_mask) if t is not None]
-        ctx.save_for_backward(xs, h0, h0d, c0, h1, c1, packed, stats, zpool, *head, *opt)
-        ctx.meta = (scale, B, mask is not None, rrelu_slope is not None, drop2_mask is not None, seed, thresh16, scale1, half_stride)
+        _save(ctx, [xs, h0, h0d, c0, h1, c1, packed, stats, zpool, *head], [mask, rrelu_slope, drop2_mask])
+        ctx.meta = (scale, B, seed, thresh16, scale1, half_stride)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        scale, B, has_d1, has_rr, has_d2, seed, thresh16, scale1, hs = ctx.meta
-        has_drop = has_d1 or thresh16 < 65536
-        sv = list(ctx.saved_tensors)
+        scale, B, seed, thresh16, scale1, hs = ctx.meta
+        sv, (d1, rr, d2) = _saved(ctx)
         xs, h0, h0d, c0, h1, c1, packed, stats, zpool = sv[:9]
-        head = sv[9:17]
-        rest = sv[17:]
-        d1 = rest.pop(0) if has_d1 else None
-        rr = rest.pop(0) if has_rr else None
-        d2 = rest.pop(0) if has_d2 else None
-        H, NC = 48, dlogits.shape[1]
-        dz, dparams = head_tail_bwd(dlogits.contiguous(), zpool, head, rr, d2, scale)      # fp32, unscaled
-        dz, s, inv_s = _scale_dz(dz)
-        in1 = h0d if has_drop else h0
-        din1, dg1, d_attn = lstm_bwd_x3(1, in1, h1, c1, None, packed, d1, seed, thresh16, scale1, [dz, stats, zpool, head[0], head[1]], B, hs)
-        dw_ih1, dw_hh1, db1 = lstm_wgrad_x3(1, dg1, in1, h1, hs)
-        del dg1
-        _, dg0, _ = lstm_bwd_x3(0, xs, h0, c0, din1, packed, None, 0, 65536, 1.0, [], B, hs)
-        dw_ih0, dw_hh0, db0 = lstm_wgrad_x3(0, dg0, xs, h0, hs)
-        del dg0
-        d_attn = d_attn.clone()                        # (a slice of the kernel's 52-float output)
-        torch._foreach_mul_([dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn], inv_s)      # ONE launch unscales every scaled gradient
-        dparams = torch.cat([d_attn, dparams[H + 1:]])
-        head_grads = split_head_grads(dparams, H, NC)
-        grads = [dw_ih0, dw_hh0, db0, db0.clone(), dw_ih1, dw_hh1, db1, db1.clone(), *head_grads]
-        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip(grads, ctx.param_dtypes)]
-        return (None, None, None, None, None, None, *grads)
+        head = sv[9:]
+        in1 = h0d if d1 is not None or thresh16 < 65536 else h0
+
+        def layers_bwd(dz):
+            din1, dg1, d_attn = lstm_bwd_x3(1, in1, h1, c1, None, packed, d1, seed, thresh16, scale1, [dz, stats, zpool, head[0], head[1]], B, hs)
+            dw_ih1, dw_hh1, db1 = lstm_wgrad_x3(1, dg1, in1, h1, hs)
+            del dg1
+            _, dg0, _ = lstm_bwd_x3(0, xs, h0, c0, din1, packed, None, 0, 65536, 1.0, [], B, hs)
+            dw_ih0, dw_hh0, db0 = lstm_wgrad_x3(0, dg0, xs, h0, hs)
+            del dg0
+            return dw_ih0, dw_hh0, db0, dw_ih1, dw_hh1, db1, d_attn.clone()     # (d_attn: a slice of the kernel's 52-float output)
+        return _tc_backward(ctx, dlogits, zpool, head, rr, d2, scale, layers_bwd)
 
 
 def decoder_train_forward_x3(x: Tensor, lstm_params, head_params, p: float, zscore: bool = False,
@@ -1621,31 +1581,23 @@ class DecoderFunctionWideTC(torch.autograd.Function):
                     layer_in = h2d
         h1 = h_rows[1].float().reshape(T, Bp, H)
         logits, _, stats, zpool = head_fwd(h1, B, head, rrelu_slope, drop2_mask, scale, False, True)
-        opt = [t for t in (mask, rrelu_slope, drop2_mask) if t is not None]
-        ctx.save_for_backward(saved[0], saved[1], saved[2], saved[3], saved[4], saved[5], saved[6], h_rows[0], h_rows[1],
-                              layer_in if mask is not None else h_rows[0], stats, zpool, *lstm, *head, *opt)
-        ctx.meta = (scale, B, T, Bp, H, mask is not None, rrelu_slope is not None, drop2_mask is not None)
+        _save(ctx, [*saved[:7], h_rows[0], h_rows[1], layer_in if mask is not None else h_rows[0], stats, zpool, *lstm, *head],
+              [mask, rrelu_slope, drop2_mask])
+        ctx.meta = (scale, B, T, Bp, H)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        scale, B, T, Bp, H, has_d1, has_rr, has_d2 = ctx.meta
-        sv = list(ctx.saved_tensors)
+        scale, B, T, Bp, H = ctx.meta
+        sv, (mask, rr, d2) = _saved(ctx)
         gates0, c0, bimg0, x2d, gates1, c1, bimg1, h0_2d, h1_2d, in1_2d, stats, zpool = sv[:12]
         lstm, head = sv[12:20], sv[20:28]
-        rest = sv[28:]
-        mask = rest.pop(0) if has_d1 else None
-        rr = rest.pop(0) if has_rr else None
-        d2 = rest.pop(0) if has_d2 else None
         dev = dlogits.device
         NC = dlogits.shape[1]
         h1 = h1_2d.float().reshape(T, Bp, H)
         dh1, dparams = head_bwd(dlogits.contiguous(), h1, stats, zpool, head, rr, d2, scale)
         del h1
-        # d(gates) are fp16: scale the gradient entering the recurrence by an exact power of two (max|dh| -> 2^6)
-        amax = dh1.detach().abs().max().clamp_min(1e-30)
-        s = torch.pow(2.0, 6.0 - torch.ceil(torch.log2(amax)))
-        inv_s = 1.0 / s
+        dh1, _, inv_s = _scale_dz(dh1)       # d(gates) are fp16: the gradient entering the recurrence, scaled (max|dh| -> 2^6)
         zeros_h = torch.zeros((Bp, H), dtype=torch.float16, device=dev)
         def layer_bwd(gates, c, bimg, dh2d, in2d, h2d, w_ih):
             dg = lstm_wide_bwd(gates, c, _to_wtl(dh2d, T, Bp, H), bimg, H)
@@ -1658,7 +1610,7 @@ class DecoderFunctionWideTC(torch.autograd.Function):
             dw_hh = _mm_f32(dgt, hprev)
             db = _mm_f32(dgt, torch.ones((dg2d.shape[0], 8), dtype=torch.float16, device=dev))[:, 0].contiguous()
             return dg2d, dw_ih, dw_hh, db
-        dg1, dw_ih1, dw_hh1, db1 = layer_bwd(gates1, c1, bimg1, (dh1 * s).reshape(T * Bp, H), in1_2d, h1_2d, lstm[4])
+        dg1, dw_ih1, dw_hh1, db1 = layer_bwd(gates1, c1, bimg1, dh1.reshape(T * Bp, H), in1_2d, h1_2d, lstm[4])
         del dh1
         din1 = _mm_f32(dg1, lstm[4].to(torch.float16))                            # [T*Bp, H] fp32 (still scaled by s)
         del dg1
@@ -1672,8 +1624,7 @@ class DecoderFunctionWideTC(torch.autograd.Function):
         head_grads = split_head_grads(dparams, H, NC)
         db0, db1 = db0 * inv_s, db1 * inv_s
         grads = [dw_ih0 * inv_s, dw_hh0 * inv_s, db0, db0.clone(), dw_ih1 * inv_s, dw_hh1 * inv_s, db1, db1.clone(), *head_grads]
-        grads = [g.to(dt) if g.dtype != dt else g for g, dt in zip(grads, ctx.param_dtypes)]
-        return (None, None, None, None, None, None, *grads)
+        return (None, None, None, None, None, None, *_cast_grads(grads, ctx.param_dtypes))
 
 
 def decoder_train_forward_wide_tc(x: Tensor, lstm_params, head_params, p: float, zscore: bool = False,
