@@ -408,6 +408,10 @@ int na_head_tail_bwd_f32(const float* dlogits, const float* zpool, const float* 
  *                         dz != NULL, the time loop of the head backward fused (dh_in must be NULL then), d_attn [52] =
  *                         d attn_w (48) | d attn_b | pad; layer 0: dh_in = din of layer 1.  zeros: >= 24,576 zero bytes.
  *                         scratch: na_train_x3_scratch_floats() floats.
+ *   na_lstm_bwd_x3_dx     na_lstm_bwd_x3 for input attributions: the same BPTT without its weight-gradient byproducts (no dg,
+ *                         no d_attn, no scratch); layer 0 also writes dx = d/dx of the layer-0 input, fp32 batch-first
+ *                         [B][T][8], rows b < B only, each multiplied by dz_inv_scale[b] ([B], the inverse of the factor
+ *                         that window's dz was scaled by).
  *   na_lstm_wgrad_x3      time-parallel dW_ih, dW_hh, db (= both biases) from dg and the saved activations; same scratch.
  * half_stride > 0 selects HALF TILES exactly as in na_lstm2_fwd_train_bf16 (64 windows per tile, rows 64..127 mirror rows
  * 0..63, B <= Bp / 2, half_stride = the dropout generator's row stride); 0 = full tiles.
@@ -424,6 +428,11 @@ int na_lstm_bwd_x3(int64_t layer, const void* act_in, const void* h, const float
                    float drop_scale, float* din, void* dg, const float* dz, const float* stats, const float* zpool,
                    const float* attn_w, const float* attn_b, int64_t B, float* d_attn, float* scratch,
                    int64_t T, int64_t Bp, int64_t half_stride, na_stream_t stream);
+int na_lstm_bwd_x3_dx(int64_t layer, const void* act_in, const void* h, const float* cstate, const float* dh_in,
+                      const void* packed_x3, const void* zeros, const unsigned char* in_mask, uint64_t seed, int64_t thresh16,
+                      float drop_scale, float* din, const float* dz, const float* stats, const float* zpool,
+                      const float* attn_w, const float* attn_b, int64_t B, float* dx, const float* dz_inv_scale,
+                      int64_t T, int64_t Bp, int64_t half_stride, na_stream_t stream);
 int na_lstm_wgrad_x3(int64_t layer, const void* dg, const void* act_in, const void* h, const void* zeros,
                      float* dw_ih, float* dw_hh, float* db, float* scratch, int64_t T, int64_t Bp, int64_t half_stride,
                      na_stream_t stream);

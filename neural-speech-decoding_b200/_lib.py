@@ -63,6 +63,7 @@ SIGNATURES = {
     "na_train_x3_scratch_floats": (c_int64, []),
     "na_train_x3_smem_bytes": (c_int64, [I64]),
     "na_lstm_bwd_x3": (c_int, [I64, P, P, P, P, P, P, P, ctypes.c_uint64, I64, F32, P, P, P, P, P, P, P, I64, P, P, I64, I64, I64, P]),
+    "na_lstm_bwd_x3_dx": (c_int, [I64, P, P, P, P, P, P, P, ctypes.c_uint64, I64, F32, P, P, P, P, P, P, I64, P, P, I64, I64, I64, P]),
     "na_lstm_wgrad_x3": (c_int, [I64, P, P, P, P, P, P, P, P, I64, I64, I64, P]),
     "na_head_tail_fwd_f32": (c_int, [P] * 9 + [P, P, F32, P, P, I64, I64, I64, P]),
     "na_head_tail_bwd_f32": (c_int, [P] * 10 + [P, P, F32, P, P, P, I64, I64, I64, P]),

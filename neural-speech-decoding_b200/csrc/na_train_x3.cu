@@ -43,6 +43,10 @@ constexpr int kTxMmaWarp = 12, kTxTmaWarp = 13;
 constexpr int kTxStages = 3;
 constexpr uint32_t kTxAccCols = 256;      // forward: TMEM column stride of the two gate accumulators (192 gates + 16 score columns)
 
+// kDx backward (layer 0): dx = dG . [W_ih | bias] as an N = 16 accumulator at TMEM column 2 x 192 + 64 (464 of 512 in use)
+constexpr uint32_t kTxDxCol = 2 * kN + 64;
+constexpr uint32_t kTxIdescDx = make_idesc(16, kFmtVal, kFmtVal, false, true);
+
 __device__ __forceinline__ int64_t tclx_off(int t, int ntiles, int tile, int chunk, int row) {       // fp16 elements
     return ((((int64_t)t * ntiles + tile) * 12 + chunk) * kRows + row) * 8;
 }
@@ -423,6 +427,8 @@ struct TxBwdSmem {
     float wa[kH];
     float ba;
     float2 xch[3][kRows];                                           // fused head backward: per-step exchange of the 3 unit-group warps
+    alignas(8) uint64_t dx_full;                                    // kDx, layer 0: the dx MMAs of a step have completed (last, so
+                                                                    // the other members keep their offsets in every instantiation)
 };
 
 // gates of one cell at fp32 accuracy: 5 ex2 + 2 rcp (the reciprocals of each group are combined)
@@ -451,7 +457,13 @@ __device__ __forceinline__ void gates_exact(float vi, float vf, float vg, float 
 // HALF: half tiles as in lstm_fwd_x3_kernel -- copy rp = q / 2 takes K chunk 2 g + rp (8 units per thread), writes its
 // d(gates) to BOTH row copies in shared memory (so D_R is complete on every row) and to the canonical row in HBM (the
 // weight-gradient kernel then reads rows 0..63 only).
-template <int LAYER, bool HALF>
+//
+// kDx (input attributions, no weight gradients): neither layer stores DGX nor the d attn partials.  Layer 0 also emits
+// dx_t = dG_t . W_ih0 into fp32 [B][T][8]: three more MMAs per K16 slice (N = 16 over image chunks 0-1 | 8-9, i.e. W_ih and the
+// bias column, whose 8 products are discarded) into their own TMEM accumulator, issued after R's commit so that they stay off
+// the d(gates) -> dh_rec chain, with their own barrier.  Every epilogue warp waits for them before it overwrites the d(gates)
+// operand they read; the g == 0 warps read dx(t+1) then, i.e. before dg_ready(t), which the next dx MMAs wait for.
+template <int LAYER, bool HALF, bool kDx = false>
 __global__ void __launch_bounds__(kTxThreads, 1)
 lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  L1: TCLX (the layer's forward input)
                    const __half* __restrict__ h,                    // TCLX: this layer's h
@@ -462,10 +474,14 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
                    const unsigned char* __restrict__ mask, uint64_t seed, uint32_t thresh16, float drop_scale,   // L1: dropout of its input
                    float* __restrict__ din,                         // TCL32, L1 only
                    __half* __restrict__ dg_out,                     // DGX
-                   const float* __restrict__ dz, const float* __restrict__ stats, const float* __restrict__ zpool,
+                   const float* __restrict__ dz,
+                   const float* __restrict__ stats,                 // L1: softmax (max, sum);  kDx L0: per-window unscale of dz [B]
+                   const float* __restrict__ zpool,
                    const float* __restrict__ attn_w, const float* __restrict__ attn_b, int64_t B,
-                   float* __restrict__ attn_partial,                // [grid][52]: d attn_w | d attn_b
+                   float* __restrict__ attn_partial,                // L1: [grid][52] d attn_w | d attn_b;  kDx L0: dx [B][T][8]
                    int T, int64_t Bp, int ntiles, int64_t drop_stride) {
+    // (kDx re-uses two pointers that layer 0 has no use for: a new parameter changes the register allocation of every
+    // instantiation, and the default ones must keep their SASS)
     using SM = TxBwdSmem<LAYER>;
     constexpr int kInChunks = LAYER == 0 ? 2 : 12;
     constexpr int kHp = LAYER == 0 ? 2 : 12;                         // first h_{t-1} chunk of the act stage
@@ -490,6 +506,7 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
             mbar_init(&S.act_full, 1); mbar_init(&S.act_free, 1);
             mbar_init(&S.g_full[0], 1); mbar_init(&S.g_full[1], 1); mbar_init(&S.r_full, 1);
             mbar_init(&S.dg_ready, 12 * 32);
+            if constexpr (kDx && LAYER == 0) mbar_init(&S.dx_full, 1);
             fence_mbar_init();
         }
         if (dz != nullptr) {
@@ -589,6 +606,19 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
                         }
                 }
                 if (leader) umma_commit(&S.r_full);            // R(t+1) done (i == 0: nothing pending)
+                if constexpr (kDx && LAYER == 0) {
+                    if (i >= 1) {                               // dx(t+1) = dG . [W_ih | bias] (N = 16; columns 8-15 unused)
+#pragma unroll
+                        for (int ks = 0; ks < 12; ++ks)
+                            if (leader) {
+                                const uint64_t ahi = desc_adv(d_dgk, 2 * ks * kAChunk), alo = desc_adv(d_dgk, (24 + 2 * ks) * kAChunk);
+                                umma_bf16_i(tmem + kTxDxCol, ahi, desc_adv(d_bm, ks * 256), kTxIdescDx, ks == 0 ? 0u : 1u);
+                                umma_bf16_i(tmem + kTxDxCol, ahi, desc_adv(d_bm, 8 * kBChunk + ks * 256), kTxIdescDx, 1u);
+                                umma_bf16_i(tmem + kTxDxCol, alo, desc_adv(d_bm, ks * 256), kTxIdescDx, 1u);
+                            }
+                        if (leader) umma_commit(&S.dx_full);
+                    }
+                }
                 if (i + 1 < T) issue_g((i + 1) & 1);           // G(t-1): accumulator (i+1)&1 was drained (and its barrier consumed) in iteration i-1
             }
         } else {
@@ -604,6 +634,24 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
             const int u0 = 8 * chunk0;                               // its first hidden unit
             const int64_t bwin = HALF ? (int64_t)tile * 64 + crow : b0 + row;
             const uint32_t xbar = HALF ? 1 + (q & 1) : 1 + q, xcnt = HALF ? 192 : 96;      // the warps that share a window
+            // dx(tx): the image's W_ih0 carries the x16 of the x / 16 input split; dz of the window was scaled by 1 / stats[b]
+            float* const dx = attn_partial;
+            const float dxs = (kDx && LAYER == 0 && bwin < B) ? kX3XScale * stats[bwin] : 0.f;
+            auto take_dx = [&](const int tx) {
+                // phase: T per tile, consumed in order -- this CTA's earlier tiles, then steps T-1 .. tx of this one
+                const uint32_t k = (uint32_t)((tile - (int)blockIdx.x) / (int)gridDim.x) * (uint32_t)T + (uint32_t)(T - 1 - tx);
+                mbar_wait(&S.dx_full, k & 1);
+                tc_fence_after();
+                if (g == 0) {                                        // one writer per window: g == 0, first row copy
+                    uint32_t r[8];
+                    tmem_ld8(tmem + kTxDxCol + lane_base, r);
+                    if (rp == 0 && bwin < B) {
+                        float4* o = reinterpret_cast<float4*>(dx + (bwin * T + tx) * 8);
+                        o[0] = make_float4(__uint_as_float(r[0]) * dxs, __uint_as_float(r[1]) * dxs, __uint_as_float(r[2]) * dxs, __uint_as_float(r[3]) * dxs);
+                        o[1] = make_float4(__uint_as_float(r[4]) * dxs, __uint_as_float(r[5]) * dxs, __uint_as_float(r[6]) * dxs, __uint_as_float(r[7]) * dxs);
+                    }
+                }
+            };
             float dc[kU], ccur[kU];
 #pragma unroll
             for (int j = 0; j < kU; ++j) dc[j] = 0.f;
@@ -667,9 +715,9 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
 #pragma unroll
                         for (int j = 0; j < kU; ++j) {
                             dh[j] = fmaf(alpha, dzr[j], ds * S.wa[u0 + j]);
-                            dwa[j] = fmaf(ds, hv[j], dwa[j]);
+                            if constexpr (!kDx) dwa[j] = fmaf(ds, hv[j], dwa[j]);
                         }
-                        dba += ds;
+                        if constexpr (!kDx) dba += ds;
                     } else {
 #pragma unroll
                         for (int j = 0; j < kU; j += 4) {
@@ -742,6 +790,8 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
                         for (int j = 0; j < kU; ++j) dh[j] += __uint_as_float(r[j]);
                     }
                 }
+                if constexpr (kDx && LAYER == 0)
+                    if (i == T) take_dx(0);
                 if (i == T) break;
 #pragma unroll
                 for (int pr = 0; pr < kNB; ++pr) {
@@ -781,14 +831,18 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
                         const float e1[8] = {pg[0], pg[1], pg[2], pg[3], po[0], po[1], po[2], po[3]};
                         uint32_t hi[4], lo[4];
                         split_pack8(e0, hi, lo);
+                        if constexpr (kDx && LAYER == 0)
+                            if (i >= 1 && pr == 0 && gi == 0) take_dx(t + 1);      // before the first overwrite of S.dg
                         st_shared_v4(S.dg + (2 * G) * kAChunk + row * 16, hi[0], hi[1], hi[2], hi[3]);
                         st_shared_v4(S.dg + (24 + 2 * G) * kAChunk + row * 16, lo[0], lo[1], lo[2], lo[3]);
                         if (HALF) {
                             st_shared_v4(S.dg + (2 * G) * kAChunk + (row ^ 64) * 16, hi[0], hi[1], hi[2], hi[3]);
                             st_shared_v4(S.dg + (24 + 2 * G) * kAChunk + (row ^ 64) * 16, lo[0], lo[1], lo[2], lo[3]);
                         }
-                        *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 2 * G, crow)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                        *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 24 + 2 * G, crow)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                        if constexpr (!kDx) {
+                            *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 2 * G, crow)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                            *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 24 + 2 * G, crow)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                        }
                         split_pack8(e1, hi, lo);
                         st_shared_v4(S.dg + (2 * G + 1) * kAChunk + row * 16, hi[0], hi[1], hi[2], hi[3]);
                         st_shared_v4(S.dg + (24 + 2 * G + 1) * kAChunk + row * 16, lo[0], lo[1], lo[2], lo[3]);
@@ -796,8 +850,10 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
                             st_shared_v4(S.dg + (2 * G + 1) * kAChunk + (row ^ 64) * 16, hi[0], hi[1], hi[2], hi[3]);
                             st_shared_v4(S.dg + (24 + 2 * G + 1) * kAChunk + (row ^ 64) * 16, lo[0], lo[1], lo[2], lo[3]);
                         }
-                        *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 2 * G + 1, crow)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                        *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 24 + 2 * G + 1, crow)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                        if constexpr (!kDx) {
+                            *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 2 * G + 1, crow)) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                            *reinterpret_cast<uint4*>(dg_out + dgx_any<HALF>(t, ntiles, tile, 24 + 2 * G + 1, crow)) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                        }
                     }
                 }
                 tc_fence_before();
@@ -809,7 +865,7 @@ lstm_bwd_x3_kernel(const __half* __restrict__ act_in,               // L0: XS;  
     }
 
     // ---- per-CTA partial of d attn_w / d attn_b (fused head backward) ---------------------------------------------
-    if (head) {
+    if (head && !kDx) {
         float* red = reinterpret_cast<float*>(S.dg);               // [12 warps][17]; every MMA has completed (tile-end barrier)
         if (warp < 12) {
 #pragma unroll
@@ -1111,6 +1167,40 @@ extern "C" int64_t na_train_x3_scratch_floats(void) {
     return sms * 52 + sms * na::tc::kRows * na::tc::kN;      // attention partials, then weight-gradient partials
 }
 
+namespace {
+// One launch of lstm_bwd_x3_kernel<layer, half, kDx> (its arguments checked by the caller).
+template <bool kDx>
+int launch_bwd_x3(const char* name, int64_t layer, const void* act_in, const void* h, const float* cstate, const float* dh_in,
+                  const void* packed_x3, const void* zeros, const unsigned char* in_mask, uint64_t seed, int64_t thresh16,
+                  float drop_scale, float* din, void* dg, const float* dz, const float* stats, const float* zpool,
+                  const float* attn_w, const float* attn_b, int64_t B, float* attn_partial, float* dx, const float* dx_scale,
+                  int64_t T, int64_t Bp, int64_t half_stride, cudaStream_t st, int* grid_out) {
+    using namespace na;
+    const int ntiles = (int)(Bp / tc::kRows);
+    const int grid = train_grid_cap(ntiles < tc::tx_sms() ? ntiles : tc::tx_sms());
+    const unsigned char* pk = reinterpret_cast<const unsigned char*>(packed_x3) + (layer == 0 ? 0 : tc::kX3B0Chunks * tc::kBChunk);
+    const int64_t dstride = half_stride > 0 ? half_stride : Bp;
+#define NA_X3_BWD(L, HF)                                                                                                              \
+    {                                                                                                                                \
+        const size_t smem = sizeof(tc::TxBwdSmem<L>);                                                                                \
+        cudaError_t e = cudaFuncSetAttribute(tc::lstm_bwd_x3_kernel<L, HF, kDx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (e != cudaSuccess) return fail((int)e, "%s: shared memory opt-in (%zu B) failed: %s", name, smem, cudaGetErrorString(e)); \
+        tc::lstm_bwd_x3_kernel<L, HF, kDx><<<grid, tc::kTxThreads, smem, st>>>(                                                      \
+            reinterpret_cast<const __half*>(act_in), reinterpret_cast<const __half*>(h), cstate, dh_in, pk,                           \
+            reinterpret_cast<const __half*>(zeros), L == 0 ? nullptr : in_mask, L == 0 ? 0 : seed, L == 0 ? 65536u : (uint32_t)thresh16, \
+            L == 0 ? 1.0f : drop_scale, L == 0 ? nullptr : din, reinterpret_cast<__half*>(dg), L == 0 ? nullptr : dz,                 \
+            L == 0 ? dx_scale : stats, L == 0 ? nullptr : zpool, L == 0 ? nullptr : attn_w, L == 0 ? nullptr : attn_b, B,           \
+            L == 0 ? dx : attn_partial, (int)T, Bp, ntiles, dstride);                                                                \
+    }
+    if (layer == 0) { if (half_stride > 0) NA_X3_BWD(0, true) else NA_X3_BWD(0, false) }
+    else { if (half_stride > 0) NA_X3_BWD(1, true) else NA_X3_BWD(1, false) }
+#undef NA_X3_BWD
+    count_launch();
+    *grid_out = grid;
+    return check_launch(name);
+}
+}  // namespace
+
 extern "C" int na_lstm_bwd_x3(int64_t layer, const void* act_in, const void* h, const float* cstate, const float* dh_in,
                               const void* packed_x3, const void* zeros, const unsigned char* in_mask, uint64_t seed, int64_t thresh16,
                               float drop_scale, float* din, void* dg, const float* dz, const float* stats, const float* zpool,
@@ -1131,31 +1221,42 @@ extern "C" int na_lstm_bwd_x3(int64_t layer, const void* act_in, const void* h, 
     NA_REQUIRE(layer == 0 || din != nullptr, NA_EINVAL, "na_lstm_bwd_x3: layer 1 needs din");
     NA_REQUIRE(thresh16 >= 0 && thresh16 <= 65536, NA_EINVAL, "na_lstm_bwd_x3: thresh16 outside [0,65536]");
     cudaStream_t st = as_stream(stream);
-    const int ntiles = (int)(Bp / tc::kRows);
-    const int grid = train_grid_cap(ntiles < tc::tx_sms() ? ntiles : tc::tx_sms());
-    const unsigned char* pk = reinterpret_cast<const unsigned char*>(packed_x3) + (layer == 0 ? 0 : tc::kX3B0Chunks * tc::kBChunk);
     float* attn_partial = scratch;
-    const int64_t dstride = half_stride > 0 ? half_stride : Bp;
-#define NA_X3_BWD(L, HF)                                                                                                              \
-    {                                                                                                                                \
-        const size_t smem = sizeof(tc::TxBwdSmem<L>);                                                                                \
-        cudaError_t e = cudaFuncSetAttribute(tc::lstm_bwd_x3_kernel<L, HF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        if (e != cudaSuccess) return fail((int)e, "na_lstm_bwd_x3: shared memory opt-in (%zu B) failed: %s", smem, cudaGetErrorString(e)); \
-        tc::lstm_bwd_x3_kernel<L, HF><<<grid, tc::kTxThreads, smem, st>>>(                                                           \
-            reinterpret_cast<const __half*>(act_in), reinterpret_cast<const __half*>(h), cstate, dh_in, pk,                           \
-            reinterpret_cast<const __half*>(zeros), L == 0 ? nullptr : in_mask, L == 0 ? 0 : seed, L == 0 ? 65536u : (uint32_t)thresh16, \
-            L == 0 ? 1.0f : drop_scale, L == 0 ? nullptr : din, reinterpret_cast<__half*>(dg), L == 0 ? nullptr : dz,                 \
-            L == 0 ? nullptr : stats, L == 0 ? nullptr : zpool, L == 0 ? nullptr : attn_w, L == 0 ? nullptr : attn_b, B,              \
-            L == 0 ? nullptr : attn_partial, (int)T, Bp, ntiles, dstride);                                                           \
-    }
-    if (layer == 0) { if (half_stride > 0) NA_X3_BWD(0, true) else NA_X3_BWD(0, false) }
-    else { if (half_stride > 0) NA_X3_BWD(1, true) else NA_X3_BWD(1, false) }
-#undef NA_X3_BWD
-    count_launch();
-    int rc = check_launch("na_lstm_bwd_x3");
+    int grid = 0;
+    int rc = launch_bwd_x3<false>("na_lstm_bwd_x3", layer, act_in, h, cstate, dh_in, packed_x3, zeros, in_mask, seed, thresh16,
+                                  drop_scale, din, dg, dz, stats, zpool, attn_w, attn_b, B, attn_partial, nullptr, nullptr, T, Bp,
+                                  half_stride, st, &grid);
     if (rc) return rc;
     if (dz != nullptr) return reduce_partials(attn_partial, d_attn, grid, 52, st);
     return NA_OK;
+}
+
+extern "C" int na_lstm_bwd_x3_dx(int64_t layer, const void* act_in, const void* h, const float* cstate, const float* dh_in,
+                                 const void* packed_x3, const void* zeros, const unsigned char* in_mask, uint64_t seed,
+                                 int64_t thresh16, float drop_scale, float* din, const float* dz, const float* stats,
+                                 const float* zpool, const float* attn_w, const float* attn_b, int64_t B, float* dx,
+                                 const float* dz_inv_scale, int64_t T, int64_t Bp, int64_t half_stride, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(layer == 0 || layer == 1, NA_EINVAL, "na_lstm_bwd_x3_dx: layer must be 0 or 1");
+    NA_REQUIRE(half_stride >= 0 && (half_stride == 0 || layer == 0 || dz != nullptr), NA_EUNSUPPORTED,
+               "na_lstm_bwd_x3_dx: half tiles need the fused head backward on layer 1");
+    NA_REQUIRE(half_stride == 0 || B <= Bp / 2, NA_EINVAL, "na_lstm_bwd_x3_dx: half tiles need B <= Bp / 2");
+    NA_REQUIRE(T >= 1 && T < (1 << 20) && Bp >= tc::kRows && Bp % tc::kRows == 0, NA_EINVAL,
+               "na_lstm_bwd_x3_dx: bad shape T=%lld Bp=%lld", (long long)T, (long long)Bp);
+    NA_REQUIRE_PTR(act_in); NA_REQUIRE_PTR(h); NA_REQUIRE_PTR(cstate); NA_REQUIRE_PTR(packed_x3); NA_REQUIRE_PTR(zeros);
+    NA_OPTIONAL_PTR(dh_in); NA_OPTIONAL_PTR(dz); NA_OPTIONAL_PTR(in_mask); NA_OPTIONAL_PTR(din);
+    NA_OPTIONAL_PTR(dx); NA_OPTIONAL_PTR(dz_inv_scale);
+    NA_REQUIRE((dz != nullptr) != (dh_in != nullptr), NA_EINVAL, "na_lstm_bwd_x3_dx: give exactly one of dh_in and dz");
+    NA_REQUIRE(dz == nullptr || (layer == 1 && stats && zpool && attn_w && attn_b), NA_EINVAL,
+               "na_lstm_bwd_x3_dx: the fused head backward is for layer 1 and needs stats, zpool, attn_w, attn_b");
+    NA_REQUIRE(B >= 1 && B <= Bp, NA_EINVAL, "na_lstm_bwd_x3_dx: need 1 <= B <= Bp, got B=%lld Bp=%lld", (long long)B, (long long)Bp);
+    NA_REQUIRE(layer == 0 || din != nullptr, NA_EINVAL, "na_lstm_bwd_x3_dx: layer 1 needs din");
+    NA_REQUIRE(layer == 1 || (dx != nullptr && dz_inv_scale != nullptr), NA_EINVAL, "na_lstm_bwd_x3_dx: layer 0 needs dx and dz_inv_scale");
+    NA_REQUIRE(thresh16 >= 0 && thresh16 <= 65536, NA_EINVAL, "na_lstm_bwd_x3_dx: thresh16 outside [0,65536]");
+    int grid = 0;
+    return launch_bwd_x3<true>("na_lstm_bwd_x3_dx", layer, act_in, h, cstate, dh_in, packed_x3, zeros, in_mask, seed, thresh16,
+                               drop_scale, din, nullptr, dz, stats, zpool, attn_w, attn_b, B, nullptr, dx, dz_inv_scale, T, Bp,
+                               half_stride, as_stream(stream), &grid);
 }
 
 extern "C" int na_lstm_wgrad_x3(int64_t layer, const void* dg, const void* act_in, const void* h, const void* zeros,

@@ -31,6 +31,14 @@ class DecoderOutputs(NamedTuple):
     embedding: torch.Tensor     # [B, H]
 
 
+class Attributions(NamedTuple):
+    """``EEG_LSTM.input_gradients`` / ``integrated_gradients``: fp32 on the device of ``x``."""
+    logits: torch.Tensor        # [B, K], at x
+    target: torch.Tensor        # [B] long, the explained class of each window
+    attributions: torch.Tensor  # [B, T, C]
+    delta: Optional[torch.Tensor] = None    # [B] integrated gradients: sum(attributions) - (F(x) - F(baseline))
+
+
 class LSTMParameters(nn.Module):
     """Parameter container with ``nn.LSTM``'s names, shapes, registration order and default init
     (U(-1/sqrt(H), 1/sqrt(H)) for every tensor, drawn in registration order), so that
@@ -347,6 +355,96 @@ class EEG_LSTM(nn.Module):
                 d2 = (torch.rand((B, 32), device=device) >= p).float()
         return d1, rr, d2
 
+    # -- input attributions -----------------------------------------------------------------
+    def _targets(self, target, B: int, device) -> Optional[torch.Tensor]:
+        if target is None:
+            return None
+        K = self.fc[3].out_features
+        t = torch.as_tensor(target, dtype=torch.long, device=device)
+        t = t.expand(B).contiguous() if t.dim() == 0 else t
+        if t.shape != (B,):
+            raise ValueError(f"target must be an int or a [B] = [{B}] tensor, got shape {tuple(t.shape)}")
+        if B and (int(t.min()) < 0 or int(t.max()) >= K):
+            raise ValueError(f"target out of range for {K} classes")
+        return t
+
+    def input_gradients(self, x: torch.Tensor, target=None) -> Attributions:
+        """Saliency: ``d logits[b, target[b]] / d x[b]`` for every window, ``x`` [B,T,C] on CUDA -> ``Attributions(logits,
+        target, attributions [B,T,C])``.  ``target``: an int or a [B] long tensor; default the argmax of each window's
+        logits.  Eval-mode arithmetic whatever ``self.training`` is; parameter ``.grad``, the module's mode and its packed
+        weights are left as they are.  ``compute_dtype`` does not apply: attributions always carry the fp32 contract.
+
+        The flagship shape without ``zscore_input`` runs on the exact tensor-core kernels (``ops.decoder_input_grad_x3``)
+        while ``ops.EXACT_TC_TRAIN`` is set.  Its accuracy is looser than the 1e-5 of the weight gradients, because a
+        per-step dx does not average over time and windows.  On the 324 shipped windows (625 steps), max|d| / max|ref|
+        against float64, on each window's own scale, is at most 4.3e-5 at the argmax class and 8.2e-5 at another class.
+        That is the fp16 hi + lo operand split over the BPTT; it is tested at 2e-4.  With ``ops.EXACT_TC_TRAIN = False``
+        every call takes the FFMA path: 9.6e-6 at the argmax class (4.8e-5 at another class, on one window).  Everything
+        but the flagship shape, and ``zscore_input``, also runs on that path: torch autograd through the FFMA kernels
+        (``ops.DecoderFunction``).  It has no gradient through the z-score stage, so ``zscore_input`` raises."""
+        return self._input_gradients(x, target)
+
+    def _input_gradients(self, x: torch.Tensor, target) -> Attributions:
+        if x.dim() != 3:
+            raise ValueError(f"expected x of shape [B,T,C], got {tuple(x.shape)}")
+        ops._require_cuda(x)
+        if x.shape[2] != self.lstm.input_size:
+            raise RuntimeError(f"input.size(-1) must be equal to input_size. Expected {self.lstm.input_size}, got {x.shape[2]}")
+        B = x.shape[0]
+        tgt = self._targets(target, B, x.device)
+        if B == 0:
+            K = self.fc[3].out_features
+            e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=x.device)
+            return Attributions(e(0, K), torch.empty((0,), dtype=torch.long, device=x.device), e(*x.shape))
+        x32 = x.detach().float().contiguous()
+        L = self.lstm.num_layers
+        lstm_params = [[p.detach() for p in self.lstm.layer(l)] for l in range(L)]
+        head = [p.detach() for p in self._head_params()]
+        if ops.EXACT_TC_TRAIN and self.tc_supported() and not self.zscore_input:
+            logits, dx = ops.decoder_input_grad_x3(x32, lstm_params, head, tgt)
+        else:
+            with torch.enable_grad():
+                xg = x32.requires_grad_(True)
+                logits = ops.decoder_train_forward(xg, lstm_params, head, self.dropout_p, self.zscore_input)
+                pick = logits.argmax(dim=1) if tgt is None else tgt
+                (dx,) = torch.autograd.grad(logits.gather(1, pick[:, None]).sum(), xg)
+            logits = logits.detach().float()
+        if tgt is None:
+            tgt = logits.argmax(dim=1)
+        return Attributions(logits, tgt, dx)
+
+    def integrated_gradients(self, x: torch.Tensor, target=None, baseline: Optional[torch.Tensor] = None,
+                             steps: int = 32) -> Attributions:
+        """Integrated gradients (Sundararajan et al., 2017) of ``logits[b, target[b]]`` from ``baseline`` (default zeros: a
+        flat signal) to ``x``, midpoint rule: ``alpha_k = (k + 1/2) / steps``, all ``B * steps`` interpolated windows as one
+        batch through ``input_gradients``' path; ``attributions = (x - baseline) * mean_k grad``.  ``delta[b] =
+        sum(attributions[b]) - (F(x) - F(baseline))`` is the completeness error.  It shrinks as ``steps`` grows once the
+        steps resolve the path: on the shipped windows from a zero baseline, from 32 steps on (not from 8 to 16)."""
+        if steps < 1:
+            raise ValueError("steps must be >= 1")
+        if x.dim() != 3:
+            raise ValueError(f"expected x of shape [B,T,C], got {tuple(x.shape)}")
+        x32 = x.detach().float()
+        if baseline is None:
+            base = torch.zeros_like(x32)
+        else:
+            if tuple(baseline.shape) != tuple(x.shape):
+                raise ValueError(f"baseline must have the shape of x {tuple(x.shape)}, got {tuple(baseline.shape)}")
+            base = baseline.detach().to(device=x32.device, dtype=torch.float32)
+        at_x = self._input_gradients(x32, target)
+        B = x.shape[0]
+        if B == 0:
+            return Attributions(at_x.logits, at_x.target, at_x.attributions, at_x.logits.new_empty((0,)))
+        alpha = (torch.arange(steps, dtype=torch.float32, device=x32.device) + 0.5) / steps
+        diff = x32 - base
+        batch = torch.cat([base, (base[None] + alpha[:, None, None, None] * diff[None]).reshape(-1, *x.shape[1:])])
+        run = self._input_gradients(batch, at_x.target.repeat(steps + 1))
+        grads = run.attributions[B:].reshape(steps, *x.shape).mean(dim=0)
+        attributions = diff * grads
+        pick = lambda lg: lg.gather(1, at_x.target[:, None])[:, 0]
+        delta = attributions.sum(dim=(1, 2)) - (pick(at_x.logits) - pick(run.logits[:B]))
+        return Attributions(at_x.logits, at_x.target, attributions, delta)
+
     # -- forward ---------------------------------------------------------------------------
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         if x.dim() != 3:
@@ -461,6 +559,19 @@ class SimplePredictor:
             attention = out.attention[0].detach().cpu().numpy().astype(np.float32)
         y_idx = int(np.argmax(probs))
         return probs, self.class_names[y_idx], attention
+
+    def attribute(self, chunk_TxC: np.ndarray, steps: int = 32):
+        """``predict`` plus integrated gradients of the predicted class (``EEG_LSTM.integrated_gradients``, zero
+        baseline): chunk [T,C] -> (probs float32[K], label, attributions float32[T,C]).  Same preprocessing as
+        ``predict``; the attributions are with respect to the preprocessed window."""
+        x = self.pre.transform(chunk_TxC)
+        x_t = torch.from_numpy(np.ascontiguousarray(x[None, ...])).float().to(self.compute_device)
+        with self._no_grad():
+            _, probs = self.model.decode(x_t, want_probs=True)
+            probs = probs[0].detach().cpu().numpy().astype(np.float32)
+        y_idx = int(np.argmax(probs))
+        out = self.model.integrated_gradients(x_t, target=y_idx, steps=steps)
+        return probs, self.class_names[y_idx], out.attributions[0].detach().cpu().numpy().astype(np.float32)
 
     def predict_batch(self, chunks_BxTxC: np.ndarray, preprocess: bool = True) -> np.ndarray:
         """Batched sibling of ``predict``: [B,T,C] -> probs [B,K] (one H2D, one launch sequence, one D2H)."""

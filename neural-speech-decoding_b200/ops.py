@@ -1387,10 +1387,37 @@ def _(layer, dg, act_in, h, half_stride=0):
     return f32(192, 8 if layer == 0 else 48), f32(192, 48), f32(192)
 
 
+def _x3_forward(x: Tensor, lstm_flat: Sequence[Tensor], head: Sequence[Tensor], p: float, zscore: bool, drop1,
+                rrelu_slope: Optional[Tensor], drop2_mask: Optional[Tensor]):
+    """Forward of the exact training tier with saves: x [B,T,8] -> (logits, saves (xs, h0, h0d, c0, h1, c1, packed, stats,
+    zpool), the layer-0 keep-mask in its tile layout or None, meta (scale, B, seed, thresh16, scale1, half_stride)).
+    ``lstm_flat`` / ``head``: detached tensors, the head ones fp32.  Used by DecoderFunctionX3 and, with no noise (eval
+    arithmetic), by decoder_input_grad_x3."""
+    B, T, C = x.shape
+    scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0          # head dropout (and mask-tensor mode)
+    mask, seed, thresh16, scale1 = _drop1_args(drop1, scale)
+    xin = x.detach()
+    if xin.dtype != torch.float32:
+        xin = xin.float()
+    if zscore:
+        xin = window_zscore(xin, T, T, True, False, NA_F32)
+    half_stride = _half_stride(B, x.device, X3_HALF_TILES)
+    Bp = ((B + 63) // 64) * TC_TILE if half_stride else padded_batch(B, TC_TILE)
+    if half_stride and mask is not None:
+        mask = _half_tile_rows(mask, B, Bp)
+    xs = x3_split_input(xin.contiguous(), Bp, half_stride)
+    packed = decoder_pack_x3(lstm_flat)
+    h0, h0d, c0, _, _ = lstm_fwd_train_x3(0, xs, packed, head[0], head[1], mask, seed, thresh16, scale1, B, half_stride)
+    has_drop = mask is not None or thresh16 < 65536
+    h1, _, c1, zpool, stats = lstm_fwd_train_x3(1, h0d if has_drop else h0, packed, head[0], head[1], None, 0, 65536, 1.0, B, half_stride)
+    logits, _ = head_tail_fwd(zpool, head, rrelu_slope, drop2_mask, scale, False)
+    return logits, (xs, h0, h0d, c0, h1, c1, packed, stats, zpool), mask, (scale, B, seed, thresh16, scale1, half_stride)
+
+
 class DecoderFunctionX3(torch.autograd.Function):
     """Training step of the flagship decoder at fp32 accuracy on the tensor cores (1e-5 contract on logits and
     gradients): operand-split tcgen05 forward with saves, fp32 head kernels, operand-split BPTT, time-parallel
-    weight-gradient GEMMs.  No d/dx (the FFMA tier provides it)."""
+    weight-gradient GEMMs.  No d/dx (the FFMA tier provides it; input attributions: decoder_input_grad_x3)."""
 
     @staticmethod
     def forward(ctx, x, p, zscore, drop1, rrelu_slope, drop2_mask, *params):
@@ -1398,27 +1425,9 @@ class DecoderFunctionX3(torch.autograd.Function):
         ctx.param_dtypes = [t.dtype for t in params]
         if ctx.needs_input_grad[0]:
             raise RuntimeError("the tensor-core exact training tier does not produce d/dx")
-        B, T, C = x.shape
         lstm_flat, head = [t.detach() for t in params[:8]], [_f32c(t.detach()) for t in params[8:]]
-        scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0          # head dropout (and mask-tensor mode)
-        mask, seed, thresh16, scale1 = _drop1_args(drop1, scale)
-        xin = x.detach()
-        if xin.dtype != torch.float32:
-            xin = xin.float()
-        if zscore:
-            xin = window_zscore(xin, T, T, True, False, NA_F32)
-        half_stride = _half_stride(B, x.device, X3_HALF_TILES)
-        Bp = ((B + 63) // 64) * TC_TILE if half_stride else padded_batch(B, TC_TILE)
-        if half_stride and mask is not None:
-            mask = _half_tile_rows(mask, B, Bp)
-        xs = x3_split_input(xin.contiguous(), Bp, half_stride)
-        packed = decoder_pack_x3(lstm_flat)
-        h0, h0d, c0, _, _ = lstm_fwd_train_x3(0, xs, packed, head[0], head[1], mask, seed, thresh16, scale1, B, half_stride)
-        has_drop = mask is not None or thresh16 < 65536
-        h1, _, c1, zpool, stats = lstm_fwd_train_x3(1, h0d if has_drop else h0, packed, head[0], head[1], None, 0, 65536, 1.0, B, half_stride)
-        logits, _ = head_tail_fwd(zpool, head, rrelu_slope, drop2_mask, scale, False)
-        _save(ctx, [xs, h0, h0d, c0, h1, c1, packed, stats, zpool, *head], [mask, rrelu_slope, drop2_mask])
-        ctx.meta = (scale, B, seed, thresh16, scale1, half_stride)
+        logits, saves, mask, ctx.meta = _x3_forward(x, lstm_flat, head, p, zscore, drop1, rrelu_slope, drop2_mask)
+        _save(ctx, [*saves, *head], [mask, rrelu_slope, drop2_mask])
         return logits
 
     @staticmethod
@@ -1444,6 +1453,75 @@ def decoder_train_forward_x3(x: Tensor, lstm_params, head_params, p: float, zsco
                              drop1=None, rrelu_slope=None, drop2_mask=None) -> Tensor:
     flat = [t for layer in lstm_params for t in layer]
     return DecoderFunctionX3.apply(x, p, zscore, drop1, rrelu_slope, drop2_mask, *flat, *head_params)
+
+
+@torch.library.custom_op("neuroalpha::lstm_bwd_x3_dx", mutates_args=(), device_types="cuda")
+@_device_guard
+def lstm_bwd_x3_dx(layer: int, act_in: Tensor, h: Tensor, c: Tensor, dh_in: Optional[Tensor], packed: Tensor,
+                   head: Sequence[Tensor], dz_inv_scale: Optional[Tensor], B: int, half_stride: int = 0) -> Tensor:
+    """BPTT of one layer for input attributions (no weight-gradient byproducts, no dropout) -> layer 1: din TCL32;
+    layer 0: dx fp32 [B, T, 8], each window's row multiplied by ``dz_inv_scale[b]``.  ``head`` as in lstm_bwd_x3."""
+    _require_cuda(act_in, h, c, dh_in, packed, dz_inv_scale, *head)
+    T, NT = c.shape[0], c.shape[1]
+    Bp, dev = NT * TC_TILE, c.device
+    out = _tcl32(T, Bp, dev) if layer == 1 else torch.empty((B, T, 8), dtype=torch.float32, device=dev)
+    fused = len(head) > 0
+    hp = [_f32c(t) for t in head]
+    zeros, _ = _train_buffers(dev, "x3", 24576, 4 * _lib.query("na_train_x3_scratch_floats"))
+    _lib.call("na_lstm_bwd_x3_dx", int(layer), act_in.data_ptr(), h.data_ptr(), c.data_ptr(), None if fused else dh_in.data_ptr(),
+              packed.data_ptr(), zeros.data_ptr(), None, 0, 65536, 1.0, out.data_ptr() if layer == 1 else None,
+              *([t.data_ptr() for t in hp] if fused else [None] * 5), int(B), out.data_ptr() if layer == 0 else None,
+              _f32c(dz_inv_scale).data_ptr() if layer == 0 else None, T, Bp, int(half_stride), _stream())
+    return out
+
+
+@lstm_bwd_x3_dx.register_fake
+def _(layer, act_in, h, c, dh_in, packed, head, dz_inv_scale, B, half_stride=0):
+    return c.new_empty(c.shape) if layer == 1 else c.new_empty((B, c.shape[0], 8))
+
+
+def _scale_dz_rows(dz: Tensor) -> Tuple[Tensor, Tensor]:
+    """_scale_dz per window, for per-window results: row b of dz is scaled by its own power of two 2^6 / 2^ceil(log2
+    max|dz_b|), so a window whose dz is far below the batch maximum (LayerNorm's 1/sigma varies per window) keeps its low
+    bits in the fp16 d(gates), and a NaN window leaves the others' scale alone.  Everything below dz is linear per
+    window.  -> (scaled dz, the inverse factors [B])."""
+    amax = dz.abs().amax(dim=1, keepdim=True).clamp_min(1e-30)
+    s = torch.pow(2.0, 6.0 - torch.ceil(torch.log2(amax)))
+    return dz * s, (1.0 / s).reshape(-1).contiguous()
+
+
+def _input_grad_x3_round(x: Tensor, lstm_flat: Sequence[Tensor], head: Sequence[Tensor], target: Optional[Tensor]):
+    logits, saves, _, meta = _x3_forward(x, lstm_flat, head, 0.0, False, None, None, None)
+    xs, h0, _, c0, h1, c1, packed, stats, zpool = saves
+    B, hs = meta[1], meta[5]
+    tgt = logits.argmax(dim=1) if target is None else target
+    dlogits = torch.zeros_like(logits).scatter_(1, tgt[:, None], 1.0)
+    dz, _ = head_tail_bwd(dlogits, zpool, head, None, None, 1.0)
+    dz, inv_s = _scale_dz_rows(dz)
+    din1 = lstm_bwd_x3_dx(1, h0, h1, c1, None, packed, [dz, stats, zpool, head[0], head[1]], None, B, hs)
+    del h1, c1
+    dx = lstm_bwd_x3_dx(0, xs, h0, c0, din1, packed, [], inv_s, B, hs)
+    return logits, tgt, dx
+
+
+def decoder_input_grad_x3(x: Tensor, lstm_params, head_params, target: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """Saliency of the flagship decoder on the exact tensor-core tier, eval arithmetic (no dropout, RReLU at its eval
+    slope): x fp32 [B,T,8] -> (logits [B,K], dx = d logits[b, target[b]] / d x[b] fp32 [B,T,8]).  ``target``: long [B], or
+    None for the argmax of each window's logits.  Runs without autograd: the forward of DecoderFunctionX3, the head tail
+    backward of a one-hot dlogits, then both layers' BPTT without weight gradients.  Batches above one round of full
+    tiles (SMs x 128 windows) run round by round; each round saves about 1 MB per 625-step window."""
+    _require_cuda(x, target)
+    B, T, C = x.shape
+    with torch.no_grad():
+        lstm_flat = [t.detach() for layer in lstm_params for t in layer]
+        head = [_f32c(t.detach()) for t in head_params]
+        rnd = _sm_count(x.device) * TC_TILE
+        if B <= rnd:
+            logits, _, dx = _input_grad_x3_round(x, lstm_flat, head, target)
+            return logits, dx
+        parts = [_input_grad_x3_round(x[i:i + rnd], lstm_flat, head, None if target is None else target[i:i + rnd])
+                 for i in range(0, B, rnd)]
+        return torch.cat([q[0] for q in parts]), torch.cat([q[2] for q in parts])
 
 
 # ------------------------------------------------------------------------------------------
