@@ -345,6 +345,15 @@ iir_chain_warp_kernel(const float* __restrict__ x, float* __restrict__ y, const 
 static int g_iir_occ3 = 2;           // LT = 20: CTAs per SM the register allocation aims at (1: 152 registers, 2: <= 128, 3: <= 80 with spills); A/B knob
 void set_iir_occ3(int v) { g_iir_occ3 = v; }
 
+// The 48 KB a launch gets without opting in covers static (s_coef, s_pm: 14,880 B) and dynamic shared memory together, so
+// the C == 8 staging of LT = 40 (41,984 B) needs the opt-in as well as that of LT = 80 (82,944 B); LT = 20 (21,504 B) fits.
+template <typename Kernel>
+static int allow_dynamic_smem(Kernel kern, size_t smem) {
+    if (smem == 0) return 0;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    return e == cudaSuccess ? 0 : fail((int)e, "na_iir_chain: shared memory opt-in failed (%s)", cudaGetErrorString(e));
+}
+
 template <int LT>
 static int launch_iir_warp(const float* x, float* y, const double* coef, const int* nsec, int nfilt, int max_sections, int64_t S, int T,
                            int C, int detrend, int round_decimals, int carry_state, cudaStream_t st) {
@@ -358,11 +367,11 @@ static int launch_iir_warp(const float* x, float* y, const double* coef, const i
                                                                                           round_decimals, carry_state);
     } else if (max_sections <= 4) {
         auto kern = iir_chain_warp_kernel<LT, 4, 1>;
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (const int rc = allow_dynamic_smem(kern, smem)) return rc;
         kern<<<grid, kIirWarps * 32, smem, st>>>(x, y, coef, nsec, nfilt, S, T, C, detrend, round_decimals, carry_state);
     } else {
         auto kern = iir_chain_warp_kernel<LT, kIirMaxS, 1>;
-        if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (const int rc = allow_dynamic_smem(kern, smem)) return rc;
         kern<<<grid, kIirWarps * 32, smem, st>>>(x, y, coef, nsec, nfilt, S, T, C, detrend, round_decimals, carry_state);
     }
     return 0;

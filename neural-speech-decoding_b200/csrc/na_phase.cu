@@ -15,7 +15,10 @@
 //
 // One CTA per window.  T = 625 = 5^4: a radix-5 Stockham FFT in shared memory (4 stages, complex double).  Two real
 // channels ride in one complex transform: H is a real linear operator, so IFFT(-i sgn(k) FFT(x_a + i x_b)) = H[x_a] + i H[x_b]
-// -- 4 forward + 4 inverse transforms per window instead of 16, and no spectrum unpacking.  The twiddle table
+// -- 4 forward + 4 inverse transforms per window instead of 16, and no spectrum unpacking.  The pair's rounding leaks
+// into each other's transform at eps times the larger channel, so every channel is first scaled by a power of two to
+// [1, 2) (exact, and the phases do not depend on it), and an all-zero channel keeps H = 0 (phase 0, as in the
+// reference) instead of taking the leak as its signal.  The twiddle table
 // exp(-2 pi i k / 625) is computed on the host in float64 and passed in.  ~0.6 MFLOP (fp64) and 40 KB of DRAM traffic
 // per window; the bound is the fp64 pipe / shared-memory latency, not HBM.
 #include "na_common.cuh"
@@ -29,6 +32,9 @@ struct PhaseSmem {
     double2 tw[kPhT];
     float x[kPhT * kPhC];
     double red[8][28];
+    float cmax[8][8];                 // per warp, per channel: max |x|
+    double cscale[kPhC];              // s = 2^-floor(log2 max|x|); 0 for an all-zero channel
+    double2 hscale[4];                // per channel pair: (1 / (N s_{2p}), -1 / (N s_{2p+1})), 0 for an all-zero channel
     double P[8][8];
     double A[8][16];                  // [A | I] for the Gauss-Jordan inverse
 };
@@ -55,7 +61,9 @@ __device__ __forceinline__ void dft5(double2 (&v)[5]) {
     v[3] = make_double2(a2.x - b2.y, a2.y + b2.x);
 }
 
-// Forward FFT of the 4 series in S.buf[0] (Stockham autosort, radix 5, 4 stages): the result is back in S.buf[0].
+// Forward FFT of the 4 series in S.buf[0] (Stockham autosort, radix 5, 4 stages): the result is back in S.buf[0],
+// with kScale: multiplied by S.hscale[p] component-wise.
+template <bool kScale>
 __device__ __forceinline__ void fft625x4(PhaseSmem& S, int tid) {
     int src = 0;
     for (int Ns = 1; Ns < kPhT; Ns *= 5) {
@@ -71,6 +79,11 @@ __device__ __forceinline__ void fft625x4(PhaseSmem& S, int tid) {
             for (int r = 1; r < 5; ++r) v[r] = cmul(in[j + r * 125], S.tw[k * r * tstep]);
             dft5(v);
             const int j0 = (j / Ns) * Ns * 5 + k;
+            if (kScale && Ns * 5 == kPhT) {
+                const double2 sc = S.hscale[p];
+#pragma unroll
+                for (int r = 0; r < 5; ++r) v[r] = make_double2(v[r].x * sc.x, v[r].y * sc.y);
+            }
 #pragma unroll
             for (int r = 0; r < 5; ++r) out[j0 + r * Ns] = v[r];
         }
@@ -87,19 +100,47 @@ phase_coupling_filter_kernel(const float* __restrict__ x, float* __restrict__ y,
     const int tid = threadIdx.x;
     const int64_t b = blockIdx.x;
     for (int i = tid; i < kPhT; i += kPhThreads) S.tw[i] = make_double2(twiddle[2 * i], twiddle[2 * i + 1]);
-    {   // the window, coalesced 16-byte loads
+    {   // the window, coalesced 16-byte loads; thread tid only sees channels 4 (tid & 1) .. 4 (tid & 1) + 3
         const float4* src = reinterpret_cast<const float4*>(x + b * kPhT * kPhC);
         float4* dst = reinterpret_cast<float4*>(S.x);
-        for (int i = tid; i < kPhT * kPhC / 4; i += kPhThreads) dst[i] = src[i];
+        float m0 = 0.f, m1 = 0.f, m2 = 0.f, m3 = 0.f;
+        for (int i = tid; i < kPhT * kPhC / 4; i += kPhThreads) {
+            const float4 q = src[i];
+            dst[i] = q;
+            m0 = fmaxf(m0, fabsf(q.x)); m1 = fmaxf(m1, fabsf(q.y)); m2 = fmaxf(m2, fabsf(q.z)); m3 = fmaxf(m3, fabsf(q.w));
+        }
+#pragma unroll
+        for (int o = 2; o < 32; o <<= 1) {
+            m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, o)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, o));
+            m2 = fmaxf(m2, __shfl_xor_sync(0xffffffffu, m2, o)); m3 = fmaxf(m3, __shfl_xor_sync(0xffffffffu, m3, o));
+        }
+        const int lane = tid & 31;
+        if (lane < 2) {
+            float* cm = &S.cmax[tid >> 5][4 * lane];
+            cm[0] = m0; cm[1] = m1; cm[2] = m2; cm[3] = m3;
+        }
     }
     __syncthreads();
-    // ---- 1. z_p = x_{2p} + i x_{2p+1};  FFT;  W = -i sgn(k) Z;  inverse FFT by conjugation -----------------------------
+    if (tid < kPhC) {       // fmaxf skips NaN; an Inf keeps scale 1 so that it reaches the output like in the reference
+        float m = 0.f;
+#pragma unroll
+        for (int w = 0; w < kPhThreads / 32; ++w) m = fmaxf(m, S.cmax[w][tid]);
+        const long long e = isfinite(m) ? ((__double_as_longlong((double)m) >> 52) & 0x7ff) - 1023 : 0;   // floor(log2 m)
+        S.cscale[tid] = m == 0.f ? 0.0 : __longlong_as_double((1023 - e) << 52);
+        // 1 / s is a power of two, so scaling by (1 / N) / s rounds like the unscaled (1 / N)
+        const double h = m == 0.f ? 0.0 : (1.0 / kPhT) * __longlong_as_double((1023 + e) << 52);
+        if (tid & 1) S.hscale[tid >> 1].y = -h;
+        else S.hscale[tid >> 1].x = h;
+    }
+    __syncthreads();
+    // ---- 1. z_p = x_{2p} + i x_{2p+1} (scaled);  FFT;  W = -i sgn(k) Z;  inverse FFT by conjugation --------------------
     for (int i = tid; i < 4 * kPhT; i += kPhThreads) {
         const int p = i / kPhT, t = i % kPhT;
-        S.buf[0][p][t] = make_double2((double)S.x[t * kPhC + 2 * p], (double)S.x[t * kPhC + 2 * p + 1]);
+        S.buf[0][p][t] = make_double2((double)S.x[t * kPhC + 2 * p] * S.cscale[2 * p],
+                                      (double)S.x[t * kPhC + 2 * p + 1] * S.cscale[2 * p + 1]);
     }
     __syncthreads();
-    fft625x4(S, tid);
+    fft625x4<false>(S, tid);
     for (int i = tid; i < 4 * kPhT; i += kPhThreads) {
         const int p = i / kPhT, k = i % kPhT;
         const double2 z = S.buf[0][p][k];
@@ -110,9 +151,10 @@ phase_coupling_filter_kernel(const float* __restrict__ x, float* __restrict__ y,
         S.buf[0][p][k] = wv;
     }
     __syncthreads();
-    fft625x4(S, tid);
-    // now H[x_{2p}](t) = Re(buf) / N,  H[x_{2p+1}](t) = -Im(buf) / N
-    // ---- 2./3. phase unit vectors and the pairwise sums ---------------------------------------------------------------
+    // H[s x_{2p}] = Re / N, H[s x_{2p+1}] = -Im / N: the last stage writes buf = (H[x_{2p}], H[x_{2p+1}]), and H = 0 for
+    // an all-zero channel instead of the leak of its pair partner
+    fft625x4<true>(S, tid);
+    // ---- 2./3. phase unit vectors and the pairwise sums: angle(0) = 0 like np.angle, a NaN phase stays NaN ---------------
     double acc[28];
 #pragma unroll
     for (int q = 0; q < 28; ++q) acc[q] = 0.0;
@@ -122,10 +164,10 @@ phase_coupling_filter_kernel(const float* __restrict__ x, float* __restrict__ y,
         for (int c = 0; c < 8; ++c) {
             const double2 hv = S.buf[0][c >> 1][t];
             const double re = (double)S.x[t * kPhC + c];
-            const double im = ((c & 1) ? -hv.y : hv.x) * (1.0 / kPhT);
+            const double im = (c & 1) ? hv.y : hv.x;
             const double r = sqrt(re * re + im * im);
-            cs[c] = r > 0.0 ? re / r : 1.0;
-            sn[c] = r > 0.0 ? im / r : 0.0;
+            cs[c] = r == 0.0 ? 1.0 : re / r;
+            sn[c] = r == 0.0 ? 0.0 : im / r;
         }
         int q = 0;
 #pragma unroll
@@ -176,7 +218,7 @@ phase_coupling_filter_kernel(const float* __restrict__ x, float* __restrict__ y,
                 const double a = fabs(S.A[r][col]);
                 if (a > best) { best = a; piv = r; }
             }
-            if (!(best > 0.0) || !isfinite(best)) singular = true;
+            if (best == 0.0) singular = true;           // an exactly zero pivot, as LAPACK's getrf reports; NaN is not singular
             __syncwarp();
             if (piv != col && tid < 16) { const double tmp = S.A[col][tid]; S.A[col][tid] = S.A[piv][tid]; S.A[piv][tid] = tmp; }
             __syncwarp();

@@ -100,7 +100,7 @@ def filter_windows(x: torch.Tensor, fs: float = 125.0, chain: Sequence[Tuple[str
     ops._require_cuda(x)
     if x.dim() != 3:
         raise ValueError(f"filter_windows expects [B,T,C], got {tuple(x.shape)}")
-    x = ops._f32c(x)
+    x = ops._aligned16(ops._f32c(x))
     B, T, C = x.shape
     sos = chain_sos(chain, fs)
     nsec = np.array([s.shape[0] for s in sos], dtype=np.int32)

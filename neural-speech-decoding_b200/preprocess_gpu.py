@@ -49,7 +49,7 @@ class PhaseCouplingFilterGPU:
         ops._require_cuda(x)
         if x.dim() != 3 or x.shape[1] != T_WINDOW or x.shape[2] != N_CHANNELS:
             raise ValueError(f"Expected windows of shape [B, {T_WINDOW}, {N_CHANNELS}], got {tuple(x.shape)}")
-        x = ops._f32c(x)
+        x = ops._aligned16(ops._f32c(x))
         y = torch.empty_like(x)
         if x.shape[0] == 0:
             return y
@@ -63,7 +63,8 @@ class PhaseCouplingFilterGPU:
 
     def check(self) -> None:
         """Raise ``numpy.linalg.LinAlgError`` (what the reference's ``np.linalg.inv`` raises) if a window of the last
-        batch had a singular system."""
+        batch had a singular system: an exactly zero pivot, as LAPACK reports it.  A window holding NaN or Inf is not
+        singular; like the reference, its output is NaN."""
         st = getattr(self, "_last_status", None)
         if st is not None and int(st[0].item()) != 0:
             raise np.linalg.LinAlgError("Singular matrix")

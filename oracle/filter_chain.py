@@ -29,10 +29,18 @@ def cascade(x, sos, state):
     return y
 
 
-def collector_chain(window_TxC, fs=125.0, sos_list=None, carry_state=True, detrend=True, decimals=7):
-    """[T, C] float -> [T, C] float32, the values the collector would write (and the loader read back)."""
+def collector_round(x, decimals):
+    """The collector's output rule: np.round(x, decimals) (skipped for decimals < 0), negative zero cleared, float32."""
+    x = np.asarray(x, dtype=np.float64)
+    if decimals >= 0:
+        x = np.round(x, decimals)
+        x[x == 0] = 0.0
+    return x.astype(np.float32)
+
+
+def zero_phase_chain(window_TxC, sos_list, carry_state=True, detrend=True):
+    """[T, C] -> [T, C] float64 before rounding: the explicit-loop restatement, one channel at a time."""
     x = np.asarray(window_TxC, dtype=np.float64)
-    sos_list = sos_list if sos_list is not None else [scipy_sos(k, lo, hi, o, fs) for k, lo, hi, o in CHAIN]
     out = np.empty_like(x)
     for c in range(x.shape[1]):
         v = x[:, c].copy()
@@ -45,7 +53,27 @@ def collector_chain(window_TxC, fs=125.0, sos_list=None, carry_state=True, detre
                 st[:] = 0.0
             v = cascade(v[::-1].copy(), sos, st)[::-1].copy()
         out[:, c] = v
-    if decimals >= 0:
-        out = np.round(out, decimals)
-        out[out == 0] = 0.0
-    return out.astype(np.float32)
+    return out
+
+
+def zero_phase_chain_sosfilt(x, sos_list, carry_state=True, detrend=True, axis=-2):
+    """zero_phase_chain for any number of series at once (default layout [..., T, C]), float64, with
+    scipy.signal.sosfilt.  Carrying sosfilt's final state into the reversed pass continues the same filter, which is
+    what carrying the DirectFormII state does; the two differ only by rounding."""
+    x = np.asarray(x, dtype=np.float64)
+    if detrend:
+        x = x - x.mean(axis=axis, keepdims=True)
+    for sos in sos_list:
+        zshape = list(x.shape)
+        zshape[axis] = 2
+        zeros = np.zeros((sos.shape[0], *zshape))
+        y, zf = signal.sosfilt(sos, x, axis=axis, zi=zeros)
+        y, _ = signal.sosfilt(sos, np.flip(y, axis), axis=axis, zi=zf if carry_state else zeros)
+        x = np.flip(y, axis)
+    return np.ascontiguousarray(x)
+
+
+def collector_chain(window_TxC, fs=125.0, sos_list=None, carry_state=True, detrend=True, decimals=7):
+    """[T, C] float -> [T, C] float32, the values the collector would write (and the loader read back)."""
+    sos_list = sos_list if sos_list is not None else [scipy_sos(k, lo, hi, o, fs) for k, lo, hi, o in CHAIN]
+    return collector_round(zero_phase_chain(window_TxC, sos_list, carry_state, detrend), decimals)
