@@ -79,6 +79,7 @@ int na_ffma_probe(float* out, int64_t blocks, int64_t iters, na_stream_t stream)
  *          (a [B,T,C] batch is the case hop == T)
  *   y      normalize ? z-scored : copied windows, fp32 or bf16 (out_dtype), in
  *          out_tmp ? TMP layout [T][Bp][C] (rows >= B zero-filled) : [B][T][C]
+ *   C      any C >= 1 for a copy; C <= 256 with normalize (NA_EUNSUPPORTED above)
  */
 int na_window_zscore(const float* x, void* y, int64_t B, int64_t T, int64_t C, int64_t hop,
                      int normalize, int out_tmp, int64_t Bp, int out_dtype, na_stream_t stream);
@@ -92,7 +93,9 @@ int na_pack_lstm_layer(const float* w_ih, const float* w_hh, const float* b_ih, 
                        float* wt, float* bias, int64_t K, int64_t H, na_stream_t stream);
 
 /* ---- K3: one LSTM layer, all timesteps, h0 = c0 = 0 -------------------------------------
- * Replaces `self.lstm(x)` (lstm_eeg_model.py:34), one layer per call.
+ * Replaces `self.lstm(x)` (lstm_eeg_model.py:34), one layer per call.  Every 1 <= K <= 4096,
+ * 1 <= H <= 1024 runs, forward and backward, with or without the initial state below (the
+ * generic kernels: at most 512 threads a CTA, a thread owns two hidden units when H > 512).
  *   in    TMP [T][Bp][K]       hout TMP [T][Bp][H]
  *   cout  TMP [T][Bp][H]  or NULL   (cell state, saved for backward)
  *   gates TMP [T][Bp][4H] or NULL   (activated i,f,g,o, saved for backward)
@@ -156,7 +159,7 @@ int na_lstm_layer_wgrad_f32_hx(const float* dgates, const float* in, const float
 
 /* ---- K4: attention pool + LayerNorm + MLP head (+ softmax) -------------------------------
  * Replaces lstm_eeg_model.py:35-39 and, when probs != NULL, F.softmax at :97.
- *   h TMP [T][Bp][H];  attn_w [H], attn_b [1], ln_w [H], ln_b [H],
+ *   h TMP [T][Bp][H] (1 <= H <= 1024, 1 <= NC <= NA_MAX_CLASSES);  attn_w [H], attn_b [1], ln_w [H], ln_b [H],
  *   fc0_w [32,H], fc0_b [32], fc3_w [NC,32], fc3_b [NC]
  *   rrelu_slope [B,32] or NULL (eval: (1/8+1/3)/2), drop_mask [B,32] 0/1 or NULL, drop_scale
  *   logits [B,NC]; probs [B,NC] or NULL

@@ -21,6 +21,26 @@ int check_launch(const char* what);   // cudaGetLastError -> code + message
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// Before a launch of `threads` per block with `smem` bytes of dynamic shared memory: fails with NA_EUNSUPPORTED when the
+// kernel as compiled cannot run that many threads (its registers decide), and opts in to shared memory beyond the 48 KB
+// default, which covers static and dynamic shared memory together.  A launch that would be refused fails here with a
+// message that names the limit instead of as "too many resources requested for launch".
+template <typename Kernel>
+int prepare_launch(Kernel kern, int threads, size_t smem, const char* what) {
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, kern);
+    if (e != cudaSuccess) return fail((int)e, "%s: cudaFuncGetAttributes failed (%s)", what, cudaGetErrorString(e));
+    if (threads > a.maxThreadsPerBlock)
+        return fail(NA_EUNSUPPORTED, "%s: %d threads per block exceed the kernel's limit of %d (%d registers per thread)", what,
+                    threads, a.maxThreadsPerBlock, a.numRegs);
+    if (a.sharedSizeBytes + smem > 48 * 1024) {
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess)
+            return fail((int)e, "%s: opt-in to %zu bytes of shared memory failed (%s)", what, smem, cudaGetErrorString(e));
+    }
+    return NA_OK;
+}
+
 #define NA_REQUIRE(cond, code, ...)                          \
     do {                                                     \
         if (!(cond)) return ::na::fail((code), __VA_ARGS__); \

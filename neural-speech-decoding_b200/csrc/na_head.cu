@@ -330,9 +330,8 @@ int launch_head_fwd(const float* h, const HeadParams& p, float* logits, float* p
                     int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, cudaStream_t st,
                     const float* zpool_in = nullptr, float* scores_tm = nullptr, float* pooled = nullptr,
                     float* embedding = nullptr) {
-    const size_t smem = sizeof(float) * (H * (kFc + 1) + kHeadWarps * H);
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(head_fwd_kernel<JPL, CH, kEx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = sizeof(float) * (H * (kFc + 1) + kHeadWarps * H);      // 164 KB at H = 1024
+    if (int rc = prepare_launch(head_fwd_kernel<JPL, CH, kEx>, kHeadWarps * 32, smem, "na_head_fwd_f32")) return rc;
     const unsigned grid = (unsigned)((B + kHeadWarps - 1) / kHeadWarps);
     head_fwd_kernel<JPL, CH, kEx><<<grid, kHeadWarps * 32, smem, st>>>(h, p, logits, probs, stats, zpool, zpool_in, (int)T, B, Bp,
                                                                      (int)H, (int)NC, scores_tm, pooled, embedding);
@@ -344,9 +343,8 @@ template <int JPL, int CH>
 int launch_head_bwd(const float* dlogits, const float* h, const float* stats, const float* zpool,
                     const HeadParams& p, float* dh, float* scratch, float* wa_partial, int64_t T, int64_t B,
                     int64_t Bp, int64_t H, int64_t NC, cudaStream_t st, float* dz_out = nullptr) {
-    const size_t smem = sizeof(float) * (H * (kFc + 1) + kHeadWarps * H + kHeadWarps * (H + 1));
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(head_bwd_kernel<JPL, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = sizeof(float) * (H * (kFc + 1) + kHeadWarps * H + kHeadWarps * (H + 1));   // 196 KB at H = 1024
+    if (int rc = prepare_launch(head_bwd_kernel<JPL, CH>, kHeadWarps * 32, smem, "na_head_bwd_f32")) return rc;
     const unsigned grid = (unsigned)(Bp / kHeadWarps);
     head_bwd_kernel<JPL, CH><<<grid, kHeadWarps * 32, smem, st>>>(dlogits, h, stats, zpool, p, dh, scratch,
                                                                 wa_partial, dz_out, (int)T, B, Bp, (int)H, (int)NC);

@@ -253,6 +253,23 @@ window_zscore_generic_kernel(const float* __restrict__ x, void* __restrict__ y, 
     }
 }
 
+// Layout copy (normalize = 0) of windows with more channels than a CTA has threads (the LSTM's input_size reaches 4096):
+// thread = channel, strided over the C channels, one time row after another.
+__global__ void __launch_bounds__(kWinThreads)
+window_copy_wide_kernel(const float* __restrict__ x, void* __restrict__ y, int64_t B, int64_t T, int64_t C, int64_t hop,
+                        int out_tmp, int64_t Bp, int out_dtype) {
+    const int64_t b = blockIdx.x;
+    const float* src = x + b * hop * C;
+    for (int64_t r = 0; r < T; ++r)
+        for (int64_t c = threadIdx.x; c < C; c += kWinThreads) {
+            const float v = (b < B) ? src[r * C + c] : 0.f;
+            const int64_t o = out_tmp ? ((r * Bp + b) * C + c) : ((b * T + r) * C + c);
+            if (out_dtype == NA_F32) reinterpret_cast<float*>(y)[o] = v;
+            else if (out_dtype == NA_F16) reinterpret_cast<__half*>(y)[o] = __float2half_rn(kF16InScale * v);
+            else reinterpret_cast<__nv_bfloat16*>(y)[o] = __float2bfloat16_rn(v);
+        }
+}
+
 }  // namespace na
 
 extern "C" int na_window_zscore(const float* x, void* y, int64_t B, int64_t T, int64_t C, int64_t hop,
@@ -262,7 +279,8 @@ extern "C" int na_window_zscore(const float* x, void* y, int64_t B, int64_t T, i
     NA_REQUIRE(B >= 0 && T >= 1 && C >= 1 && hop >= 1, NA_EINVAL,
                "na_window_zscore: bad shape B=%lld T=%lld C=%lld hop=%lld", (long long)B, (long long)T,
                (long long)C, (long long)hop);
-    NA_REQUIRE(C <= kWinThreads, NA_EUNSUPPORTED, "na_window_zscore: C=%lld > %d", (long long)C, kWinThreads);
+    NA_REQUIRE(C <= kWinThreads || !normalize, NA_EUNSUPPORTED, "na_window_zscore: C=%lld > %d with normalize", (long long)C,
+               kWinThreads);
     NA_REQUIRE(out_dtype == NA_F32 || out_dtype == NA_BF16 || out_dtype == NA_F16, NA_EINVAL, "na_window_zscore: bad out_dtype");
     if (!out_tmp) Bp = B;
     NA_REQUIRE(Bp >= B, NA_EINVAL, "na_window_zscore: Bp < B");
@@ -273,7 +291,9 @@ extern "C" int na_window_zscore(const float* x, void* y, int64_t B, int64_t T, i
     const dim3 grid((unsigned)Bp), block(kWinThreads);
     const int64_t nvec = (C % 4 == 0) ? T * (C / 4) : 0;
     const bool hop_ok = ((hop * C) % 4) == 0;   // every window start stays 16-byte aligned
-    if (C == 8 && hop_ok && out_tmp && out_dtype != NA_F32 && Bp % kPackWin == 0 && nvec <= 5 * kWinThreads &&
+    if (C > kWinThreads) {
+        window_copy_wide_kernel<<<grid, block, 0, st>>>(x, y, B, T, C, hop, out_tmp, Bp, out_dtype);
+    } else if (C == 8 && hop_ok && out_tmp && out_dtype != NA_F32 && Bp % kPackWin == 0 && nvec <= 5 * kWinThreads &&
         (size_t)T * kPackWin * 16 <= 200 * 1024) {
         const size_t smem = (size_t)T * kPackWin * 16;
         // the attribute is per device: set it on every launch (cheap), like the other wrappers do

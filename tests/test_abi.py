@@ -44,6 +44,7 @@ def test_error_codes_without_gpu(lib):
     assert lib.na_trial_mean_f32(ctypes.c_void_p(8), ctypes.c_void_p(16), 10, 5, None) == -2   # alignment
     assert lib.na_window_zscore(None, None, 4, 625, 8, 0, 1, 0, 4, 0, None) == -1
     assert lib.na_window_zscore(None, None, 4, 625, 1000, 625, 1, 0, 4, 0, None) == -3
+    assert lib.na_window_zscore(None, None, 4, 625, 1000, 625, 0, 0, 4, 0, None) == -1   # a copy takes any C: null pointer
     assert lib.na_lstm_layer_fwd_f32(*([None] * 7), 1.0, None, 625, 33, 8, 48, None) == -1   # Bp % 32
     assert lib.na_lstm_layer_fwd_f32(*([None] * 7), 1.0, None, 625, 32, 8, 4096, None) == -3  # H too large
     assert lib.na_head_fwd_f32(*([None] * 11), 1.0, *([None] * 4), 625, 4, 32, 48, 99, None) == -3
