@@ -194,6 +194,12 @@ int na_head_fwd_f32_ex(const float* h, const float* attn_w, const float* attn_b,
                        float* stats, float* zpool,
                        int64_t T, int64_t B, int64_t Bp, int64_t H, int64_t NC, na_stream_t stream);
 int na_attention_softmax_f32(const float* scores_tm, float* attn, int64_t T, int64_t B, na_stream_t stream);
+/* The attention pool of every prefix (lstm_eeg_model.py:35-37 on h[:, :t_j]): h TMP [T][Bp][H] (1 <= H <= 1024) ->
+ * pooled [B][P][H] fp32, P = ceil(T / stride), row j = the pooled vector of steps [0, t_j), t_j = min((j + 1) * stride, T).
+ * One warp per window runs the online softmax over time a step at a time and stores z / l at every prefix end; the rows
+ * go to na_head_tail_fwd_f32 as for na_decoder_prefix_pool_x3.  stride >= 1; only rows b < B of `pooled` are written. */
+int na_attention_pool_prefix_f32(const float* h, const float* attn_w, const float* attn_b, float* pooled, int64_t T,
+                                 int64_t B, int64_t Bp, int64_t H, int64_t stride, na_stream_t stream);
 
 /* Backward of na_head_fwd_f32.  dlogits [B,NC] -> dh TMP [T][Bp][H] (padding rows zeroed)
  * and the 8 head parameter gradients, packed in `dparams` as
@@ -309,6 +315,16 @@ int na_decoder_infer_x3_ex(const float* x, const void* packed,
  * Only rows b < B are written; every pointer 16-byte aligned. */
 int na_decoder_lstm_x3(const float* x, const void* packed, const float* h_init, const float* c_init, float* out,
                        float* h_n, float* c_n, int64_t T, int64_t B, na_stream_t stream);
+/* The attention-pooled vector of every prefix x[:, :t_j] of the windows, t_j = min((j + 1) * stride, T) for j < P =
+ * ceil(T / stride) (the last prefix is the whole window), from one pass of the same kernel and arithmetic: the LSTM is
+ * causal and the attention pool is an online softmax, so after the pool has taken in step t its state is the pooled
+ * vector of x[:, :t+1].  No head: pooled [B][P][48] fp32 (row j = sum_{t < t_j} alpha_t h_t with alpha the softmax of
+ * the scores over the prefix) is the input of na_head_tail_fwd_f32 over B * P rows, which gives the logits of
+ * lstm_eeg_model.py:32-39 on every prefix (EEG_LSTM.decode_prefixes).  The last prefix's row is bit-identical to the
+ * pooled output of na_decoder_infer_x3_ex.  stride >= 1 (a stride >= T gives one prefix); only rows b < B are written;
+ * every pointer 16-byte aligned. */
+int na_decoder_prefix_pool_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                              float* pooled, int64_t T, int64_t B, int64_t stride, na_stream_t stream);
 
 /* ---- tensor-core tier, wide hidden sizes (H = 96, 144, 192; BASELINE configs[4]: H = 192, T = 2500) --------
  * Same contract as na_decoder_infer_bf16 (lstm_eeg_model.py:32-39 + :97, eval mode; input_size 8, 2 layers),

@@ -27,6 +27,8 @@
 //   B1 (25 chunks x 208 rows): Wih_hi x6 | Whh_hi x6 | bias(hi,lo) | Wih_lo x6 | Whh_lo x6;  rows 192.. = attention
 //   K16 MMAs pair two chunks through the descriptor's leading-byte-offset, so (x_lo | zeros), (x_hi | zeros) and
 //   (ones | zeros) pairs need no copies.  220 KB of shared memory; head parameters are read from global memory.
+// Instantiations: the default (logits / probs), kEx (+ scores, pooled vector, LayerNorm output; DESIGN 10c), kSeq (the two
+// LSTM layers alone, model.lstm; 10d) and kPrefix (the pooled vector of every prefix x[:, :t_j], no head; 10f).
 #include "na_x3_common.cuh"
 
 namespace na {
@@ -142,6 +144,20 @@ __device__ __forceinline__ void x3_seq_init(SmemX3& S, const int q, const int g,
     }
 }
 
+// kPrefix: the pooled vector z / l of this thread's units (computed as the kEx pooled store computes it) to the prefix row
+// `pout` when the window is live; `pout` moves on to the next prefix's row.
+template <int kU>
+__device__ __forceinline__ void x3_store_prefix(float*& pout, const float* z, const float l, const bool live) {
+    if (live) {
+        float zp[kU];
+        const float inv = 1.0f / l;
+#pragma unroll
+        for (int j = 0; j < kU; ++j) zp[j] = z[j] * inv;
+        store_row<kU>(pout, zp);
+    }
+    pout += kH;
+}
+
 // TMEM loads without the wait: a phase issues all of its loads and waits once (x3_drained).
 __device__ __forceinline__ void x3_tmem_ld16_nowait(uint32_t taddr, uint32_t* v) {
     asm volatile(
@@ -183,7 +199,11 @@ __device__ __forceinline__ void x3_drained(uint64_t* bar, const int lane) {
 // kSeq (never together with kEx): no pooling and no head.  The cell states start from c_init [2][B][48] when it is given,
 // and every thread stores, for its own units and rows b < B, the last layer's h of every step into seq_out [B][T][48]
 // and both layers' h and c of the last step into h_n / c_n [2][B][48].
-template <int R, int NR, bool kEx, bool kSeq>
+// kPrefix (never together with kEx or kSeq): no head.  The online softmax pool holds, after it has taken in step t, the
+// pooled vector z / l of the prefix x[:, :t+1] (the LSTM is causal), so at every prefix end (t + 1 a multiple of
+// `stride`, and t = T - 1) every thread stores z / l of its own units and rows b < B into prefix_out [B][P][48],
+// P = ceil(T / stride).
+template <int R, int NR, bool kEx, bool kSeq, bool kPrefix>
 __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const int g, const int lane, const int nq, const int T,
                                                  const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                                  const int64_t b0, const int64_t B, const int NC,
@@ -193,7 +213,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                                                  float* __restrict__ logits, float* __restrict__ probs,
                                                  float* __restrict__ scores_tm, float* __restrict__ pooled,
                                                  float* __restrict__ embedding, const float* __restrict__ c_init,
-                                                 float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
+                                                 float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n,
+                                                 const int stride, float* __restrict__ prefix_out) {
     constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
@@ -233,6 +254,12 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             }
         }
     float mx = -INFINITY, l = 0.f;
+    float* pout = nullptr;                         // kPrefix: this thread's units of the next prefix to store,
+    int left = 0;                                  // and the steps the pool takes in until that prefix ends
+    if constexpr (kPrefix) {
+        pout = prefix_out + brow * ((T + stride - 1) / stride) * kH + gr0 * 4;
+        left = stride;
+    }
     auto pool = [&](float score) {                 // online softmax over time (lstm_eeg_model.py:35-37), fp32
         if (score > mx) {
             const float sc = expf(mx - score);
@@ -304,6 +331,11 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             cells(v, c1, S.h1, hprev);
             fence_proxy_async_smem();
             mbar_arrive(&S.h1_ready);
+            if constexpr (kPrefix)                 // after the arrival: the pooled state is final until the next pool
+                if (t >= 2 && --left == 0) {
+                    x3_store_prefix<kU>(pout, z, l, brow < B);
+                    left = stride;
+                }
             if constexpr (kSeq)
                 if (brow < B) {
                     store_row<kU>(seq_out + (brow * T + (t - 1)) * kH + gr0 * 4, hprev);
@@ -324,6 +356,10 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         pool(__uint_as_float(sc2[0]));
         if constexpr (kEx)
             if (ex_writer && scores_tm) scores_tm[(int64_t)(T - 1) * B + b0 + wrow] = __uint_as_float(sc2[0]);
+    }
+    if constexpr (kPrefix) {                       // the whole window is the last prefix; no head
+        x3_store_prefix<kU>(pout, z, l, brow < B);
+        return;
     }
     // ---- head: LN -> fc0 -> RReLU(eval) -> fc3 -> softmax (fp32; parameters from global memory) ------
     float* zx = reinterpret_cast<float*>(S.h0[0]);             // [128][49] floats <= the two h0 buffers
@@ -388,7 +424,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
 // Barrier 0 over the whole CTA from code that differs between warps (the tile loops of the two register budgets).
 __device__ __forceinline__ void x3_cta_sync() { asm volatile("barrier.sync 0;" ::: "memory"); }
 
-template <int NR, bool kEx = false, bool kSeq = false>
+template <int NR, bool kEx = false, bool kSeq = false, bool kPrefix = false>
 __global__ void __launch_bounds__(kX3InferThreads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
@@ -397,13 +433,14 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         const float* __restrict__ fc0_w, const float* __restrict__ fc0_b,
                         const float* __restrict__ fc3_w, const float* __restrict__ fc3_b,
                         float* __restrict__ logits, float* __restrict__ probs,
-                        int T, int64_t B, int NC, int nquarters,
+                        int T, int64_t B, int NC, int nquarters,    // kPrefix: NC = the prefix stride
                         float* __restrict__ scores_tm,              // kEx: [T][B] scores, [B][48] pooled / LayerNorm output
-                        float* __restrict__ pooled, float* __restrict__ embedding,
+                        float* __restrict__ pooled, float* __restrict__ embedding,   // kPrefix: pooled = [B][P][48]
                         const float* __restrict__ h_init,           // kSeq: initial state [2][B][48] (both or neither),
                         const float* __restrict__ c_init,           // the last layer's h [B][T][48], final state [2][B][48]
                         float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
     static_assert(!(kEx && kSeq), "the intermediates and the sequence output are separate instantiations");
+    static_assert(!(kPrefix && (kEx || kSeq)), "the prefix pool is an instantiation of its own");
     constexpr int kMmaWarp = 12, kProdWarp = 13, kTmemWarp = 15;     // producers: warps 13 and 14
     const bool seq_init = kSeq && h_init != nullptr;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -647,9 +684,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                 fence_proxy_async_smem();
                 x3_cta_sync();     // the previous tile is complete (barrier at its end): h0 / h1 are free
             }
-            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
-            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
-            else x3_epilogue_tile<4, NR, kEx, kSeq>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n);
+            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
+            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
+            else x3_epilogue_tile<4, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
         });
     }
 
@@ -774,4 +811,37 @@ extern "C" int na_decoder_lstm_x3(const float* x, const void* packed, const floa
 #undef NA_X3_SEQ_LAUNCH
     count_launch();
     return check_launch("na_decoder_lstm_x3");
+}
+
+extern "C" int na_decoder_prefix_pool_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                         float* pooled, int64_t T, int64_t B, int64_t stride, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_prefix_pool_x3: bad shape T=%lld B=%lld", (long long)T,
+               (long long)B);
+    NA_REQUIRE(stride >= 1, NA_EINVAL, "na_decoder_prefix_pool_x3: stride=%lld < 1", (long long)stride);
+    NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(pooled);
+    NA_REQUIRE(attn_w && attn_b, NA_EINVAL, "na_decoder_prefix_pool_x3: null parameter pointer");
+    const int st = (int)(stride < T ? stride : T);          // a stride past the window: one prefix, the whole window
+    const size_t smem = sizeof(tc::SmemX3) + 1024;
+    const int nquarters = (int)((B + 31) / 32);
+    const int sms = tc::x3_sms();
+    const int grid = nquarters < sms ? nquarters : sms;
+#define NA_X3_PREFIX_LAUNCH(NRV)                                                                                                     \
+    {                                                                                                                                \
+        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, false, false, true>,                                   \
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                                \
+        if (e != cudaSuccess) return fail((int)e, "na_decoder_prefix_pool_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e)); \
+        tc::decoder_infer_x3_kernel<NRV, false, false, true><<<grid, tc::kX3InferThreads, smem, as_stream(stream)>>>(                \
+            x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, \
+            nullptr, nullptr, (int)T, B, st, nquarters, nullptr, pooled, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);       \
+    }
+    switch (tc::g_x3_rcp_fma) {
+        case 0: NA_X3_PREFIX_LAUNCH(0) break;
+        case 2: NA_X3_PREFIX_LAUNCH(2) break;
+        case 3: NA_X3_PREFIX_LAUNCH(3) break;
+        default: NA_X3_PREFIX_LAUNCH(1) break;
+    }
+#undef NA_X3_PREFIX_LAUNCH
+    count_launch();
+    return check_launch("na_decoder_prefix_pool_x3");
 }

@@ -404,6 +404,110 @@ extern "C" int na_head_fwd_f32(const float* h, const float* attn_w, const float*
 }
 
 namespace na {
+// Attention pool of every prefix of the windows (EEG_LSTM.decode_prefixes on the FFMA path): h TMP [T][Bp][H] -> pooled
+// [B][P][H], row j = the softmax-over-time pool of steps [0, t_j), t_j = min((j + 1) stride, T), P = ceil(T / stride).  One
+// warp per window, h read once (rows of CH steps in flight, as in head_fwd_kernel).  The online softmax takes one step at a
+// time -- score attn_w . h_t + attn_b, the running max raised with the rescale exp(m_old - m_new) -- so that z / l is the
+// pooled vector of the prefix that ends at the step just taken in; it is stored at every prefix end.
+template <int JPL, int CH>
+__global__ void __launch_bounds__(kHeadWarps * 32)
+attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restrict__ attn_w, const float* __restrict__ attn_b,
+                             float* __restrict__ pooled, int T, int64_t B, int64_t Bp, int H, int stride) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t b = (int64_t)blockIdx.x * kHeadWarps + warp;
+    if (b >= B) return;
+    float wa[JPL], z[JPL];
+#pragma unroll
+    for (int i = 0; i < JPL; ++i) {
+        const int j = lane + 32 * i;
+        wa[i] = (j < H) ? attn_w[j] : 0.f;
+        z[i] = 0.f;
+    }
+    const float ba = attn_b[0];
+    float* out = pooled + b * ((T + stride - 1) / stride) * H;
+    float m = -INFINITY, l = 0.f;
+    int left = stride;                            // steps until the next prefix end
+    for (int t0 = 0; t0 < T; t0 += CH) {
+        float hv[CH][JPL];
+#pragma unroll
+        for (int u = 0; u < CH; ++u) {
+            const int t = t0 + u;
+            const float* row = h + ((int64_t)t * Bp + b) * H;
+#pragma unroll
+            for (int i = 0; i < JPL; ++i) {
+                const int j = lane + 32 * i;
+                hv[u][i] = (t < T && j < H) ? __ldg(row + j) : 0.f;
+            }
+        }
+        float s[CH];
+#pragma unroll
+        for (int u = 0; u < CH; ++u) {
+            float d = 0.f;
+#pragma unroll
+            for (int i = 0; i < JPL; ++i) d = fmaf(hv[u][i], wa[i], d);
+            s[u] = warp_sum(d) + ba;
+        }
+#pragma unroll
+        for (int u = 0; u < CH; ++u) {
+            const int t = t0 + u;
+            if (t >= T) break;
+            if (s[u] > m) {                       // first step: exp(-inf) = 0
+                const float sc = expf(m - s[u]);
+                l *= sc;
+#pragma unroll
+                for (int i = 0; i < JPL; ++i) z[i] *= sc;
+                m = s[u];
+            }
+            const float e = expf(s[u] - m);
+            l += e;
+#pragma unroll
+            for (int i = 0; i < JPL; ++i) z[i] = fmaf(e, hv[u][i], z[i]);
+            if (--left == 0 || t == T - 1) {
+                const float inv = 1.0f / l;
+#pragma unroll
+                for (int i = 0; i < JPL; ++i) {
+                    const int j = lane + 32 * i;
+                    if (j < H) out[j] = z[i] * inv;
+                }
+                out += H;
+                left = stride;
+            }
+        }
+    }
+}
+
+template <int JPL, int CH>
+int launch_attention_pool_prefix(const float* h, const float* attn_w, const float* attn_b, float* pooled, int64_t T, int64_t B,
+                                 int64_t Bp, int64_t H, int stride, cudaStream_t st) {
+    if (int rc = prepare_launch(attention_pool_prefix_kernel<JPL, CH>, kHeadWarps * 32, 0, "na_attention_pool_prefix_f32"))
+        return rc;
+    const unsigned grid = (unsigned)((B + kHeadWarps - 1) / kHeadWarps);
+    attention_pool_prefix_kernel<JPL, CH><<<grid, kHeadWarps * 32, 0, st>>>(h, attn_w, attn_b, pooled, (int)T, B, Bp, (int)H,
+                                                                           stride);
+    count_launch();
+    return check_launch("na_attention_pool_prefix_f32");
+}
+}  // namespace na
+
+extern "C" int na_attention_pool_prefix_f32(const float* h, const float* attn_w, const float* attn_b, float* pooled, int64_t T,
+                                            int64_t B, int64_t Bp, int64_t H, int64_t stride, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T <= INT32_MAX && B >= 1 && Bp >= B && Bp % NA_BATCH_ALIGN == 0, NA_EINVAL,
+               "na_attention_pool_prefix_f32: bad shape T=%lld B=%lld Bp=%lld", (long long)T, (long long)B, (long long)Bp);
+    NA_REQUIRE(H >= 1 && H <= 1024, NA_EUNSUPPORTED, "na_attention_pool_prefix_f32: H=%lld outside [1,1024]", (long long)H);
+    NA_REQUIRE(stride >= 1, NA_EINVAL, "na_attention_pool_prefix_f32: stride=%lld < 1", (long long)stride);
+    NA_REQUIRE_PTR(h); NA_REQUIRE_PTR(pooled);
+    NA_REQUIRE(attn_w && attn_b, NA_EINVAL, "na_attention_pool_prefix_f32: null parameter pointer");
+    const int sd = (int)(stride < T ? stride : T);          // a stride past the window: one prefix, the whole window
+    cudaStream_t st = as_stream(stream);
+    if (H <= 64) return launch_attention_pool_prefix<2, 8>(h, attn_w, attn_b, pooled, T, B, Bp, H, sd, st);
+    if (H <= 128) return launch_attention_pool_prefix<4, 4>(h, attn_w, attn_b, pooled, T, B, Bp, H, sd, st);
+    if (H <= 256) return launch_attention_pool_prefix<8, 2>(h, attn_w, attn_b, pooled, T, B, Bp, H, sd, st);
+    if (H <= 512) return launch_attention_pool_prefix<16, 1>(h, attn_w, attn_b, pooled, T, B, Bp, H, sd, st);
+    return launch_attention_pool_prefix<32, 1>(h, attn_w, attn_b, pooled, T, B, Bp, H, sd, st);
+}
+
+namespace na {
 // Attention weights from the time-major scores the inference kernels wrote: scores [T][B] -> attn [B][T], per window
 // alpha_t = exp(s_t - max_t s) / sum_t exp(s_t - max_t s) in fp32 (torch.softmax's two passes; a NaN score makes the
 // window's whole row NaN, as in torch).  A CTA owns 32 windows: lane = window for the reads (one 128-byte run per step),

@@ -9,6 +9,7 @@ hand-written sm_100a kernels (libneuroalpha_b200.so).  There is no CPU compute p
 from __future__ import annotations
 
 import math
+import operator
 from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import numpy as np
@@ -29,6 +30,14 @@ class DecoderOutputs(NamedTuple):
     attention: torch.Tensor     # [B, T]
     pooled: torch.Tensor        # [B, H]
     embedding: torch.Tensor     # [B, H]
+
+
+class PrefixOutputs(NamedTuple):
+    """``EEG_LSTM.decode_prefixes``: the eval forward of every prefix ``x[:, :t]`` of the windows, fp32 on the device of
+    ``x``.  ``logits[:, j]`` is ``decode(x[:, :lengths[j]])[0]``."""
+    lengths: torch.Tensor       # [P] long, t_j = min((j + 1) * stride, T); the last is T
+    logits: torch.Tensor        # [B, P, K]
+    probs: torch.Tensor         # [B, P, K]
 
 
 class Attributions(NamedTuple):
@@ -314,6 +323,49 @@ class EEG_LSTM(nn.Module):
             e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=x.device)
             return DecoderOutputs(e(0, K), e(0, K), e(0, T), e(0, H), e(0, H))
         return DecoderOutputs(*self._decode(x, True))
+
+    def decode_prefixes(self, x: torch.Tensor, stride: int = 1) -> PrefixOutputs:
+        """The decoder's output on every prefix of the windows, from one pass over them: ``x`` [B,T,C] on CUDA (T >= 1)
+        -> ``PrefixOutputs(lengths, logits, probs)`` for the P = ceil(T / stride) prefixes ``x[:, :t_j]``, ``t_j =
+        min((j + 1) * stride, T)`` (the last prefix is the whole window; a ``stride`` above T gives P = 1).  For an
+        accuracy-versus-decision-time curve, or to stop as soon as the decoder is confident.
+
+        ``logits[:, j]`` is ``decode(x[:, :t_j])[0]``, the reference's eval forward on the prefix, under the exact tier's
+        1e-5 contract: the LSTM is causal and the attention pool is an online softmax, so the pool's state after step t
+        is the pooled vector of ``x[:, :t+1]``; it is stored at every prefix end and the head runs on those vectors.  Eval
+        arithmetic whatever ``self.training`` is; ``compute_dtype`` does not apply (a float16 / bfloat16 ``x`` is
+        converted to fp32).  The flagship shape runs on the exact tensor-core kernel while ``ops.EXACT_TC`` is set, every
+        other shape on the FFMA kernels.  ``zscore_input`` raises ``ValueError``: the z-score takes its statistics from
+        the whole window, so a prefix of a normalised window is not a normalised prefix."""
+        if x.dim() != 3:
+            raise ValueError(f"expected x of shape [B,T,C], got {tuple(x.shape)}")
+        ops._require_cuda(x)
+        if x.shape[2] != self.lstm.input_size:
+            raise RuntimeError(f"input.size(-1) must be equal to input_size. Expected {self.lstm.input_size}, got {x.shape[2]}")
+        stride = operator.index(stride)
+        if stride < 1:
+            raise ValueError(f"stride must be >= 1, got {stride}")
+        B, T = x.shape[0], x.shape[1]
+        if T < 1:
+            raise ValueError("decode_prefixes needs windows of at least one step")
+        if self.zscore_input:
+            raise ValueError("decode_prefixes: zscore_input normalises with the statistics of the whole window, so a "
+                             "prefix of a normalised window is not a normalised prefix")
+        lengths = ops.prefix_lengths(T, stride, x.device)
+        if B == 0:
+            K = self.fc[3].out_features
+            e = torch.empty((0, lengths.numel(), K), dtype=torch.float32, device=x.device)
+            return PrefixOutputs(lengths, e, e.clone())
+        x32 = ops._aligned16(x.detach().float().contiguous())
+        head = [p.detach() for p in self._head_params()]
+        with torch.no_grad():
+            if ops.EXACT_TC and self.tc_supported():
+                logits, probs = ops.decoder_prefixes_x3(x32, self._packed_x3(), head, stride)
+            else:
+                L = self.lstm.num_layers
+                logits, probs = ops.decoder_prefixes(x32, [self.lstm.layer(l) for l in range(L)], head, stride,
+                                                     [self._packed(l) for l in range(L)])
+        return PrefixOutputs(lengths, logits, probs)
 
     def inject_noise(self, drop1: Optional[torch.Tensor] = None, rrelu_slope: Optional[torch.Tensor] = None,
                      drop2: Optional[torch.Tensor] = None) -> None:

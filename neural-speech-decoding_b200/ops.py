@@ -101,7 +101,7 @@ def all_custom_ops():
             decoder_pack_wide_bf16, decoder_infer_wide_bf16, x3_split_input, lstm_fwd_train_x3, lstm_bwd_x3, lstm_wgrad_x3,
             lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
             decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex, lstm_layer_fwd_hx, lstm_layer_bwd_hx,
-            lstm_layer_wgrad_hx, decoder_lstm_x3]
+            lstm_layer_wgrad_hx, decoder_lstm_x3, decoder_prefix_pool_x3, attention_pool_prefix]
 
 
 def launch_count() -> int:
@@ -691,6 +691,52 @@ def decoder_infer_x3_intermediates(x: Tensor, packed: Tensor,
     return _with_attention(decoder_infer_x3_ex(x, packed, list(head_params)))
 
 
+def num_prefixes(T: int, stride: int) -> int:
+    """P = ceil(T / stride): prefixes x[:, :t_j] with t_j = min((j + 1) * stride, T), the last one the whole window."""
+    return -(-T // stride)
+
+
+def prefix_lengths(T: int, stride: int, device=None) -> Tensor:
+    """The lengths t_j = min((j + 1) * stride, T) of the P prefixes, long [P]."""
+    return torch.clamp(torch.arange(1, num_prefixes(T, stride) + 1, dtype=torch.long, device=device) * stride, max=T)
+
+
+@torch.library.custom_op("neuroalpha::decoder_prefix_pool_x3", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_prefix_pool_x3(x: Tensor, packed: Tensor, attn_w: Tensor, attn_b: Tensor, stride: int) -> Tensor:
+    """The attention-pooled vector of every prefix of the windows from one pass of decoder_infer_x3's kernel and
+    arithmetic (no head): x [B,T,8] fp32 -> pooled [B,P,48], row j = the pool of x[:, :t_j] (see prefix_lengths)."""
+    _require_cuda(x, packed, attn_w, attn_b)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8:
+        raise RuntimeError("decoder_prefix_pool_x3: x must be fp32 [B, T, 8]")
+    x = _aligned16(x.contiguous())
+    pooled = torch.empty((B, num_prefixes(T, stride), 48), dtype=torch.float32, device=x.device)
+    _lib.call("na_decoder_prefix_pool_x3", x.data_ptr(), packed.data_ptr(), _f32c(attn_w).data_ptr(),
+              _f32c(attn_b).data_ptr(), pooled.data_ptr(), T, B, stride, _stream())
+    return pooled
+
+
+@decoder_prefix_pool_x3.register_fake
+def _(x, packed, attn_w, attn_b, stride):
+    return x.new_empty((x.shape[0], num_prefixes(x.shape[1], stride), 48), dtype=torch.float32)
+
+
+def _prefix_head(pooled: Tensor, head: Sequence[Tensor]) -> Tuple[Tensor, Tensor]:
+    """pooled [B,P,H] -> (logits [B,P,K], probs [B,P,K]): the head tail in eval arithmetic over the B * P rows."""
+    B, P, H = pooled.shape
+    logits, probs = head_tail_fwd(pooled.reshape(B * P, H), list(head), None, None, 1.0, True)
+    K = logits.shape[1]
+    return logits.view(B, P, K), probs.view(B, P, K)
+
+
+def decoder_prefixes_x3(x: Tensor, packed: Tensor, head_params: Sequence[Tensor], stride: int) -> Tuple[Tensor, Tensor]:
+    """Eval forward of every prefix of x [B,T,8] fp32 on the exact tensor-core kernel: (logits [B,P,K], probs [B,P,K]),
+    [:, j] = decoder_infer_x3 of x[:, :t_j].  head_params in EEG_LSTM._head_params() order."""
+    head = [_f32c(t) for t in head_params]
+    return _prefix_head(decoder_prefix_pool_x3(x, packed, head[0], head[1], stride), head)
+
+
 WIDE_HIDDEN = (96, 144, 192)          # hidden sizes of the streamed-weight tensor-core kernel (na_decoder_wide.cu)
 
 
@@ -822,6 +868,39 @@ def decoder_infer_intermediates(x: Tensor, lstm_params: Sequence[Sequence[Tensor
     """decoder_infer with the intermediates of the head: (logits, probs, attention [B,T], pooled [B,H], embedding [B,H]).
     The LSTM layers are the same launches; the head kernel writes the scores, the pooled vector and the LayerNorm output."""
     return _infer_ffma(x, lstm_params, head_params, True, zscore, packed, True)
+
+
+@torch.library.custom_op("neuroalpha::attention_pool_prefix", mutates_args=(), device_types="cuda")
+@_device_guard
+def attention_pool_prefix(h: Tensor, B: int, attn_w: Tensor, attn_b: Tensor, stride: int) -> Tensor:
+    """The attention pool of every prefix: h TMP [T,Bp,H] (the last LSTM layer's output) -> pooled [B,P,H], row j = the
+    softmax-over-time pool of steps [0, t_j) (see prefix_lengths)."""
+    _require_cuda(h, attn_w, attn_b)
+    T, Bp, H = h.shape
+    pooled = torch.empty((B, num_prefixes(T, stride), H), dtype=torch.float32, device=h.device)
+    _lib.call("na_attention_pool_prefix_f32", h.data_ptr(), _f32c(attn_w).data_ptr(), _f32c(attn_b).data_ptr(),
+              pooled.data_ptr(), T, B, Bp, H, stride, _stream())
+    return pooled
+
+
+@attention_pool_prefix.register_fake
+def _(h, B, attn_w, attn_b, stride):
+    return h.new_empty((B, num_prefixes(h.shape[0], stride), h.shape[2]), dtype=torch.float32)
+
+
+def decoder_prefixes(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor], stride: int,
+                     packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None) -> Tuple[Tensor, Tensor]:
+    """Eval forward of every prefix of x [B,T,C] on the FFMA kernels, any shape: the LSTM layers once over the whole
+    window as decoder_infer runs them, then attention_pool_prefix and the head tail over the B * P pooled rows ->
+    (logits [B,P,K], probs [B,P,K])."""
+    _require_cuda(x)
+    B, T, C = x.shape
+    cur = window_zscore(x, T, T, False, True, False)
+    for l, (w_ih, w_hh, b_ih, b_hh) in enumerate(lstm_params):
+        wt, bias = packed[l] if packed is not None else pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
+        cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
+    head = [_f32c(t) for t in head_params]
+    return _prefix_head(attention_pool_prefix(cur, B, head[0], head[1], stride), head)
 
 
 def _save(ctx, tensors: Sequence[Tensor], optional: Sequence[Optional[Tensor]]) -> None:
