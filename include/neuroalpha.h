@@ -200,6 +200,14 @@ int na_attention_softmax_f32(const float* scores_tm, float* attn, int64_t T, int
  * go to na_head_tail_fwd_f32 as for na_decoder_prefix_pool_x3.  stride >= 1; only rows b < B of `pooled` are written. */
 int na_attention_pool_prefix_f32(const float* h, const float* attn_w, const float* attn_b, float* pooled, int64_t T,
                                  int64_t B, int64_t Bp, int64_t H, int64_t stride, na_stream_t stream);
+/* The attention pool continued from a carried online-softmax state (EEG_LSTM.decode_stream on the FFMA path): h TMP
+ * [T][Bp][H] (1 <= H <= 1024) of the next chunk; m_in / l_in [B], z_in [B][H] = the running max, sum_t exp(s_t - m)
+ * and the unnormalised sum_t exp(s_t - m) h_t after the earlier chunks (all three or none: a fresh pool, m = -inf).
+ * -> pooled [B][H] = z / l after the chunk (the input of na_head_tail_fwd_f32) and the state m_out, l_out, z_out.  One
+ * warp per window, one step at a time, as na_attention_pool_prefix_f32 does.  Only rows b < B are written. */
+int na_attention_pool_stream_f32(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
+                                 const float* l_in, const float* z_in, float* pooled, float* m_out, float* l_out,
+                                 float* z_out, int64_t T, int64_t B, int64_t Bp, int64_t H, na_stream_t stream);
 
 /* Backward of na_head_fwd_f32.  dlogits [B,NC] -> dh TMP [T][Bp][H] (padding rows zeroed)
  * and the 8 head parameter gradients, packed in `dparams` as
@@ -325,6 +333,21 @@ int na_decoder_lstm_x3(const float* x, const void* packed, const float* h_init, 
  * every pointer 16-byte aligned. */
 int na_decoder_prefix_pool_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
                               float* pooled, int64_t T, int64_t B, int64_t stride, na_stream_t stream);
+/* The chunk x [B][T][8] of B streams, continuing each from its state after the chunks before (EEG_LSTM.decode_stream):
+ * logits / probs [B][NC] of everything each stream has received, the same kernel and arithmetic as
+ * na_decoder_infer_x3, and the state after this chunk.  The state is both LSTM layers' h and c (h_in / c_in, h_out /
+ * c_out [2][B][48]) and the attention pool's online softmax: m [B] = the running max of the scores, l [B] = sum_t
+ * exp(s_t - m), z [B][48] = sum_t exp(s_t - m) h_t (unnormalised; the pooled vector is z / l).  h_in, c_in, m_in, l_in
+ * and z_in are all given or all NULL (a fresh stream: zeros, and m = -inf).  Accuracy: streaming a window chunk by
+ * chunk gives, after each chunk, logits and probs bit-identical to na_decoder_infer_x3 on everything streamed so far,
+ * and h_out / c_out bit-identical to na_decoder_lstm_x3's h_n / c_n.  No output may overlap an input or another output
+ * (NA_EINVAL); probs may be NULL; only rows b < B are written; every pointer 16-byte aligned. */
+int na_decoder_stream_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                         const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                         const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
+                         const float* m_in, const float* l_in, const float* z_in, float* logits, float* probs,
+                         float* h_out, float* c_out, float* m_out, float* l_out, float* z_out, int64_t T, int64_t B,
+                         int64_t NC, na_stream_t stream);
 
 /* ---- tensor-core tier, wide hidden sizes (H = 96, 144, 192; BASELINE configs[4]: H = 192, T = 2500) --------
  * Same contract as na_decoder_infer_bf16 (lstm_eeg_model.py:32-39 + :97, eval mode; input_size 8, 2 layers),

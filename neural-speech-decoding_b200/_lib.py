@@ -35,6 +35,7 @@ SIGNATURES = {
     "na_head_fwd_f32_ex": (c_int, [P] * 9 + [P, P, F32, P, P, P, P, P, P, P, I64, I64, I64, I64, I64, P]),
     "na_attention_softmax_f32": (c_int, [P, P, I64, I64, P]),
     "na_attention_pool_prefix_f32": (c_int, [P, P, P, P, I64, I64, I64, I64, I64, P]),
+    "na_attention_pool_stream_f32": (c_int, [P] * 10 + [I64, I64, I64, I64, P]),
     "na_head_param_floats": (c_int64, [I64, I64]),
     "na_head_partial_floats": (c_int64, [I64, I64, I64]),
     "na_head_bwd_f32": (c_int, [P] * 12 + [P, P, F32, P, P, P, I64, I64, I64, I64, I64, P]),
@@ -50,6 +51,7 @@ SIGNATURES = {
     "na_decoder_infer_x3_ex": (c_int, [P] * 15 + [I64, I64, I64, P]),
     "na_decoder_lstm_x3": (c_int, [P] * 7 + [I64, I64, P]),
     "na_decoder_prefix_pool_x3": (c_int, [P] * 5 + [I64, I64, I64, P]),
+    "na_decoder_stream_x3": (c_int, [P] * 22 + [I64, I64, I64, P]),
     "na_decoder_wide_packed_bytes": (c_int64, [I64]),
     "na_decoder_wide_state_bytes": (c_int64, [I64]),
     "na_decoder_pack_wide_bf16": (c_int, [P] * 11 + [I64, P]),

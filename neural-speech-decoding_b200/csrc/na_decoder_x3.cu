@@ -28,7 +28,8 @@
 //   K16 MMAs pair two chunks through the descriptor's leading-byte-offset, so (x_lo | zeros), (x_hi | zeros) and
 //   (ones | zeros) pairs need no copies.  220 KB of shared memory; head parameters are read from global memory.
 // Instantiations: the default (logits / probs), kEx (+ scores, pooled vector, LayerNorm output; DESIGN 10c), kSeq (the two
-// LSTM layers alone, model.lstm; 10d) and kPrefix (the pooled vector of every prefix x[:, :t_j], no head; 10f).
+// LSTM layers alone, model.lstm; 10d), kPrefix (the pooled vector of every prefix x[:, :t_j], no head; 10f) and kStream
+// (the default's outputs from a carried LSTM and pool state, which it also returns; 10g).
 #include "na_x3_common.cuh"
 
 namespace na {
@@ -158,6 +159,39 @@ __device__ __forceinline__ void x3_store_prefix(float*& pout, const float* z, co
     pout += kH;
 }
 
+// kStream: the pool state of this thread's units and row b < B after the stream's earlier chunks -- the running max and
+// sum of exp(s - max) of the row, the unnormalised weighted sum z of the units -- when a state is given.  Otherwise the
+// registers keep the fresh state (-inf, 0, 0) they were initialised with.
+template <int kU>
+__device__ __forceinline__ void x3_stream_load(float& mx, float& l, float* z, const float* __restrict__ m_in,
+                                               const float* __restrict__ l_in, const float* __restrict__ z_in,
+                                               const int64_t b, const int64_t B, const int gr0) {
+    if (z_in && b < B) {
+        mx = m_in[b];
+        l = l_in[b];
+#pragma unroll
+        for (int j = 0; j < kU; j += 4) {
+            const float4 v = *reinterpret_cast<const float4*>(z_in + b * kH + gr0 * 4 + j);
+            z[j] = v.x; z[j + 1] = v.y; z[j + 2] = v.z; z[j + 3] = v.w;
+        }
+    }
+}
+
+// kStream: the pool state after the last step, for row b < B: z of this thread's units, and (max, sum) from one writer
+// per window (`writer`: g == 0, first row copy).
+template <int kU>
+__device__ __forceinline__ void x3_stream_store(const float* z, const float mx, const float l, float* __restrict__ m_out,
+                                                float* __restrict__ l_out, float* __restrict__ z_out, const int64_t b,
+                                                const int64_t B, const int gr0, const bool writer) {
+    if (b < B) {
+        store_row<kU>(z_out + b * kH + gr0 * 4, z);
+        if (writer) {
+            m_out[b] = mx;
+            l_out[b] = l;
+        }
+    }
+}
+
 // TMEM loads without the wait: a phase issues all of its loads and waits once (x3_drained).
 __device__ __forceinline__ void x3_tmem_ld16_nowait(uint32_t taddr, uint32_t* v) {
     asm volatile(
@@ -203,7 +237,12 @@ __device__ __forceinline__ void x3_drained(uint64_t* bar, const int lane) {
 // pooled vector z / l of the prefix x[:, :t+1] (the LSTM is causal), so at every prefix end (t + 1 a multiple of
 // `stride`, and t = T - 1) every thread stores z / l of its own units and rows b < B into prefix_out [B][P][48],
 // P = ceil(T / stride).
-template <int R, int NR, bool kEx, bool kSeq, bool kPrefix>
+// kStream (never together with the others): the default's pooling, flush and head, continuing a stream.  With a state,
+// the cell states start from c_init [2][B][48] as in kSeq (the caller has stored h_init) and the pool from
+// (m_in, l_in, z_in) [B], [B], [B][48]; every thread stores, for its own units and rows b < B, both layers' h and c of
+// the last step into h_n / c_n [2][B][48] and the pool's z after the last step into z_out [B][48]; the head's thread
+// stores the pool's max and sum into m_out / l_out [B].
+template <int R, int NR, bool kEx, bool kSeq, bool kPrefix, bool kStream>
 __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const int g, const int lane, const int nq, const int T,
                                                  const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                                  const int64_t b0, const int64_t B, const int NC,
@@ -214,7 +253,10 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                                                  float* __restrict__ scores_tm, float* __restrict__ pooled,
                                                  float* __restrict__ embedding, const float* __restrict__ c_init,
                                                  float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n,
-                                                 const int stride, float* __restrict__ prefix_out) {
+                                                 const int stride, float* __restrict__ prefix_out,
+                                                 const float* __restrict__ m_in, const float* __restrict__ l_in,
+                                                 const float* __restrict__ z_in, float* __restrict__ m_out,
+                                                 float* __restrict__ l_out, float* __restrict__ z_out) {
     constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
@@ -243,7 +285,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
 #pragma unroll
     for (int j = 0; j < kU; ++j) { c0[j] = 0.f; c1[j] = 0.f; z[j] = 0.f; hprev[j] = 0.f; }
     const int64_t brow = b0 + wrow;
-    if constexpr (kSeq)
+    if constexpr (kSeq || kStream)
         if (c_init && brow < B) {
 #pragma unroll
             for (int j = 0; j < kU; j += 4) {
@@ -254,6 +296,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             }
         }
     float mx = -INFINITY, l = 0.f;
+    if constexpr (kStream) x3_stream_load<kU>(mx, l, z, m_in, l_in, z_in, brow, B, gr0);
     float* pout = nullptr;                         // kPrefix: this thread's units of the next prefix to store,
     int left = 0;                                  // and the steps the pool takes in until that prefix ends
     if constexpr (kPrefix) {
@@ -310,7 +353,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             cells(v, c0, S.h0[n & 1], hl0);
             fence_proxy_async_smem();
             mbar_arrive(&S.h0_ready[n & 1]);
-            if constexpr (kSeq)
+            if constexpr (kSeq || kStream)
                 if (t == T - 1 && brow < B) {
                     store_row<kU>(h_n + brow * kH + gr0 * 4, hl0);
                     store_row<kU>(c_n + brow * kH + gr0 * 4, c0);
@@ -344,6 +387,11 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                         store_row<kU>(c_n + (B + brow) * kH + gr0 * 4, c1);
                     }
                 }
+            if constexpr (kStream)
+                if (t == T && brow < B) {
+                    store_row<kU>(h_n + (B + brow) * kH + gr0 * 4, hprev);
+                    store_row<kU>(c_n + (B + brow) * kH + gr0 * 4, c1);
+                }
         }
     }
     if constexpr (kSeq) return;
@@ -361,6 +409,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         x3_store_prefix<kU>(pout, z, l, brow < B);
         return;
     }
+    if constexpr (kStream) x3_stream_store<kU>(z, mx, l, m_out, l_out, z_out, brow, B, gr0, g == 0 && rp == 0);
     // ---- head: LN -> fc0 -> RReLU(eval) -> fc3 -> softmax (fp32; parameters from global memory) ------
     float* zx = reinterpret_cast<float*>(S.h0[0]);             // [128][49] floats <= the two h0 buffers
 #pragma unroll
@@ -424,7 +473,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
 // Barrier 0 over the whole CTA from code that differs between warps (the tile loops of the two register budgets).
 __device__ __forceinline__ void x3_cta_sync() { asm volatile("barrier.sync 0;" ::: "memory"); }
 
-template <int NR, bool kEx = false, bool kSeq = false, bool kPrefix = false>
+template <int NR, bool kEx = false, bool kSeq = false, bool kPrefix = false, bool kStream = false>
 __global__ void __launch_bounds__(kX3InferThreads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
@@ -438,11 +487,16 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         float* __restrict__ pooled, float* __restrict__ embedding,   // kPrefix: pooled = [B][P][48]
                         const float* __restrict__ h_init,           // kSeq: initial state [2][B][48] (both or neither),
                         const float* __restrict__ c_init,           // the last layer's h [B][T][48], final state [2][B][48]
-                        float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n) {
+                        float* __restrict__ seq_out, float* __restrict__ h_n, float* __restrict__ c_n,
+                        const float* __restrict__ m_in = nullptr,   // kStream: pool state in [B], [B], [B][48] (with h_init,
+                        const float* __restrict__ l_in = nullptr,   // c_init, or none), and out (with h_n, c_n)
+                        const float* __restrict__ z_in = nullptr, float* __restrict__ m_out = nullptr,
+                        float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr) {
     static_assert(!(kEx && kSeq), "the intermediates and the sequence output are separate instantiations");
     static_assert(!(kPrefix && (kEx || kSeq)), "the prefix pool is an instantiation of its own");
+    static_assert(!(kStream && (kEx || kSeq || kPrefix)), "the stream is an instantiation of its own");
     constexpr int kMmaWarp = 12, kProdWarp = 13, kTmemWarp = 15;     // producers: warps 13 and 14
-    const bool seq_init = kSeq && h_init != nullptr;
+    const bool seq_init = (kSeq || kStream) && h_init != nullptr;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     SmemX3& S = *reinterpret_cast<SmemX3*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
@@ -684,9 +738,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                 fence_proxy_async_smem();
                 x3_cta_sync();     // the previous tile is complete (barrier at its end): h0 / h1 are free
             }
-            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
-            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
-            else x3_epilogue_tile<4, NR, kEx, kSeq, kPrefix>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr);
+            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
+            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
+            else x3_epilogue_tile<4, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
         });
     }
 
@@ -844,4 +898,72 @@ extern "C" int na_decoder_prefix_pool_x3(const float* x, const void* packed, con
 #undef NA_X3_PREFIX_LAUNCH
     count_launch();
     return check_launch("na_decoder_prefix_pool_x3");
+}
+
+namespace na { namespace tc {
+// [p, p + n floats) and [q, q + m floats) share a byte (a NULL range shares none).
+static bool x3_overlap(const void* p, int64_t n, const void* q, int64_t m) {
+    if (!p || !q || n <= 0 || m <= 0) return false;
+    const uintptr_t a = reinterpret_cast<uintptr_t>(p), b = reinterpret_cast<uintptr_t>(q);
+    return a < b + (uintptr_t)m * 4 && b < a + (uintptr_t)n * 4;
+}
+} }
+
+extern "C" int na_decoder_stream_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                    const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                    const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
+                                    const float* m_in, const float* l_in, const float* z_in, float* logits, float* probs,
+                                    float* h_out, float* c_out, float* m_out, float* l_out, float* z_out, int64_t T,
+                                    int64_t B, int64_t NC, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_stream_x3: bad shape T=%lld B=%lld", (long long)T,
+               (long long)B);
+    NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_stream_x3: num_classes=%lld", (long long)NC);
+    NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(logits);
+    NA_OPTIONAL_PTR(probs);
+    NA_REQUIRE_PTR(h_out); NA_REQUIRE_PTR(c_out); NA_REQUIRE_PTR(m_out); NA_REQUIRE_PTR(l_out); NA_REQUIRE_PTR(z_out);
+    NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
+               "na_decoder_stream_x3: null parameter pointer");
+    const int given = (h_in != nullptr) + (c_in != nullptr) + (m_in != nullptr) + (l_in != nullptr) + (z_in != nullptr);
+    NA_REQUIRE(given == 0 || given == 5, NA_EINVAL,
+               "na_decoder_stream_x3: h_in, c_in, m_in, l_in and z_in must be given together (or all NULL)");
+    NA_OPTIONAL_PTR(h_in); NA_OPTIONAL_PTR(c_in); NA_OPTIONAL_PTR(m_in); NA_OPTIONAL_PTR(l_in); NA_OPTIONAL_PTR(z_in);
+    // The kernel's pointers are __restrict__: no output may share memory with an input or with another output.
+    const int64_t S = 2 * B * tc::kH;
+    const void* in[] = {x, h_in, c_in, m_in, l_in, z_in};
+    const int64_t in_n[] = {B * T * 8, S, S, B, B, B * tc::kH};
+    float* out[] = {logits, probs, h_out, c_out, m_out, l_out, z_out};
+    const int64_t out_n[] = {B * NC, B * NC, S, S, B, B, B * tc::kH};
+    const char* out_name[] = {"logits", "probs", "h_out", "c_out", "m_out", "l_out", "z_out"};
+    for (int i = 0; i < 7; ++i) {
+        for (int j = 0; j < 6; ++j)
+            NA_REQUIRE(!tc::x3_overlap(out[i], out_n[i], in[j], in_n[j]), NA_EINVAL,
+                       "na_decoder_stream_x3: %s overlaps an input", out_name[i]);
+        for (int j = 0; j < i; ++j)
+            NA_REQUIRE(!tc::x3_overlap(out[i], out_n[i], out[j], out_n[j]), NA_EINVAL,
+                       "na_decoder_stream_x3: %s overlaps %s", out_name[i], out_name[j]);
+    }
+    const size_t smem = sizeof(tc::SmemX3) + 1024;
+    const int nquarters = (int)((B + 31) / 32);
+    const int sms = tc::x3_sms();
+    const int grid = nquarters < sms ? nquarters : sms;
+#define NA_X3_STREAM_LAUNCH(NRV)                                                                                                     \
+    {                                                                                                                                \
+        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, false, false, false, true>,                            \
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                                \
+        if (e != cudaSuccess) return fail((int)e, "na_decoder_stream_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e)); \
+        tc::decoder_infer_x3_kernel<NRV, false, false, false, true><<<grid, tc::kX3InferThreads, smem, as_stream(stream)>>>(          \
+            x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, \
+            (int)T, B, (int)NC, nquarters, nullptr, nullptr, nullptr, h_in, c_in, nullptr, h_out, c_out, m_in, l_in, z_in, m_out,   \
+            l_out, z_out);                                                                                                           \
+    }
+    switch (tc::g_x3_rcp_fma) {
+        case 0: NA_X3_STREAM_LAUNCH(0) break;
+        case 2: NA_X3_STREAM_LAUNCH(2) break;
+        case 3: NA_X3_STREAM_LAUNCH(3) break;
+        default: NA_X3_STREAM_LAUNCH(1) break;
+    }
+#undef NA_X3_STREAM_LAUNCH
+    count_launch();
+    return check_launch("na_decoder_stream_x3");
 }

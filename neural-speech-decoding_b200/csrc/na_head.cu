@@ -409,10 +409,16 @@ namespace na {
 // warp per window, h read once (rows of CH steps in flight, as in head_fwd_kernel).  The online softmax takes one step at a
 // time -- score attn_w . h_t + attn_b, the running max raised with the rescale exp(m_old - m_new) -- so that z / l is the
 // pooled vector of the prefix that ends at the step just taken in; it is stored at every prefix end.
-template <int JPL, int CH>
+// kState (EEG_LSTM.decode_stream, with stride = T: one pooled row): the online softmax starts from the state (m, l, z)
+// the earlier chunks of the stream left, when m_in / l_in / z_in are given, and its state after the last step is stored
+// to m_out / l_out [B] and z_out [B][H].
+template <int JPL, int CH, bool kState = false>
 __global__ void __launch_bounds__(kHeadWarps * 32)
 attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restrict__ attn_w, const float* __restrict__ attn_b,
-                             float* __restrict__ pooled, int T, int64_t B, int64_t Bp, int H, int stride) {
+                             float* __restrict__ pooled, int T, int64_t B, int64_t Bp, int H, int stride,
+                             const float* __restrict__ m_in = nullptr, const float* __restrict__ l_in = nullptr,
+                             const float* __restrict__ z_in = nullptr, float* __restrict__ m_out = nullptr,
+                             float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t b = (int64_t)blockIdx.x * kHeadWarps + warp;
     if (b >= B) return;
@@ -426,6 +432,16 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
     const float ba = attn_b[0];
     float* out = pooled + b * ((T + stride - 1) / stride) * H;
     float m = -INFINITY, l = 0.f;
+    if constexpr (kState)
+        if (z_in) {
+            m = m_in[b];
+            l = l_in[b];
+#pragma unroll
+            for (int i = 0; i < JPL; ++i) {
+                const int j = lane + 32 * i;
+                if (j < H) z[i] = z_in[b * H + j];
+            }
+        }
     int left = stride;                            // steps until the next prefix end
     for (int t0 = 0; t0 < T; t0 += CH) {
         float hv[CH][JPL];
@@ -474,6 +490,17 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
             }
         }
     }
+    if constexpr (kState) {
+#pragma unroll
+        for (int i = 0; i < JPL; ++i) {
+            const int j = lane + 32 * i;
+            if (j < H) z_out[b * H + j] = z[i];
+        }
+        if (lane == 0) {
+            m_out[b] = m;
+            l_out[b] = l;
+        }
+    }
 }
 
 template <int JPL, int CH>
@@ -488,6 +515,45 @@ int launch_attention_pool_prefix(const float* h, const float* attn_w, const floa
     return check_launch("na_attention_pool_prefix_f32");
 }
 }  // namespace na
+
+namespace na {
+template <int JPL, int CH>
+int launch_attention_pool_stream(const float* h, const float* attn_w, const float* attn_b, const float* m_in, const float* l_in,
+                                 const float* z_in, float* pooled, float* m_out, float* l_out, float* z_out, int64_t T,
+                                 int64_t B, int64_t Bp, int64_t H, cudaStream_t st) {
+    if (int rc = prepare_launch(attention_pool_prefix_kernel<JPL, CH, true>, kHeadWarps * 32, 0, "na_attention_pool_stream_f32"))
+        return rc;
+    const unsigned grid = (unsigned)((B + kHeadWarps - 1) / kHeadWarps);
+    attention_pool_prefix_kernel<JPL, CH, true><<<grid, kHeadWarps * 32, 0, st>>>(
+        h, attn_w, attn_b, pooled, (int)T, B, Bp, (int)H, (int)T, m_in, l_in, z_in, m_out, l_out, z_out);
+    count_launch();
+    return check_launch("na_attention_pool_stream_f32");
+}
+}  // namespace na
+
+extern "C" int na_attention_pool_stream_f32(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
+                                            const float* l_in, const float* z_in, float* pooled, float* m_out, float* l_out,
+                                            float* z_out, int64_t T, int64_t B, int64_t Bp, int64_t H, na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T <= INT32_MAX && B >= 1 && Bp >= B && Bp % NA_BATCH_ALIGN == 0, NA_EINVAL,
+               "na_attention_pool_stream_f32: bad shape T=%lld B=%lld Bp=%lld", (long long)T, (long long)B, (long long)Bp);
+    NA_REQUIRE(H >= 1 && H <= 1024, NA_EUNSUPPORTED, "na_attention_pool_stream_f32: H=%lld outside [1,1024]", (long long)H);
+    NA_REQUIRE_PTR(h); NA_REQUIRE_PTR(pooled); NA_REQUIRE_PTR(m_out); NA_REQUIRE_PTR(l_out); NA_REQUIRE_PTR(z_out);
+    NA_REQUIRE(attn_w && attn_b, NA_EINVAL, "na_attention_pool_stream_f32: null parameter pointer");
+    const int given = (m_in != nullptr) + (l_in != nullptr) + (z_in != nullptr);
+    NA_REQUIRE(given == 0 || given == 3, NA_EINVAL,
+               "na_attention_pool_stream_f32: m_in, l_in and z_in must be given together (or all NULL)");
+    NA_OPTIONAL_PTR(m_in); NA_OPTIONAL_PTR(l_in); NA_OPTIONAL_PTR(z_in);
+    cudaStream_t st = as_stream(stream);
+#define NA_POOL_STREAM(JPL, CH) \
+    launch_attention_pool_stream<JPL, CH>(h, attn_w, attn_b, m_in, l_in, z_in, pooled, m_out, l_out, z_out, T, B, Bp, H, st)
+    if (H <= 64) return NA_POOL_STREAM(2, 8);
+    if (H <= 128) return NA_POOL_STREAM(4, 4);
+    if (H <= 256) return NA_POOL_STREAM(8, 2);
+    if (H <= 512) return NA_POOL_STREAM(16, 1);
+    return NA_POOL_STREAM(32, 1);
+#undef NA_POOL_STREAM
+}
 
 extern "C" int na_attention_pool_prefix_f32(const float* h, const float* attn_w, const float* attn_b, float* pooled, int64_t T,
                                             int64_t B, int64_t Bp, int64_t H, int64_t stride, na_stream_t stream) {

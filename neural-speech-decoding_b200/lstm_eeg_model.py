@@ -40,6 +40,28 @@ class PrefixOutputs(NamedTuple):
     probs: torch.Tensor         # [B, P, K]
 
 
+class DecoderState(NamedTuple):
+    """The state of B streams after the chunks ``EEG_LSTM.decode_stream`` has taken in, fp32 on the device of the chunks.
+    ``h`` / ``c`` have nn.LSTM's ``h_n`` / ``c_n`` layout (the same as ``model.lstm``'s), batch dimension 1; the three
+    attention-pool fields are the pool's online softmax over the steps seen so far, batch dimension 0: the running max
+    ``m`` of the scores s_t = attn(h_t), ``sum_t exp(s_t - m)`` and ``sum_t exp(s_t - m) h_t`` (the pooled vector is
+    ``pool_z / pool_sum[:, None]``).  Rows are independent: index, concatenate or reset them with plain torch (a fresh
+    row is ``EEG_LSTM.initial_stream_state``'s: zeros, ``pool_max = -inf``)."""
+    h: torch.Tensor             # [L, B, H]
+    c: torch.Tensor             # [L, B, H]
+    pool_max: torch.Tensor      # [B]
+    pool_sum: torch.Tensor      # [B]
+    pool_z: torch.Tensor        # [B, H]
+
+
+class StreamOutputs(NamedTuple):
+    """``EEG_LSTM.decode_stream``: the eval forward of everything each stream has received, and the state after the
+    chunk (fp32 on the device of ``x``)."""
+    logits: torch.Tensor        # [B, K]
+    probs: torch.Tensor         # [B, K]
+    state: DecoderState
+
+
 class Attributions(NamedTuple):
     """``EEG_LSTM.input_gradients`` / ``integrated_gradients``: fp32 on the device of ``x``."""
     logits: torch.Tensor        # [B, K], at x
@@ -366,6 +388,80 @@ class EEG_LSTM(nn.Module):
                 logits, probs = ops.decoder_prefixes(x32, [self.lstm.layer(l) for l in range(L)], head, stride,
                                                      [self._packed(l) for l in range(L)])
         return PrefixOutputs(lengths, logits, probs)
+
+    def initial_stream_state(self, B: int, device=None) -> DecoderState:
+        """The ``DecoderState`` of B streams that have seen nothing: zeros, except ``pool_max = -inf``.  ``device``
+        defaults to the parameters' device.  ``decode_stream(x, initial_stream_state(B))`` is ``decode_stream(x)`` bit
+        for bit."""
+        L, H = self.lstm.num_layers, self.lstm.hidden_size
+        dev = self.attn.weight.device if device is None else torch.device(device)
+        z = lambda *shape: torch.zeros(shape, dtype=torch.float32, device=dev)
+        return DecoderState(z(L, B, H), z(L, B, H), torch.full((B,), -math.inf, dtype=torch.float32, device=dev),
+                            z(B), z(B, H))
+
+    def _check_stream_state(self, state, B: int, device) -> DecoderState:
+        """``state`` as a ``DecoderState`` whose fields match chunks of B streams on ``device``; raises otherwise, naming
+        the field: ``ValueError`` for the wrong number of fields or a dtype other than float32, ``RuntimeError`` for a
+        shape or a device that does not match."""
+        if not isinstance(state, tuple) or len(state) != 5:
+            raise ValueError("state must be a DecoderState (h, c, pool_max, pool_sum, pool_z)")
+        state = DecoderState(*state)
+        L, H = self.lstm.num_layers, self.lstm.hidden_size
+        want = {"h": (L, B, H), "c": (L, B, H), "pool_max": (B,), "pool_sum": (B,), "pool_z": (B, H)}
+        for name, shape in want.items():
+            t = getattr(state, name)
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"state.{name} must be a tensor, got {type(t).__name__}")
+            if tuple(t.shape) != shape:
+                raise RuntimeError(f"state.{name} must have shape {list(shape)} for {B} streams, got {list(t.shape)}")
+            if t.dtype != torch.float32:
+                raise ValueError(f"state.{name} must be float32, got {t.dtype}")
+            if t.device != device:
+                raise RuntimeError(f"state.{name} is on {t.device}, the chunk on {device}")
+        return state
+
+    def decode_stream(self, x: torch.Tensor, state: Optional[DecoderState] = None) -> StreamOutputs:
+        """The decoder on recordings that arrive a chunk at a time: ``x`` [B,T,C] on CUDA (T >= 1) is the next chunk of
+        each of B streams, ``state`` the ``DecoderState`` the previous call returned (None: fresh streams) ->
+        ``StreamOutputs(logits, probs, state)``.  ``logits`` is ``decode(torch.cat(chunks, dim=1))[0]``, the eval
+        forward of everything each stream has received, at the cost of the new steps only: the LSTM carries its (h, c)
+        and the attention pool its online softmax (max, sum, weighted sum) from chunk to chunk.  The returned state is
+        new; the one passed in is never written.  For dynamic stopping on a live recording: after each chunk, compare
+        ``probs.max(1)`` with a threshold (``scripts/accuracy_vs_time.py``).
+
+        On the exact tier (``ops.EXACT_TC`` and the flagship shape) one fused kernel runs per call, and after each chunk
+        the logits and probs are bit-identical to ``decode`` of everything streamed so far, and ``state.h`` /
+        ``state.c`` to ``model.lstm``'s ``h_n`` / ``c_n``; every other shape runs on the FFMA kernels under the 1e-5
+        contract.  Eval arithmetic whatever ``self.training`` is; ``compute_dtype`` does not apply (a float16 /
+        bfloat16 ``x`` is converted to fp32).  ``zscore_input`` raises ``ValueError``: the z-score takes its statistics
+        from the whole window, which a stream does not have."""
+        if x.dim() != 3:
+            raise ValueError(f"expected x of shape [B,T,C], got {tuple(x.shape)}")
+        ops._require_cuda(x)
+        if x.shape[2] != self.lstm.input_size:
+            raise RuntimeError(f"input.size(-1) must be equal to input_size. Expected {self.lstm.input_size}, got {x.shape[2]}")
+        B, T = x.shape[0], x.shape[1]
+        if T < 1:
+            raise ValueError("decode_stream needs chunks of at least one step")
+        if self.zscore_input:
+            raise ValueError("decode_stream: zscore_input normalises with the statistics of the whole window, which a "
+                             "stream does not have")
+        if state is not None:
+            state = self._check_stream_state(state, B, x.device)
+        if B == 0:
+            K = self.fc[3].out_features
+            e = torch.empty((0, K), dtype=torch.float32, device=x.device)
+            return StreamOutputs(e, e.clone(), self.initial_stream_state(0, x.device))
+        x32 = ops._aligned16(x.detach().float().contiguous())
+        head = [p.detach() for p in self._head_params()]
+        with torch.no_grad():
+            if ops.EXACT_TC and self.tc_supported():
+                out = ops.decoder_stream_chunk_x3(x32, self._packed_x3(), head, state)
+            else:
+                L = self.lstm.num_layers
+                out = ops.decoder_stream_chunk(x32, [self.lstm.layer(l) for l in range(L)], head, state,
+                                               [self._packed(l) for l in range(L)])
+        return StreamOutputs(out[0], out[1], DecoderState(*out[2:]))
 
     def inject_noise(self, drop1: Optional[torch.Tensor] = None, rrelu_slope: Optional[torch.Tensor] = None,
                      drop2: Optional[torch.Tensor] = None) -> None:

@@ -101,7 +101,8 @@ def all_custom_ops():
             decoder_pack_wide_bf16, decoder_infer_wide_bf16, x3_split_input, lstm_fwd_train_x3, lstm_bwd_x3, lstm_wgrad_x3,
             lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
             decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex, lstm_layer_fwd_hx, lstm_layer_bwd_hx,
-            lstm_layer_wgrad_hx, decoder_lstm_x3, decoder_prefix_pool_x3, attention_pool_prefix]
+            lstm_layer_wgrad_hx, decoder_lstm_x3, decoder_prefix_pool_x3, attention_pool_prefix, decoder_stream_x3,
+            attention_pool_stream]
 
 
 def launch_count() -> int:
@@ -737,6 +738,58 @@ def decoder_prefixes_x3(x: Tensor, packed: Tensor, head_params: Sequence[Tensor]
     return _prefix_head(decoder_prefix_pool_x3(x, packed, head[0], head[1], stride), head)
 
 
+def _state_in(state: Optional[Sequence[Tensor]]) -> List[Optional[Tensor]]:
+    """The five fields of a stream state (h, c, pool max, pool sum, pool z) as contiguous 16-byte aligned tensors, or
+    five Nones for a fresh stream."""
+    if state is None:
+        return [None] * 5
+    return [_aligned16(_f32c(t)) for t in state]
+
+
+@torch.library.custom_op("neuroalpha::decoder_stream_x3", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_stream_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], h: Optional[Tensor], c: Optional[Tensor],
+                      m: Optional[Tensor], l: Optional[Tensor], z: Optional[Tensor]
+                      ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """The next chunk x [B,T,8] fp32 of B streams on decoder_infer_x3's kernel and arithmetic, continuing from the
+    stream state h / c [2,B,48], m / l [B], z [B,48] (all five or none: a fresh stream) -> (logits [B,K], probs [B,K],
+    and the state after the chunk: h, c, m, l, z).  The logits are those of decoder_infer_x3 on everything the streams
+    have received."""
+    _require_cuda(x, packed, h, c, m, l, z)
+    B, T, C = x.shape
+    if x.dtype != torch.float32 or C != 8:
+        raise RuntimeError("decoder_stream_x3: x must be fp32 [B, T, 8]")
+    x = _aligned16(x.contiguous())
+    h, c, m, l, z = _state_in(None if h is None else (h, c, m, l, z))
+    head = [_f32c(t) for t in head]
+    dev, f = x.device, torch.float32
+    NC = head[6].shape[0]
+    logits, probs = torch.empty((B, NC), dtype=f, device=dev), torch.empty((B, NC), dtype=f, device=dev)
+    h_out, c_out = torch.empty((2, B, 48), dtype=f, device=dev), torch.empty((2, B, 48), dtype=f, device=dev)
+    m_out, l_out = torch.empty((B,), dtype=f, device=dev), torch.empty((B,), dtype=f, device=dev)
+    z_out = torch.empty((B, 48), dtype=f, device=dev)
+    _lib.call("na_decoder_stream_x3", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              _ptr(h), _ptr(c), _ptr(m), _ptr(l), _ptr(z), logits.data_ptr(), probs.data_ptr(), h_out.data_ptr(),
+              c_out.data_ptr(), m_out.data_ptr(), l_out.data_ptr(), z_out.data_ptr(), T, B, NC, _stream())
+    return logits, probs, h_out, c_out, m_out, l_out, z_out
+
+
+@decoder_stream_x3.register_fake
+def _(x, packed, head, h, c, m, l, z):
+    B, NC, f = x.shape[0], head[6].shape[0], torch.float32
+    return (x.new_empty((B, NC), dtype=f), x.new_empty((B, NC), dtype=f), x.new_empty((2, B, 48), dtype=f),
+            x.new_empty((2, B, 48), dtype=f), x.new_empty((B,), dtype=f), x.new_empty((B,), dtype=f),
+            x.new_empty((B, 48), dtype=f))
+
+
+def decoder_stream_chunk_x3(x: Tensor, packed: Tensor, head_params: Sequence[Tensor],
+                            state: Optional[Sequence[Tensor]]) -> Tuple[Tensor, ...]:
+    """Eval forward of the next chunk x [B,T,8] fp32 of B streams on the exact tensor-core kernel, from ``state`` =
+    (h, c, pool max, pool sum, pool z) or None (fresh streams) -> (logits, probs, h, c, pool max, pool sum, pool z).
+    head_params in EEG_LSTM._head_params() order."""
+    return decoder_stream_x3(x, packed, list(head_params), *([None] * 5 if state is None else state))
+
+
 WIDE_HIDDEN = (96, 144, 192)          # hidden sizes of the streamed-weight tensor-core kernel (na_decoder_wide.cu)
 
 
@@ -901,6 +954,57 @@ def decoder_prefixes(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_pa
         cur = lstm_layer_fwd(cur, wt, bias, None, 1.0, False)[0]
     head = [_f32c(t) for t in head_params]
     return _prefix_head(attention_pool_prefix(cur, B, head[0], head[1], stride), head)
+
+
+@torch.library.custom_op("neuroalpha::attention_pool_stream", mutates_args=(), device_types="cuda")
+@_device_guard
+def attention_pool_stream(h: Tensor, B: int, attn_w: Tensor, attn_b: Tensor, m: Optional[Tensor], l: Optional[Tensor],
+                          z: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """The attention pool continued from the online-softmax state m / l [B], z [B,H] (all three or none: a fresh
+    pool) over the chunk h TMP [T,Bp,H] -> (pooled [B,H] = z / l after the chunk, m, l, z after the chunk)."""
+    _require_cuda(h, attn_w, attn_b, m, l, z)
+    T, Bp, H = h.shape
+    dev, f = h.device, torch.float32
+    pooled, z_out = torch.empty((B, H), dtype=f, device=dev), torch.empty((B, H), dtype=f, device=dev)
+    m_out, l_out = torch.empty((B,), dtype=f, device=dev), torch.empty((B,), dtype=f, device=dev)
+    _lib.call("na_attention_pool_stream_f32", h.data_ptr(), _f32c(attn_w).data_ptr(), _f32c(attn_b).data_ptr(), _ptr(m),
+              _ptr(l), _ptr(z), pooled.data_ptr(), m_out.data_ptr(), l_out.data_ptr(), z_out.data_ptr(), T, B, Bp, H,
+              _stream())
+    return pooled, m_out, l_out, z_out
+
+
+@attention_pool_stream.register_fake
+def _(h, B, attn_w, attn_b, m, l, z):
+    H, f = h.shape[2], torch.float32
+    return h.new_empty((B, H), dtype=f), h.new_empty((B,), dtype=f), h.new_empty((B,), dtype=f), h.new_empty((B, H), dtype=f)
+
+
+def decoder_stream_chunk(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
+                         state: Optional[Sequence[Tensor]], packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None
+                         ) -> Tuple[Tensor, ...]:
+    """Eval forward of the next chunk x [B,T,C] of B streams on the FFMA kernels, any shape: every LSTM layer from the
+    state's (h, c) (zeros for a fresh stream), then attention_pool_stream from the state's pool and the head tail ->
+    (logits, probs, h [L,B,H], c [L,B,H], pool max [B], pool sum [B], pool z [B,H])."""
+    _require_cuda(x)
+    B, T, C = x.shape
+    Bp = padded_batch(B)
+    h0, c0, m, l, z = _state_in(state)
+    cur = window_zscore(x, T, T, False, True, False)
+    h_n, c_n = [], []
+    for i, (w_ih, w_hh, b_ih, b_hh) in enumerate(lstm_params):
+        wt, bias = packed[i] if packed is not None else pack_lstm_layer(w_ih, w_hh, b_ih, b_hh)
+        H = bias.numel() // 4
+        hp = torch.zeros((Bp, H), dtype=torch.float32, device=x.device)      # TMP rows of the initial state
+        cp = torch.zeros((Bp, H), dtype=torch.float32, device=x.device)
+        if h0 is not None:
+            hp[:B], cp[:B] = h0[i], c0[i]
+        cur, c, _, _ = lstm_layer_fwd_hx(cur, wt, bias, None, 1.0, hp, cp)
+        h_n.append(cur[T - 1, :B])
+        c_n.append(c[T - 1, :B])
+    head = [_f32c(t) for t in head_params]
+    pooled, m, l, z = attention_pool_stream(cur, B, head[0], head[1], m, l, z)
+    logits, probs = head_tail_fwd(pooled, head, None, None, 1.0, True)
+    return logits, probs, torch.stack(h_n), torch.stack(c_n), m, l, z
 
 
 def _save(ctx, tensors: Sequence[Tensor], optional: Sequence[Optional[Tensor]]) -> None:
