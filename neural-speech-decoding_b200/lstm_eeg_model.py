@@ -284,13 +284,17 @@ class EEG_LSTM(nn.Module):
         (``ops.EXACT_TC_TRAIN``) and also takes fp16 / bf16 ``x``; otherwise the eval path of ``decode``."""
         half = (self.compute_dtype == torch.bfloat16 or x.dtype == torch.bfloat16
                 or self.attn.weight.dtype == torch.bfloat16)
+        # a dropout rate within 1.5 / 65536 of 1 scales h0 past fp16's range on the flagship tensor-core tiers
+        injected = (self._injected_noise or {}).get("drop1") is not None
+        tc_train_ok = (not (train and self.training and self.lstm.dropout > 0.0)
+                       or ops.tc_train_dropout_ok(self.dropout_p, mask_tensor=injected))
         if half and not (train and x.requires_grad):
-            if self.tc_supported():
+            if self.tc_supported() and tc_train_ok:
                 return "tc"
             if self.tc_wide_supported():
                 return "wide"
         if train:
-            if (ops.EXACT_TC_TRAIN and not half and self.tc_supported() and not x.requires_grad
+            if (ops.EXACT_TC_TRAIN and not half and self.tc_supported() and tc_train_ok and not x.requires_grad
                     and x.dtype in (torch.float32, torch.float16, torch.bfloat16)):
                 return "x3"
         elif ops.EXACT_TC and not half and self.tc_supported() and x.dtype == torch.float32 and x.shape[0] > 0:
@@ -625,7 +629,7 @@ class EEG_LSTM(nn.Module):
                     elif self.lstm.dropout > 0.0:
                         # no mask tensor: the kernels generate (and the backward re-generates) the keep-bits from
                         # a counter-based hash; the seed comes from torch's CPU generator (torch.manual_seed)
-                        drop1 = (int(torch.randint(0, 2 ** 62, (1,)).item()), int(round((1.0 - self.dropout_p) * 65536)))
+                        drop1 = (int(torch.randint(0, 2 ** 62, (1,)).item()), ops.drop1_thresh16(self.dropout_p))
                 train_forward = ops.decoder_train_forward_tc if tier == "tc" else ops.decoder_train_forward_x3
                 logits = train_forward(x, lstm_params, head, self.dropout_p, self.zscore_input, drop1, rr, d2)
             elif tier == "wide":

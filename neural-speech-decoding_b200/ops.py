@@ -97,7 +97,7 @@ def _device_guard(fn):
 def all_custom_ops():
     return [window_zscore, pack_lstm_layer, lstm_layer_fwd, lstm_layer_bwd, lstm_layer_wgrad, head_fwd,
             head_bwd, trial_mean, decoder_pack_bf16, decoder_infer_bf16, lstm2_fwd_train_bf16, lstm_bwd_bf16,
-            dropout_mask_u8, head_tail_fwd, head_tail_bwd, decoder_infer_bf16_x32, decoder_pack_x3, decoder_infer_x3,
+            _dropout_mask_u8, head_tail_fwd, head_tail_bwd, decoder_infer_bf16_x32, decoder_pack_x3, decoder_infer_x3,
             decoder_pack_wide_bf16, decoder_infer_wide_bf16, x3_split_input, lstm_fwd_train_x3, lstm_bwd_x3, lstm_wgrad_x3,
             lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
             decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex, lstm_layer_fwd_hx, lstm_layer_bwd_hx,
@@ -1256,19 +1256,33 @@ def _(dlogits, zpool, params, rrelu_slope, drop_mask, drop_scale):
     return zpool.new_empty(zpool.shape), zpool.new_empty((n,))
 
 
+def _seed_i64(seed: int) -> int:
+    """A dropout seed in [-2**63, 2**64) as the int64 with the same 64 bits: torch custom ops take int64 arguments, and the
+    C ABI's uint64_t parameter reads those bits back as the unsigned seed."""
+    seed = int(seed)
+    if not -2 ** 63 <= seed < 2 ** 64:
+        raise ValueError(f"dropout seed {seed} does not fit 64 bits")
+    return seed - 2 ** 64 if seed >= 2 ** 63 else seed
+
+
 @torch.library.custom_op("neuroalpha::dropout_mask_u8", mutates_args=(), device_types="cuda")
 @_device_guard
-def dropout_mask_u8(like: Tensor, seed: int, thresh16: int, T: int, Bp: int) -> Tensor:
-    """The keep-mask the in-kernel generator produces for (seed, thresh16): u8 [T,Bp,48] on like.device."""
+def _dropout_mask_u8(like: Tensor, seed: int, thresh16: int, T: int, Bp: int) -> Tensor:
     _require_cuda(like)
     out = torch.empty((T, Bp, 48), dtype=torch.uint8, device=like.device)
     _lib.call("na_dropout_mask_u8", int(seed), int(thresh16), T, Bp, out.data_ptr(), _stream())
     return out
 
 
-@dropout_mask_u8.register_fake
+@_dropout_mask_u8.register_fake
 def _(like, seed, thresh16, T, Bp):
     return like.new_empty((T, Bp, 48), dtype=torch.uint8)
+
+
+def dropout_mask_u8(like: Tensor, seed: int, thresh16: int, T: int, Bp: int) -> Tensor:
+    """The keep-mask the in-kernel generator produces for (seed, thresh16): u8 [T,Bp,48] on like.device.  ``seed``: any
+    uint64 (or its int64 bit pattern)."""
+    return _dropout_mask_u8(like, _seed_i64(seed), thresh16, T, Bp)
 
 
 @torch.library.custom_op("neuroalpha::lstm_bwd_bf16", mutates_args=(), device_types="cuda")
@@ -1344,16 +1358,43 @@ def _sm_count(device) -> int:
     return _SM_COUNT[idx]
 
 
+F16_MAX = 65504.0
+
+
+def drop1_thresh16(p: float) -> int:
+    """thresh16 of the in-kernel inter-layer dropout for dropout probability ``p``: P(keep) = thresh16 / 65536."""
+    return int(round((1.0 - p) * 65536))
+
+
+def tc_train_dropout_ok(p: float, mask_tensor: bool = False) -> bool:
+    """Whether the flagship tensor-core training tiers can apply inter-layer dropout ``p``.  Both store the kept h0 * scale
+    in fp16 (the 16-bit tier as its layer-1 operand, the exact tier as that operand's hi half), so the scale times |h0| <= 1
+    must stay within fp16's 65504.  The scale is 65536 / thresh16 for the in-kernel generator (thresh16 = 1 fails: p within
+    1.5 / 65536 of 1, not counting the p that round thresh16 to 0, which drop everything at scale 0), or 1 / (1 - p) for a
+    mask tensor (``mask_tensor``; fails for p > 1 - 1 / 65504).  The FFMA tier (fp32 throughout) trains those rates."""
+    if p >= 1.0:
+        return True
+    if mask_tensor:
+        return 1.0 / (1.0 - p) <= F16_MAX
+    th = drop1_thresh16(p)
+    return th == 0 or 65536.0 / th <= F16_MAX
+
+
 def _drop1_args(drop1, scale: float) -> Tuple[Optional[Tensor], int, int, float]:
     """``drop1`` of DecoderFunctionTC / X3 -> (mask, seed, thresh16, scale1) of the layer-0 training kernels: None (no
     inter-layer dropout), a u8 keep-mask (scaled like the head dropout), or ``(seed, thresh16)`` of the in-kernel
-    counter-based generator."""
+    counter-based generator (any uint64 seed).  A scale past fp16's range (see tc_train_dropout_ok) raises ValueError."""
     if isinstance(drop1, tuple):
-        seed, thresh16 = int(drop1[0]), int(drop1[1])
-        return None, seed, thresh16, 65536.0 / thresh16 if thresh16 > 0 else 0.0   # exactly unbiased for the quantised keep-rate
-    if drop1 is not None:
-        return drop1, 0, 65536, scale
-    return None, 0, 65536, 1.0
+        mask, seed, thresh16 = None, _seed_i64(drop1[0]), int(drop1[1])
+        scale1 = 65536.0 / thresh16 if thresh16 > 0 else 0.0      # exactly unbiased for the quantised keep-rate
+    elif drop1 is not None:
+        mask, seed, thresh16, scale1 = drop1, 0, 65536, scale
+    else:
+        return None, 0, 65536, 1.0
+    if scale1 > F16_MAX:
+        raise ValueError(f"inter-layer dropout scale {scale1} overflows the tensor-core tiers' fp16 operands (max {F16_MAX}); "
+                         "train this dropout rate on the FFMA tier")
+    return mask, seed, thresh16, scale1
 
 
 def _half_stride(B: int, device, half_tiles: bool) -> int:

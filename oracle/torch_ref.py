@@ -38,11 +38,15 @@ class RefEEGLSTM(nn.Module):
         return self.fc(self.ln(out))
 
 
-def explicit_forward(x, sd, num_layers=2, p=0.6, drop1_mask=None, rrelu_slope=None, drop2_mask=None):
+def explicit_forward(x, sd, num_layers=2, p=0.6, drop1_mask=None, rrelu_slope=None, drop2_mask=None, drop1_scale=None):
     """x [B,T,C]; sd: name -> tensor (may require grad).  Returns logits [B,K].
 
-    Masks are 0/1 tensors; scaling by 1/(1-p) is applied here, as torch's dropout does.
+    Masks are 0/1 tensors; scaling by 1/(1-p) (0 for p = 1) is applied here, as torch's dropout does.  ``drop1_scale``
+    replaces that factor for the inter-layer dropout (the in-kernel generator of the tensor-core tiers scales by
+    65536 / thresh16).
     """
+    scale = 1.0 / (1.0 - p) if p < 1.0 else 0.0
+    scale1 = scale if drop1_scale is None else drop1_scale
     inp = x
     for l in range(num_layers):
         w_ih, w_hh = sd[f"lstm.weight_ih_l{l}"], sd[f"lstm.weight_hh_l{l}"]
@@ -61,7 +65,7 @@ def explicit_forward(x, sd, num_layers=2, p=0.6, drop1_mask=None, rrelu_slope=No
             hs.append(h)
         inp = torch.stack(hs, dim=1)
         if drop1_mask is not None and l < num_layers - 1:
-            inp = inp * drop1_mask / (1.0 - p)
+            inp = inp * drop1_mask * scale1
     out = inp
     scores = out @ sd["attn.weight"][0] + sd["attn.bias"][0]
     w = torch.softmax(scores, dim=1)
@@ -71,5 +75,5 @@ def explicit_forward(x, sd, num_layers=2, p=0.6, drop1_mask=None, rrelu_slope=No
     slope = RRELU_EVAL_SLOPE if rrelu_slope is None else rrelu_slope
     a = torch.where(a >= 0, a, a * slope)
     if drop2_mask is not None:
-        a = a * drop2_mask / (1.0 - p)
+        a = a * drop2_mask * scale
     return a @ sd["fc.3.weight"].t() + sd["fc.3.bias"]

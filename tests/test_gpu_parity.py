@@ -596,7 +596,9 @@ def test_exact_tc_training_train_mode_injected_noise(dev, checkpoint):
 
 def test_exact_tc_training_in_kernel_dropout_equals_mask_mode(dev, checkpoint):
     """Counter-based in-kernel dropout of the exact tensor-core tier == the mask-tensor mode fed with the materialised
-    mask, bit for bit (logits and all gradients); the result is reproducible run to run."""
+    mask, bit for bit (logits and all gradients); the result is reproducible run to run.  Both runs pass p' = 1 -
+    thresh16 / 65536, so the mask mode's scale 1 / (1 - p') is exactly the generator's 65536 / thresh16 (and the head
+    dropout is scaled alike in both).  tests/test_gpu_dropout.py covers more shapes, layouts and both tiers."""
     from neural_speech_decoding_b200 import ops
     torch.manual_seed(4)
     B, T = 140, 21
@@ -607,19 +609,21 @@ def test_exact_tc_training_in_kernel_dropout_equals_mask_mode(dev, checkpoint):
     m = make_model(dev, checkpoint).train()
     lstm, head = [m.lstm.layer(l) for l in range(2)], m._head_params()
     seed, th = 123456789, int(round(0.4 * 65536))
+    p = 1.0 - th / 65536
     def run(drop1):
         m.zero_grad()
-        out = ops.decoder_train_forward_x3(x, lstm, head, 0.6, False, drop1, rr, d2)
+        out = ops.decoder_train_forward_x3(x, lstm, head, p, False, drop1, rr, d2)
         torch.nn.functional.cross_entropy(out, y).backward()
         return out.detach().clone(), [p.grad.clone() for p in m.parameters()]
     a, ga = run((seed, th))
     Bp = ops.padded_batch(B, ops.TC_TILE)
     mask = ops.dropout_mask_u8(x, seed, th, T, Bp)
-    # mask-tensor mode scales by 1 / (1 - p); the counter mode by 65536 / thresh16 (exactly unbiased for the quantised rate):
-    # identical here because 0.4 * 65536 rounds to 26214 and both are applied as the same fp32 factor only if equal -- so
-    # compare against the mask mode run with that exact factor
-    b, gb = run((seed, th))
-    assert torch.equal(a, b) and all(torch.equal(p, q) for p, q in zip(ga, gb))          # run-to-run reproducible
+    b, gb = run(mask)
+    assert torch.isfinite(a).all() and torch.equal(a, b), (a - b).abs().max().item()
+    for (k, _), u, v in zip(m.named_parameters(), ga, gb):
+        assert torch.equal(u, v), (k, (u - v).abs().max().item())
+    c, gc = run((seed, th))
+    assert torch.equal(a, c) and all(torch.equal(u, v) for u, v in zip(ga, gc))          # run-to-run reproducible
     assert abs(mask[:, :B].float().mean().item() - 0.4) < 0.01
 
 

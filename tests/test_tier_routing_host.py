@@ -286,3 +286,54 @@ def test_train_noise_seeded_and_injected(cpu_backend, monkeypatch, tier, inject)
         (call,) = rec.take()
         assert call["tier"] == tier
         _check_noise(call, tier, m, B, injected)
+
+
+@pytest.mark.parametrize("cdt", [F32, BF16])
+def test_dropout_rates_past_fp16_train_on_ffma(cpu_backend, monkeypatch, cdt):
+    """The flagship tensor-core tiers store the kept h0 * scale in fp16: a dropout rate whose scale passes 65504 trains on
+    the FFMA tier instead.  The scale is the generator's 65536 / thresh16 (thresh16 = 1 fails; thresh16 = 0, scale 0, does
+    not), or 1 / (1 - p) when an injected mask tensor replaces the generator.  Eval mode with gradients applies no dropout
+    and keeps its tier; p = 1 (scale 0) and thresh16 = 2 (scale 32768) stay on the tensor cores."""
+    from neural_speech_decoding_b200 import ops
+    rec = Recorder(monkeypatch)
+    monkeypatch.setattr(ops, "EXACT_TC_TRAIN", True)
+    tc = "tc" if cdt == BF16 else "x3"
+    B = 3
+    x = torch.randn(B, T, 8)
+    mask = (torch.rand(1, B, T, 48) >= 0.5).float()
+    # p -> (generator fits, mask tensor fits)
+    for p, ok_gen, ok_mask in [(1.0, True, True), (1 - 2 / 65536, True, True), (1 - 1.45 / 65536, False, True),
+                               (1 - 1 / 65536, False, False), (1 - 0.55 / 65536, False, False),
+                               (1 - 0.45 / 65536, True, False), (1 - 1e-9, True, False), (0.6, True, True)]:
+        assert ops.tc_train_dropout_ok(p) == ok_gen and ops.tc_train_dropout_ok(p, mask_tensor=True) == ok_mask, p
+        m = _model("flagship", F32)
+        m.compute_dtype, m.dropout_p, m.lstm.dropout = cdt, p, p
+        for inject, ok in ((None, ok_gen), (mask, ok_mask)):
+            m.inject_noise(drop1=inject)
+            for train in (True, False):
+                m.train(train)
+                m(x)
+                (call,) = rec.take()
+                assert call["tier"] == (tc if ok or not train else "ffma"), (p, inject is not None, train)
+    assert ops.drop1_thresh16(1 - 1 / 65536) == 1 and ops.drop1_thresh16(1 - 0.45 / 65536) == 0
+    assert ops.drop1_thresh16(0.6) == 26214
+
+
+def test_drop1_args_seed_bits_and_scale_limit():
+    from neural_speech_decoding_b200 import ops
+    for seed, want in [(0, 0), (2 ** 63 - 1, 2 ** 63 - 1), (2 ** 63, -2 ** 63), (2 ** 64 - 1, -1), (-5, -5)]:
+        assert ops._seed_i64(seed) == want
+        assert ops._drop1_args((seed, 26214), 2.5)[1] == want
+    for bad in (2 ** 64, -2 ** 63 - 1):
+        with pytest.raises(ValueError):
+            ops._seed_i64(bad)
+    assert ops._drop1_args((7, 26214), 2.5) == (None, 7, 26214, 65536 / 26214)
+    assert ops._drop1_args((7, 0), 0.0) == (None, 7, 0, 0.0)
+    assert ops._drop1_args((7, 2), 2.5)[3] == 32768.0
+    with pytest.raises(ValueError, match="fp16"):
+        ops._drop1_args((7, 1), 65536.0)                       # scale 65536
+    mask = torch.ones(1, dtype=torch.uint8)
+    assert ops._drop1_args(mask, 65504.0)[3] == 65504.0
+    with pytest.raises(ValueError, match="fp16"):
+        ops._drop1_args(mask, 65505.0)
+    assert ops._drop1_args(None, 2.5) == (None, 0, 65536, 1.0)
