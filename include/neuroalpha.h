@@ -208,6 +208,13 @@ int na_attention_pool_prefix_f32(const float* h, const float* attn_w, const floa
 int na_attention_pool_stream_f32(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
                                  const float* l_in, const float* z_in, float* pooled, float* m_out, float* l_out,
                                  float* z_out, int64_t T, int64_t B, int64_t Bp, int64_t H, na_stream_t stream);
+/* na_attention_pool_stream_f32 with a length per window (EEG_LSTM.decode_stream / decode with lengths on the FFMA path):
+ * window b takes in steps t < lengths[b] of h only (int32 [B] on the device, clamped to [0, T]); a window given no
+ * steps keeps its state, and its pooled row is the state's z / l (NaN for a fresh pool).  Only rows b < B are written. */
+int na_attention_pool_stream_ragged_f32(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
+                                        const float* l_in, const float* z_in, const int32_t* lengths, float* pooled,
+                                        float* m_out, float* l_out, float* z_out, int64_t T, int64_t B, int64_t Bp,
+                                        int64_t H, na_stream_t stream);
 
 /* Backward of na_head_fwd_f32.  dlogits [B,NC] -> dh TMP [T][Bp][H] (padding rows zeroed)
  * and the 8 head parameter gradients, packed in `dparams` as
@@ -348,6 +355,17 @@ int na_decoder_stream_x3(const float* x, const void* packed, const float* attn_w
                          const float* m_in, const float* l_in, const float* z_in, float* logits, float* probs,
                          float* h_out, float* c_out, float* m_out, float* l_out, float* z_out, int64_t T, int64_t B,
                          int64_t NC, na_stream_t stream);
+/* na_decoder_stream_x3 with a length per stream: row b takes only x[b, :lengths[b]] (int32 [B] on the device, required,
+ * clamped to [0, T]; x past a row's length is ignored, NaN included).  Its logits, probs and state are those of
+ * na_decoder_stream_x3 on the chunk x[b, :lengths[b]], bit for bit; a row given 0 steps returns its state unchanged, and
+ * the logits of that state (NaN for a fresh stream).  Same checks as na_decoder_stream_x3; no output may overlap
+ * `lengths` either. */
+int na_decoder_stream_ragged_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
+                                const float* m_in, const float* l_in, const float* z_in, const int32_t* lengths,
+                                float* logits, float* probs, float* h_out, float* c_out, float* m_out, float* l_out,
+                                float* z_out, int64_t T, int64_t B, int64_t NC, na_stream_t stream);
 
 /* ---- tensor-core tier, wide hidden sizes (H = 96, 144, 192; BASELINE configs[4]: H = 192, T = 2500) --------
  * Same contract as na_decoder_infer_bf16 (lstm_eeg_model.py:32-39 + :97, eval mode; input_size 8, 2 layers),

@@ -36,6 +36,7 @@ SIGNATURES = {
     "na_attention_softmax_f32": (c_int, [P, P, I64, I64, P]),
     "na_attention_pool_prefix_f32": (c_int, [P, P, P, P, I64, I64, I64, I64, I64, P]),
     "na_attention_pool_stream_f32": (c_int, [P] * 10 + [I64, I64, I64, I64, P]),
+    "na_attention_pool_stream_ragged_f32": (c_int, [P] * 11 + [I64, I64, I64, I64, P]),
     "na_head_param_floats": (c_int64, [I64, I64]),
     "na_head_partial_floats": (c_int64, [I64, I64, I64]),
     "na_head_bwd_f32": (c_int, [P] * 12 + [P, P, F32, P, P, P, I64, I64, I64, I64, I64, P]),
@@ -52,6 +53,7 @@ SIGNATURES = {
     "na_decoder_lstm_x3": (c_int, [P] * 7 + [I64, I64, P]),
     "na_decoder_prefix_pool_x3": (c_int, [P] * 5 + [I64, I64, I64, P]),
     "na_decoder_stream_x3": (c_int, [P] * 22 + [I64, I64, I64, P]),
+    "na_decoder_stream_ragged_x3": (c_int, [P] * 23 + [I64, I64, I64, P]),
     "na_decoder_wide_packed_bytes": (c_int64, [I64]),
     "na_decoder_wide_state_bytes": (c_int64, [I64]),
     "na_decoder_pack_wide_bf16": (c_int, [P] * 11 + [I64, P]),

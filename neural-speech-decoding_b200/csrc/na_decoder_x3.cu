@@ -28,8 +28,9 @@
 //   K16 MMAs pair two chunks through the descriptor's leading-byte-offset, so (x_lo | zeros), (x_hi | zeros) and
 //   (ones | zeros) pairs need no copies.  220 KB of shared memory; head parameters are read from global memory.
 // Instantiations: the default (logits / probs), kEx (+ scores, pooled vector, LayerNorm output; DESIGN 10c), kSeq (the two
-// LSTM layers alone, model.lstm; 10d), kPrefix (the pooled vector of every prefix x[:, :t_j], no head; 10f) and kStream
-// (the default's outputs from a carried LSTM and pool state, which it also returns; 10g).
+// LSTM layers alone, model.lstm; 10d), kPrefix (the pooled vector of every prefix x[:, :t_j], no head; 10f), kStream
+// (the default's outputs from a carried LSTM and pool state, which it also returns; 10g) and kStream + kRagged (the same
+// with a length per window row: row b takes only x[b, :lengths[b]]; 10h).
 #include "na_x3_common.cuh"
 
 namespace na {
@@ -192,6 +193,27 @@ __device__ __forceinline__ void x3_stream_store(const float* z, const float mx, 
     }
 }
 
+// kRagged, a row b < B given no steps (len == 0): its h_n / c_n are the state it came with -- h_init [2][B][48] (zeros
+// when NULL) and the cell states c0 / c1 as loaded from c_init -- stored before the tile's loop, which never reaches
+// the stores at steps len - 1 and len.
+template <int kU>
+__device__ __forceinline__ void x3_ragged_empty(const float* c0, const float* c1, const float* __restrict__ h_init,
+                                                float* __restrict__ h_n, float* __restrict__ c_n, const int64_t b,
+                                                const int64_t B, const int gr0) {
+#pragma unroll
+    for (int l = 0; l < 2; ++l) {
+        float hv[kU];
+#pragma unroll
+        for (int j = 0; j < kU; j += 4) {
+            const float4 v = h_init ? *reinterpret_cast<const float4*>(h_init + (l * B + b) * kH + gr0 * 4 + j)
+                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+            hv[j] = v.x; hv[j + 1] = v.y; hv[j + 2] = v.z; hv[j + 3] = v.w;
+        }
+        store_row<kU>(h_n + (l * B + b) * kH + gr0 * 4, hv);
+        store_row<kU>(c_n + (l * B + b) * kH + gr0 * 4, l == 0 ? c0 : c1);
+    }
+}
+
 // TMEM loads without the wait: a phase issues all of its loads and waits once (x3_drained).
 __device__ __forceinline__ void x3_tmem_ld16_nowait(uint32_t taddr, uint32_t* v) {
     asm volatile(
@@ -242,7 +264,12 @@ __device__ __forceinline__ void x3_drained(uint64_t* bar, const int lane) {
 // (m_in, l_in, z_in) [B], [B], [B][48]; every thread stores, for its own units and rows b < B, both layers' h and c of
 // the last step into h_n / c_n [2][B][48] and the pool's z after the last step into z_out [B][48]; the head's thread
 // stores the pool's max and sum into m_out / l_out [B].
-template <int R, int NR, bool kEx, bool kSeq, bool kPrefix, bool kStream>
+// kRagged (with kStream only): row b < B ends at len = lengths[b] (clamped to [0, T]) instead of T.  The tile still runs
+// all T steps, since its rows share the MMAs; a row's h_n / c_n are stored at layer-0 step len - 1 and loop step len
+// (layer-1 step len - 1), its pool takes in steps t - 2 < len only and the flush only when len == T, so nothing derived
+// from x[b, len:] reaches an output.  The pool and head code are the default's, so the row's outputs equal kStream's on
+// x[b, :len] bit for bit.
+template <int R, int NR, bool kEx, bool kSeq, bool kPrefix, bool kStream, bool kRagged>
 __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const int g, const int lane, const int nq, const int T,
                                                  const int n0, uint32_t& k1, const uint32_t tmem_d0, const uint32_t tmem_d1,
                                                  const int64_t b0, const int64_t B, const int NC,
@@ -256,7 +283,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                                                  const int stride, float* __restrict__ prefix_out,
                                                  const float* __restrict__ m_in, const float* __restrict__ l_in,
                                                  const float* __restrict__ z_in, float* __restrict__ m_out,
-                                                 float* __restrict__ l_out, float* __restrict__ z_out) {
+                                                 float* __restrict__ l_out, float* __restrict__ z_out,
+                                                 const int32_t* __restrict__ lengths, const float* __restrict__ h_init) {
     constexpr int kQ = 4 / R, kSlots = 4 / R, kU = 4 * kSlots;
     const int qs = q % kQ, rp = q / kQ;
     const int wrow = qs * 32 + lane;               // window row of the tile (first copy)
@@ -297,6 +325,13 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         }
     float mx = -INFINITY, l = 0.f;
     if constexpr (kStream) x3_stream_load<kU>(mx, l, z, m_in, l_in, z_in, brow, B, gr0);
+    int len = T;                                   // kRagged: the steps row brow takes in (T for rows b >= B)
+    if constexpr (kRagged)
+        if (brow < B) {
+            len = min(max(lengths[brow], 0), T);
+            if (len == 0) x3_ragged_empty<kU>(c0, c1, h_init, h_n, c_n, brow, B, gr0);
+        }
+    const int t_end = kRagged ? len : T;
     float* pout = nullptr;                         // kPrefix: this thread's units of the next prefix to store,
     int left = 0;                                  // and the steps the pool takes in until that prefix ends
     if constexpr (kPrefix) {
@@ -327,15 +362,24 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             for (int pr = 0; pr < kSlots / 2; ++pr) x3_tmem_ld32_nowait(tmem_d + lane_base + (gr0 + 2 * pr) * 16, v + 32 * pr);
         }
     };
-    auto cells = [&](const uint32_t* v, float* c, unsigned char* buf, float* hout) {
+    // `past` (kRagged, layer 0 at steps t >= len): zeros go to `buf` instead of h.  The layer-1 MMA that gives the score
+    // of the row's last step also reads the next step's layer-0 h, with zero weights; a NaN there (x past the length is
+    // not read for any output, and may hold anything) would make that score NaN.
+    auto cells = [&](const uint32_t* v, float* c, unsigned char* buf, float* hout, const bool past = false) {
         if constexpr (R == 4) {
             cell_granule_exact<NR>(v, c, hout);
+            if (past)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) hout[j] = 0.f;
             x3_store_h<R>(buf, gr0, wrow, 0, hout);
         } else {
 #pragma unroll
             for (int pr = 0; pr < kSlots / 2; ++pr) {       // pairs of granules = one 8-unit K chunk
                 cell_granule_exact<NR>(v + 32 * pr, c + pr * 8, hout + pr * 8);
                 cell_granule_exact<NR>(v + 32 * pr + 16, c + pr * 8 + 4, hout + pr * 8 + 4);
+                if (past)
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) hout[pr * 8 + j] = 0.f;
                 x3_store_h<R>(buf, gr0, wrow, pr, hout + pr * 8);
             }
         }
@@ -350,11 +394,11 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             gates_ld(tmem_d0, v);
             x3_drained(&S.d0_drained, lane);
             float hl0[kU];                         // layer-0 h: the next step reads it from shared memory
-            cells(v, c0, S.h0[n & 1], hl0);
+            cells(v, c0, S.h0[n & 1], hl0, kRagged && t >= len);
             fence_proxy_async_smem();
             mbar_arrive(&S.h0_ready[n & 1]);
             if constexpr (kSeq || kStream)
-                if (t == T - 1 && brow < B) {
+                if (t == t_end - 1 && brow < B) {
                     store_row<kU>(h_n + brow * kH + gr0 * 4, hl0);
                     store_row<kU>(c_n + brow * kH + gr0 * 4, c0);
                 }
@@ -367,7 +411,8 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
             if constexpr (!kSeq) x3_tmem_ld2_nowait(tmem_d1 + lane_base + kN, sc2);
             x3_drained(&S.d1_drained, lane);
             if constexpr (!kSeq) {
-                if (t >= 2) pool(__uint_as_float(sc2[0]));     // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
+                if (t >= 2 && (!kRagged || t - 2 < len))        // pooling of step t-2 (h_{t-2} in hprev) first: frees hprev
+                    pool(__uint_as_float(sc2[0]));
                 if constexpr (kEx)
                     if (t >= 2 && ex_writer && scores_tm) scores_tm[(int64_t)(t - 2) * B + b0 + wrow] = __uint_as_float(sc2[0]);
             }
@@ -388,7 +433,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
                     }
                 }
             if constexpr (kStream)
-                if (t == T && brow < B) {
+                if (t == t_end && brow < B) {
                     store_row<kU>(h_n + (B + brow) * kH + gr0 * 4, hprev);
                     store_row<kU>(c_n + (B + brow) * kH + gr0 * 4, c1);
                 }
@@ -401,7 +446,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
         uint32_t sc2[2];
         x3_tmem_ld2(tmem_d1 + lane_base + kN, sc2);
         tc_fence_before();
-        pool(__uint_as_float(sc2[0]));
+        if (!kRagged || len == T) pool(__uint_as_float(sc2[0]));
         if constexpr (kEx)
             if (ex_writer && scores_tm) scores_tm[(int64_t)(T - 1) * B + b0 + wrow] = __uint_as_float(sc2[0]);
     }
@@ -473,7 +518,7 @@ __device__ __forceinline__ void x3_epilogue_tile(SmemX3& S, const int q, const i
 // Barrier 0 over the whole CTA from code that differs between warps (the tile loops of the two register budgets).
 __device__ __forceinline__ void x3_cta_sync() { asm volatile("barrier.sync 0;" ::: "memory"); }
 
-template <int NR, bool kEx = false, bool kSeq = false, bool kPrefix = false, bool kStream = false>
+template <int NR, bool kEx = false, bool kSeq = false, bool kPrefix = false, bool kStream = false, bool kRagged = false>
 __global__ void __launch_bounds__(kX3InferThreads, 1)
 decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8] fp32, batch-first
                         const unsigned char* __restrict__ packed,   // pack_decoder_x3_kernel image
@@ -491,10 +536,12 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                         const float* __restrict__ m_in = nullptr,   // kStream: pool state in [B], [B], [B][48] (with h_init,
                         const float* __restrict__ l_in = nullptr,   // c_init, or none), and out (with h_n, c_n)
                         const float* __restrict__ z_in = nullptr, float* __restrict__ m_out = nullptr,
-                        float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr) {
+                        float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr,
+                        const int32_t* __restrict__ lengths = nullptr) {   // kRagged: [B] steps of each row
     static_assert(!(kEx && kSeq), "the intermediates and the sequence output are separate instantiations");
     static_assert(!(kPrefix && (kEx || kSeq)), "the prefix pool is an instantiation of its own");
     static_assert(!(kStream && (kEx || kSeq || kPrefix)), "the stream is an instantiation of its own");
+    static_assert(!kRagged || kStream, "per-row lengths are a variant of the stream");
     constexpr int kMmaWarp = 12, kProdWarp = 13, kTmemWarp = 15;     // producers: warps 13 and 14
     const bool seq_init = (kSeq || kStream) && h_init != nullptr;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -738,9 +785,9 @@ decoder_infer_x3_kernel(const float* __restrict__ x32,              // [B][T][8]
                 fence_proxy_async_smem();
                 x3_cta_sync();     // the previous tile is complete (barrier at its end): h0 / h1 are free
             }
-            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
-            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
-            else x3_epilogue_tile<4, NR, kEx, kSeq, kPrefix, kStream>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr);
+            if (R == 1) x3_epilogue_tile<1, NR, kEx, kSeq, kPrefix, kStream, kRagged>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr, kRagged ? lengths : nullptr, kRagged ? h_init : nullptr);
+            else if (R == 2) x3_epilogue_tile<2, NR, kEx, kSeq, kPrefix, kStream, kRagged>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr, kRagged ? lengths : nullptr, kRagged ? h_init : nullptr);
+            else x3_epilogue_tile<4, NR, kEx, kSeq, kPrefix, kStream, kRagged>(S, q, g, lane, nq, T, n0, k1, tmem_d0, tmem_d1, b0, B, NC, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, scores_tm, pooled, embedding, c_init, seq_out, h_n, c_n, NC, kPrefix ? pooled : nullptr, kStream ? m_in : nullptr, kStream ? l_in : nullptr, kStream ? z_in : nullptr, kStream ? m_out : nullptr, kStream ? l_out : nullptr, kStream ? z_out : nullptr, kRagged ? lengths : nullptr, kRagged ? h_init : nullptr);
         });
     }
 
@@ -909,55 +956,68 @@ static bool x3_overlap(const void* p, int64_t n, const void* q, int64_t m) {
 }
 } }
 
-extern "C" int na_decoder_stream_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
-                                    const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
-                                    const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
-                                    const float* m_in, const float* l_in, const float* z_in, float* logits, float* probs,
-                                    float* h_out, float* c_out, float* m_out, float* l_out, float* z_out, int64_t T,
-                                    int64_t B, int64_t NC, na_stream_t stream) {
-    using namespace na;
-    NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "na_decoder_stream_x3: bad shape T=%lld B=%lld", (long long)T,
-               (long long)B);
-    NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "na_decoder_stream_x3: num_classes=%lld", (long long)NC);
-    NA_REQUIRE_PTR(x); NA_REQUIRE_PTR(packed); NA_REQUIRE_PTR(logits);
-    NA_OPTIONAL_PTR(probs);
-    NA_REQUIRE_PTR(h_out); NA_REQUIRE_PTR(c_out); NA_REQUIRE_PTR(m_out); NA_REQUIRE_PTR(l_out); NA_REQUIRE_PTR(z_out);
+namespace na { namespace tc {
+// na_decoder_stream_x3 (lengths == NULL) and na_decoder_stream_ragged_x3 (`fn`): the argument checks, then the kStream
+// or kStream + kRagged instantiation for the x3_rcp_fma knob.
+template <bool kRagged>
+static int x3_stream(const char* fn, const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                     const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b, const float* fc3_w,
+                     const float* fc3_b, const float* h_in, const float* c_in, const float* m_in, const float* l_in,
+                     const float* z_in, const int32_t* lengths, float* logits, float* probs, float* h_out, float* c_out,
+                     float* m_out, float* l_out, float* z_out, int64_t T, int64_t B, int64_t NC, na_stream_t stream) {
+#define NA_X3S_PTR(p)                                                                                              \
+    do {                                                                                                           \
+        if ((p) == nullptr) return fail(NA_EINVAL, "%s: null pointer " #p, fn);                                    \
+        if (!aligned16(p)) return fail(NA_EALIGN, "%s: " #p " not 16-byte aligned", fn);                           \
+    } while (0)
+#define NA_X3S_OPT(p)                                                                                              \
+    do {                                                                                                           \
+        if ((p) != nullptr && !aligned16(p)) return fail(NA_EALIGN, "%s: " #p " not 16-byte aligned", fn);        \
+    } while (0)
+    NA_REQUIRE(T >= 1 && T < (1 << 20) && B >= 1, NA_EINVAL, "%s: bad shape T=%lld B=%lld", fn, (long long)T, (long long)B);
+    NA_REQUIRE(NC >= 1 && NC <= NA_MAX_CLASSES, NA_EUNSUPPORTED, "%s: num_classes=%lld", fn, (long long)NC);
+    NA_X3S_PTR(x); NA_X3S_PTR(packed); NA_X3S_PTR(logits);
+    NA_X3S_OPT(probs);
+    NA_X3S_PTR(h_out); NA_X3S_PTR(c_out); NA_X3S_PTR(m_out); NA_X3S_PTR(l_out); NA_X3S_PTR(z_out);
+    if (kRagged) NA_X3S_PTR(lengths);
     NA_REQUIRE(attn_w && attn_b && ln_w && ln_b && fc0_w && fc0_b && fc3_w && fc3_b, NA_EINVAL,
-               "na_decoder_stream_x3: null parameter pointer");
+               "%s: null parameter pointer", fn);
     const int given = (h_in != nullptr) + (c_in != nullptr) + (m_in != nullptr) + (l_in != nullptr) + (z_in != nullptr);
     NA_REQUIRE(given == 0 || given == 5, NA_EINVAL,
-               "na_decoder_stream_x3: h_in, c_in, m_in, l_in and z_in must be given together (or all NULL)");
-    NA_OPTIONAL_PTR(h_in); NA_OPTIONAL_PTR(c_in); NA_OPTIONAL_PTR(m_in); NA_OPTIONAL_PTR(l_in); NA_OPTIONAL_PTR(z_in);
+               "%s: h_in, c_in, m_in, l_in and z_in must be given together (or all NULL)", fn);
+    NA_X3S_OPT(h_in); NA_X3S_OPT(c_in); NA_X3S_OPT(m_in); NA_X3S_OPT(l_in); NA_X3S_OPT(z_in);
+#undef NA_X3S_PTR
+#undef NA_X3S_OPT
     // The kernel's pointers are __restrict__: no output may share memory with an input or with another output.
-    const int64_t S = 2 * B * tc::kH;
-    const void* in[] = {x, h_in, c_in, m_in, l_in, z_in};
-    const int64_t in_n[] = {B * T * 8, S, S, B, B, B * tc::kH};
+    const int64_t S = 2 * B * kH;
+    const void* in[] = {x, h_in, c_in, m_in, l_in, z_in, kRagged ? lengths : nullptr};    // lengths: 4-byte elements
+    const int64_t in_n[] = {B * T * 8, S, S, B, B, B * kH, B};
     float* out[] = {logits, probs, h_out, c_out, m_out, l_out, z_out};
-    const int64_t out_n[] = {B * NC, B * NC, S, S, B, B, B * tc::kH};
+    const int64_t out_n[] = {B * NC, B * NC, S, S, B, B, B * kH};
     const char* out_name[] = {"logits", "probs", "h_out", "c_out", "m_out", "l_out", "z_out"};
     for (int i = 0; i < 7; ++i) {
-        for (int j = 0; j < 6; ++j)
-            NA_REQUIRE(!tc::x3_overlap(out[i], out_n[i], in[j], in_n[j]), NA_EINVAL,
-                       "na_decoder_stream_x3: %s overlaps an input", out_name[i]);
+        for (int j = 0; j < 7; ++j)
+            NA_REQUIRE(!x3_overlap(out[i], out_n[i], in[j], in_n[j]), NA_EINVAL, "%s: %s overlaps an input", fn,
+                       out_name[i]);
         for (int j = 0; j < i; ++j)
-            NA_REQUIRE(!tc::x3_overlap(out[i], out_n[i], out[j], out_n[j]), NA_EINVAL,
-                       "na_decoder_stream_x3: %s overlaps %s", out_name[i], out_name[j]);
+            NA_REQUIRE(!x3_overlap(out[i], out_n[i], out[j], out_n[j]), NA_EINVAL, "%s: %s overlaps %s", fn, out_name[i],
+                       out_name[j]);
     }
-    const size_t smem = sizeof(tc::SmemX3) + 1024;
+    const size_t smem = sizeof(SmemX3) + 1024;
     const int nquarters = (int)((B + 31) / 32);
-    const int sms = tc::x3_sms();
+    const int sms = x3_sms();
     const int grid = nquarters < sms ? nquarters : sms;
 #define NA_X3_STREAM_LAUNCH(NRV)                                                                                                     \
     {                                                                                                                                \
-        cudaError_t e = cudaFuncSetAttribute(tc::decoder_infer_x3_kernel<NRV, false, false, false, true>,                            \
+        cudaError_t e = cudaFuncSetAttribute(decoder_infer_x3_kernel<NRV, false, false, false, true, kRagged>,                       \
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                                \
-        if (e != cudaSuccess) return fail((int)e, "na_decoder_stream_x3: shared memory opt-in failed (%s)", cudaGetErrorString(e)); \
-        tc::decoder_infer_x3_kernel<NRV, false, false, false, true><<<grid, tc::kX3InferThreads, smem, as_stream(stream)>>>(          \
+        if (e != cudaSuccess) return fail((int)e, "%s: shared memory opt-in failed (%s)", fn, cudaGetErrorString(e));             \
+        decoder_infer_x3_kernel<NRV, false, false, false, true, kRagged><<<grid, kX3InferThreads, smem, as_stream(stream)>>>(     \
             x, reinterpret_cast<const unsigned char*>(packed), attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w, fc3_b, logits, probs, \
             (int)T, B, (int)NC, nquarters, nullptr, nullptr, nullptr, h_in, c_in, nullptr, h_out, c_out, m_in, l_in, z_in, m_out,   \
-            l_out, z_out);                                                                                                           \
+            l_out, z_out, kRagged ? lengths : nullptr);                                                                              \
     }
-    switch (tc::g_x3_rcp_fma) {
+    switch (g_x3_rcp_fma) {
         case 0: NA_X3_STREAM_LAUNCH(0) break;
         case 2: NA_X3_STREAM_LAUNCH(2) break;
         case 3: NA_X3_STREAM_LAUNCH(3) break;
@@ -965,5 +1025,29 @@ extern "C" int na_decoder_stream_x3(const float* x, const void* packed, const fl
     }
 #undef NA_X3_STREAM_LAUNCH
     count_launch();
-    return check_launch("na_decoder_stream_x3");
+    return check_launch(fn);
+}
+} }
+
+extern "C" int na_decoder_stream_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                    const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                    const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
+                                    const float* m_in, const float* l_in, const float* z_in, float* logits, float* probs,
+                                    float* h_out, float* c_out, float* m_out, float* l_out, float* z_out, int64_t T,
+                                    int64_t B, int64_t NC, na_stream_t stream) {
+    return na::tc::x3_stream<false>("na_decoder_stream_x3", x, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b, fc3_w,
+                                    fc3_b, h_in, c_in, m_in, l_in, z_in, nullptr, logits, probs, h_out, c_out, m_out,
+                                    l_out, z_out, T, B, NC, stream);
+}
+
+extern "C" int na_decoder_stream_ragged_x3(const float* x, const void* packed, const float* attn_w, const float* attn_b,
+                                           const float* ln_w, const float* ln_b, const float* fc0_w, const float* fc0_b,
+                                           const float* fc3_w, const float* fc3_b, const float* h_in, const float* c_in,
+                                           const float* m_in, const float* l_in, const float* z_in,
+                                           const int32_t* lengths, float* logits, float* probs, float* h_out,
+                                           float* c_out, float* m_out, float* l_out, float* z_out, int64_t T,
+                                           int64_t B, int64_t NC, na_stream_t stream) {
+    return na::tc::x3_stream<true>("na_decoder_stream_ragged_x3", x, packed, attn_w, attn_b, ln_w, ln_b, fc0_w, fc0_b,
+                                   fc3_w, fc3_b, h_in, c_in, m_in, l_in, z_in, lengths, logits, probs, h_out, c_out,
+                                   m_out, l_out, z_out, T, B, NC, stream);
 }

@@ -412,16 +412,21 @@ namespace na {
 // kState (EEG_LSTM.decode_stream, with stride = T: one pooled row): the online softmax starts from the state (m, l, z)
 // the earlier chunks of the stream left, when m_in / l_in / z_in are given, and its state after the last step is stored
 // to m_out / l_out [B] and z_out [B][H].
-template <int JPL, int CH, bool kState = false>
+// kRagged (with kState; EEG_LSTM.decode_stream with lengths): window b takes in steps t < lengths[b] (clamped to [0, T])
+// only, and its pooled row z / l is stored after them: the pool state it came with when it takes in none.
+template <int JPL, int CH, bool kState = false, bool kRagged = false>
 __global__ void __launch_bounds__(kHeadWarps * 32)
 attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restrict__ attn_w, const float* __restrict__ attn_b,
                              float* __restrict__ pooled, int T, int64_t B, int64_t Bp, int H, int stride,
                              const float* __restrict__ m_in = nullptr, const float* __restrict__ l_in = nullptr,
                              const float* __restrict__ z_in = nullptr, float* __restrict__ m_out = nullptr,
-                             float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr) {
+                             float* __restrict__ l_out = nullptr, float* __restrict__ z_out = nullptr,
+                             const int32_t* __restrict__ lengths = nullptr) {
+    static_assert(!kRagged || kState, "per-row lengths are a variant of the stream pool");
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t b = (int64_t)blockIdx.x * kHeadWarps + warp;
     if (b >= B) return;
+    const int Tb = kRagged ? min(max(lengths[b], 0), T) : T;    // the steps window b takes in
     float wa[JPL], z[JPL];
 #pragma unroll
     for (int i = 0; i < JPL; ++i) {
@@ -443,7 +448,7 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
             }
         }
     int left = stride;                            // steps until the next prefix end
-    for (int t0 = 0; t0 < T; t0 += CH) {
+    for (int t0 = 0; t0 < Tb; t0 += CH) {
         float hv[CH][JPL];
 #pragma unroll
         for (int u = 0; u < CH; ++u) {
@@ -452,7 +457,7 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
 #pragma unroll
             for (int i = 0; i < JPL; ++i) {
                 const int j = lane + 32 * i;
-                hv[u][i] = (t < T && j < H) ? __ldg(row + j) : 0.f;
+                hv[u][i] = (t < Tb && j < H) ? __ldg(row + j) : 0.f;
             }
         }
         float s[CH];
@@ -466,7 +471,7 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
 #pragma unroll
         for (int u = 0; u < CH; ++u) {
             const int t = t0 + u;
-            if (t >= T) break;
+            if (t >= Tb) break;
             if (s[u] > m) {                       // first step: exp(-inf) = 0
                 const float sc = expf(m - s[u]);
                 l *= sc;
@@ -478,7 +483,7 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
             l += e;
 #pragma unroll
             for (int i = 0; i < JPL; ++i) z[i] = fmaf(e, hv[u][i], z[i]);
-            if (--left == 0 || t == T - 1) {
+            if (!kRagged && (--left == 0 || t == T - 1)) {
                 const float inv = 1.0f / l;
 #pragma unroll
                 for (int i = 0; i < JPL; ++i) {
@@ -488,6 +493,14 @@ attention_pool_prefix_kernel(const float* __restrict__ h, const float* __restric
                 out += H;
                 left = stride;
             }
+        }
+    }
+    if constexpr (kRagged) {                      // the one pooled row (stride T), after the row's last step
+        const float inv = 1.0f / l;
+#pragma unroll
+        for (int i = 0; i < JPL; ++i) {
+            const int j = lane + 32 * i;
+            if (j < H) out[j] = z[i] * inv;
         }
     }
     if constexpr (kState) {
@@ -530,6 +543,53 @@ int launch_attention_pool_stream(const float* h, const float* attn_w, const floa
     return check_launch("na_attention_pool_stream_f32");
 }
 }  // namespace na
+
+namespace na {
+template <int JPL, int CH>
+int launch_attention_pool_stream_ragged(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
+                                        const float* l_in, const float* z_in, const int32_t* lengths, float* pooled,
+                                        float* m_out, float* l_out, float* z_out, int64_t T, int64_t B, int64_t Bp,
+                                        int64_t H, cudaStream_t st) {
+    if (int rc = prepare_launch(attention_pool_prefix_kernel<JPL, CH, true, true>, kHeadWarps * 32, 0,
+                                "na_attention_pool_stream_ragged_f32"))
+        return rc;
+    const unsigned grid = (unsigned)((B + kHeadWarps - 1) / kHeadWarps);
+    attention_pool_prefix_kernel<JPL, CH, true, true><<<grid, kHeadWarps * 32, 0, st>>>(
+        h, attn_w, attn_b, pooled, (int)T, B, Bp, (int)H, (int)T, m_in, l_in, z_in, m_out, l_out, z_out, lengths);
+    count_launch();
+    return check_launch("na_attention_pool_stream_ragged_f32");
+}
+}  // namespace na
+
+extern "C" int na_attention_pool_stream_ragged_f32(const float* h, const float* attn_w, const float* attn_b,
+                                                   const float* m_in, const float* l_in, const float* z_in,
+                                                   const int32_t* lengths, float* pooled, float* m_out, float* l_out,
+                                                   float* z_out, int64_t T, int64_t B, int64_t Bp, int64_t H,
+                                                   na_stream_t stream) {
+    using namespace na;
+    NA_REQUIRE(T >= 1 && T <= INT32_MAX && B >= 1 && Bp >= B && Bp % NA_BATCH_ALIGN == 0, NA_EINVAL,
+               "na_attention_pool_stream_ragged_f32: bad shape T=%lld B=%lld Bp=%lld", (long long)T, (long long)B,
+               (long long)Bp);
+    NA_REQUIRE(H >= 1 && H <= 1024, NA_EUNSUPPORTED, "na_attention_pool_stream_ragged_f32: H=%lld outside [1,1024]",
+               (long long)H);
+    NA_REQUIRE_PTR(h); NA_REQUIRE_PTR(lengths);
+    NA_REQUIRE_PTR(pooled); NA_REQUIRE_PTR(m_out); NA_REQUIRE_PTR(l_out); NA_REQUIRE_PTR(z_out);
+    NA_REQUIRE(attn_w && attn_b, NA_EINVAL, "na_attention_pool_stream_ragged_f32: null parameter pointer");
+    const int given = (m_in != nullptr) + (l_in != nullptr) + (z_in != nullptr);
+    NA_REQUIRE(given == 0 || given == 3, NA_EINVAL,
+               "na_attention_pool_stream_ragged_f32: m_in, l_in and z_in must be given together (or all NULL)");
+    NA_OPTIONAL_PTR(m_in); NA_OPTIONAL_PTR(l_in); NA_OPTIONAL_PTR(z_in);
+    cudaStream_t st = as_stream(stream);
+#define NA_POOL_RAGGED(JPL, CH)                                                                                        \
+    launch_attention_pool_stream_ragged<JPL, CH>(h, attn_w, attn_b, m_in, l_in, z_in, lengths, pooled, m_out, l_out, \
+                                                 z_out, T, B, Bp, H, st)
+    if (H <= 64) return NA_POOL_RAGGED(2, 8);
+    if (H <= 128) return NA_POOL_RAGGED(4, 4);
+    if (H <= 256) return NA_POOL_RAGGED(8, 2);
+    if (H <= 512) return NA_POOL_RAGGED(16, 1);
+    return NA_POOL_RAGGED(32, 1);
+#undef NA_POOL_RAGGED
+}
 
 extern "C" int na_attention_pool_stream_f32(const float* h, const float* attn_w, const float* attn_b, const float* m_in,
                                             const float* l_in, const float* z_in, float* pooled, float* m_out, float* l_out,

@@ -327,11 +327,24 @@ class EEG_LSTM(nn.Module):
             return op(x, [self.lstm.layer(l) for l in range(L)], [ops._f32c(t) for t in self._head_params()], *probs,
                       z, [self._packed(l) for l in range(L)])
 
-    def decode(self, x: torch.Tensor, want_probs: bool = True):
+    def decode(self, x: torch.Tensor, want_probs: bool = True, lengths=None):
         """Eval-mode forward without autograd: x [B,T,C] on CUDA -> (logits fp32 [B,K], probs fp32 [B,K] or
-        empty).  Picks the tier from ``compute_dtype`` / the dtype of ``x`` / the parameters."""
+        empty).  Picks the tier from ``compute_dtype`` / the dtype of ``x`` / the parameters.
+
+        ``lengths`` (a length-B sequence or 1-D integer tensor on any device, values in [1, T]) batches windows of
+        different durations, as ``pack_padded_sequence`` does for nn.LSTM: row b is the forward of ``x[b, :lengths[b]]``
+        alone, and ``x`` past a row's length is ignored whatever it holds, NaN included.  It runs ``decode_stream(x,
+        lengths=lengths)`` from fresh streams and drops the state, so it has that call's contract: on the exact tier
+        (``ops.EXACT_TC`` and the flagship shape) row b is ``decode(x[:, :lengths[b]])[b]`` bit for bit (whose error in
+        mid-window is up to 2e-5 of float64, DESIGN 10f), elsewhere the FFMA kernels within 1e-5.  Eval arithmetic whatever
+        ``self.training`` is; ``compute_dtype`` does not apply (a float16 / bfloat16 ``x`` is converted to fp32);
+        ``zscore_input`` raises ``ValueError`` (its statistics would come from the whole padded window).  Reading the
+        lengths for validation synchronises with the device once."""
         ops._require_cuda(x)
-        return self._decode(x, False, want_probs)
+        if lengths is None:
+            return self._decode(x, False, want_probs)
+        out = self._stream(x, None, lengths, 1, "decode")
+        return out.logits, out.probs if want_probs else torch.empty((0,), dtype=torch.float32, device=x.device)
 
     def decode_intermediates(self, x: torch.Tensor) -> DecoderOutputs:
         """Eval-mode forward without autograd that also returns the attention weights over time, the pooled vector and
@@ -424,7 +437,7 @@ class EEG_LSTM(nn.Module):
                 raise RuntimeError(f"state.{name} is on {t.device}, the chunk on {device}")
         return state
 
-    def decode_stream(self, x: torch.Tensor, state: Optional[DecoderState] = None) -> StreamOutputs:
+    def decode_stream(self, x: torch.Tensor, state: Optional[DecoderState] = None, lengths=None) -> StreamOutputs:
         """The decoder on recordings that arrive a chunk at a time: ``x`` [B,T,C] on CUDA (T >= 1) is the next chunk of
         each of B streams, ``state`` the ``DecoderState`` the previous call returned (None: fresh streams) ->
         ``StreamOutputs(logits, probs, state)``.  ``logits`` is ``decode(torch.cat(chunks, dim=1))[0]``, the eval
@@ -438,20 +451,55 @@ class EEG_LSTM(nn.Module):
         ``state.c`` to ``model.lstm``'s ``h_n`` / ``c_n``; every other shape runs on the FFMA kernels under the 1e-5
         contract.  Eval arithmetic whatever ``self.training`` is; ``compute_dtype`` does not apply (a float16 /
         bfloat16 ``x`` is converted to fp32).  ``zscore_input`` raises ``ValueError``: the z-score takes its statistics
-        from the whole window, which a stream does not have."""
+        from the whole window, which a stream does not have.
+
+        ``lengths`` serves streams that delivered different numbers of samples since the last call in one batch: a
+        length-B sequence or 1-D integer tensor on any device, values in [0, T].  Row b then takes only ``x[b,
+        :lengths[b]]``; ``x`` past a row's length is ignored whatever it holds, NaN included.  Row b's logits, probs and
+        state are those of ``decode_stream(x[b:b+1, :lengths[b]], its state)``: on the exact tier bit for bit, with the
+        logits of ``decode`` of everything the stream has received (error up to 2e-5 of float64 in mid-window, DESIGN
+        10f / 10g), on the FFMA kernels within 1e-5.  A row given 0 steps returns its state unchanged, bit for bit, and
+        the logits of that state: NaN for a stream that has seen nothing.  Reading the lengths for validation
+        synchronises with the device once.  ``lengths=None`` is the call without them."""
+        return self._stream(x, state, lengths, 0, "decode_stream")
+
+    def _check_lengths(self, lengths, B: int, T: int, low: int, device) -> torch.Tensor:
+        """``lengths`` as int32 [B] on ``device``; ``ValueError`` unless it is a length-B sequence or 1-D tensor of
+        integers in [low, T].  Reads the values on the host (one synchronisation)."""
+        t = lengths
+        if not isinstance(t, torch.Tensor):
+            t = torch.as_tensor(lengths)
+            if t.numel() == 0:                     # an empty sequence has no dtype to tell
+                t = t.long()
+        if t.dtype == torch.bool or t.dtype.is_floating_point or t.dtype.is_complex:
+            raise ValueError(f"lengths must hold integers, got {t.dtype}")
+        if tuple(t.shape) != (B,):
+            raise ValueError(f"lengths must have shape [{B}] (one per row of x), got {list(t.shape)}")
+        if B > 0:
+            lo, hi = (int(v) for v in torch.stack(torch.aminmax(t)).tolist())
+            if lo < low or hi > T:
+                raise ValueError(f"lengths must lie in [{low}, {T}], got values in [{lo}, {hi}]")
+        return t.to(device=device, dtype=torch.int32)
+
+    def _stream(self, x: torch.Tensor, state, lengths, low: int, name: str) -> StreamOutputs:
+        """``decode_stream``, and ``decode`` with ``lengths`` (``low`` = the smallest length allowed, ``name`` the
+        caller's name in errors)."""
         if x.dim() != 3:
             raise ValueError(f"expected x of shape [B,T,C], got {tuple(x.shape)}")
         ops._require_cuda(x)
         if x.shape[2] != self.lstm.input_size:
             raise RuntimeError(f"input.size(-1) must be equal to input_size. Expected {self.lstm.input_size}, got {x.shape[2]}")
         B, T = x.shape[0], x.shape[1]
+        stream = name == "decode_stream"
         if T < 1:
-            raise ValueError("decode_stream needs chunks of at least one step")
+            raise ValueError(f"{name} needs {'chunks' if stream else 'windows'} of at least one step")
         if self.zscore_input:
-            raise ValueError("decode_stream: zscore_input normalises with the statistics of the whole window, which a "
-                             "stream does not have")
+            why = "which a stream does not have" if stream else "not those of each row's first lengths[b] steps"
+            raise ValueError(f"{name}: zscore_input normalises with the statistics of the whole window, {why}")
         if state is not None:
             state = self._check_stream_state(state, B, x.device)
+        if lengths is not None:
+            lengths = self._check_lengths(lengths, B, T, low, x.device)
         if B == 0:
             K = self.fc[3].out_features
             e = torch.empty((0, K), dtype=torch.float32, device=x.device)
@@ -459,12 +507,18 @@ class EEG_LSTM(nn.Module):
         x32 = ops._aligned16(x.detach().float().contiguous())
         head = [p.detach() for p in self._head_params()]
         with torch.no_grad():
+            L = self.lstm.num_layers
             if ops.EXACT_TC and self.tc_supported():
-                out = ops.decoder_stream_chunk_x3(x32, self._packed_x3(), head, state)
-            else:
-                L = self.lstm.num_layers
+                if lengths is None:
+                    out = ops.decoder_stream_chunk_x3(x32, self._packed_x3(), head, state)
+                else:
+                    out = ops.decoder_stream_chunk_ragged_x3(x32, self._packed_x3(), head, state, lengths)
+            elif lengths is None:
                 out = ops.decoder_stream_chunk(x32, [self.lstm.layer(l) for l in range(L)], head, state,
                                                [self._packed(l) for l in range(L)])
+            else:
+                out = ops.decoder_stream_chunk_ragged(x32, [self.lstm.layer(l) for l in range(L)], head, state, lengths,
+                                                      [self._packed(l) for l in range(L)])
         return StreamOutputs(out[0], out[1], DecoderState(*out[2:]))
 
     def inject_noise(self, drop1: Optional[torch.Tensor] = None, rrelu_slope: Optional[torch.Tensor] = None,

@@ -102,7 +102,7 @@ def all_custom_ops():
             lstm_wide_fwd_train, lstm_wide_bwd, head_fwd_ex, attention_softmax, decoder_infer_bf16_ex,
             decoder_infer_bf16_x32_ex, decoder_infer_x3_ex, decoder_infer_wide_bf16_ex, lstm_layer_fwd_hx, lstm_layer_bwd_hx,
             lstm_layer_wgrad_hx, decoder_lstm_x3, decoder_prefix_pool_x3, attention_pool_prefix, decoder_stream_x3,
-            attention_pool_stream]
+            attention_pool_stream, decoder_stream_ragged_x3, attention_pool_stream_ragged]
 
 
 def launch_count() -> int:
@@ -755,12 +755,19 @@ def decoder_stream_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], h: Opti
     stream state h / c [2,B,48], m / l [B], z [B,48] (all five or none: a fresh stream) -> (logits [B,K], probs [B,K],
     and the state after the chunk: h, c, m, l, z).  The logits are those of decoder_infer_x3 on everything the streams
     have received."""
-    _require_cuda(x, packed, h, c, m, l, z)
+    return _stream_x3("decoder_stream_x3", x, packed, head, (h, c, m, l, z), None)
+
+
+def _stream_x3(op: str, x: Tensor, packed: Tensor, head: Sequence[Tensor], state: Sequence[Optional[Tensor]],
+               lengths: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """Body of decoder_stream_x3 (``lengths`` None: entry point na_decoder_stream_x3) and decoder_stream_ragged_x3
+    (na_decoder_stream_ragged_x3)."""
+    _require_cuda(x, packed, *state, lengths)
     B, T, C = x.shape
     if x.dtype != torch.float32 or C != 8:
-        raise RuntimeError("decoder_stream_x3: x must be fp32 [B, T, 8]")
+        raise RuntimeError(f"{op}: x must be fp32 [B, T, 8]")
     x = _aligned16(x.contiguous())
-    h, c, m, l, z = _state_in(None if h is None else (h, c, m, l, z))
+    h, c, m, l, z = _state_in(None if state[0] is None else state)
     head = [_f32c(t) for t in head]
     dev, f = x.device, torch.float32
     NC = head[6].shape[0]
@@ -768,10 +775,16 @@ def decoder_stream_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], h: Opti
     h_out, c_out = torch.empty((2, B, 48), dtype=f, device=dev), torch.empty((2, B, 48), dtype=f, device=dev)
     m_out, l_out = torch.empty((B,), dtype=f, device=dev), torch.empty((B,), dtype=f, device=dev)
     z_out = torch.empty((B, 48), dtype=f, device=dev)
-    _lib.call("na_decoder_stream_x3", x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
-              _ptr(h), _ptr(c), _ptr(m), _ptr(l), _ptr(z), logits.data_ptr(), probs.data_ptr(), h_out.data_ptr(),
+    lens = [] if lengths is None else [_lengths_in(lengths)]          # held until the call returns
+    _lib.call("na_" + op, x.data_ptr(), packed.data_ptr(), *[t.data_ptr() for t in head],
+              _ptr(h), _ptr(c), _ptr(m), _ptr(l), _ptr(z), *[t.data_ptr() for t in lens], logits.data_ptr(), probs.data_ptr(), h_out.data_ptr(),
               c_out.data_ptr(), m_out.data_ptr(), l_out.data_ptr(), z_out.data_ptr(), T, B, NC, _stream())
     return logits, probs, h_out, c_out, m_out, l_out, z_out
+
+
+def _lengths_in(lengths: Tensor) -> Tensor:
+    """Per-row lengths as the contiguous, 16-byte aligned int32 [B] the ragged entry points read."""
+    return _aligned16(lengths.to(torch.int32).contiguous())
 
 
 @decoder_stream_x3.register_fake
@@ -788,6 +801,31 @@ def decoder_stream_chunk_x3(x: Tensor, packed: Tensor, head_params: Sequence[Ten
     (h, c, pool max, pool sum, pool z) or None (fresh streams) -> (logits, probs, h, c, pool max, pool sum, pool z).
     head_params in EEG_LSTM._head_params() order."""
     return decoder_stream_x3(x, packed, list(head_params), *([None] * 5 if state is None else state))
+
+
+@torch.library.custom_op("neuroalpha::decoder_stream_ragged_x3", mutates_args=(), device_types="cuda")
+@_device_guard
+def decoder_stream_ragged_x3(x: Tensor, packed: Tensor, head: Sequence[Tensor], h: Optional[Tensor],
+                             c: Optional[Tensor], m: Optional[Tensor], l: Optional[Tensor], z: Optional[Tensor],
+                             lengths: Tensor) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """decoder_stream_x3 with a length per stream: row b takes only x[b, :lengths[b]] (integer [B], values in [0, T];
+    x past a row's length is ignored, NaN included), and its outputs are decoder_stream_x3's on that chunk bit for bit.
+    A row given 0 steps keeps its state."""
+    return _stream_x3("decoder_stream_ragged_x3", x, packed, head, (h, c, m, l, z), lengths)
+
+
+@decoder_stream_ragged_x3.register_fake
+def _(x, packed, head, h, c, m, l, z, lengths):
+    B, NC, f = x.shape[0], head[6].shape[0], torch.float32
+    return (x.new_empty((B, NC), dtype=f), x.new_empty((B, NC), dtype=f), x.new_empty((2, B, 48), dtype=f),
+            x.new_empty((2, B, 48), dtype=f), x.new_empty((B,), dtype=f), x.new_empty((B,), dtype=f),
+            x.new_empty((B, 48), dtype=f))
+
+
+def decoder_stream_chunk_ragged_x3(x: Tensor, packed: Tensor, head_params: Sequence[Tensor],
+                                   state: Optional[Sequence[Tensor]], lengths: Tensor) -> Tuple[Tensor, ...]:
+    """decoder_stream_chunk_x3 where row b takes only x[b, :lengths[b]]."""
+    return decoder_stream_ragged_x3(x, packed, list(head_params), *([None] * 5 if state is None else state), lengths)
 
 
 WIDE_HIDDEN = (96, 144, 192)          # hidden sizes of the streamed-weight tensor-core kernel (na_decoder_wide.cu)
@@ -986,6 +1024,19 @@ def decoder_stream_chunk(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], hea
     state's (h, c) (zeros for a fresh stream), then attention_pool_stream from the state's pool and the head tail ->
     (logits, probs, h [L,B,H], c [L,B,H], pool max [B], pool sum [B], pool z [B,H])."""
     _require_cuda(x)
+    T = x.shape[1]
+    cur, h_n, c_n, (m, l, z) = _stream_layers(x, lstm_params, state, packed, lambda seq, init: seq[T - 1, :x.shape[0]])
+    head = [_f32c(t) for t in head_params]
+    pooled, m, l, z = attention_pool_stream(cur, x.shape[0], head[0], head[1], m, l, z)
+    logits, probs = head_tail_fwd(pooled, head, None, None, 1.0, True)
+    return logits, probs, h_n, c_n, m, l, z
+
+
+def _stream_layers(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], state: Optional[Sequence[Tensor]],
+                   packed: Optional[Sequence[Tuple[Tensor, Tensor]]], last) -> Tuple[Tensor, Tensor, Tensor, List]:
+    """The LSTM layers of decoder_stream_chunk / decoder_stream_chunk_ragged on the chunk x [B,T,C], each from the state's
+    (h, c) -> (the last layer's h TMP [T,Bp,H], h_n [L,B,H], c_n [L,B,H], the state's pool fields).  ``last(seq,
+    init)`` picks a layer's final h or c [B,H] from its sequence TMP [T,Bp,H] and its initial value [B,H] (None: zeros)."""
     B, T, C = x.shape
     Bp = padded_batch(B)
     h0, c0, m, l, z = _state_in(state)
@@ -999,12 +1050,57 @@ def decoder_stream_chunk(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], hea
         if h0 is not None:
             hp[:B], cp[:B] = h0[i], c0[i]
         cur, c, _, _ = lstm_layer_fwd_hx(cur, wt, bias, None, 1.0, hp, cp)
-        h_n.append(cur[T - 1, :B])
-        c_n.append(c[T - 1, :B])
+        h_n.append(last(cur, None if h0 is None else h0[i]))
+        c_n.append(last(c, None if h0 is None else c0[i]))
+    return cur, torch.stack(h_n), torch.stack(c_n), [m, l, z]
+
+
+@torch.library.custom_op("neuroalpha::attention_pool_stream_ragged", mutates_args=(), device_types="cuda")
+@_device_guard
+def attention_pool_stream_ragged(h: Tensor, B: int, attn_w: Tensor, attn_b: Tensor, m: Optional[Tensor],
+                                 l: Optional[Tensor], z: Optional[Tensor], lengths: Tensor
+                                 ) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """attention_pool_stream where window b takes in steps t < lengths[b] of the chunk h TMP [T,Bp,H] only (integer [B],
+    values in [0, T]); a window given no steps keeps its state and pools it (NaN for a fresh pool)."""
+    _require_cuda(h, attn_w, attn_b, m, l, z, lengths)
+    T, Bp, H = h.shape
+    dev, f = h.device, torch.float32
+    pooled, z_out = torch.empty((B, H), dtype=f, device=dev), torch.empty((B, H), dtype=f, device=dev)
+    m_out, l_out = torch.empty((B,), dtype=f, device=dev), torch.empty((B,), dtype=f, device=dev)
+    lengths = _lengths_in(lengths)
+    _lib.call("na_attention_pool_stream_ragged_f32", h.data_ptr(), _f32c(attn_w).data_ptr(), _f32c(attn_b).data_ptr(),
+              _ptr(m), _ptr(l), _ptr(z), lengths.data_ptr(), pooled.data_ptr(), m_out.data_ptr(),
+              l_out.data_ptr(), z_out.data_ptr(), T, B, Bp, H, _stream())
+    return pooled, m_out, l_out, z_out
+
+
+@attention_pool_stream_ragged.register_fake
+def _(h, B, attn_w, attn_b, m, l, z, lengths):
+    H, f = h.shape[2], torch.float32
+    return h.new_empty((B, H), dtype=f), h.new_empty((B,), dtype=f), h.new_empty((B,), dtype=f), h.new_empty((B, H), dtype=f)
+
+
+def decoder_stream_chunk_ragged(x: Tensor, lstm_params: Sequence[Sequence[Tensor]], head_params: Sequence[Tensor],
+                                state: Optional[Sequence[Tensor]], lengths: Tensor,
+                                packed: Optional[Sequence[Tuple[Tensor, Tensor]]] = None) -> Tuple[Tensor, ...]:
+    """decoder_stream_chunk where row b takes only x[b, :lengths[b]] (integer [B] on x's device, values in [0, T]).  The
+    layers run over all T steps -- rows are independent, so the steps past a row's length reach nothing of that row's
+    outputs -- and h_n / c_n are gathered at step lengths[b] - 1, or taken from the state where lengths[b] == 0; then
+    attention_pool_stream_ragged and the head tail."""
+    _require_cuda(x, lengths)
+    B = x.shape[0]
+    lengths = lengths.to(device=x.device)
+    rows, at_step = torch.arange(B, device=x.device), (lengths.long() - 1).clamp(min=0)
+    empty = (lengths == 0)[:, None]
+
+    def last(seq, init):
+        at = seq[at_step, rows]
+        return torch.where(empty, torch.zeros_like(at) if init is None else init, at)
+    cur, h_n, c_n, (m, l, z) = _stream_layers(x, lstm_params, state, packed, last)
     head = [_f32c(t) for t in head_params]
-    pooled, m, l, z = attention_pool_stream(cur, B, head[0], head[1], m, l, z)
+    pooled, m, l, z = attention_pool_stream_ragged(cur, B, head[0], head[1], m, l, z, lengths)
     logits, probs = head_tail_fwd(pooled, head, None, None, 1.0, True)
-    return logits, probs, torch.stack(h_n), torch.stack(c_n), m, l, z
+    return logits, probs, h_n, c_n, m, l, z
 
 
 def _save(ctx, tensors: Sequence[Tensor], optional: Sequence[Optional[Tensor]]) -> None:
